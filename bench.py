@@ -51,6 +51,9 @@ def parse():
                    help="cross-shard threshold exchange of the doc-sharded index (N > 1): 1 on, 0 off, -1 the library default")
     p.add_argument("--opt", action="append", default=[], metavar="NAME=INT",
                    help="br_set_option on the index (tuning experiments, e.g. defer_pm=800); not used by the driver")
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the ids and scores the last timed step returned as DIR/ids.npy and "
+                        "DIR/scores.npy (float64), so that two builds can be compared output for output")
     return p.parse_args()
 
 
@@ -183,6 +186,15 @@ def gen_queries(args, doc_offsets, token_ids, doc_lo, doc_hi, rank, world):
     q_off = np.zeros(args.queries + 1, np.int32)
     np.cumsum([t.size for t in terms], out=q_off[1:])
     return np.concatenate(terms).astype(np.int32), q_off, src
+
+
+def dump_outputs(path, ids, scores):
+    """The [Q, k] ids and scores of a retrieval call as path/ids.npy and path/scores.npy, both float64 (exact for doc ids
+    below 2^53; -1 pads stay -1)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("ids", ids), ("scores", scores)):
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
 
 
 def cpu_sample_size(args, threads):
@@ -513,8 +525,10 @@ def main():
             co.topk_batch(q_terms[:qo[-1]], qo, args.k, dedup=True, n_threads=threads)
         t0 = time.time()
         for _ in range(args.steps):
-            co.topk_batch(q_terms[:qo[-1]], qo, args.k, dedup=True, n_threads=threads)
+            ids, sc, _ = co.topk_batch(q_terms[:qo[-1]], qo, args.k, dedup=True, n_threads=threads)
         dt = (time.time() - t0) / args.steps
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ids, sc)
         qps = n_sample / dt
         sample = f"{n_sample} of {args.queries} queries at full N={args.docs} per step, index resident in host RAM"
         _emit(({
@@ -579,11 +593,13 @@ def main():
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms for all `steps` calls, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        out = None
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -591,7 +607,7 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -602,13 +618,13 @@ def main():
     model.set_profiling(True)
     step_device()                            # creates the profiling events outside the timed region
     sampler.mark()
-    ms_total = timed(step_device, args.steps)
+    ms_total, (ids_last, sc_last) = timed(step_device, args.steps)
     qstats = model.query_stats()            # last step's counters (identical every step)
     clocks = sampler.stop() if rank == 0 else None
     model.set_profiling(False)
     for _ in range(max(1, args.warmup // 2)):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     ids_e2e = h_out.clone()
     assert torch.equal(ids_e2e, ids_ref.cpu()), "e2e and device-resident results differ"
 
@@ -627,7 +643,7 @@ def main():
         return h_out
 
     step_text()
-    ms_text = timed(step_text, args.steps)
+    ms_text, _ = timed(step_text, args.steps)
     assert torch.equal(h_out, ids_ref.cpu()), "text-surface and device-resident results differ"
     del voc
 
@@ -727,6 +743,8 @@ def main():
                                 "sample": f"first {n_sample} of {args.queries} queries at full N={args.docs} "
                                           f"({cpu_s:.1f} s; host index build {cpu_build_s:.1f} s untimed)",
                                 "top10_ids_identical_to_gpu": same}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, ids_last, sc_last)
     if rank == 0:
         _emit(line)
     if dist_on:

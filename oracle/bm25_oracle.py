@@ -6,8 +6,8 @@ This module is the *checker*: only ``tests/``, ``__graft_entry__.smoke()`` and t
 
 Parity pinning: the reference holds no golden vectors (SURVEY 4), so this restatement is pinned
 against the *unmodified reference functions executed in the authoring container*
-(``oracle/ref_loader.py``) - see ``tests/golden/make_golden.py`` (fixtures) and
-``tests/test_oracle_vs_reference.py`` (live check where /root/reference exists).
+(``oracle/ref_loader.py``) - ``tests/golden/make_golden.py`` stores their outputs as the fixtures
+under ``tests/golden/`` that ``tests/test_oracle.py`` checks this module against.
 
 Every function cites the reference lines it restates.  Arithmetic is float64 with the
 reference's own operation order, so per-posting contributions are bit-identical to the Python
