@@ -1,5 +1,5 @@
 #!/bin/bash
-# development helper: GPU tests, then bench lines for a list of option sets ("defer_pm=700 tile_tpb=8" ...)
+# development helper: GPU tests, then bench lines for a list of option sets ("defer_pm=500" "defer_pm=800 fused_long=0" ...)
 tag=$1; shift
 python -m pytest tests -m gpu -x -q > gpurun_out/pytest_$tag.log 2>&1; echo pytest_rc=$?
 tail -5 gpurun_out/pytest_$tag.log

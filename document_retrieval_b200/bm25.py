@@ -370,7 +370,8 @@ class BM25:
         check(_lib.load().br_set_profiling(self._h, int(bool(on))), "br_set_profiling")
 
     def set_option(self, name, value):
-        """Library tuning / test switches: "fused" (0 = dense path only), "tile_g" (0 auto, 1/2/4/8)."""
+        """Library tuning / test switches: "fused" (0 = dense path only), "fused_long" (0 = no long-query tiled pass),
+        "defer_pm" (MaxScore deferral budget, per mille of the threshold, 0-1000)."""
         check(_lib.load().br_set_option(self._h, name.encode(), int(value)), "br_set_option")
 
     def query_stats(self):

@@ -19,7 +19,8 @@ def _bf16(x, dev):
 
 
 def set_cosine_option(name, value):
-    """br_set_cosine_option: process-wide kernel-variant / schedule switches of the brute-force path (tests, sweeps)."""
+    """br_set_cosine_option: process-wide test switch of the brute-force path: "kernel" (0 auto, 1 forces the
+    2-CTA multicast kernel that serves d > 768; both return bit-identical results)."""
     check(_lib.load().br_set_cosine_option(name.encode(), int(value)), "br_set_cosine_option")
 
 

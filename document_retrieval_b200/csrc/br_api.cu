@@ -101,28 +101,10 @@ int br_set_option(br_index* ix, const char* name, int value) {
     BR_REQUIRE(ix && name, BR_ERR_INVALID, "br_set_option: null pointer");
     const std::string n(name);
     if (n == "fused") ix->allow_fused = value != 0;
-    else if (n == "fused_bigk") ix->allow_fused_bigk = value != 0;
     else if (n == "fused_long") ix->allow_fused_long = value != 0;
-    else if (n == "seed_thr") ix->seed_thr = value != 0;
-    else if (n == "tile_g") {
-        BR_REQUIRE(value == 0 || value == 1 || value == 2 || value == 4 || value == 8, BR_ERR_INVALID,
-                   "br_set_option: tile_g must be 0, 1, 2, 4 or 8");
-        ix->tile_g = value;
-    } else if (n == "defer_pm") {
+    else if (n == "defer_pm") {
         BR_REQUIRE(value >= 0 && value <= 1000, BR_ERR_INVALID, "br_set_option: defer_pm must be in [0, 1000]");
         ix->defer_pm = value;
-    } else if (n == "tile_growth") {
-        BR_REQUIRE(value >= 2 && value <= 16, BR_ERR_INVALID, "br_set_option: tile_growth must be in [2, 16]");
-        ix->tile_growth = value;
-    } else if (n == "tile_dense_min") {
-        BR_REQUIRE(value >= 1 && value <= 512, BR_ERR_INVALID, "br_set_option: tile_dense_min must be in [1, 512]");
-        ix->tile_dense_min = value;
-    } else if (n == "sparse_mode") {
-        BR_REQUIRE(value >= 0 && value <= 1, BR_ERR_INVALID, "br_set_option: sparse_mode must be 0 or 1");
-        ix->sparse_mode = value;
-    } else if (n == "tile_tpb") {
-        BR_REQUIRE(value >= 1 && value <= 64, BR_ERR_INVALID, "br_set_option: tile_tpb must be in [1, 64]");
-        ix->tile_tpb = value;
     } else {
         br::set_error("br_set_option: unknown option " + n);
         return BR_ERR_INVALID;

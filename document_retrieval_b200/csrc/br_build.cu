@@ -593,7 +593,7 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
         BR_CUDA(cudaStreamSynchronize(st));
     }
     if (!ix->sig_bit) {
-        // the 32 most frequent terms: queries are grouped by which of them they contain (br_tile.cu)
+        // the 32 most frequent terms: the tiled scorer orders its queries by which of them they contain (br_tile.cu)
         std::vector<int32_t> order(V);
         for (size_t t = 0; t < V; ++t) order[t] = (int32_t)t;
         const size_t top = std::min<size_t>(32, V);

@@ -8,14 +8,10 @@
 
 #include "../../include/br_b200.h"
 
-// docs per skip-table sub-range = docs per warp of the tile kernel (2^kSubShift)
-#ifndef BR_TILE_SHIFT
-#define BR_TILE_SHIFT 11
-#endif
-
 namespace br {
 
-constexpr int kSubShift = BR_TILE_SHIFT;
+// docs per skip-table sub-range = docs per warp of the tile kernel (2^kSubShift; why 2048: br_tile.cu)
+constexpr int kSubShift = 11;
 
 void set_error(const std::string& msg);
 
@@ -159,21 +155,14 @@ struct br_index {
     br::DevBuf ws_prep, ws_dense, ws_sel, ws_cand, ws_misc, ws_tile, ws_sort, ws_cold, ws_rec;
     br_query_stats stats{};
 
-    bool allow_fused = true, allow_fused_bigk = true, allow_fused_long = true;
-    int tile_g = 0;
+    bool allow_fused = true, allow_fused_long = true;
     // doc-sharded callers: callback that max-reduces thr[Q] over the shards (br_set_thr_exchange), user pointer, and the
     // number of tile launches after which it is called (plus once after seeding); rounds < 0: off
     br_thr_exchange_fn thr_exchange = nullptr;
     void* thr_exchange_user = nullptr;
     int thr_exchange_rounds = -1;
     int thr_exchange_world = 1;
-    bool seed_thr = true;           // threshold seeding before the first launch of the tiled scorer
     int defer_pm = 650;             // MaxScore deferral budget of the tiled scorer, per mille of the threshold (0 = off)
-    int tile_growth = 2;            // every launch covers this many times the tiles of the one before
-    int sparse_mode = 1;            // sparse phase of the tile kernel: 0 next non-empty slice pulled over by shuffles, 1 term list walked from shared memory
-    int tile_tpb = 16;              // consecutive tiles per CTA in the large launches
-    int tile_dense_min = 32;        // average postings of a term per sub-range from which its slices are walked
-                                    // term by term (whole warp, pipelined) instead of concatenated with the sparse ones
 
     // optional event timing of the scoring kernel
     bool profiling = false;

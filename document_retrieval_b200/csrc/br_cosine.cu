@@ -2,12 +2,14 @@
 //   e_hat = e / (||e|| + 1e-10) on both sides, sims = E_hat . q_hat, top-k per query.
 //
 //   k_row_inv_norm      1/(||x||_2 + 1e-10) per row, fp32                        (HBM-bound, one pass)
-//   k_cosine_gemm       brute force: bf16 tcgen05 (UMMA) GEMM  docs[256-row tile] x queries[256-col tile],
-//                       TMA (128B swizzle) -> 3-stage smem ring -> tcgen05.mma, fp32 accumulators in TMEM
-//                       (2 x 256 columns: two 128-row UMMAs share each query tile); epilogue warps read TMEM with tcgen05.ld,
-//                       apply 1/(||d||+eps) * 1/(||q||+eps) and keep only scores above the query's running
-//                       threshold - the [Q, N] score matrix is never written.  Persistent, warp-specialised
+//   k_cosine_gemm_qs    brute force, d <= 768: bf16 tcgen05 (UMMA) GEMM on CTA pairs, the pair's block of 224 queries
+//                       resident in shared memory while doc tiles stream past it (TMA, 128B swizzle, 3-stage ring);
+//                       fp32 accumulators in TMEM; epilogue warps read TMEM with tcgen05.ld, apply
+//                       1/(||d||+eps) * 1/(||q||+eps) and keep only scores above the query's running threshold - the
+//                       [Q, N] score matrix is never written.  Persistent, warp-specialised
 //                       (warp 0 TMA, warp 1 MMA + TMEM alloc, warps 2-9 epilogue).        (tensor-bound)
+//   k_cosine_gemm_mc    the same for d > 768 (the query block no longer fits): docs[256-row tile] x queries[256-col
+//                       tile] per CTA, the doc tile multicast to a CTA pair
 //   k_tighten_cos       between doc chunks of doubling size: threshold := k-th best so far, compact list
 //   k_cosine_rerank     per query its own c candidate rows (BM25 top-1000 -> cosine): one warp per
 //                       (query, candidate) dot product with 128-bit loads              (gather / HBM-bound)
@@ -175,166 +177,10 @@ struct CosArgs {
     int32_t window;                 // query-stationary kernel: doc tiles per L2 window
 };
 
-__global__ void __launch_bounds__(CG_THREADS, 1) k_cosine_gemm(const __grid_constant__ CUtensorMap map_docs,
-                                                               const __grid_constant__ CUtensorMap map_q, CosArgs a) {
-    extern __shared__ unsigned char smem_raw[];
-    const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;             // 128B swizzle needs 1024-byte alignment
-    unsigned char* gen = smem_raw + (base - smem_u32(smem_raw));
-    const uint32_t s_tiles = base;
-    float* s_thr = reinterpret_cast<float*>(gen + CG_STAGES * CG_STAGE_BYTES);          // [CG_BN] scaled thresholds
-    float* s_inq = s_thr + CG_BN;                                                        // [CG_BN] 1/(||q||+eps)
-    uint64_t* bars = reinterpret_cast<uint64_t*>(s_inq + CG_BN);                        // full[S] empty[S] tfull[2] tempty[2]
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 12);
-    const uint32_t bar0 = smem_u32(bars);
-    auto full_bar = [&](int s) { return bar0 + 8u * s; };
-    auto empty_bar = [&](int s) { return bar0 + 8u * (CG_STAGES + s); };
-    auto tfull_bar = [&](int b) { return bar0 + 8u * (2 * CG_STAGES + b); };
-    auto tempty_bar = [&](int b) { return bar0 + 8u * (2 * CG_STAGES + 2 + b); };
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_qt = (a.nq + CG_BN - 1) / CG_BN;
-    const int64_t n_tiles = (int64_t)(a.tile_end - a.tile_begin) * n_qt;
-    const int n_kb = (a.d + CG_BK - 1) / CG_BK;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < CG_STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-        for (int b = 0; b < 2; ++b) { mbar_init(tfull_bar(b), 1); mbar_init(tempty_bar(b), 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(s_tmem)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *s_tmem;
-
-    if (warp == 0) {
-        // ===== TMA producer =====
-        if (lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0;
-            for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-                const int dt = a.tile_begin + (int)(t / n_qt), qt = (int)(t % n_qt);
-                for (int kb = 0; kb < n_kb; ++kb) {
-                    mbar_wait(empty_bar(stage), phase ^ 1);
-                    mbar_expect_tx(full_bar(stage), CG_STAGE_BYTES);
-                    const uint32_t sa = s_tiles + stage * CG_STAGE_BYTES;
-                    tma_load_2d(sa, &map_docs, full_bar(stage), kb * CG_BK, dt * CG_BM);          // 256 doc rows
-                    tma_load_2d(sa + CG_A_BYTES, &map_q, full_bar(stage), kb * CG_BK, qt * CG_BN);
-                    if (++stage == CG_STAGES) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ===== MMA issuer (one elected lane) =====
-        if (lane == 0) {
-            int stage = 0;
-            uint32_t phase = 0, acc_phase = 0;
-            for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-                // both accumulator halves (TMEM columns [0,256) and [256,512)) must have been drained
-                mbar_wait(tempty_bar(0), acc_phase ^ 1);
-                mbar_wait(tempty_bar(1), acc_phase ^ 1);
-                acc_phase ^= 1;
-                tc_fence_after();
-                for (int kb = 0; kb < n_kb; ++kb) {
-                    mbar_wait(full_bar(stage), phase);
-                    tc_fence_after();
-                    const uint32_t sa = s_tiles + stage * CG_STAGE_BYTES;
-                    const uint64_t da0 = umma_desc_sw128(sa), da1 = umma_desc_sw128(sa + CG_A_BYTES / 2);
-                    const uint64_t db = umma_desc_sw128(sa + CG_A_BYTES);
-#pragma unroll
-                    for (int k = 0; k < CG_BK / 16; ++k) {        // UMMA_K = 16 bf16 = 32 bytes: +2 in the >>4 address field
-                        tc_mma_bf16(tmem_base, da0 + (uint64_t)(2 * k), db + (uint64_t)(2 * k), CG_IDESC, (kb | k) != 0);
-                        tc_mma_bf16(tmem_base + CG_BN, da1 + (uint64_t)(2 * k), db + (uint64_t)(2 * k), CG_IDESC, (kb | k) != 0);
-                    }
-                    tc_commit(empty_bar(stage));                    // smem slot free once these MMAs retire
-                    if (++stage == CG_STAGES) { stage = 0; phase ^= 1; }
-                }
-                tc_commit(tfull_bar(0));                            // accumulators ready for the epilogue warps
-                tc_commit(tfull_bar(1));
-            }
-        }
-    } else {
-        // ===== epilogue warps: half h = (warp-2)/4 owns doc rows [128h, 128h+128) = TMEM columns [256h, 256h+256);
-        //       a warp reads TMEM lanes [32*(warp%4), +32) =====
-        const int quarter = warp & 3, half = (warp - 2) >> 2;
-        const int et = (int)threadIdx.x - 64;                       // 0..255
-        uint32_t acc_phase = 0;
-        for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-            const int dt = a.tile_begin + (int)(t / n_qt), qt = (int)(t % n_qt);
-            asm volatile("bar.sync 1, 256;" ::: "memory");          // previous tile's thresholds no longer in use
-            {
-                const int c = et;
-                const int q = qt * CG_BN + c;
-                float th = CUDART_INF_F, iq = 0.f;
-                if (q < a.nq) {
-                    iq = a.inv_nq[q];
-                    const float raw = __ldcg(a.thr + q) / iq;          // compare acc*inv_d against thr/inv_q
-                    th = raw - fabsf(raw) * 4e-6f;                      // superset: rounding of the division
-                }
-                s_thr[c] = th;
-                s_inq[c] = iq;
-            }
-            asm volatile("bar.sync 1, 256;" ::: "memory");          // epilogue warps only
-            mbar_wait(tfull_bar(half), acc_phase);
-            acc_phase ^= 1;
-            tc_fence_after();
-            const int64_t doc = (int64_t)dt * CG_BM + half * 128 + quarter * 32 + lane;
-            const float inv_d = doc < a.n_docs ? a.inv_nd[doc] : 0.f;
-            const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)half * CG_BN;
-            // Common case (nothing passes) is branch-free: m = max_j (acc_j * inv_d - thr_j) over 32 columns with the
-            // thresholds read as float4; the next 32 columns are already on their way from TMEM.  Only when m >= 0
-            // are the 32 columns rescanned and emitted.
-            uint32_t v[2][32];
-            tc_ld_32x32(taddr, v[0]);
-#pragma unroll
-            for (int b = 0; b < (CG_BN / 32); ++b) {
-                tc_wait_ld();
-                if (b + 1 < CG_BN / 32) tc_ld_32x32(taddr + (b + 1) * 32, v[(b + 1) & 1]);
-                const uint32_t (&cur)[32] = v[b & 1];
-                const float4* t4 = reinterpret_cast<const float4*>(s_thr + b * 32);
-                float m = -CUDART_INF_F;
-#pragma unroll
-                for (int j4 = 0; j4 < 8; ++j4) {
-                    const float4 th = t4[j4];
-                    m = fmaxf(m, fmaf(__uint_as_float(cur[4 * j4 + 0]), inv_d, -th.x));
-                    m = fmaxf(m, fmaf(__uint_as_float(cur[4 * j4 + 1]), inv_d, -th.y));
-                    m = fmaxf(m, fmaf(__uint_as_float(cur[4 * j4 + 2]), inv_d, -th.z));
-                    m = fmaxf(m, fmaf(__uint_as_float(cur[4 * j4 + 3]), inv_d, -th.w));
-                }
-                if (m >= 0.f && doc < a.n_docs) {
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        const float sc = __uint_as_float(cur[j]) * inv_d;
-                        if (sc >= s_thr[b * 32 + j]) {
-                            const int q = qt * CG_BN + b * 32 + j;
-                            const int pos = atomicAdd(a.cand_cnt + q, 1);
-                            if (pos < COS_CAP) {
-                                a.cand[(int64_t)q * COS_CAP + pos] = (int32_t)doc;
-                                a.cand_h[(int64_t)q * COS_CAP + pos] = sc * s_inq[b * 32 + j];
-                            }
-                        }
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tempty_bar(half));
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-    }
-}
-
-// Cluster variant: CTA pairs share every doc (A) tile - rank r loads rows [128r, 128r+128) of it and multicasts them to both
-// CTAs, so the doc operand crosses L2->SM once per pair; each CTA loads its own query (B) tile.  Stage release is cluster-wide
-// (both CTAs' UMMAs arrive on both CTAs' empty barriers).
+// Multicast kernel (d > 768): a CTA computes docs[256-row tile] x queries[256-col tile] with two 128-row UMMAs sharing the
+// query tile, fp32 accumulators in 2 x 256 TMEM columns.  CTA pairs share every doc (A) tile - rank r loads rows
+// [128r, 128r+128) of it and multicasts them to both CTAs, so the doc operand crosses L2->SM once per pair; each CTA loads
+// its own query (B) tile.  Stage release is cluster-wide (both CTAs' UMMAs arrive on both CTAs' empty barriers).
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cosine_gemm_mc(const __grid_constant__ CUtensorMap map_docs,
                                                                const __grid_constant__ CUtensorMap map_q, CosArgs a) {
     extern __shared__ unsigned char smem_raw[];
@@ -515,16 +361,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cos
 constexpr int QS_NKB = 12;
 constexpr int QS_A_BYTES = 128 * CG_BK * 2;            // 16 KB: this CTA's 128 doc rows of one k-block
 constexpr int QS_THREADS = 320;                        // warp 0 TMA, warp 1 MMA / TMEM alloc, warps 2-9 epilogue
-template <int BN, int STAGES>
-struct QsCfg {
-    static constexpr int BNH = BN / 2;                                  // query rows held by each CTA
-    static constexpr int B_BYTES = BNH * CG_BK * 2;                     // one k-block of them
-    static constexpr size_t SMEM = 1024 + (size_t)QS_NKB * B_BYTES + (size_t)STAGES * QS_A_BYTES + 2 * BN * sizeof(float) + 8 * (2 * STAGES + 6) + 16;
-    // instruction descriptor: D=f32, A=B=bf16 K-major, N=BN (>>3 at bit 17), M=256 (>>4 at bit 24; the pair's M)
-    static constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
-    static_assert(SMEM <= 232448, "query block + doc ring exceed the shared memory of one SM");
-    static_assert(BN % 32 == 0 && BN <= 256, "BN: multiple of 32 (epilogue column chunks), two accumulator stages in 512 TMEM columns");
-};
+// Query block width and doc ring depth: 224 x 3 fills the shared memory; 128 x 8, 160 x 6 and 192 x 5 measured within
+// noise of it or slower (DESIGN.md 3.5).
+constexpr int QS_BN = 224, QS_STAGES = 3;
+constexpr int QS_BNH = QS_BN / 2;                      // query rows held by each CTA
+constexpr int QS_B_BYTES = QS_BNH * CG_BK * 2;         // one k-block of them
+constexpr size_t QS_SMEM = 1024 + (size_t)QS_NKB * QS_B_BYTES + (size_t)QS_STAGES * QS_A_BYTES + 2 * QS_BN * sizeof(float) + 8 * (2 * QS_STAGES + 6) + 16;
+// instruction descriptor: D=f32, A=B=bf16 K-major, N=QS_BN (>>3 at bit 17), M=256 (>>4 at bit 24; the pair's M)
+constexpr uint32_t QS_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(QS_BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
+constexpr int QS_WINDOW = 64;                          // doc tiles per L2 window (~25 MB of embeddings at d = 768)
+static_assert(QS_SMEM <= 232448, "query block + doc ring exceed the shared memory of one SM");
+static_assert(QS_BN % 32 == 0 && QS_BN <= 256, "QS_BN: multiple of 32 (epilogue column chunks), two accumulator stages in 512 TMEM columns");
 
 __device__ __forceinline__ uint32_t mapa_rank(uint32_t addr, uint32_t rank) {   // shared::cta address -> shared::cluster address in CTA `rank`
     uint32_t r;
@@ -595,12 +442,8 @@ struct QsIter {
     }
 };
 
-template <int QS_BN, int QS_STAGES, int EPI = 0>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cosine_gemm_qs(const __grid_constant__ CUtensorMap map_docs,
                                                                const __grid_constant__ CUtensorMap map_q, CosArgs a) {
-    using Cfg = QsCfg<QS_BN, QS_STAGES>;
-    constexpr int QS_BNH = Cfg::BNH, QS_B_BYTES = Cfg::B_BYTES;
-    constexpr uint32_t QS_IDESC = Cfg::IDESC;
     extern __shared__ unsigned char smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;             // 128B swizzle needs 1024-byte alignment
     unsigned char* gen = smem_raw + (base - smem_u32(smem_raw));
@@ -736,130 +579,72 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
             acc_phase[acc] ^= 1;
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)acc * 256u + (uint32_t)col0;
-            if constexpr (EPI == 0) {
-                // common case (nothing passes) is branch-free: per 16-column chunk mc = max_j (acc_j * inv_d - thr_j)
-                float mc[NCH];
-                {
-                    uint32_t v[NCH][16];
+            // All of the warp's columns are in registers after one wait.  The filter is straight-line code: per chunk
+            // the maximum of acc*inv_d - thr, and a predicated copy of the chunk's 16 accumulators when it holds a
+            // passing column.  The emission code exists ONCE (ncu on the first version, which emitted from 7 x 16
+            // unrolled copies: 35 % of all stall samples were instruction-cache misses on the emission lines).
+            // A lane with passing columns in two or more chunks (thresholds still loose) sends its warp through the
+            // chunk loop, which reads each chunk again from TMEM; otherwise the accumulator stage goes back to the MMA
+            // issuer before anything is emitted.
+            uint32_t hv[16];
+            int hc = 0, nhc = 0;
+            {
+                uint32_t v[NCH][16];
 #pragma unroll
-                    for (int c = 0; c < NCH; ++c) tc_ld_32x16(taddr + c * 16, v[c]);
-                    tc_wait_ld();
+                for (int c = 0; c < NCH; ++c) tc_ld_32x16(taddr + c * 16, v[c]);
+                tc_wait_ld();
 #pragma unroll
-                    for (int c = 0; c < NCH; ++c) {
-                        const float4* t4 = reinterpret_cast<const float4*>(s_thr + col0 + c * 16);
-                        float m = -CUDART_INF_F;
-                        {
-#pragma unroll
-                            for (int j4 = 0; j4 < 4; ++j4) {
-                                const float4 th = t4[j4];
-                                m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 0]), inv_d, -th.x));
-                                m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 1]), inv_d, -th.y));
-                                m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 2]), inv_d, -th.z));
-                                m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 3]), inv_d, -th.w));
-                            }
-                        }
-                        mc[c] = doc < a.n_docs ? m : -CUDART_INF_F;
-                    }
-                }
-                // rare (about k ln 2 docs per query per launch): a chunk in which some doc row of this warp has a passing
-                // column is read again from TMEM (the tcgen05.ld is warp-collective, so the whole warp takes the branch)
-                // and its passing (doc, query) pairs are appended to the queries' candidate lists
+                for (int j = 0; j < 16; ++j) hv[j] = 0u;
 #pragma unroll
                 for (int c = 0; c < NCH; ++c) {
-                    if (!__any_sync(0xffffffffu, mc[c] >= 0.f)) continue;
-                    uint32_t e[16];
-                    tc_ld_32x16(taddr + c * 16, e);
-                    tc_wait_ld();
-                    if (mc[c] >= 0.f) {
+                    const float4* t4 = reinterpret_cast<const float4*>(s_thr + col0 + c * 16);
+                    float m = -CUDART_INF_F;
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            const float sc = __uint_as_float(e[j]) * inv_d;
-                            const int col = col0 + c * 16 + j;
-                            if (sc >= s_thr[col]) {
-                                const int q = un.qb * QS_BN + col;
-                                const int pos = atomicAdd(a.cand_cnt + q, 1);
-                                if (pos < COS_CAP) {
-                                    a.cand[(int64_t)q * COS_CAP + pos] = (int32_t)doc;
-                                    a.cand_h[(int64_t)q * COS_CAP + pos] = sc * s_inq[col];
-                                }
-                            }
-                        }
+                    for (int j4 = 0; j4 < 4; ++j4) {
+                        const float4 th = t4[j4];
+                        m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 0]), inv_d, -th.x));
+                        m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 1]), inv_d, -th.y));
+                        m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 2]), inv_d, -th.z));
+                        m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 3]), inv_d, -th.w));
                     }
+                    const bool hit = doc < a.n_docs && m >= 0.f;
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) hv[j] = hit ? v[c][j] : hv[j];
+                    hc = hit ? c : hc;
+                    nhc += hit ? 1 : 0;
                 }
             }
-            if constexpr (EPI != 0) {
-                // All of the warp's columns are in registers after one wait.  The filter is straight-line code: per chunk
-                // the maximum of acc*inv_d - thr, and a predicated copy of the chunk's 16 accumulators when it holds a
-                // passing column.  The emission code exists ONCE (ncu on the first version, which emitted from 7 x 16
-                // unrolled copies: 35 % of all stall samples were instruction-cache misses on the emission lines).
-                // A lane with passing columns in two or more chunks (thresholds still loose) sends its warp through the
-                // chunk loop, which reads each chunk again from TMEM; otherwise the accumulator stage goes back to the MMA
-                // issuer before anything is emitted.
-                uint32_t hv[16];
-                int hc = 0, nhc = 0;
-                {
-                    uint32_t v[NCH][16];
-#pragma unroll
-                    for (int c = 0; c < NCH; ++c) tc_ld_32x16(taddr + c * 16, v[c]);
-                    tc_wait_ld();
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) hv[j] = 0u;
-#pragma unroll
-                    for (int c = 0; c < NCH; ++c) {
-                        const float4* t4 = reinterpret_cast<const float4*>(s_thr + col0 + c * 16);
-                        float m = -CUDART_INF_F;
-#pragma unroll
-                        for (int j4 = 0; j4 < 4; ++j4) {
-                            const float4 th = t4[j4];
-                            m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 0]), inv_d, -th.x));
-                            m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 1]), inv_d, -th.y));
-                            m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 2]), inv_d, -th.z));
-                            m = fmaxf(m, fmaf(__uint_as_float(v[c][4 * j4 + 3]), inv_d, -th.w));
-                        }
-                        const bool hit = doc < a.n_docs && m >= 0.f;
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) hv[j] = hit ? v[c][j] : hv[j];
-                        hc = hit ? c : hc;
-                        nhc += hit ? 1 : 0;
-                    }
-                }
-                const bool multi = __any_sync(0xffffffffu, nhc > 1);
-                if (!multi) {
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive_cluster(acc ? l_tempty1 : l_tempty0);
-                }
-                const int c_begin = multi ? 0 : hc, c_end = multi ? NCH : hc + nhc;
+            const bool multi = __any_sync(0xffffffffu, nhc > 1);
+            if (!multi) {
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_cluster(acc ? l_tempty1 : l_tempty0);
+            }
+            const int c_begin = multi ? 0 : hc, c_end = multi ? NCH : hc + nhc;
 #pragma unroll 1
-                for (int c = c_begin; c < c_end; ++c) {
-                    if (multi) {                                    // warp-uniform
-                        tc_ld_32x16(taddr + c * 16, hv);
-                        tc_wait_ld();
-                    }
-                    if (doc < a.n_docs) {
-                        const float* thc = s_thr + col0 + c * 16;
+            for (int c = c_begin; c < c_end; ++c) {
+                if (multi) {                                    // warp-uniform
+                    tc_ld_32x16(taddr + c * 16, hv);
+                    tc_wait_ld();
+                }
+                if (doc < a.n_docs) {
+                    const float* thc = s_thr + col0 + c * 16;
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            const float sc = __uint_as_float(hv[j]) * inv_d;
-                            if (sc >= thc[j]) {
-                                const int col = col0 + c * 16 + j;
-                                const int q = un.qb * QS_BN + col;
-                                const int pos = atomicAdd(a.cand_cnt + q, 1);
-                                if (pos < COS_CAP) {
-                                    a.cand[(int64_t)q * COS_CAP + pos] = (int32_t)doc;
-                                    a.cand_h[(int64_t)q * COS_CAP + pos] = sc * s_inq[col];
-                                }
+                    for (int j = 0; j < 16; ++j) {
+                        const float sc = __uint_as_float(hv[j]) * inv_d;
+                        if (sc >= thc[j]) {
+                            const int col = col0 + c * 16 + j;
+                            const int q = un.qb * QS_BN + col;
+                            const int pos = atomicAdd(a.cand_cnt + q, 1);
+                            if (pos < COS_CAP) {
+                                a.cand[(int64_t)q * COS_CAP + pos] = (int32_t)doc;
+                                a.cand_h[(int64_t)q * COS_CAP + pos] = sc * s_inq[col];
                             }
                         }
                     }
                 }
-                if (multi) {
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive_cluster(acc ? l_tempty1 : l_tempty0);
-                }
             }
-            if constexpr (EPI == 0) {
+            if (multi) {
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive_cluster(acc ? l_tempty1 : l_tempty0);
@@ -1081,32 +866,14 @@ __global__ void k_cos_patch(const int32_t* __restrict__ rows, int32_t nr, int32_
     out_sims[o] = sims[i];
 }
 
-// Process-wide tuning / test switches of br_cosine_topk (br_set_cosine_option): every setting returns bit-identical results.
-struct CosOptions {
-    int kernel = 0;          // 0 auto (query-stationary CTA pairs when d <= 768, else 2-CTA multicast), 1 multicast, 2 one CTA per tile
-    int qs_bn = 224;         // query block width of the query-stationary kernel: 128, 160, 192 or 224
-    int qs_window = 64;      // doc tiles per L2 window
-    int chunk0 = 1;          // doc tiles of the first launch
-    int chunk_mult = 2;      // growth of the launches
-    int tighten_threads = 64;
-    int qs_epi = 1;          // epilogue of the 224-wide query-stationary kernel: 0 filter + re-read of every passing chunk (7 x 16 unrolled emission sites), 1 compact: one emission site, accumulator stage released before the emission
-};
-static CosOptions g_cos;
+// br_set_cosine_option("kernel", v): 0 auto (query-stationary CTA pairs when d <= 768, else 2-CTA multicast), 1 always
+// multicast.  Both kernels return bit-identical results; the switch lets a test pin them against each other.
+static int g_cos_kernel = 0;
 
 int set_cosine_option(const char* name, int value) {
     BR_REQUIRE(name, BR_ERR_INVALID, "br_set_cosine_option: null name");
     const std::string n(name);
-    if (n == "kernel") { BR_REQUIRE(value >= 0 && value <= 2, BR_ERR_INVALID, "br_set_cosine_option: kernel must be 0, 1 or 2"); g_cos.kernel = value; }
-    else if (n == "qs_bn") { BR_REQUIRE(value == 128 || value == 160 || value == 192 || value == 224, BR_ERR_INVALID, "br_set_cosine_option: qs_bn must be 128, 160, 192 or 224"); g_cos.qs_bn = value; }
-    else if (n == "qs_window") { BR_REQUIRE(value >= 1 && value <= 4096, BR_ERR_INVALID, "br_set_cosine_option: qs_window must be in [1, 4096]"); g_cos.qs_window = value; }
-    else if (n == "chunk0") {
-        // the first launch runs without thresholds: every row is a candidate, and a query's list holds COS_CAP of them
-        BR_REQUIRE(value >= 1 && value * CG_BM <= COS_CAP, BR_ERR_INVALID, "br_set_cosine_option: chunk0 must be in [1, 4]");
-        g_cos.chunk0 = value;
-    }
-    else if (n == "chunk_mult") { BR_REQUIRE(value >= 2 && value <= 64, BR_ERR_INVALID, "br_set_cosine_option: chunk_mult must be in [2, 64]"); g_cos.chunk_mult = value; }
-    else if (n == "qs_epi") { BR_REQUIRE(value >= 0 && value <= 1, BR_ERR_INVALID, "br_set_cosine_option: qs_epi must be 0 or 1"); g_cos.qs_epi = value; }
-    else if (n == "tighten_threads") { BR_REQUIRE(value >= 32 && value <= TC_T && value % 32 == 0, BR_ERR_INVALID, "br_set_cosine_option: tighten_threads must be a multiple of 32 up to 256"); g_cos.tighten_threads = value; }
+    if (n == "kernel") { BR_REQUIRE(value >= 0 && value <= 1, BR_ERR_INVALID, "br_set_cosine_option: kernel must be 0 or 1"); g_cos_kernel = value; }
     else { set_error("br_set_cosine_option: unknown option " + n); return BR_ERR_INVALID; }
     return BR_OK;
 }
@@ -1119,20 +886,12 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     BR_REQUIRE(k >= 1 && k <= 256, BR_ERR_INVALID, "br_cosine_topk: k must be in [1, 256]");
     BR_REQUIRE(((uintptr_t)docs & 15) == 0 && ((uintptr_t)queries & 15) == 0, BR_ERR_INVALID, "br_cosine_topk: 16-byte alignment required");
     if (nq == 0) return BR_OK;
-    // kernel choice: "qs" query-stationary CTA pairs (default when the query block fits: d <= 768), "mc" 2-CTA multicast,
-    // "plain" one CTA per tile (br_set_cosine_option("kernel", ...) overrides)
-    const bool use_mc = g_cos.kernel != 2;
-    const bool use_qs = d <= QS_NKB * CG_BK && g_cos.kernel == 0;
-    const int qs_bn = g_cos.qs_bn, qs_window = g_cos.qs_window;
+    // kernel choice: query-stationary CTA pairs when the query block fits (d <= 768), else 2-CTA multicast
+    const bool use_qs = d <= QS_NKB * CG_BK && g_cos_kernel == 0;
     CUtensorMap map_d, map_q;
-    BR_TRY(make_map(&map_d, docs, n_docs, d, (use_mc || use_qs) ? 128 : CG_BM));
-    BR_TRY(make_map(&map_q, queries, nq, d, use_qs ? qs_bn / 2 : CG_BN));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QsCfg<128, 8>::SMEM));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<192, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QsCfg<192, 5>::SMEM));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<224, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QsCfg<224, 3>::SMEM));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<224, 3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QsCfg<224, 3>::SMEM));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<160, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QsCfg<160, 6>::SMEM));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG_SMEM));      // per device
+    BR_TRY(make_map(&map_d, docs, n_docs, d, 128));
+    BR_TRY(make_map(&map_q, queries, nq, d, use_qs ? QS_BNH : CG_BN));
+    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QS_SMEM));   // per device
     BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_mc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG_SMEM));
     const size_t Q = (size_t)nq;
     AsyncBuf b_inq(st), b_thr(st), b_cnt(st), b_prev(st), b_ovf(st), b_cand(st), b_h(st);
@@ -1150,35 +909,30 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     // doc chunks of growing size: thresholds learnt on the docs so far filter the next chunk.  A launch emits about
     // k (growth - 1) candidates per query whatever its size; measured on the config-5 shard an emission costs ~1.7 ns of
     // wall time, which makes doubling (13 launches, ~120 emissions per query) faster than 3x / 4x / 8x growth
-    const int chunk0 = g_cos.chunk0, growth = g_cos.chunk_mult;
+    // The first launch runs without thresholds: every row is a candidate, and one doc tile (CG_BM rows) fits a query's
+    // list of COS_CAP.
+    static_assert(CG_BM <= COS_CAP, "the first launch must fit the candidate lists");
     // candidate lists are ~2k long after the first rounds: small CTAs (more of them resident, cheaper barriers)
-    const int tighten_t = g_cos.tighten_threads;
-    int t0 = 0, chunk = chunk0;
+    constexpr int tighten_t = 64;
+    int t0 = 0, chunk = 1;
     while (t0 < n_dt) {
         const int nt = std::min(chunk, n_dt - t0);
         CosArgs a{inv_nd, inv_nq, thr, (int32_t*)b_cnt.p, (int32_t*)b_cand.p, (float*)b_h.p, n_docs, nq, d, t0, t0 + nt,
-                  qs_window};
+                  QS_WINDOW};
         if (use_qs) {
-            const int64_t units = (int64_t)nt * ((nq + qs_bn - 1) / qs_bn);
+            const int64_t units = (int64_t)nt * ((nq + QS_BN - 1) / QS_BN);
             const int grid = 2 * (int)std::min<int64_t>(units, kNumSMs / 2);
-            if (qs_bn == 128) k_cosine_gemm_qs<128, 8><<<grid, QS_THREADS, QsCfg<128, 8>::SMEM, st>>>(map_d, map_q, a);
-            else if (qs_bn == 192) k_cosine_gemm_qs<192, 5><<<grid, QS_THREADS, QsCfg<192, 5>::SMEM, st>>>(map_d, map_q, a);
-            else if (qs_bn == 224 && g_cos.qs_epi == 1) k_cosine_gemm_qs<224, 3, 1><<<grid, QS_THREADS, QsCfg<224, 3>::SMEM, st>>>(map_d, map_q, a);
-            else if (qs_bn == 224) k_cosine_gemm_qs<224, 3><<<grid, QS_THREADS, QsCfg<224, 3>::SMEM, st>>>(map_d, map_q, a);
-            else k_cosine_gemm_qs<160, 6><<<grid, QS_THREADS, QsCfg<160, 6>::SMEM, st>>>(map_d, map_q, a);
-        } else if (use_mc) {
+            k_cosine_gemm_qs<<<grid, QS_THREADS, QS_SMEM, st>>>(map_d, map_q, a);
+        } else {
             const int grid = 2 * (int)std::min<int64_t>((int64_t)nt * ((n_qt + 1) / 2), kNumSMs / 2);
             k_cosine_gemm_mc<<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
-        } else {
-            const int grid = (int)std::min<int64_t>((int64_t)nt * n_qt, kNumSMs);
-            k_cosine_gemm<<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
         }
         BR_CUDA(cudaGetLastError());
         k_tighten_cos<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, k,
                                            (int32_t*)b_ovf.p);
         BR_CUDA(cudaGetLastError());
         t0 += nt;
-        chunk *= growth;
+        chunk *= 2;
     }
     k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, nq, k,
                                                                     doc_base, out_ids, out_sims);

@@ -222,10 +222,8 @@ int br_row_inv_norms(const void* emb_bf16_dev, int64_t n, int32_t d, float* out_
 int br_cosine_topk(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                    const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base,
                    int64_t* out_ids_dev, float* out_sims_dev, void* stream);
-/* Process-wide tuning / test switches of br_cosine_topk; every setting returns bit-identical results.  name = "kernel"
- * (0 auto: query-stationary CTA pairs for d <= 768, else 2-CTA multicast; 1 multicast; 2 one CTA per tile), "qs_bn" (query
- * block width 128/160/192/224), "qs_window" (doc tiles per L2 window), "chunk0", "chunk_mult" (launch schedule),
- * "tighten_threads". */
+/* Process-wide test switch of br_cosine_topk: name = "kernel" (0 auto: query-stationary CTA pairs for d <= 768, else
+ * 2-CTA multicast; 1 always multicast).  Both kernels return bit-identical results.  Any other name: BR_ERR_INVALID. */
 int br_set_cosine_option(const char* name, int value);
 /* Re-rank: query q against its own candidates cand_ids_dev[q, 0..c) (local rows, -1 = empty slot),
  * e.g. the BM25 top-1000 (text_preprocessing_and_embedding_setup.py:342).  doc_inv_norm_dev may be
@@ -263,8 +261,10 @@ int br_last_query_stats(const br_index* ix, br_query_stats* out);
 /* Bracket every launch of the scoring kernel with CUDA events on the call's stream (bench.py's
  * live roofline measurement).  Off by default. */
 int br_set_profiling(br_index* ix, int on);
-/* Tuning / test switches.  name = "fused" (0 forces the dense path for every query; default 1),
- * "tile_g" (queries per group of the tiled kernel: 0 auto, 1, 2, 4 or 8). */
+/* Tuning / test switches.  name = "fused" (0 forces the dense path for every query; default 1), "fused_long" (0 sends
+ * the queries the regular tiled pass cannot serve straight to the dense path instead of the long-query tiled pass;
+ * default 1), "defer_pm" (MaxScore deferral budget of the tiled scorer in per mille of the threshold, 0-1000, 0 = off;
+ * default 650).  Any other name: BR_ERR_INVALID. */
 int br_set_option(br_index* ix, const char* name, int value);
 
 /* ---------------------------------------------------------------------------------------------

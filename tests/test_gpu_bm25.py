@@ -215,28 +215,40 @@ def test_recall_and_routing(golden):
     assert [o.tolist() for o in out] == [orc.retrieve_top_n(oracles[any_lang], q, 10)[0].tolist() for q in some]
 
 
-@pytest.mark.parametrize("g", [0, 1, 2, 4, 8])
-def test_fused_path_equals_dense_path(g):
-    """The tiled smem-accumulator path and the dense path must return identical ids / scores."""
+@pytest.mark.parametrize("k", [3, 5, 10, 16, 32])
+def test_fused_path_equals_dense_path(k):
+    """The tiled smem-accumulator path and the dense path must return identical ids / scores, for k across the k <= 32
+    path (threshold seeding at k, in-kernel k-th lane bound, first-launch size TILE_CAP / (24 k))."""
     c = synth.make_config("C1")
     from document_retrieval_b200 import BM25
     m = BM25.from_token_ids(c["doc_offsets"], c["token_ids"], c["vocab"])
     q = (c["q_terms"], c["q_offsets"])
     m.set_option("fused", 0)
-    ids_d, sc_d = m.retrieve_top_n_batch(q, 10)
+    ids_d, sc_d = m.retrieve_top_n_batch(q, k)
     assert m.query_stats()["queries_fused"] == 0
     m.set_option("fused", 1)
-    m.set_option("tile_g", g)
-    ids_f, sc_f = m.retrieve_top_n_batch(q, 10)
+    ids_f, sc_f = m.retrieve_top_n_batch(q, k)
     st = m.query_stats()
     assert st["queries_fused"] > 0.9 * c["q_offsets"].size
     assert torch.equal(ids_d, ids_f) and torch.equal(sc_d, sc_f)
+    # the tile kernel makes exactly the launches br_tile_launch_count announces (a doc-sharded caller sizes its threshold
+    # exchange by it): a batch of short queries served wholly by the regular fused pass, counted on its second call
+    from document_retrieval_b200 import _lib
+    short = [i for i in range(c["q_offsets"].size - 1) if np.unique(_q(c, i)).size <= 20][:500]
+    qs = (np.concatenate([_q(c, i) for i in short]), np.concatenate([[0], np.cumsum([_q(c, i).size for i in short])]))
+    m.set_option("fused_long", 0)
+    for kk in (k, 100):
+        m.retrieve_top_n_batch(qs, kk)
+        m.retrieve_top_n_batch(qs, kk)
+        st = m.query_stats()
+        assert st["queries_fused"] == len(short) and st["queries_dense"] == 0
+        assert st["score_launches"] == _lib.load().br_tile_launch_count(m._h, kk) >= 1
+    m.set_option("fused_long", 1)
     # okapi / duplicates counted / only docs with a hit
     m2 = BM25.from_token_ids(c["doc_offsets"], c["token_ids"], c["vocab"], variant="okapi", dedup_query=False)
-    m2.set_option("tile_g", g)
-    a = m2.retrieve_top_n_batch(q, 10, positive_only=True, return_counts=True)
+    a = m2.retrieve_top_n_batch(q, k, positive_only=True, return_counts=True)
     m2.set_option("fused", 0)
-    b = m2.retrieve_top_n_batch(q, 10, positive_only=True, return_counts=True)
+    b = m2.retrieve_top_n_batch(q, k, positive_only=True, return_counts=True)
     assert all(torch.equal(x, y) for x, y in zip(a, b))
 
 
