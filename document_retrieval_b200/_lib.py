@@ -34,6 +34,9 @@ SIGNATURES = {
     "br_score_batch": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int, _P, _P]),
     "br_topk_batch": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, _P, _P, _P, _P]),
     "br_topk_batch_records": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, _P, _P, _P]),
+    "br_topk_batch_filtered": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
+    "br_topk_batch_records_filtered": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, _P, _P, _P,
+                                                 _P]),
     "br_topk_merge_records": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),
     "br_rescore_docs": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int, _P, _P, _P, _P]),
     "br_index_enable_tfidf": (C.c_int, [_P, _P]),
@@ -42,6 +45,8 @@ SIGNATURES = {
     "br_topk_merge": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P]),
     "br_row_inv_norms": (C.c_int, [_P, C.c_int64, C.c_int32, _P, _P]),
     "br_cosine_topk": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P]),
+    "br_cosine_topk_filtered": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P,
+                                          _P]),
     "br_set_cosine_option": (C.c_int, [C.c_char_p, C.c_int]),
     "br_cosine_rerank": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "br_dedupe_first_docs": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
@@ -70,8 +75,55 @@ class QueryStats(C.Structure):
                 ("score_ms", C.c_double)]
 
 
+class DocFilterC(C.Structure):
+    """br_doc_filter (include/br_b200.h)."""
+    _fields_ = [("bits_dev", C.c_void_p), ("words", C.c_int64), ("n_rows", C.c_int32), ("query_row_dev", C.c_void_p)]
+
+
 class BRError(RuntimeError):
     pass
+
+
+def _bit_weights(dev):
+    return torch.bitwise_left_shift(torch.ones(32, dtype=torch.int64, device=dev), torch.arange(32, device=dev))
+
+
+def pack_doc_filter(doc_filter, query_filter, nq: int, n_docs: int, device):
+    """``doc_filter`` bool [N] (one allow-list for the whole batch) or [F, N] with ``query_filter`` int [Q] (the row each
+    query uses, -1 = unfiltered) -> (br_doc_filter struct, tensors it points to).  The bits are packed on the device:
+    bit (d & 31) of word (d >> 5) of row f = doc_filter[f, d].  Shape mismatches raise ValueError; a query_filter value
+    outside [-1, F) is left to the library, which rejects it (BRError)."""
+    f = torch.as_tensor(doc_filter)
+    if f.dtype != torch.bool:
+        raise ValueError(f"doc_filter must be a bool array, got {f.dtype}")
+    if f.dim() not in (1, 2) or f.shape[-1] != n_docs:
+        raise ValueError(f"doc_filter must have shape [{n_docs}] or [F, {n_docs}], got {tuple(f.shape)}")
+    if f.dim() == 1:
+        if query_filter is not None:
+            raise ValueError("query_filter needs a 2-D doc_filter [F, N]")
+        f = f[None]
+    elif query_filter is None:
+        raise ValueError("a 2-D doc_filter [F, N] needs query_filter (int [Q], the row of each query, -1 = unfiltered)")
+    n_rows = f.shape[0]
+    if n_rows < 1:
+        raise ValueError("doc_filter has no rows")
+    f = f.to(device).contiguous()
+    words = max(1, (n_docs + 31) // 32)
+    pad = words * 32 - n_docs
+    if pad:
+        f = torch.nn.functional.pad(f, (0, pad))
+    packed = (f.view(n_rows, words, 32).to(torch.int64) * _bit_weights(f.device)).sum(-1)
+    bits = torch.where(packed >= 2 ** 31, packed - 2 ** 32, packed).to(torch.int32).contiguous()
+    rows = None
+    if query_filter is not None:
+        rows = torch.as_tensor(query_filter)
+        if rows.dim() != 1 or rows.shape[0] != nq:
+            raise ValueError(f"query_filter must have shape [{nq}], got {tuple(rows.shape)}")
+        if rows.dtype.is_floating_point or rows.dtype == torch.bool:
+            raise ValueError(f"query_filter must be an integer array, got {rows.dtype}")
+        rows = rows.to(device=device, dtype=torch.int32).contiguous()
+    st = DocFilterC(bits.data_ptr(), words, n_rows, 0 if rows is None else rows.data_ptr())
+    return st, (bits, rows)
 
 
 class VocabularyNotDistinct(BRError):

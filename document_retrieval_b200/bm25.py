@@ -264,9 +264,15 @@ class BM25:
 
     calculate_scores = get_scores          # final_implementation.py:127
 
-    def retrieve_top_n_batch(self, queries, n=10, positive_only=False, return_counts=False):
+    def retrieve_top_n_batch(self, queries, n=10, positive_only=False, return_counts=False, doc_filter=None,
+                             query_filter=None):
         """Batched retrieve_top_n -> (ids int32[Q, n] local doc ids (-1 pads), scores float64[Q, n])
-        as CUDA tensors, ordered by (float64 score desc, doc id asc)."""
+        as CUDA tensors, ordered by (float64 score desc, doc id asc).
+
+        ``doc_filter`` restricts what may be returned: a bool [N] allow-list for the whole batch, or bool [F, N] rows
+        with ``query_filter`` int [Q] (the row of each query, -1 = unfiltered).  A filtered query's result is the
+        result over its allowed docs only - same scores (N, avgdl and idf stay those of the whole index), -1 padding
+        when fewer than n docs are allowed."""
         self._require()
         lib = _lib.load()
         n = int(n)
@@ -276,17 +282,28 @@ class BM25:
         nq = q_off.numel() - 1
         dev = self._device
         with torch.cuda.device(dev):
+            filt = None
+            if doc_filter is not None or query_filter is not None:
+                if doc_filter is None:
+                    raise ValueError("query_filter needs a doc_filter")
+                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
             ids = torch.empty((nq, n), dtype=torch.int32, device=dev)
             sc = torch.empty((nq, n), dtype=torch.float64, device=dev)
             cnt = torch.empty((nq,), dtype=torch.int32, device=dev)
-            check(lib.br_topk_batch(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                    int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
-                                    _lib.stream_ptr(dev)), "br_topk_batch")
+            if filt is None:
+                check(lib.br_topk_batch(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                        int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
+                                        _lib.stream_ptr(dev)), "br_topk_batch")
+            else:
+                check(lib.br_topk_batch_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                                 int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
+                                                 C.byref(filt), _lib.stream_ptr(dev)), "br_topk_batch_filtered")
         return (ids, sc, cnt) if return_counts else (ids, sc)
 
-    def retrieve_records_batch(self, queries, n=10, positive_only=False):
+    def retrieve_records_batch(self, queries, n=10, positive_only=False, doc_filter=None, query_filter=None):
         """retrieve_top_n_batch as packed records int64[Q, n, 2]: [..., 0] = global doc id (doc_base + local id, -1
-        pads), [..., 1] = the float64 score's bits - what a doc-sharded caller all-gathers in one collective."""
+        pads), [..., 1] = the float64 score's bits - what a doc-sharded caller all-gathers in one collective.
+        ``doc_filter`` / ``query_filter``: as in retrieve_top_n_batch (over this index's local doc ids)."""
         self._require()
         lib = _lib.load()
         n = int(n)
@@ -296,10 +313,21 @@ class BM25:
         nq = q_off.numel() - 1
         dev = self._device
         with torch.cuda.device(dev):
+            filt = None
+            if doc_filter is not None or query_filter is not None:
+                if doc_filter is None:
+                    raise ValueError("query_filter needs a doc_filter")
+                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
             rec = torch.empty((nq, n, 2), dtype=torch.int64, device=dev)
-            check(lib.br_topk_batch_records(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                            int(self.dedup_query), int(positive_only), ptr(rec), None,
-                                            _lib.stream_ptr(dev)), "br_topk_batch_records")
+            if filt is None:
+                check(lib.br_topk_batch_records(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                                int(self.dedup_query), int(positive_only), ptr(rec), None,
+                                                _lib.stream_ptr(dev)), "br_topk_batch_records")
+            else:
+                check(lib.br_topk_batch_records_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                                         int(self.dedup_query), int(positive_only), ptr(rec), None,
+                                                         C.byref(filt), _lib.stream_ptr(dev)),
+                      "br_topk_batch_records_filtered")
         return rec
 
     def exact_scores(self, query):
@@ -349,20 +377,33 @@ class BM25:
                                           _lib.stream_ptr(dev)), "br_rerank_v3_scores")
         return out
 
-    def retrieve_top_n(self, query, n=10):
+    def retrieve_top_n(self, query, n=10, doc_filter=None):
         """bm25_ranking.ipynb:206-213 -> np.ndarray[int64] of local doc indices, best first.
-        ``n >= N`` returns the full ranking (:208-209).  Ties: doc id ascending."""
+        ``n >= N`` returns the full ranking (:208-209).  Ties: doc id ascending.  ``doc_filter`` (bool [N]): rank only
+        the allowed docs (the result then holds at most as many ids as docs are allowed)."""
         self._require()
         n = int(n)
         N = self.corpus_size
+        if doc_filter is not None:
+            f = torch.as_tensor(doc_filter)
+            if f.dtype != torch.bool or f.dim() != 1 or f.shape[0] != N:
+                raise ValueError(f"doc_filter must be a bool array of shape [{N}]")
         if n >= N or n > _lib.BR_MAX_K:
             s = self.exact_scores(query)
-            order = torch.sort(-s, stable=True).indices[:min(n, N)]     # stable: ties keep id order
+            if doc_filter is None:
+                order = torch.sort(-s, stable=True).indices[:min(n, N)]     # stable: ties keep id order
+            else:
+                allowed = torch.nonzero(f.to(s.device)).flatten()
+                order = allowed[torch.sort(-s[allowed], stable=True).indices][:min(n, N)]
             return order.cpu().numpy().astype(np.int64)
         if n <= 0:
             return np.zeros(0, dtype=np.int64)
-        ids, _ = self.retrieve_top_n_batch([query], n)
-        return ids[0].cpu().numpy().astype(np.int64)
+        if doc_filter is None:
+            ids, _ = self.retrieve_top_n_batch([query], n)
+            return ids[0].cpu().numpy().astype(np.int64)
+        ids, _ = self.retrieve_top_n_batch([query], n, doc_filter=f)
+        row = ids[0].cpu().numpy().astype(np.int64)
+        return row[row >= 0]
 
     get_top_n = retrieve_top_n             # BASELINE.json's wording (rank_bm25 style)
 

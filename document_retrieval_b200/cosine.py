@@ -5,6 +5,8 @@ the B200: a bf16 tcgen05 GEMM with the L2-normalisation and the top-k filter fus
 cosine top-10).  Host code here only moves tensors; all arithmetic is in libbr_b200.so."""
 from __future__ import annotations
 
+import ctypes as C
+
 import torch
 
 from . import _lib
@@ -40,16 +42,28 @@ class CosineIndex:
             check(lib.br_row_inv_norms(ptr(self.docs), self.n_docs, self.dim, ptr(self.inv_norm), _lib.stream_ptr(dev)),
                   "br_row_inv_norms")
 
-    def topk(self, query_embeddings, k=10):
-        """Brute-force cosine top-k -> (ids int64[Q, k] (doc_base + row), sims float32[Q, k]) on the device."""
+    def topk(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
+        """Brute-force cosine top-k -> (ids int64[Q, k] (doc_base + row), sims float32[Q, k]) on the device.
+        ``doc_filter`` restricts the rows a query may return: bool [n] for the whole batch, or bool [F, n] with
+        ``query_filter`` int [Q] (row of each query, -1 = unfiltered); exact, -1 pads when fewer than k rows are allowed."""
         lib = _lib.load()
         q = _bf16(query_embeddings, self.device)
         nq = q.shape[0]
         with torch.cuda.device(self.device):
+            filt = None
+            if doc_filter is not None or query_filter is not None:
+                if doc_filter is None:
+                    raise ValueError("query_filter needs a doc_filter")
+                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_docs, self.device)
             ids = torch.empty((nq, k), dtype=torch.int64, device=self.device)
             sims = torch.empty((nq, k), dtype=torch.float32, device=self.device)
-            check(lib.br_cosine_topk(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq, int(k),
-                                     self.doc_base, ptr(ids), ptr(sims), _lib.stream_ptr(self.device)), "br_cosine_topk")
+            if filt is None:
+                check(lib.br_cosine_topk(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq, int(k),
+                                         self.doc_base, ptr(ids), ptr(sims), _lib.stream_ptr(self.device)), "br_cosine_topk")
+            else:
+                check(lib.br_cosine_topk_filtered(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq,
+                                                  int(k), self.doc_base, ptr(ids), ptr(sims), C.byref(filt),
+                                                  _lib.stream_ptr(self.device)), "br_cosine_topk_filtered")
         return ids, sims
 
     def rerank(self, query_embeddings, candidate_ids, k=10):

@@ -17,20 +17,34 @@ int br_score_batch(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_of
     return br::score_batch(ix, q_terms_dev, q_offsets_dev, nq, dedup, out_scores_dev, (cudaStream_t)stream);
 }
 
+int br_topk_batch_filtered(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq,
+                           int32_t n_terms, int32_t k, int dedup, int positive_only, int32_t* out_ids_dev,
+                           double* out_scores_dev, int32_t* out_counts_dev, const br_doc_filter* filter, void* stream) {
+    BR_REQUIRE(out_ids_dev && out_scores_dev, BR_ERR_INVALID, "br_topk_batch: null pointer");
+    return br::topk_batch(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only, out_ids_dev, out_scores_dev,
+                          out_counts_dev, nullptr, filter, (cudaStream_t)stream);
+}
+
 int br_topk_batch(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq, int32_t n_terms,
                   int32_t k, int dedup, int positive_only, int32_t* out_ids_dev, double* out_scores_dev,
                   int32_t* out_counts_dev, void* stream) {
-    BR_REQUIRE(out_ids_dev && out_scores_dev, BR_ERR_INVALID, "br_topk_batch: null pointer");
-    return br::topk_batch(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only, out_ids_dev, out_scores_dev,
-                          out_counts_dev, nullptr, (cudaStream_t)stream);
+    return br_topk_batch_filtered(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only, out_ids_dev,
+                                  out_scores_dev, out_counts_dev, nullptr, stream);
+}
+
+int br_topk_batch_records_filtered(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq,
+                                   int32_t n_terms, int32_t k, int dedup, int positive_only, br_record* out_records_dev,
+                                   int32_t* out_counts_dev, const br_doc_filter* filter, void* stream) {
+    BR_REQUIRE(out_records_dev, BR_ERR_INVALID, "br_topk_batch_records: null pointer");
+    return br::topk_batch(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only, nullptr, nullptr,
+                          out_counts_dev, out_records_dev, filter, (cudaStream_t)stream);
 }
 
 int br_topk_batch_records(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq,
                           int32_t n_terms, int32_t k, int dedup, int positive_only, br_record* out_records_dev,
                           int32_t* out_counts_dev, void* stream) {
-    BR_REQUIRE(out_records_dev, BR_ERR_INVALID, "br_topk_batch_records: null pointer");
-    return br::topk_batch(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only, nullptr, nullptr,
-                          out_counts_dev, out_records_dev, (cudaStream_t)stream);
+    return br_topk_batch_records_filtered(ix, q_terms_dev, q_offsets_dev, nq, n_terms, k, dedup, positive_only,
+                                          out_records_dev, out_counts_dev, nullptr, stream);
 }
 
 int br_topk_merge_records(const br_record* records_dev, int32_t n_parts, int32_t nq, int32_t k, int64_t* out_ids_dev,

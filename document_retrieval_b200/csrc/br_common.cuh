@@ -99,6 +99,27 @@ inline int scratch_alloc(void** p, size_t bytes, cudaStream_t st) {
 constexpr int kNumSMs = 148;          // B200
 constexpr float kBandRel = 1e-5f;     // fp32 candidate band kept below the k-th fp32 score (see DESIGN.md)
 
+// Per-query doc filter of a batch (br_doc_filter after validation): query q may return local doc d iff row[q] < 0 or bit
+// (d & 31) of word (d >> 5) of bitmap row row[q] is set.  row[] is indexed like the kernel's query index (a sub-batch gets
+// its own remapped copy) and holds only values in [-1, n_rows).
+struct DocFilter {
+    const uint32_t* bits;
+    int64_t words;
+    const int32_t* row;
+#ifdef __CUDACC__
+    __device__ __forceinline__ const uint32_t* row_of(int q) const {
+        const int32_t r = row[q];
+        return r < 0 ? nullptr : bits + (int64_t)r * words;
+    }
+#endif
+};
+#ifdef __CUDACC__
+// fr: the query's bitmap row (nullptr: unfiltered); doc < n_docs
+__device__ __forceinline__ bool doc_allowed(const uint32_t* fr, uint32_t doc) {
+    return !fr || ((__ldg(fr + (doc >> 5)) >> (doc & 31)) & 1u) != 0u;
+}
+#endif
+
 }  // namespace br
 
 // One posting: doc id + precomputed fp32 BM25 weight, 8 bytes, read as one 64-bit word
@@ -153,6 +174,7 @@ struct br_index {
 
     // query-time scratch
     br::DevBuf ws_prep, ws_dense, ws_sel, ws_cand, ws_misc, ws_tile, ws_sort, ws_cold, ws_rec;
+    br::DevBuf ws_filt;             // filtered batches: validated filter rows of the batch and of its redo sub-batch
     br_query_stats stats{};
 
     bool allow_fused = true, allow_fused_long = true;
@@ -208,7 +230,7 @@ int score_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_offsets, 
                 float* out_scores, cudaStream_t st);
 int topk_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_offsets, int32_t nq, int32_t n_terms, int32_t k,
                int dedup, int positive_only, int32_t* out_ids, double* out_scores, int32_t* out_counts,
-               br_record* out_recs, cudaStream_t st);
+               br_record* out_recs, const br_doc_filter* filter, cudaStream_t st);
 int rescore_docs(br_index* ix, const int32_t* q_terms, const int32_t* q_offsets, int32_t nq, int dedup,
                  const int32_t* cand_ids, const int64_t* cand_off, double* out_scores, cudaStream_t st);
 int enable_tfidf(br_index* ix, cudaStream_t st);

@@ -175,12 +175,23 @@ struct CosArgs {
     int32_t d;
     int32_t tile_begin, tile_end;   // doc tiles [tile_begin, tile_end) of CG_BM rows
     int32_t window;                 // query-stationary kernel: doc tiles per L2 window
+    // row filter (the <true> instantiations only; appended so that the fields above keep their offsets)
+    const uint32_t* fbits;          // bitmap rows [n_rows, fwords]
+    int64_t fwords;
+    const int32_t* frow;            // [nq] row of query q, -1 = unfiltered
 };
+
+// The filtered kernels keep each query column's filter row in shared memory behind the barriers (beyond the unfiltered
+// layout, so that it stays as it is); a row is tested only where a score has passed the threshold.
+__device__ __forceinline__ bool cos_row_allowed(const CosArgs& a, int32_t frow, int64_t doc) {
+    return frow < 0 || ((__ldg(a.fbits + (int64_t)frow * a.fwords + (doc >> 5)) >> (doc & 31)) & 1u) != 0u;
+}
 
 // Multicast kernel (d > 768): a CTA computes docs[256-row tile] x queries[256-col tile] with two 128-row UMMAs sharing the
 // query tile, fp32 accumulators in 2 x 256 TMEM columns.  CTA pairs share every doc (A) tile - rank r loads rows
 // [128r, 128r+128) of it and multicasts them to both CTAs, so the doc operand crosses L2->SM once per pair; each CTA loads
 // its own query (B) tile.  Stage release is cluster-wide (both CTAs' UMMAs arrive on both CTAs' empty barriers).
+template <bool FILT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cosine_gemm_mc(const __grid_constant__ CUtensorMap map_docs,
                                                                const __grid_constant__ CUtensorMap map_q, CosArgs a) {
     extern __shared__ unsigned char smem_raw[];
@@ -191,6 +202,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cos
     float* s_inq = s_thr + CG_BN;                                                        // [CG_BN] 1/(||q||+eps)
     uint64_t* bars = reinterpret_cast<uint64_t*>(s_inq + CG_BN);                        // full[S] empty[S] tfull[2] tempty[2]
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 12);
+    int32_t* s_frow = reinterpret_cast<int32_t*>(bars + 14);                            // [CG_BN] (FILT) filter rows
     const uint32_t bar0 = smem_u32(bars);
     auto full_bar = [&](int s) { return bar0 + 8u * s; };
     auto empty_bar = [&](int s) { return bar0 + 8u * (CG_STAGES + s); };
@@ -286,6 +298,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cos
                 }
                 s_thr[c] = th;
                 s_inq[c] = iq;
+                if constexpr (FILT) s_frow[c] = q < a.nq ? a.frow[q] : -1;
             }
             asm volatile("bar.sync 1, 256;" ::: "memory");          // epilogue warps only
             mbar_wait(tfull_bar(half), acc_phase);
@@ -318,7 +331,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cos
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
                         const float sc = __uint_as_float(cur[j]) * inv_d;
-                        if (sc >= s_thr[b * 32 + j]) {
+                        bool pass = sc >= s_thr[b * 32 + j];
+                        if constexpr (FILT) pass = pass && cos_row_allowed(a, s_frow[b * 32 + j], doc);
+                        if (pass) {
                             const int q = qt * CG_BN + b * 32 + j;
                             const int pos = atomicAdd(a.cand_cnt + q, 1);
                             if (pos < COS_CAP) {
@@ -442,6 +457,7 @@ struct QsIter {
     }
 };
 
+template <bool FILT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cosine_gemm_qs(const __grid_constant__ CUtensorMap map_docs,
                                                                const __grid_constant__ CUtensorMap map_q, CosArgs a) {
     extern __shared__ unsigned char smem_raw[];
@@ -453,6 +469,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
     float* s_inq = s_thr + QS_BN;                                                                   // [QS_BN]
     uint64_t* bars = reinterpret_cast<uint64_t*>(s_inq + QS_BN);
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + 2 * QS_STAGES + 6);
+    int32_t* s_frow = reinterpret_cast<int32_t*>(bars + 2 * QS_STAGES + 8);             // [QS_BN] (FILT) filter rows
     const uint32_t bar0 = smem_u32(bars);
     auto full_bar = [&](int s) { return bar0 + 8u * s; };                      // leader: doc stage filled (both CTAs' bytes)
     auto empty_bar = [&](int s) { return bar0 + 8u * (QS_STAGES + s); };       // each CTA: doc stage consumed
@@ -570,6 +587,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
                     }
                     s_thr[et] = th;
                     s_inq[et] = iq;
+                    if constexpr (FILT) s_frow[et] = q < a.nq ? a.frow[q] : -1;
                 }
                 asm volatile("bar.sync 1, 256;" ::: "memory");
             }
@@ -632,7 +650,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
 #pragma unroll
                     for (int j = 0; j < 16; ++j) {
                         const float sc = __uint_as_float(hv[j]) * inv_d;
-                        if (sc >= thc[j]) {
+                        bool pass = sc >= thc[j];
+                        if constexpr (FILT) pass = pass && cos_row_allowed(a, s_frow[col0 + c * 16 + j], doc);
+                        if (pass) {
                             const int col = col0 + c * 16 + j;
                             const int q = un.qb * QS_BN + col;
                             const int pos = atomicAdd(a.cand_cnt + q, 1);
@@ -855,6 +875,26 @@ __global__ void k_iota_rows(int32_t* __restrict__ out, int32_t rows, int64_t n) 
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x)
         out[i] = (int32_t)(i % n);
 }
+// the same for filtered queries: row r of the list holds the doc rows query qs[r] may return, -1 (an empty slot of the
+// gather pass) for the others
+__global__ void k_iota_rows_filtered(int32_t* __restrict__ out, int32_t rows, int64_t n, const int32_t* __restrict__ qs,
+                                     DocFilter f) {
+    const int64_t total = (int64_t)rows * n;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = i / n, d = i - r * n;
+        out[i] = doc_allowed(f.row_of(qs[r]), (uint32_t)d) ? (int32_t)d : -1;
+    }
+}
+// validated filter rows (the same rule as br_topk_batch_filtered): a value outside [-1, n_rows) sets *bad and becomes -1
+__global__ void k_cos_filter_rows(const int32_t* __restrict__ in, int32_t nq, int32_t n_rows, int32_t* __restrict__ out,
+                                  int32_t* __restrict__ bad) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const int32_t r = in ? in[q] : 0;
+    const bool ok = r >= -1 && r < n_rows;
+    if (!ok) atomicOr(bad, 1);
+    out[q] = ok ? r : -1;
+}
 __global__ void k_cos_patch(const int32_t* __restrict__ rows, int32_t nr, int32_t k, const int32_t* __restrict__ ids,
                             const float* __restrict__ sims, int64_t doc_base, int64_t* __restrict__ out_ids,
                             float* __restrict__ out_sims) {
@@ -879,24 +919,47 @@ int set_cosine_option(const char* name, int value) {
 }
 
 int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries, int32_t nq,
-                int32_t k, int64_t doc_base, int64_t* out_ids, float* out_sims, cudaStream_t st) {
+                int32_t k, int64_t doc_base, int64_t* out_ids, float* out_sims, const br_doc_filter* filter, cudaStream_t st) {
     BR_REQUIRE(docs && inv_nd && queries && out_ids && out_sims, BR_ERR_INVALID, "br_cosine_topk: null pointer");
     BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31) && nq >= 0, BR_ERR_INVALID, "br_cosine_topk: bad sizes");
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, "br_cosine_topk: embedding dim must be a multiple of 8 (16-byte rows for TMA)");
     BR_REQUIRE(k >= 1 && k <= 256, BR_ERR_INVALID, "br_cosine_topk: k must be in [1, 256]");
     BR_REQUIRE(((uintptr_t)docs & 15) == 0 && ((uintptr_t)queries & 15) == 0, BR_ERR_INVALID, "br_cosine_topk: 16-byte alignment required");
+    if (filter) {
+        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, "br_cosine_topk: filter bitmap is null");
+        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, "br_cosine_topk: filter n_rows must be >= 1");
+        BR_REQUIRE(filter->words >= (n_docs + 31) / 32, BR_ERR_INVALID, "br_cosine_topk: filter words < ceil(n_docs / 32)");
+    }
     if (nq == 0) return BR_OK;
     // kernel choice: query-stationary CTA pairs when the query block fits (d <= 768), else 2-CTA multicast
     const bool use_qs = d <= QS_NKB * CG_BK && g_cos_kernel == 0;
     CUtensorMap map_d, map_q;
     BR_TRY(make_map(&map_d, docs, n_docs, d, 128));
     BR_TRY(make_map(&map_q, queries, nq, d, use_qs ? QS_BNH : CG_BN));
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QS_SMEM));   // per device
-    BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_mc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG_SMEM));
+    const bool filt = filter != nullptr;
+    // the filtered kernels keep the filter rows of their query columns behind the unfiltered layout
+    const size_t qs_smem = QS_SMEM + (filt ? sizeof(int32_t) * QS_BN : 0), mc_smem = CG_SMEM + (filt ? sizeof(int32_t) * CG_BN : 0);
+    if (filt) {
+        BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)qs_smem));
+        BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_mc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mc_smem));
+    } else {
+        BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_qs<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QS_SMEM));   // per device
+        BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_mc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG_SMEM));
+    }
     const size_t Q = (size_t)nq;
-    AsyncBuf b_inq(st), b_thr(st), b_cnt(st), b_prev(st), b_ovf(st), b_cand(st), b_h(st);
+    AsyncBuf b_inq(st), b_thr(st), b_cnt(st), b_prev(st), b_ovf(st), b_cand(st), b_h(st), b_frow(st);
     BR_TRY(b_inq.alloc(4 * Q)); BR_TRY(b_thr.alloc(4 * Q)); BR_TRY(b_cnt.alloc(4 * Q)); BR_TRY(b_prev.alloc(4 * Q));
     BR_TRY(b_ovf.alloc(4 * Q)); BR_TRY(b_cand.alloc(4 * Q * COS_CAP)); BR_TRY(b_h.alloc(4 * Q * COS_CAP));
+    DocFilter fv{};
+    int32_t* f_bad = nullptr;
+    if (filt) {                                           // [nq] validated rows + the "bad row" flag
+        BR_TRY(b_frow.alloc(4 * Q + 16));
+        f_bad = (int32_t*)b_frow.p + Q;
+        BR_CUDA(cudaMemsetAsync(f_bad, 0, 4, st));
+        k_cos_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, (int32_t*)b_frow.p, f_bad);
+        BR_CUDA(cudaGetLastError());
+        fv = DocFilter{filter->bits_dev, filter->words, (const int32_t*)b_frow.p};
+    }
     float* inv_nq = (float*)b_inq.p;
     float* thr = (float*)b_thr.p;
     BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
@@ -918,14 +981,16 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     while (t0 < n_dt) {
         const int nt = std::min(chunk, n_dt - t0);
         CosArgs a{inv_nd, inv_nq, thr, (int32_t*)b_cnt.p, (int32_t*)b_cand.p, (float*)b_h.p, n_docs, nq, d, t0, t0 + nt,
-                  QS_WINDOW};
+                  QS_WINDOW, fv.bits, fv.words, fv.row};
         if (use_qs) {
             const int64_t units = (int64_t)nt * ((nq + QS_BN - 1) / QS_BN);
             const int grid = 2 * (int)std::min<int64_t>(units, kNumSMs / 2);
-            k_cosine_gemm_qs<<<grid, QS_THREADS, QS_SMEM, st>>>(map_d, map_q, a);
+            if (filt) k_cosine_gemm_qs<true><<<grid, QS_THREADS, qs_smem, st>>>(map_d, map_q, a);
+            else k_cosine_gemm_qs<false><<<grid, QS_THREADS, QS_SMEM, st>>>(map_d, map_q, a);
         } else {
             const int grid = 2 * (int)std::min<int64_t>((int64_t)nt * ((n_qt + 1) / 2), kNumSMs / 2);
-            k_cosine_gemm_mc<<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
+            if (filt) k_cosine_gemm_mc<true><<<grid, CG_THREADS, mc_smem, st>>>(map_d, map_q, a);
+            else k_cosine_gemm_mc<false><<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
         }
         BR_CUDA(cudaGetLastError());
         k_tighten_cos<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, k,
@@ -938,8 +1003,11 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
                                                                     doc_base, out_ids, out_sims);
     BR_CUDA(cudaGetLastError());
     std::vector<int32_t> ovf(Q);
+    int32_t h_fbad = 0;
     BR_CUDA(cudaMemcpyAsync(ovf.data(), b_ovf.p, 4 * Q, cudaMemcpyDeviceToHost, st));
+    if (f_bad) BR_CUDA(cudaMemcpyAsync(&h_fbad, f_bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
+    BR_REQUIRE(!h_fbad, BR_ERR_INVALID, "br_cosine_topk: a filter query_row is outside [-1, n_rows)");
     // A query with more than COS_CAP candidates at or above its threshold in one launch (masses of duplicate / exactly tied
     // embeddings) cannot be served by the filter: those few queries are answered exactly by scoring every doc row with the
     // gather kernel (same normalisation, ties by doc id) - slow (one pass over the embeddings per query) but exact.
@@ -957,14 +1025,20 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         const int32_t nr_max = (int32_t)std::min<size_t>(redo.size(), (size_t)sub);
         BR_TRY(b_q.alloc((size_t)nr_max * d * 2)); BR_TRY(b_c.alloc(4 * (size_t)nr_max * (size_t)n_docs));
         BR_TRY(b_oi.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_os.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_rows.alloc(4 * (size_t)nr_max));
-        k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr_max, n_docs);
-        BR_CUDA(cudaGetLastError());
+        if (!filt) {
+            k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr_max, n_docs);
+            BR_CUDA(cudaGetLastError());
+        }
         for (size_t r0 = 0; r0 < redo.size(); r0 += (size_t)sub) {
             const int32_t nr = (int32_t)std::min<size_t>((size_t)sub, redo.size() - r0);
             for (int32_t i = 0; i < nr; ++i)
                 BR_CUDA(cudaMemcpyAsync((char*)b_q.p + (size_t)i * d * 2, (const char*)queries + (size_t)redo[r0 + (size_t)i] * d * 2,
                                         (size_t)d * 2, cudaMemcpyDeviceToDevice, st));
             BR_CUDA(cudaMemcpyAsync(b_rows.p, redo.data() + r0, 4 * (size_t)nr, cudaMemcpyHostToDevice, st));
+            if (filt) {                                   // each redone query gathers only the rows it may return
+                k_iota_rows_filtered<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr, n_docs, (const int32_t*)b_rows.p, fv);
+                BR_CUDA(cudaGetLastError());
+            }
             BR_TRY(cosine_rerank(docs, inv_nd, n_docs, d, b_q.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs, k, (int32_t*)b_oi.p,
                                  (float*)b_os.p, st));             // synchronises: b_rows / b_q may be reused afterwards
             k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_rows.p, nr, k, (const int32_t*)b_oi.p,
@@ -1023,7 +1097,14 @@ int br_cosine_topk(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int
                    const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base, int64_t* out_ids_dev,
                    float* out_sims_dev, void* stream) {
     return br::cosine_topk(docs_bf16_dev, doc_inv_norm_dev, n_docs, d, queries_bf16_dev, nq, k, doc_base, out_ids_dev,
-                           out_sims_dev, (cudaStream_t)stream);
+                           out_sims_dev, nullptr, (cudaStream_t)stream);
+}
+
+int br_cosine_topk_filtered(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
+                            const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base, int64_t* out_ids_dev,
+                            float* out_sims_dev, const br_doc_filter* filter, void* stream) {
+    return br::cosine_topk(docs_bf16_dev, doc_inv_norm_dev, n_docs, d, queries_bf16_dev, nq, k, doc_base, out_ids_dev,
+                           out_sims_dev, filter, (cudaStream_t)stream);
 }
 
 int br_set_cosine_option(const char* name, int value) { return br::set_cosine_option(name, value); }

@@ -157,14 +157,20 @@ struct SelView {
 
 constexpr int SEL_T = 1024;
 
+// FILT: a doc the query's filter row excludes gets key 0, below every allowed doc, so kth_key == 0 means "fewer than k
+// allowed docs (with a hit, for positive_only)": mode 2 then takes every allowed doc (with a hit).  Disallowed docs are
+// neither counted nor emitted, so the zero-score tail of mode 1 is made of allowed docs in doc-id order.
+template <bool FILT>
 __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict__ scores, int64_t n_docs, int32_t k,
                                                         int positive_only, SelView sv, int32_t q_begin,
-                                                        const int32_t* __restrict__ n_terms) {
+                                                        const int32_t* __restrict__ n_terms, DocFilter f) {
     __shared__ uint32_t hist[2048];
     __shared__ uint32_t s_bin, s_above;
     __shared__ unsigned long long s_cnt[2];
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
+    const uint32_t* fr = nullptr;
+    if constexpr (FILT) fr = f.row_of(q);
     uint32_t prefix = 0, mask = 0;
     uint32_t k_rem = (uint32_t)min((int64_t)k, n_docs);
     const int shifts[3] = {21, 10, 0};
@@ -175,7 +181,8 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
         for (int i = threadIdx.x; i < 2048; i += SEL_T) hist[i] = 0;
         __syncthreads();
         for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
-            const uint32_t u = score_key(row[i], positive_only);
+            uint32_t u = score_key(row[i], positive_only);
+            if constexpr (FILT) u = doc_allowed(fr, (uint32_t)i) ? u : 0u;
             if ((u & mask) == prefix) atomicAdd(&hist[(u >> shift) & (nb - 1)], 1u);
         }
         __syncthreads();
@@ -196,7 +203,9 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     const uint32_t kth_key = prefix;
     int mode = 0;
     float lo = 0.f;
-    if (positive_only && kth_key == 0u) {
+    bool take_all = positive_only && kth_key == 0u;
+    if constexpr (FILT) take_all = kth_key == 0u;  // fewer than k allowed docs (with a hit): take them all
+    if (take_all) {
         mode = 2;                                   // fewer than k docs with a hit: take them all
     } else {
         const float kth = key_score(kth_key);
@@ -210,9 +219,16 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     unsigned long long c_band = 0, c_pos = 0;
     for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
         const float s = row[i];
-        if (mode == 2) c_band += (s != 0.0f);
-        else if (mode == 1) c_pos += (s > 0.0f);
-        else c_band += (s >= lo && !(positive_only && s == 0.0f));
+        if constexpr (FILT) {
+            const bool ok = doc_allowed(fr, (uint32_t)i);
+            if (mode == 2) c_band += (ok && (!positive_only || s != 0.0f));
+            else if (mode == 1) c_pos += (ok && s > 0.0f);
+            else c_band += (ok && s >= lo && !(positive_only && s == 0.0f));
+        } else {
+            if (mode == 2) c_band += (s != 0.0f);
+            else if (mode == 1) c_pos += (s > 0.0f);
+            else c_band += (s >= lo && !(positive_only && s == 0.0f));
+        }
     }
     for (int o = 16; o > 0; o >>= 1) {
         c_band += __shfl_xor_sync(0xffffffffu, c_band, o);
@@ -234,11 +250,15 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     }
 }
 
+template <bool FILT>
 __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ scores, int64_t n_docs,
                                                       int positive_only, SelView sv, int32_t q_begin,
-                                                      const int64_t* __restrict__ cand_off, int32_t* __restrict__ cand) {
+                                                      const int64_t* __restrict__ cand_off, int32_t* __restrict__ cand,
+                                                      DocFilter f) {
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
+    const uint32_t* fr = nullptr;
+    if constexpr (FILT) fr = f.row_of(q);
     const int mode = sv.mode[q];
     const float lo = sv.lo[q];
     const uint32_t zfill = (uint32_t)sv.zfill[q];
@@ -248,9 +268,16 @@ __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ 
         const int64_t i = base + threadIdx.x;
         const float s = i < n_docs ? row[i] : -CUDART_INF_F;
         bool take, zero = false;
-        if (mode == 2) take = i < n_docs && s != 0.0f;
-        else if (mode == 1) { take = s > 0.0f; zero = i < n_docs && s == 0.0f; }
-        else take = i < n_docs && s >= lo && !(positive_only && s == 0.0f);
+        if constexpr (FILT) {
+            const bool ok = i < n_docs && doc_allowed(fr, (uint32_t)i);
+            if (mode == 2) take = ok && (!positive_only || s != 0.0f);
+            else if (mode == 1) { take = ok && s > 0.0f; zero = ok && s == 0.0f; }
+            else take = ok && s >= lo && !(positive_only && s == 0.0f);
+        } else {
+            if (mode == 2) take = i < n_docs && s != 0.0f;
+            else if (mode == 1) { take = s > 0.0f; zero = i < n_docs && s == 0.0f; }
+            else take = i < n_docs && s >= lo && !(positive_only && s == 0.0f);
+        }
         uint32_t total, ztotal = 0, zex = 0;
         if (mode == 1) {
             zex = block_excl_scan(zero ? 1u : 0u, &ztotal);
@@ -696,7 +723,8 @@ int score_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
 // Dense path for queries [q_begin, q_begin + nq) of a prepared batch; results into out_* rows.
 static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, const int64_t* chunk_start,
                       int32_t q_begin, int32_t nq, int32_t k, int dedup, int positive_only, int32_t* out_ids,
-                      double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table = nullptr) {
+                      double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table = nullptr,
+                      const DocFilter* filt = nullptr) {
     // post_table != nullptr: score with that weight table and rank by the fp32 dense scores themselves
     // (TF-IDF cosine stage); otherwise BM25 weights + exact float64 re-score of the candidate band.
     const bool fp32_rank = post_table != nullptr;
@@ -723,7 +751,9 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
         k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(post, ix->row_ptr, q_off, pv, chunk_start, b0, bn, dense, N);
         BR_CUDA(cudaGetLastError());
         ix->prof_end(st);
-        k_select_radix<<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt);
+        // (query chunks keep batch-wide query indices b0 + i, so the filter rows need no remapping here)
+        if (filt) k_select_radix<true><<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, *filt);
+        else k_select_radix<false><<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, DocFilter{});
         BR_CUDA(cudaGetLastError());
         BR_CUDA(cudaMemcpyAsync(h_cnt.data(), sv.cnt + b0, sizeof(int64_t) * (size_t)bn, cudaMemcpyDeviceToHost, st));
         BR_CUDA(cudaStreamSynchronize(st));
@@ -734,7 +764,8 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
         BR_TRY(ix->ws_cand.reserve((size_t)(total + 1) * (sizeof(int32_t) + sizeof(double)) + 256));
         int32_t* cand = ix->ws_cand.as<int32_t>();
         double* cand_sc = (double*)(ix->ws_cand.as<char>() + (((size_t)(total + 1) * sizeof(int32_t) + 255) & ~(size_t)255));
-        k_emit_cands<<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand);
+        if (filt) k_emit_cands<true><<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, *filt);
+        else k_emit_cands<false><<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, DocFilter{});
         BR_CUDA(cudaGetLastError());
         if (total > 0 && fp32_rank) {
             // TF-IDF stage: the fp32 row only selects the band; the candidates are re-scored in float64
@@ -763,16 +794,38 @@ __global__ void k_pack_records(const int32_t* __restrict__ ids, const double* __
     out[i] = br_record{d >= 0 ? (int64_t)d + doc_base : (int64_t)-1, sc[i]};
 }
 
+// Filter rows of a batch (br_doc_filter::query_row_dev, NULL = row 0 for every query), validated on the device: a value
+// outside [-1, n_rows) sets *bad (reported when the call returns) and becomes -1, so no kernel ever addresses a row that
+// does not exist.
+__global__ void k_filter_rows(const int32_t* __restrict__ in, int32_t nq, int32_t n_rows, int32_t* __restrict__ out,
+                              int32_t* __restrict__ bad) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const int32_t r = in ? in[q] : 0;
+    const bool ok = r >= -1 && r < n_rows;
+    if (!ok) atomicOr(bad, 1);
+    out[q] = ok ? r : -1;
+}
+// filter rows of a compacted sub-batch: out[i] = in[idx[i]]
+__global__ void k_gather_rows(const int32_t* __restrict__ idx, int32_t n, const int32_t* __restrict__ in, int32_t* __restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = in[idx[i]];
+}
+
 // A prepared batch through the tiled path, then - for the queries it cannot serve exactly - the long-query pass and the
-// dense path.  post_table: weight table of the TF-IDF cosine stage (nullptr: BM25).
+// dense path.  post_table: weight table of the TF-IDF cosine stage (nullptr: BM25).  filt: the batch's doc filter
+// (nullptr: none); sub_rows: int32[nq] scratch for the filter rows of the compacted sub-batches.
 static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int32_t T, int32_t k, int dedup,
                           int positive_only, const PrepView& pv, const int64_t* chunk_start, int32_t* out_ids,
-                          double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table) {
+                          double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table,
+                          const DocFilter* filt = nullptr, int32_t* sub_rows = nullptr) {
     if (!fused_supported(ix, k, nq, post_table != nullptr)) {
-        BR_TRY(topk_dense(ix, q_off, pv, chunk_start, 0, nq, k, dedup, positive_only, out_ids, out_scores, out_counts, st, post_table));
+        BR_TRY(topk_dense(ix, q_off, pv, chunk_start, 0, nq, k, dedup, positive_only, out_ids, out_scores, out_counts, st, post_table,
+                          filt));
     } else {
         std::vector<int32_t> flags;
-        BR_TRY(topk_fused(ix, q_off, pv, nq, k, dedup, positive_only, out_ids, out_scores, out_counts, st, &flags, false, post_table));
+        BR_TRY(topk_fused(ix, q_off, pv, nq, k, dedup, positive_only, out_ids, out_scores, out_counts, st, &flags, false, post_table,
+                          filt));
         {   // offsets past n_terms make queries empty: report before the scratch of this batch is reused below
             int32_t h_bad = 0;
             BR_CUDA(cudaMemcpyAsync(&h_bad, pv.bad, 4, cudaMemcpyDeviceToHost, st));
@@ -812,6 +865,16 @@ static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q
                 BR_CUDA(cudaMemcpyAsync(d_t, s_terms.data(), 4 * s_terms.size(), cudaMemcpyHostToDevice, st));
                 BR_CUDA(cudaMemcpyAsync(d_o, s_off.data(), 4 * ((size_t)ns + 1), cudaMemcpyHostToDevice, st));
                 BR_CUDA(cudaMemcpyAsync(d_q, redo.data(), 4 * (size_t)ns, cudaMemcpyHostToDevice, st));
+                // sub-batch query i is batch query redo[i]: its filter row is the batch's row of redo[i]
+                DocFilter sfilt{};
+                if (filt) {
+                    sfilt = *filt;
+                    sfilt.row = sub_rows;
+                    k_gather_rows<<<blocks_for(ns, 256), 256, 0, st>>>(d_q, ns, filt->row, sub_rows);
+                    BR_CUDA(cudaGetLastError());
+                    ix->stats.kernel_launches += 1;
+                }
+                const DocFilter* sf = filt ? &sfilt : nullptr;
                 PrepView spv;
                 int64_t* s_chunk;
                 int32_t sT;
@@ -819,11 +882,11 @@ static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q
                 std::vector<int32_t> next;
                 if (long_pass) {
                     std::vector<int32_t> f2;
-                    BR_TRY(topk_fused(ix, d_o, spv, ns, k, dedup, positive_only, d_i, d_s, d_c, st, &f2, true, post_table));
+                    BR_TRY(topk_fused(ix, d_o, spv, ns, k, dedup, positive_only, d_i, d_s, d_c, st, &f2, true, post_table, sf));
                     for (int32_t i = 0; i < ns; ++i) if (f2[(size_t)i]) next.push_back(redo[(size_t)i]);
                     ix->stats.queries_fused += ns - (int64_t)next.size();
                 } else {
-                    BR_TRY(topk_dense(ix, d_o, spv, s_chunk, 0, ns, k, dedup, positive_only, d_i, d_s, d_c, st, post_table));
+                    BR_TRY(topk_dense(ix, d_o, spv, s_chunk, 0, ns, k, dedup, positive_only, d_i, d_s, d_c, st, post_table, sf));
                 }
                 // rows of queries that go on to the next pass are overwritten there (same stream)
                 k_scatter_rows<<<blocks_for((int64_t)ns * k, 256), 256, 0, st>>>(d_q, ns, k, d_i, d_s, d_c, out_ids, out_scores,
@@ -840,14 +903,38 @@ static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q
 
 int topk_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int32_t n_terms, int32_t k, int dedup,
                int positive_only, int32_t* out_ids, double* out_scores, int32_t* out_counts, br_record* out_recs,
-               cudaStream_t st) {
+               const br_doc_filter* filter, cudaStream_t st) {
     BR_REQUIRE(ix && q_terms && q_off && ((out_ids && out_scores) || out_recs), BR_ERR_INVALID, "br_topk_batch: null pointer");
     BR_REQUIRE(ix->finalized, BR_ERR_STATE, "br_topk_batch: call br_index_finalize first");
     BR_REQUIRE(k >= 1 && k <= BR_MAX_K, BR_ERR_INVALID, "br_topk_batch: k must be in [1, BR_MAX_K]");
     BR_REQUIRE(nq >= 0, BR_ERR_INVALID, "br_topk_batch: nq < 0");
+    if (filter) {
+        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, "br_topk_batch: filter bitmap is null");
+        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, "br_topk_batch: filter n_rows must be >= 1");
+        BR_REQUIRE(filter->words >= (ix->n_docs + 31) / 32, BR_ERR_INVALID, "br_topk_batch: filter words < ceil(n_docs / 32)");
+    }
     if (nq == 0) return BR_OK;
     BR_CUDA(cudaSetDevice(ix->device));
     ix->stats = br_query_stats{};
+    // filter rows: [nq] of the batch, [nq] of its redo sub-batches, the device-side "bad row" flag
+    DocFilter fv{};
+    const DocFilter* filt = nullptr;
+    int32_t* f_sub = nullptr;
+    int32_t* f_bad = nullptr;
+    if (filter) {
+        const size_t rb = ((size_t)nq * 4 + 255) & ~(size_t)255;
+        BR_TRY(ix->ws_filt.reserve(2 * rb + 256));
+        char* fp = ix->ws_filt.as<char>();
+        int32_t* rows = (int32_t*)fp;
+        f_sub = (int32_t*)(fp + rb);
+        f_bad = (int32_t*)(fp + 2 * rb);
+        BR_CUDA(cudaMemsetAsync(f_bad, 0, 4, st));
+        k_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, rows, f_bad);
+        BR_CUDA(cudaGetLastError());
+        ix->stats.kernel_launches += 1;
+        fv = DocFilter{filter->bits_dev, filter->words, rows};
+        filt = &fv;
+    }
     if (!out_ids || !out_scores) {                         // records only: ids / scores go to scratch
         BR_TRY(ix->ws_rec.reserve((size_t)nq * k * 12 + 512));
         out_ids = ix->ws_rec.as<int32_t>();
@@ -861,17 +948,20 @@ int topk_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32
     std::vector<int64_t> hP((size_t)nq);
     BR_CUDA(cudaMemcpyAsync(hP.data(), pv.P, sizeof(int64_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
     BR_TRY(serve_prepared(ix, q_terms, q_off, nq, T, k, dedup, positive_only, pv, chunk_start, out_ids, out_scores, out_counts, st,
-                          nullptr));
+                          nullptr, filt, f_sub));
     if (out_recs) {
         k_pack_records<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, out_scores, (int64_t)nq * k, ix->doc_base, out_recs);
         BR_CUDA(cudaGetLastError());
         ix->stats.kernel_launches += 1;
     }
+    int32_t h_fbad = 0;
+    if (f_bad) BR_CUDA(cudaMemcpyAsync(&h_fbad, f_bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
     int64_t sum = 0;
     for (int64_t v : hP) sum += v;
     ix->stats.postings_bytes = 8 * sum;
     ix->prof_collect();
+    BR_REQUIRE(!h_fbad, BR_ERR_INVALID, "br_topk_batch: a filter query_row is outside [-1, n_rows)");
     return BR_OK;
 }
 

@@ -32,6 +32,7 @@ bool fused_supported(const br_index* ix, int32_t k, int32_t nq, bool cos = false
 int fused_launch_count(const br_index* ix, int32_t k);
 int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t nq, int32_t k, int dedup,
                int positive_only, int32_t* out_ids, double* out_scores, int32_t* out_counts, cudaStream_t st,
-               std::vector<int32_t>* h_flags, bool long_pass = false, const br_posting* post_table = nullptr);
+               std::vector<int32_t>* h_flags, bool long_pass = false, const br_posting* post_table = nullptr,
+               const DocFilter* filt = nullptr);
 
 }  // namespace br

@@ -267,7 +267,23 @@ struct TileArgs {
     const uint32_t* defer_mask;   // [nq] bit j: the j-th unique term of the query is deferred in this launch
     const float* ne_ub;           // [nq] sum of the deferred terms' upper bounds (rounded up)
     const int16_t* row_slot;      // [V] look-up row of a term (every deferred term has one)
+    // doc filter (k_tile_score<QT, true> only; appended so that the fields above keep their offsets)
+    const uint32_t* fbits;        // bitmap rows [n_rows, fwords]
+    int64_t fwords;
+    const int32_t* frow;          // [nq] row of query qi, -1 = unfiltered
 };
+
+// the 4 docs doc .. doc+3 (doc a multiple of 4) of one lane share a bitmap word: zero the accumulators of the docs the
+// filter excludes (they then neither pass the threshold nor raise it); docs >= n_docs are never read from the bitmap
+__device__ __forceinline__ float4 filter4(float4 f, const uint32_t* fr, uint32_t doc, int64_t n_docs) {
+    if (!fr) return f;
+    const uint32_t b = (int64_t)doc < n_docs ? (__ldg(fr + (doc >> 5)) >> (doc & 31)) : 0u;
+    f.x = (b & 1u) ? f.x : 0.f;
+    f.y = (b & 2u) ? f.y : 0.f;
+    f.z = (b & 4u) ? f.z : 0.f;
+    f.w = (b & 8u) ? f.w : 0.f;
+    return f;
+}
 
 constexpr int LIST_CAP = 64;         // crossing-list slots per warp and sub-range (overflow -> full scan of the sub-range)
 
@@ -285,7 +301,10 @@ constexpr int LIST_CAP = 64;         // crossing-list slots per warp and sub-ran
 // threshold yet, or when the crossing list overflows.
 // After the CTA prologue there is no block barrier: every warp fetches the slice bounds of its own sub-range (one tile
 // ahead, into registers) and its own copy of the threshold.
-template <int QT>
+// FILT (filtered batches): a doc the query's filter row excludes is never emitted and never raises the threshold - the
+// crossing list tests its bit before the completion, the scan epilogue zeroes its accumulator - so every threshold stays
+// the score of k distinct ALLOWED docs, a valid lower bound of the filtered k-th best score.
+template <int QT, bool FILT>
 __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     float* acc = reinterpret_cast<float*>(smem_raw);                                     // [W][S]
@@ -310,6 +329,8 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
     const int qi = a.perm[g];
     if (!a.elig[qi]) return;                                            // served by the long pass / the dense path
     const float neub = a.ne_ub[qi];
+    const uint32_t* frow = nullptr;                                     // the query's filter row (nullptr: unfiltered)
+    if constexpr (FILT) frow = a.frow[qi] >= 0 ? a.fbits + (int64_t)a.frow[qi] * a.fwords : nullptr;
 
     if (w == 0) {
         // split the query's entries into streamed and deferred ones (stable: rows, dense postings, sparse)
@@ -566,7 +587,9 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
                 const uint32_t idx = s_list[i];
                 // a doc is listed once per update at or above t1: the first taker marks the accumulator
                 float full = atomicExch(my + idx, -1.f);
-                if (full > 0.f) {
+                bool live = full > 0.f;
+                if constexpr (FILT) live = live && doc_allowed(frow, doc0 + idx);
+                if (live) {
                     const float* col = a.rows + (doc0 + idx);
                     for (int x0 = 0; x0 < nne; x0 += 4) {          // lists are padded to a multiple of 4
                         float wv[4], mm[4];
@@ -598,7 +621,8 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
         float mx = 0.f;
 #pragma unroll
         for (int s = 0; s < TILE_S / 128; ++s) {
-            const float4 f = reinterpret_cast<const float4*>(my)[s * 32 + lane];
+            float4 f = reinterpret_cast<const float4*>(my)[s * 32 + lane];
+            if constexpr (FILT) f = filter4(f, frow, doc0 + s * 128 + lane * 4, a.n_docs);
             v[4 * s + 0] = f.x; v[4 * s + 1] = f.y; v[4 * s + 2] = f.z; v[4 * s + 3] = f.w;
             mx = fmaxf(fmaxf(mx, fmaxf(f.x, f.y)), fmaxf(f.z, f.w));
         }
@@ -623,7 +647,8 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
             mx = 0.f;
 #pragma unroll
             for (int s = 0; s < TILE_S / 128; ++s) {
-                const float4 f = reinterpret_cast<const float4*>(my)[s * 32 + lane];
+                float4 f = reinterpret_cast<const float4*>(my)[s * 32 + lane];
+                if constexpr (FILT) f = filter4(f, frow, doc0 + s * 128 + lane * 4, a.n_docs);
                 v[4 * s + 0] = f.x; v[4 * s + 1] = f.y; v[4 * s + 2] = f.z; v[4 * s + 3] = f.w;
                 mx = fmaxf(fmaxf(mx, fmaxf(f.x, f.y)), fmaxf(f.z, f.w));
             }
@@ -740,13 +765,17 @@ __device__ __forceinline__ void make_plan(const PlanArgs& pa, int q, float thr, 
 // is a valid lower bound of the K-th best score, and the first launches already run with a deferral plan instead of
 // streaming every term against a zero threshold.  One warp per query; a running top-32 is kept sorted across the lanes
 // (each batch of 32 weights is sorted, reversed and merged bitonically).
+// FILT: only the postings of docs the query's filter row allows count (K distinct ALLOWED docs score at least the seed).
 constexpr int SEED_MAX = 256;
+template <bool FILT>
 __global__ void __launch_bounds__(128) k_seed_thr(const br_posting* __restrict__ post, const int64_t* __restrict__ row_ptr,
                                                   int32_t nq, int K, const int32_t* __restrict__ elig, float* __restrict__ thr,
-                                                  PlanArgs pa) {
+                                                  PlanArgs pa, DocFilter f) {
     const int lane = threadIdx.x & 31;
     const int q = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (q >= nq || !elig[q]) return;
+    const uint32_t* fr = nullptr;
+    if constexpr (FILT) fr = f.row_of(q);
     const int32_t off = pa.q_off[q], nu = pa.u_cnt[q];
     float best = 0.f;
     for (int j = nu - 1; j >= 0; --j) {         // descending term id: in a frequency-ranked vocabulary the rare (high-bound)
@@ -757,7 +786,8 @@ __global__ void __launch_bounds__(128) k_seed_thr(const br_posting* __restrict__
         const int n = (int)min(df, (int64_t)SEED_MAX);
         float run = 0.f;                                            // lane i: i-th largest weight so far
         for (int base = 0; base < n; base += 32) {
-            const float wv = base + lane < n ? post[lo + base + lane].w * m : 0.f;
+            float wv = base + lane < n ? post[lo + base + lane].w * m : 0.f;
+            if constexpr (FILT) wv = base + lane < n && doc_allowed(fr, post[lo + base + lane].doc) ? wv : 0.f;
             const float srt = warp_sort_desc(fmaxf(wv, 0.f), lane);
             float x = fmaxf(run, __shfl_sync(0xffffffffu, srt, 31 - lane));     // bitonic: top 32 of the union
 #pragma unroll
@@ -1046,10 +1076,10 @@ static int for_each_launch(int n_sub, int k, F&& f) {
     return BR_OK;
 }
 
-template <int QT>
+template <int QT, bool FILT>
 static int launch_tiles(const TileArgs& a0, size_t smem, cudaStream_t st, br_index* ix, int32_t* prev_cnt,
                         int32_t* overflow, const PlanArgs& pa, int exchange_rounds, float* x_local, float* x_gathered) {
-    BR_CUDA(cudaFuncSetAttribute(k_tile_score<QT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));   // per device
+    BR_CUDA(cudaFuncSetAttribute(k_tile_score<QT, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));   // per device
     const bool big = a0.cap > TILE_CAP;
     if (big) BR_CUDA(cudaFuncSetAttribute(k_tighten_big, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * TILE_CAP_BIG));
     int round = 0;
@@ -1064,7 +1094,7 @@ static int launch_tiles(const TileArgs& a0, size_t smem, cudaStream_t st, br_ind
         a.tpb = 1;
         while (a.tpb * 2 <= TILE_TPB && ny >= 4 * a.tpb) a.tpb *= 2;
         ix->prof_begin(st);
-        k_tile_score<QT><<<dim3((unsigned)a0.nq, (unsigned)((ny + a.tpb - 1) / a.tpb)), TILE_W * 32, smem, st>>>(a);
+        k_tile_score<QT, FILT><<<dim3((unsigned)a0.nq, (unsigned)((ny + a.tpb - 1) / a.tpb)), TILE_W * 32, smem, st>>>(a);
         BR_CUDA(cudaGetLastError());
         ix->prof_end(st);
         if (big) k_tighten_big<<<a0.nq, TG_T, 8 * (size_t)a0.cap, st>>>(a0.thr, a0.cand_cnt, prev_cnt, a0.cand, a0.cand_h, a0.K, a0.cap, a0.cap, overflow, pa);
@@ -1095,7 +1125,7 @@ bool fused_supported(const br_index* ix, int32_t k, int32_t nq, bool cos) {
 // long_pass: the second pass for queries with up to 64 terms / 40 hot terms.
 int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t nq, int32_t k, int dedup,
                int positive_only, int32_t* out_ids, double* out_scores, int32_t* out_counts, cudaStream_t st,
-               std::vector<int32_t>* h_flags, bool long_pass, const br_posting* post_table) {
+               std::vector<int32_t>* h_flags, bool long_pass, const br_posting* post_table, const DocFilter* filt) {
     // post_table != nullptr: the TF-IDF cosine stage (br_tfidf_cosine_topk) - same kernels over the weight table
     // tf*idf^2/||d|| (all weights >= 0 whatever the idf variant), no deferral (the look-up rows and upper bounds hold
     // BM25 weights), candidates re-scored by k_rescore_cos
@@ -1203,7 +1233,8 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
         cold_off = b_off;
     }
     TileArgs a{post, ix->row_ptr, ix->skip, ix->n_sub, ix->n_docs, entries, n_entries, umax, nq, elig,
-               cold_off, cold, cold_cap, ix->dense_rows, ix->n_pad, thr, cand_cnt, cand, cand_h, cap, (int)k, 0, 0, 0, 0, 1, dedup ? 0 : 1, perm, defer_mask, ne_ub, ix->row_slot};
+               cold_off, cold, cold_cap, ix->dense_rows, ix->n_pad, thr, cand_cnt, cand, cand_h, cap, (int)k, 0, 0, 0, 0, 1, dedup ? 0 : 1, perm, defer_mask, ne_ub, ix->row_slot,
+               filt ? filt->bits : nullptr, filt ? filt->words : 0, filt ? filt->row : nullptr};
     const PlanArgs pa{q_off, pv.u_terms, pv.u_mult, pv.u_cnt, ix->ub, ix->row_slot, n_srows, cos ? 0.f : (float)ix->defer_pm * 1e-3f, defer_mask, ne_ub};
     const size_t smem = sizeof(float) * TILE_W * TILE_S + (size_t)umax * (sizeof(TileEntry) + sizeof(int64_t) + sizeof(float) +
                                                                         sizeof(uint32_t) + sizeof(uint2) * TILE_W) +
@@ -1214,13 +1245,18 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
                           ix->thr_exchange_world * (int)k <= 32 * XCHG_PER;
     const int xr = exchange ? ix->thr_exchange_rounds : 0;
     if (k <= 32) {
-        k_seed_thr<<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa);
+        if (filt) k_seed_thr<true><<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa, *filt);
+        else k_seed_thr<false><<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa, DocFilter{});
         BR_CUDA(cudaGetLastError());
         ix->stats.kernel_launches += 1;
     }
+    // The thresholds, plans, k_tighten(_big) and the exchange only ever see emitted candidates, which the filtered kernels
+    // restrict to allowed docs: they need no filter of their own.
     if (exchange) BR_TRY(exchange_thr(ix, thr, nq, elig, pa, st, nullptr, x_local, x_gathered));
-    if (long_pass) BR_TRY(launch_tiles<TILE_QT_LONG>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered));
-    else BR_TRY(launch_tiles<TILE_QT>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered));
+    if (long_pass && filt) BR_TRY((launch_tiles<TILE_QT_LONG, true>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
+    else if (long_pass) BR_TRY((launch_tiles<TILE_QT_LONG, false>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
+    else if (filt) BR_TRY((launch_tiles<TILE_QT, true>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
+    else BR_TRY((launch_tiles<TILE_QT, false>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
     BR_TRY(launch_rescore_heads(ix, q_off, pv, dedup, nq, cap, cand_cnt, cand, cand_sc, st, cos));
     BR_TRY(launch_final_select(cand, cand_sc, cand_off, 0, nq, k, positive_only, out_ids, out_scores, cnt_tmp, st, cand_cnt));
     // with shared thresholds a shard legitimately returns fewer than k docs (the rest of the corpus holds better ones)

@@ -90,6 +90,16 @@ def merge_topk_cuda(all_ids: torch.Tensor, all_sc: torch.Tensor, k: int):
     return out_ids, out_sc
 
 
+def local_filter_slice(doc_filter, lo: int, n_local: int):
+    """A filter over GLOBAL doc ids (bool [N] or [F, N]) -> this shard's columns [lo, lo + n_local)."""
+    if doc_filter is None:
+        return None
+    f = torch.as_tensor(doc_filter)
+    if f.dtype != torch.bool or f.dim() not in (1, 2) or f.shape[-1] < lo + n_local:
+        raise ValueError("doc_filter must be a bool array [N] or [F, N] over the global doc ids")
+    return f[..., lo:lo + n_local]
+
+
 class ShardedBM25:
     """One rank's view of a doc-sharded index.  ``local`` is this rank's ``BM25`` shard (built with
     ``doc_base`` = first global doc id of the shard and the all-reduced statistics)."""
@@ -162,8 +172,13 @@ class ShardedBM25:
         self.n_docs_global = n_stat
         return self
 
-    def retrieve_top_n_batch(self, queries, n=10):
-        """-> (global ids int64[Q, n], float64 scores[Q, n]) identical on every rank."""
+    def retrieve_top_n_batch(self, queries, n=10, doc_filter=None, query_filter=None):
+        """-> (global ids int64[Q, n], float64 scores[Q, n]) identical on every rank.  ``doc_filter``: bool [N] or
+        [F, N] over the GLOBAL doc ids (with ``query_filter`` int [Q] for [F, N]); each rank uses its own columns."""
+        fkw = {}
+        if doc_filter is not None or query_filter is not None:
+            fkw = dict(doc_filter=local_filter_slice(doc_filter, self.local.doc_base, self.local.corpus_size),
+                       query_filter=query_filter)
         if hasattr(self.local, "retrieve_records_batch") and self.merge is merge_topk_cuda:
             # CUDA shard: the library emits packed {global id, score} records - one all-gather, merged straight from
             # the gathered buffer
@@ -171,7 +186,7 @@ class ShardedBM25:
             if rounds >= 0:
                 self._set_exchange(rounds)
             try:
-                rec = self.local.retrieve_records_batch(queries, n)
+                rec = self.local.retrieve_records_batch(queries, n, **fkw)
             finally:
                 if rounds >= 0:
                     self._set_exchange(-1)
@@ -181,20 +196,35 @@ class ShardedBM25:
             ids, sc = merge_records_cuda(allr, n)
             if rounds >= 0:
                 # with shared thresholds a query that has fewer than n matching docs in the WHOLE corpus comes back short:
-                # those (rare) queries are repeated with local thresholds, whose zero-score fill is exact
-                total = getattr(self, "n_docs_global", None)
-                short = torch.nonzero(ids[:, min(n, total or n) - 1] < 0).flatten()
+                # those (rare) queries are repeated with local thresholds, whose zero-score fill is exact.  A filtered
+                # query can return at most as many docs as its filter allows, so "short" is measured against that.
+                total = getattr(self, "n_docs_global", None) or n
+                need = torch.full((ids.shape[0],), min(n, total), dtype=torch.int64, device=ids.device)
+                if fkw:
+                    f = torch.as_tensor(doc_filter)
+                    allowed = f.to(ids.device).reshape(-1, f.shape[-1]).sum(-1)          # [F] allowed docs per row
+                    if query_filter is None:
+                        need = torch.clamp(need, max=int(allowed[0]))
+                    else:
+                        qf = torch.as_tensor(query_filter).to(device=ids.device, dtype=torch.int64)
+                        per_q = torch.where(qf >= 0, allowed[qf.clamp(min=0, max=allowed.numel() - 1)], need)
+                        need = torch.minimum(need, per_q)
+                last = ids.gather(1, (need - 1).clamp(min=0)[:, None])[:, 0]
+                short = torch.nonzero((need > 0) & (last < 0)).flatten()
                 if short.numel():
                     q_terms, q_off = self.local.pack_queries(queries)
                     q_terms, q_off = q_terms.cpu(), q_off.cpu()
                     rows = short.cpu().tolist()
                     sub_t = torch.cat([q_terms[int(q_off[r]):int(q_off[r + 1])] for r in rows]) if rows else q_terms[:0]
                     sub_o = torch.tensor([0] + [int(q_off[r + 1] - q_off[r]) for r in rows], dtype=torch.int32).cumsum(0).to(torch.int32)
-                    rec2 = self.local.retrieve_records_batch((sub_t.to(torch.int32), sub_o), n)
+                    sub_kw = dict(fkw)
+                    if fkw and query_filter is not None:
+                        sub_kw["query_filter"] = torch.as_tensor(query_filter)[short.cpu()]
+                    rec2 = self.local.retrieve_records_batch((sub_t.to(torch.int32), sub_o), n, **sub_kw)
                     i2, s2 = merge_records_cuda(gather_records(rec2, self.group), n)
                     ids[short], sc[short] = i2, s2
             return ids, sc
-        ids, sc = self.local.retrieve_top_n_batch(queries, n)
+        ids, sc = self.local.retrieve_top_n_batch(queries, n, **fkw)
         gids = torch.where(ids >= 0, ids.to(torch.int64) + self.local.doc_base, torch.full_like(ids, -1, dtype=torch.int64))
         all_ids, all_sc = gather_candidates(gids, sc, self.group)
         if all_ids.shape[0] == 1:
@@ -216,9 +246,14 @@ class ShardedCosineIndex:
             local = CosineIndex(local_embeddings, device=device, doc_base=row_base)
         self.local, self.group, self.merge = local, group, merge
 
-    def topk(self, query_embeddings, k=10):
-        """-> (global rows int64[Q, k], cosine float64[Q, k] (fp32 values widened)) on every rank."""
-        ids, sims = self.local.topk(query_embeddings, k)
+    def topk(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
+        """-> (global rows int64[Q, k], cosine float64[Q, k] (fp32 values widened)) on every rank.  ``doc_filter``: bool
+        [N] or [F, N] over the GLOBAL rows (with ``query_filter`` int [Q] for [F, N]); each rank uses its own columns."""
+        fkw = {}
+        if doc_filter is not None or query_filter is not None:
+            fkw = dict(doc_filter=local_filter_slice(doc_filter, self.local.doc_base, self.local.n_docs),
+                       query_filter=query_filter)
+        ids, sims = self.local.topk(query_embeddings, k, **fkw)
         sims = sims.to(torch.float64)
         all_ids, all_sc = gather_candidates(ids, sims, self.group)
         if all_ids.shape[0] == 1:

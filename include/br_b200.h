@@ -145,6 +145,32 @@ int br_topk_batch_records(br_index* ix, const int32_t* q_terms_dev, const int32_
                           int32_t n_terms, int32_t k, int dedup, int positive_only, br_record* out_records_dev,
                           int32_t* out_counts_dev, void* stream);
 
+/* Filtered top-k: restrict what a query may return to an allow-list of docs (one language, one tenant, a date range,
+ * "not deleted").  A filter is a set of bitmap rows over the handle's LOCAL doc ids; every query selects one row or none.
+ *   bits_dev       uint32[n_rows, words], device: bit (d & 31) of word (d >> 5) of row f set = local doc d may be
+ *                  returned by a query that uses row f; bits at d >= n_docs are ignored
+ *   words          row stride in words, >= ceil(n_docs / 32)
+ *   query_row_dev  int32[nq], device: the row query q uses, -1 = unfiltered; NULL = row 0 for every query
+ * The result of a filtered query is the unfiltered call's result on the corpus restricted to its allowed docs: doc ids,
+ * N, avgdl, df and idf are unchanged (scores are bit-identical to the unfiltered scores of the same docs), the order is
+ * (float64 score desc, doc id asc), positive_only == 0 fills a short tail with allowed zero-score docs in doc-id order,
+ * and a query with fewer than k allowed docs gets -1 padding (out_counts = number of valid entries).  An all-ones row
+ * gives exactly the unfiltered result.  A null bits pointer, words < ceil(n_docs / 32) or n_rows < 1 is BR_ERR_INVALID;
+ * a query_row value outside [-1, n_rows) is detected on the device, never used to address the bitmap, and reported as
+ * BR_ERR_INVALID when the call returns.  filter == NULL: the unfiltered call.  The filter's arrays are only read. */
+typedef struct br_doc_filter {
+    const uint32_t* bits_dev;
+    int64_t words;
+    int32_t n_rows;
+    const int32_t* query_row_dev;
+} br_doc_filter;
+int br_topk_batch_filtered(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq,
+                           int32_t n_terms, int32_t k, int dedup, int positive_only, int32_t* out_ids_dev,
+                           double* out_scores_dev, int32_t* out_counts_dev, const br_doc_filter* filter, void* stream);
+int br_topk_batch_records_filtered(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq,
+                                   int32_t n_terms, int32_t k, int dedup, int positive_only, br_record* out_records_dev,
+                                   int32_t* out_counts_dev, const br_doc_filter* filter, void* stream);
+
 /* Exact float64 BM25 of explicit (query, doc) pairs - the arithmetic of the loop body at
  * bm25_ranking.ipynb:199-203 / team_run1.py:188-194 evaluated doc-at-a-time: query q owns the
  * candidate docs cand_ids_dev[cand_off_dev[q] .. cand_off_dev[q+1]) (local ids, int32; cand_off
@@ -222,6 +248,12 @@ int br_row_inv_norms(const void* emb_bf16_dev, int64_t n, int32_t d, float* out_
 int br_cosine_topk(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                    const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base,
                    int64_t* out_ids_dev, float* out_sims_dev, void* stream);
+/* The same restricted to per-query allow-lists of rows (br_doc_filter over the local rows 0..n_docs-1, same rules as
+ * br_topk_batch_filtered): a filtered query's result is br_cosine_topk over its allowed rows only - exact, no
+ * over-fetch; fewer than k allowed rows pad with -1.  filter == NULL: br_cosine_topk. */
+int br_cosine_topk_filtered(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
+                            const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base,
+                            int64_t* out_ids_dev, float* out_sims_dev, const br_doc_filter* filter, void* stream);
 /* Process-wide test switch of br_cosine_topk: name = "kernel" (0 auto: query-stationary CTA pairs for d <= 768, else
  * 2-CTA multicast; 1 always multicast).  Both kernels return bit-identical results.  Any other name: BR_ERR_INVALID. */
 int br_set_cosine_option(const char* name, int value);
