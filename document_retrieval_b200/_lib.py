@@ -47,6 +47,8 @@ SIGNATURES = {
     "br_cosine_topk": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P]),
     "br_cosine_topk_filtered": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int64, _P, _P, _P,
                                           _P]),
+    "br_cosine_topk_grouped": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int64,
+                                         _P, _P, _P, _P]),
     "br_set_cosine_option": (C.c_int, [C.c_char_p, C.c_int]),
     "br_cosine_rerank": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "br_dedupe_first_docs": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P]),

@@ -26,10 +26,33 @@ def set_cosine_option(name, value):
     check(_lib.load().br_set_cosine_option(name.encode(), int(value)), "br_set_cosine_option")
 
 
-class CosineIndex:
-    """Doc embeddings resident in HBM with their inverse norms (``1/(||e||+1e-10)``, computed once)."""
+def _row_group(row_group, n_rows, n_groups, dev):
+    """-> (int32 device copy of ``row_group``, n_groups).  Shape, dtype and int32 range are checked here; the layout
+    itself (non-decreasing, values in [0, n_groups)) is checked by the library on every grouped call."""
+    rg = torch.as_tensor(row_group)
+    if rg.dim() != 1 or rg.shape[0] != n_rows:
+        raise ValueError(f"row_group must have shape [{n_rows}] (one group id per embedding row), got {tuple(rg.shape)}")
+    if rg.dtype.is_floating_point or rg.dtype == torch.bool:
+        raise ValueError(f"row_group must be an integer array, got {rg.dtype}")
+    rg = rg.to(dev)
+    lo, hi = (int(rg.min()), int(rg.max())) if n_rows else (0, -1)
+    if lo < -2 ** 31 or hi >= 2 ** 31 - 1:
+        raise ValueError("row_group values must fit int32")
+    n_groups = hi + 1 if n_groups is None else int(n_groups)
+    if not 1 <= n_groups < 2 ** 31:
+        raise ValueError(f"n_groups must be in [1, 2^31), got {n_groups}")
+    return rg.to(torch.int32).contiguous(), n_groups
 
-    def __init__(self, doc_embeddings, device=None, doc_base=0):
+
+class CosineIndex:
+    """Doc embeddings resident in HBM with their inverse norms (``1/(||e||+1e-10)``, computed once).
+
+    ``row_group`` (optional, int [n]): the group (document) of every row, non-decreasing - e.g. ``sentence_to_doc`` of a
+    sentence-level index, whose rows are a document's sentences in order.  It enables ``topk_groups``.  ``n_groups``
+    defaults to ``max(row_group) + 1``; pass the document count to include trailing documents without rows (filters over
+    groups have that width).  ``group_base`` (default ``doc_base``) is added to the group ids ``topk_groups`` returns."""
+
+    def __init__(self, doc_embeddings, device=None, doc_base=0, row_group=None, n_groups=None, group_base=None):
         lib = _lib.load()
         dev = _lib.require_cuda(device)
         self.device, self.doc_base = dev, int(doc_base)
@@ -37,6 +60,12 @@ class CosineIndex:
         if self.docs.dim() != 2 or self.docs.shape[1] % 8:
             raise ValueError("embeddings must be [n, d] with d a multiple of 8")
         self.n_docs, self.dim = self.docs.shape
+        self.row_group, self.n_groups = None, None
+        self.group_base = self.doc_base if group_base is None else int(group_base)
+        if row_group is not None:
+            self.row_group, self.n_groups = _row_group(row_group, self.n_docs, n_groups, dev)
+        elif n_groups is not None:
+            raise ValueError("n_groups needs row_group")
         with torch.cuda.device(dev):
             self.inv_norm = torch.empty(self.n_docs, dtype=torch.float32, device=dev)
             check(lib.br_row_inv_norms(ptr(self.docs), self.n_docs, self.dim, ptr(self.inv_norm), _lib.stream_ptr(dev)),
@@ -64,6 +93,30 @@ class CosineIndex:
                 check(lib.br_cosine_topk_filtered(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq,
                                                   int(k), self.doc_base, ptr(ids), ptr(sims), C.byref(filt),
                                                   _lib.stream_ptr(self.device)), "br_cosine_topk_filtered")
+        return ids, sims
+
+    def topk_groups(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
+        """Exact group-level top-k ("max-sim"): a group scores the best cosine of its rows (each computed as ``topk``
+        computes it) -> (ids int64[Q, k] (group_base + group id), sims float32[Q, k]), ordered by (score desc, group id
+        asc); groups without rows are never returned, -1 pads when fewer than k groups qualify.  ``doc_filter`` is over
+        GROUP ids: bool [G] for the whole batch, or bool [F, G] with ``query_filter`` int [Q] (-1 = unfiltered)."""
+        if self.row_group is None:
+            raise ValueError("topk_groups needs an index built with row_group")
+        lib = _lib.load()
+        q = _bf16(query_embeddings, self.device)
+        nq = q.shape[0]
+        with torch.cuda.device(self.device):
+            filt = None
+            if doc_filter is not None or query_filter is not None:
+                if doc_filter is None:
+                    raise ValueError("query_filter needs a doc_filter")
+                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_groups, self.device)
+            ids = torch.empty((nq, k), dtype=torch.int64, device=self.device)
+            sims = torch.empty((nq, k), dtype=torch.float32, device=self.device)
+            check(lib.br_cosine_topk_grouped(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(self.row_group),
+                                             self.n_groups, ptr(q), nq, int(k), self.group_base, ptr(ids), ptr(sims),
+                                             None if filt is None else C.byref(filt), _lib.stream_ptr(self.device)),
+                  "br_cosine_topk_grouped")
         return ids, sims
 
     def rerank(self, query_embeddings, candidate_ids, k=10):

@@ -750,6 +750,197 @@ __global__ void k_cos_output(const int32_t* __restrict__ cand, const float* __re
 }
 
 // ------------------------------------------------------------------------------------------
+// grouped (document-level) top-k: row r belongs to group row_group[r], a non-decreasing map, so a group's rows are one
+// contiguous run and, between rows of different groups, "row asc" is "group asc".  A group scores the best of its rows.
+// ------------------------------------------------------------------------------------------
+// bitonic sort of s_h / s_id / s_g [0, n_sort) by `before(y, x)` (true: entry y goes first); n_sort a power of two
+template <class Before>
+__device__ __forceinline__ void cos_sort3(float* s_h, int32_t* s_id, int32_t* s_g, int n_sort, Before before) {
+    for (int size = 2; size <= n_sort; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < n_sort / 2; i += blockDim.x) {
+                const int x = 2 * i - (i & (stride - 1)), y = x + stride;
+                const bool up = (x & size) == 0;
+                if (before(y, x) == up) {
+                    const float h = s_h[x]; s_h[x] = s_h[y]; s_h[y] = h;
+                    const int32_t id = s_id[x]; s_id[x] = s_id[y]; s_id[y] = id;
+                    const int32_t g = s_g[x]; s_g[x] = s_g[y]; s_g[y] = g;
+                }
+            }
+        }
+    }
+    __syncthreads();
+}
+
+// k_tighten_cos for a grouped corpus: the list (rows) keeps one entry per group - its best row, the lowest row on ties -,
+// threshold := the k-th best DISTINCT-group score so far (only raised), and the groups at or above it stay, sorted
+// (score desc, row asc) = (score desc, group asc).  Every threshold is the score of k distinct groups, so it never
+// exceeds the final k-th best group score and no row of a final top-k group is ever filtered out; rows of a group that
+// is already in the list are merged by the next call.  Same overflow rule as k_tighten_cos.
+__global__ void __launch_bounds__(TC_T) k_tighten_cos_grouped(float* __restrict__ thr, int32_t* __restrict__ cand_cnt,
+                                                              int32_t* __restrict__ prev_cnt, int32_t* __restrict__ cand,
+                                                              float* __restrict__ cand_h, const int32_t* __restrict__ row_group,
+                                                              int K, int32_t* __restrict__ overflow) {
+    __shared__ float s_h[COS_CAP];
+    __shared__ int32_t s_id[COS_CAP];
+    __shared__ int32_t s_g[COS_CAP];
+    __shared__ int s_keep, s_nd;
+    const int q = blockIdx.x;
+    int n = cand_cnt[q];
+    if (n == prev_cnt[q]) return;
+    if (n > COS_CAP) {
+        if (threadIdx.x == 0) overflow[q] = 1;
+        n = COS_CAP;
+    }
+    int32_t* ids = cand + (int64_t)q * COS_CAP;
+    float* hs = cand_h + (int64_t)q * COS_CAP;
+    int n_sort = 32;
+    while (n_sort < n) n_sort <<= 1;
+    for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
+        const int32_t row = i < n ? ids[i] : 0x7fffffff;
+        s_h[i] = i < n ? hs[i] : -CUDART_INF_F;
+        s_id[i] = row;
+        s_g[i] = i < n ? __ldg(row_group + row) : 0x7fffffff;
+    }
+    if (threadIdx.x == 0) { s_keep = 0; s_nd = 0; }
+    // 1. (group asc, score desc, row asc): the first entry of every group run is the group's best row
+    cos_sort3(s_h, s_id, s_g, n_sort, [&](int y, int x) {
+        return s_g[y] < s_g[x] || (s_g[y] == s_g[x] && (s_h[y] > s_h[x] || (s_h[y] == s_h[x] && s_id[y] < s_id[x])));
+    });
+    int nd = 0;                                        // only s_h / s_id change here; s_g is only read
+    for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
+        const bool first = i < n && (i == 0 || s_g[i] != s_g[i - 1]);
+        nd += first ? 1 : 0;
+        if (!first) { s_h[i] = -CUDART_INF_F; s_id[i] = 0x7fffffff; }
+    }
+    for (int o = 16; o > 0; o >>= 1) nd += __shfl_xor_sync(0xffffffffu, nd, o);
+    if ((threadIdx.x & 31) == 0 && nd) atomicAdd(&s_nd, nd);
+    // 2. the distinct groups first, (score desc, row asc); the dropped entries (-inf, INT_MAX) last
+    cos_sort3(s_h, s_id, s_g, n_sort, [&](int y, int x) {
+        return s_h[y] > s_h[x] || (s_h[y] == s_h[x] && s_id[y] < s_id[x]);
+    });
+    nd = s_nd;
+    float th = thr[q];
+    if (nd >= K && s_h[K - 1] > th) th = s_h[K - 1];
+    int keep = 0;
+    for (int i = threadIdx.x; i < nd; i += blockDim.x) keep += (s_h[i] >= th) ? 1 : 0;
+    for (int o = 16; o > 0; o >>= 1) keep += __shfl_xor_sync(0xffffffffu, keep, o);
+    if ((threadIdx.x & 31) == 0 && keep) atomicAdd(&s_keep, keep);
+    __syncthreads();
+    keep = s_keep;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        ids[i] = i < keep ? s_id[i] : -1;
+        hs[i] = i < keep ? s_h[i] : 0.f;
+    }
+    if (threadIdx.x == 0) {
+        thr[q] = th;
+        cand_cnt[q] = keep;
+        prev_cnt[q] = keep;
+    }
+}
+
+__global__ void k_cos_output_grouped(const int32_t* __restrict__ cand, const float* __restrict__ cand_h,
+                                     const int32_t* __restrict__ cand_cnt, const int32_t* __restrict__ row_group, int32_t nq,
+                                     int32_t k, int64_t doc_base, int64_t* __restrict__ out_ids, float* __restrict__ out_sims) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)nq * k) return;
+    const int q = (int)(i / k), j = (int)(i - (int64_t)q * k);
+    const bool ok = j < cand_cnt[q] && j < COS_CAP;           // one row per group, sorted by k_tighten_cos_grouped
+    out_ids[i] = ok ? (int64_t)row_group[cand[(int64_t)q * COS_CAP + j]] + doc_base : -1;
+    out_sims[i] = ok ? cand_h[(int64_t)q * COS_CAP + j] : 0.f;
+}
+
+// Layout check, pass 1: block b looks at rows [b * GC_ROWS, (b + 1) * GC_ROWS): a value outside [0, n_groups) or below
+// its predecessor sets info[0]; blk_starts[b] = the rows of the block that start a group run.
+constexpr int GC_ROWS = 1024;
+__global__ void __launch_bounds__(256) k_group_check(const int32_t* __restrict__ rg, int64_t n_rows, int32_t n_groups,
+                                                     int32_t* __restrict__ blk_starts, int32_t* __restrict__ info) {
+    __shared__ int s_cnt;
+    if (threadIdx.x == 0) s_cnt = 0;
+    __syncthreads();
+    int cnt = 0;
+    bool bad = false;
+    for (int i = threadIdx.x; i < GC_ROWS; i += blockDim.x) {
+        const int64_t r = (int64_t)blockIdx.x * GC_ROWS + i;
+        if (r >= n_rows) break;
+        const int32_t g = rg[r], p = r > 0 ? rg[r - 1] : -1;
+        bad |= g < 0 || g >= n_groups || g < p;
+        cnt += g != p ? 1 : 0;
+    }
+    if (bad) atomicOr(info, 1);
+    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(&s_cnt, cnt);
+    __syncthreads();
+    if (threadIdx.x == 0) blk_starts[blockIdx.x] = s_cnt;
+}
+// Pass 2 (after k_exscan of blk_starts into excl[n_blk + 1]): info[2] = non-empty groups; info[1] = R_k, the shortest
+// row prefix holding k distinct groups (the row after the k-th run start), or every row when fewer than k groups are
+// non-empty.  Only the block holding the k-th run start does any work.
+__global__ void __launch_bounds__(GC_ROWS) k_group_prefix(const int32_t* __restrict__ rg, int64_t n_rows,
+                                                          const int64_t* __restrict__ excl, int32_t n_blk, int32_t k,
+                                                          int32_t* __restrict__ info) {
+    const int64_t total = excl[n_blk];
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        info[2] = (int32_t)total;
+        if (total < k) info[1] = (int32_t)n_rows;
+    }
+    if (!(excl[blockIdx.x] < k && k <= excl[blockIdx.x + 1])) return;     // block-uniform
+    const int64_t r = (int64_t)blockIdx.x * GC_ROWS + threadIdx.x;
+    const bool start = r < n_rows && (r == 0 || rg[r] != rg[r - 1]);
+    uint32_t tot;
+    const uint32_t ex = block_excl_scan(start ? 1u : 0u, &tot);
+    if (start && excl[blockIdx.x] + ex + 1 == k) info[1] = (int32_t)(r + 1);
+}
+
+// off[g] = first row of group g (lower bound in the non-decreasing map), g in [0, n_groups]
+__global__ void k_group_offsets(const int32_t* __restrict__ rg, int64_t n_rows, int32_t n_groups, int32_t* __restrict__ off) {
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g > n_groups) return;
+    int64_t lo = 0, hi = n_rows;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (rg[mid] < g) lo = mid + 1; else hi = mid;
+    }
+    off[g] = (int32_t)lo;
+}
+
+// A filter over groups -> the same filter over rows: bit r of row f = bit row_group[r] of group row f.  One warp per
+// output word.
+__global__ void k_group_filter_rows(const uint32_t* __restrict__ gbits, int64_t gwords, int32_t n_frows,
+                                    const int32_t* __restrict__ rg, int64_t n_rows, int64_t rwords, uint32_t* __restrict__ rbits) {
+    const int lane = threadIdx.x & 31;
+    const int64_t n_words = (int64_t)n_frows * rwords;
+    for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_words;
+         w += ((int64_t)gridDim.x * blockDim.x) >> 5) {
+        const int64_t f = w / rwords, r = (w - f * rwords) * 32 + lane;
+        bool on = false;
+        if (r < n_rows) {
+            const int32_t g = rg[r];
+            on = ((__ldg(gbits + f * gwords + (g >> 5)) >> (g & 31)) & 1u) != 0u;
+        }
+        const uint32_t word = __ballot_sync(0xffffffffu, on);
+        if (lane == 0) rbits[w] = word;
+    }
+}
+
+// Exact pass: per (query, group) the best of the group's row sims ([nr, n_rows], -inf = a row the query may not return)
+// -> candidate (group id, score); a group without rows or without an allowed row is an empty slot (-1).
+__global__ void k_group_max(const float* __restrict__ sims, int32_t nr, int64_t n_rows, const int32_t* __restrict__ off,
+                            int32_t n_groups, int32_t* __restrict__ gid, double* __restrict__ gsc) {
+    const int64_t total = (int64_t)nr * n_groups;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = i / n_groups;
+        const int32_t g = (int32_t)(i - r * n_groups);
+        const float* s = sims + r * n_rows;
+        float m = -CUDART_INF_F;
+        for (int32_t row = off[g]; row < off[g + 1]; ++row) m = fmaxf(m, s[row]);
+        gid[i] = m > -CUDART_INF_F ? g : -1;
+        gsc[i] = (double)m;
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // candidate re-rank: query q against its own candidate rows
 // ------------------------------------------------------------------------------------------
 // One CTA per query: each warp keeps the query row in registers (d <= 1024: 4 x 16 B per lane) and walks the
@@ -918,19 +1109,113 @@ int set_cosine_option(const char* name, int value) {
     return BR_OK;
 }
 
+// The launch schedule of the brute-force pass, for the grouped and the ungrouped call: fn(t0, nt) covers doc tiles
+// [t0, t0 + nt).  The first `warm_tiles` tiles go in launches of at most `warm_cap` tiles: a query may have no threshold
+// there yet, so such a launch can emit every row it covers, and `warm_cap` tiles plus what the list already holds fit its
+// COS_CAP slots.  After that the launch size doubles, starting from twice the last warm-up launch.  A launch emits about
+// k (growth - 1) candidates per query when a candidate is one row; `grow` < 1 replaces the doubling by launches of
+// grow x the tiles covered so far (for groups whose rows pass the threshold together, see cosine_topk).
+// Ungrouped: warm_tiles = warm_cap = 1, grow = 1 - one tile, then 2, 4, 8, ...
+template <class F>
+static int for_each_cos_launch(int n_dt, int warm_tiles, int warm_cap, double grow, F&& fn) {
+    int t0 = 0, chunk = 1;
+    while (t0 < n_dt) {
+        int nt;
+        if (t0 < warm_tiles) nt = chunk = std::min(warm_tiles - t0, warm_cap);
+        else if (grow >= 1.0) nt = chunk;
+        else nt = std::max(1, (int)(t0 * grow));
+        nt = std::min(nt, n_dt - t0);
+        BR_TRY(fn(t0, nt));
+        t0 += nt;
+        chunk *= 2;
+    }
+    return BR_OK;
+}
+
+// the gather kernel over explicit candidate rows cand[q, 0..c) -> out[q, c] fp32 cosines (-inf for an empty slot)
+static int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries,
+                             const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, cudaStream_t st) {
+    BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim > 1024");
+    const int nv = (d / 8 + 31) / 32;
+    auto launch = [&](auto kern) {
+        kern<<<nq, 256, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, n_docs, d, (const __nv_bfloat16*)queries, inv_nq, cand, c, out);
+    };
+    if (nv <= 1) launch(k_cosine_rerank<1>);
+    else if (nv == 2) launch(k_cosine_rerank<2>);
+    else if (nv == 3) launch(k_cosine_rerank<3>);
+    else launch(k_cosine_rerank<4>);
+    BR_CUDA(cudaGetLastError());
+    return BR_OK;
+}
+
+// Grouped call: row r belongs to group row_group[r] (device, non-decreasing, in [0, n_groups)).
+struct CosGroups {
+    const int32_t* row_group;
+    int32_t n_groups;
+};
+
 int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries, int32_t nq,
-                int32_t k, int64_t doc_base, int64_t* out_ids, float* out_sims, const br_doc_filter* filter, cudaStream_t st) {
-    BR_REQUIRE(docs && inv_nd && queries && out_ids && out_sims, BR_ERR_INVALID, "br_cosine_topk: null pointer");
-    BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31) && nq >= 0, BR_ERR_INVALID, "br_cosine_topk: bad sizes");
-    BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, "br_cosine_topk: embedding dim must be a multiple of 8 (16-byte rows for TMA)");
-    BR_REQUIRE(k >= 1 && k <= 256, BR_ERR_INVALID, "br_cosine_topk: k must be in [1, 256]");
-    BR_REQUIRE(((uintptr_t)docs & 15) == 0 && ((uintptr_t)queries & 15) == 0, BR_ERR_INVALID, "br_cosine_topk: 16-byte alignment required");
+                int32_t k, int64_t doc_base, int64_t* out_ids, float* out_sims, const br_doc_filter* filter, cudaStream_t st,
+                const CosGroups* grp = nullptr) {
+    const std::string fn = grp ? "br_cosine_topk_grouped" : "br_cosine_topk";
+    BR_REQUIRE(docs && inv_nd && queries && out_ids && out_sims, BR_ERR_INVALID, fn + ": null pointer");
+    BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31) && nq >= 0, BR_ERR_INVALID, fn + ": bad sizes");
+    BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, fn + ": embedding dim must be a multiple of 8 (16-byte rows for TMA)");
+    BR_REQUIRE(k >= 1 && k <= 256, BR_ERR_INVALID, fn + ": k must be in [1, 256]");
+    BR_REQUIRE(((uintptr_t)docs & 15) == 0 && ((uintptr_t)queries & 15) == 0, BR_ERR_INVALID, fn + ": 16-byte alignment required");
+    if (grp) {
+        BR_REQUIRE(grp->row_group, BR_ERR_INVALID, fn + ": row_group is null");
+        BR_REQUIRE(grp->n_groups >= 1, BR_ERR_INVALID, fn + ": n_groups must be >= 1");
+    }
+    // a filter is over the ids the call returns: rows, or groups for a grouped call
+    const int64_t n_ids = grp ? (int64_t)grp->n_groups : n_docs;
     if (filter) {
-        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, "br_cosine_topk: filter bitmap is null");
-        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, "br_cosine_topk: filter n_rows must be >= 1");
-        BR_REQUIRE(filter->words >= (n_docs + 31) / 32, BR_ERR_INVALID, "br_cosine_topk: filter words < ceil(n_docs / 32)");
+        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, fn + ": filter bitmap is null");
+        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, fn + ": filter n_rows must be >= 1");
+        BR_REQUIRE(filter->words >= (n_ids + 31) / 32, BR_ERR_INVALID,
+                   fn + (grp ? ": filter words < ceil(n_groups / 32)" : ": filter words < ceil(n_docs / 32)"));
     }
     if (nq == 0) return BR_OK;
+    const int n_dt = (int)((n_docs + CG_BM - 1) / CG_BM), n_qt = (nq + CG_BN - 1) / CG_BN;
+    // Launch schedule.  Ungrouped, the first launch runs without thresholds: every row is a candidate, and one doc tile
+    // (CG_BM rows) fits a query's list of COS_CAP.
+    static_assert(CG_BM <= COS_CAP, "the first launch must fit the candidate lists");
+    int warm_tiles = 1, warm_cap = 1;
+    double grow = 1.0;
+    AsyncBuf b_lay(st);
+    if (grp) {
+        // One pass over the layout before any GEMM: a decreasing or out-of-range value fails the call, and R_k (the
+        // shortest row prefix with k distinct groups) bounds the warm-up.  Until R_k rows are covered a query holds
+        // fewer than k groups and no threshold: its list keeps <= k - 1 entries and a launch can emit every row it
+        // covers, so warm-up launches cover at most (COS_CAP - (k - 1)) / CG_BM tiles (>= 3).  With singleton groups
+        // R_k = k <= CG_BM: one tile, then the ungrouped doubling - the same launches as br_cosine_topk.
+        const int32_t n_blk = (int32_t)((n_docs + GC_ROWS - 1) / GC_ROWS);
+        BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 8 * ((size_t)n_blk + 1) + 16));
+        int64_t* excl = (int64_t*)b_lay.p;
+        int32_t* blk = (int32_t*)(excl + n_blk + 1);
+        int32_t* info = blk + n_blk;
+        BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
+        k_group_check<<<n_blk, 256, 0, st>>>(grp->row_group, n_docs, grp->n_groups, blk, info);
+        BR_CUDA(cudaGetLastError());
+        k_exscan<int32_t><<<1, 1024, 0, st>>>(blk, n_blk, excl);
+        BR_CUDA(cudaGetLastError());
+        k_group_prefix<<<n_blk, GC_ROWS, 0, st>>>(grp->row_group, n_docs, excl, n_blk, k, info);
+        BR_CUDA(cudaGetLastError());
+        int32_t h_info[4] = {0, 0, 0, 0};
+        BR_CUDA(cudaMemcpyAsync(h_info, info, 16, cudaMemcpyDeviceToHost, st));
+        BR_CUDA(cudaStreamSynchronize(st));
+        BR_REQUIRE(!h_info[0], BR_ERR_INVALID, fn + ": row_group must be non-decreasing with values in [0, n_groups)");
+        const int64_t r_k = h_info[1], n_nonempty = std::max<int64_t>(h_info[2], 1);
+        warm_tiles = (int)((r_k + CG_BM - 1) / CG_BM);
+        warm_cap = (COS_CAP - (k - 1)) / CG_BM;
+        // After the warm-up a launch over R new rows passes about k R / S of the groups seen in S rows, and the rows of
+        // a passing group tend to pass together (sentences of one document are alike): about k s R / S rows for groups
+        // of s rows on average.  Doubling (R = S) keeps that at <= COS_CAP / 4 while k s <= 256 (always, ungrouped);
+        // beyond it launches grow by 256 / (k s) of the rows covered so far, so that a launch still fits the lists.
+        const double ks = (double)k * (double)n_docs / (double)n_nonempty;
+        grow = std::min(1.0, (COS_CAP / 4) / ks);
+    }
+    static_assert(COS_CAP - 255 >= 3 * CG_BM, "a warm-up launch covers at least 3 tiles for every k <= 256");
     // kernel choice: query-stationary CTA pairs when the query block fits (d <= 768), else 2-CTA multicast
     const bool use_qs = d <= QS_NKB * CG_BK && g_cos_kernel == 0;
     CUtensorMap map_d, map_q;
@@ -960,6 +1245,16 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         BR_CUDA(cudaGetLastError());
         fv = DocFilter{filter->bits_dev, filter->words, (const int32_t*)b_frow.p};
     }
+    AsyncBuf b_rbits(st);
+    if (filt && grp) {                                    // the group filter as a row filter: the GEMMs test rows
+        const int64_t rwords = (n_docs + 31) / 32, n_words = (int64_t)filter->n_rows * rwords;
+        BR_TRY(b_rbits.alloc(4 * (size_t)n_words));
+        k_group_filter_rows<<<(unsigned)std::min<int64_t>((n_words + 7) / 8, kNumSMs * 64), 256, 0, st>>>(
+            filter->bits_dev, filter->words, filter->n_rows, grp->row_group, n_docs, rwords, (uint32_t*)b_rbits.p);
+        BR_CUDA(cudaGetLastError());
+        fv.bits = (const uint32_t*)b_rbits.p;
+        fv.words = rwords;
+    }
     float* inv_nq = (float*)b_inq.p;
     float* thr = (float*)b_thr.p;
     BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
@@ -968,18 +1263,12 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     BR_CUDA(cudaMemsetAsync(b_cnt.p, 0, 4 * Q, st));
     BR_CUDA(cudaMemsetAsync(b_prev.p, 0, 4 * Q, st));
     BR_CUDA(cudaMemsetAsync(b_ovf.p, 0, 4 * Q, st));
-    const int n_dt = (int)((n_docs + CG_BM - 1) / CG_BM), n_qt = (nq + CG_BN - 1) / CG_BN;
     // doc chunks of growing size: thresholds learnt on the docs so far filter the next chunk.  A launch emits about
     // k (growth - 1) candidates per query whatever its size; measured on the config-5 shard an emission costs ~1.7 ns of
     // wall time, which makes doubling (13 launches, ~120 emissions per query) faster than 3x / 4x / 8x growth
-    // The first launch runs without thresholds: every row is a candidate, and one doc tile (CG_BM rows) fits a query's
-    // list of COS_CAP.
-    static_assert(CG_BM <= COS_CAP, "the first launch must fit the candidate lists");
     // candidate lists are ~2k long after the first rounds: small CTAs (more of them resident, cheaper barriers)
     constexpr int tighten_t = 64;
-    int t0 = 0, chunk = 1;
-    while (t0 < n_dt) {
-        const int nt = std::min(chunk, n_dt - t0);
+    BR_TRY(for_each_cos_launch(n_dt, warm_tiles, warm_cap, grow, [&](int t0, int nt) {
         CosArgs a{inv_nd, inv_nq, thr, (int32_t*)b_cnt.p, (int32_t*)b_cand.p, (float*)b_h.p, n_docs, nq, d, t0, t0 + nt,
                   QS_WINDOW, fv.bits, fv.words, fv.row};
         if (use_qs) {
@@ -993,21 +1282,28 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
             else k_cosine_gemm_mc<false><<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
         }
         BR_CUDA(cudaGetLastError());
-        k_tighten_cos<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, k,
-                                           (int32_t*)b_ovf.p);
+        if (grp)
+            k_tighten_cos_grouped<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p,
+                                                            (float*)b_h.p, grp->row_group, k, (int32_t*)b_ovf.p);
+        else
+            k_tighten_cos<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, k,
+                                               (int32_t*)b_ovf.p);
         BR_CUDA(cudaGetLastError());
-        t0 += nt;
-        chunk *= 2;
-    }
-    k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, nq, k,
-                                                                    doc_base, out_ids, out_sims);
+        return BR_OK;
+    }));
+    if (grp)
+        k_cos_output_grouped<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p,
+                                                                                grp->row_group, nq, k, doc_base, out_ids, out_sims);
+    else
+        k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, nq, k,
+                                                                        doc_base, out_ids, out_sims);
     BR_CUDA(cudaGetLastError());
     std::vector<int32_t> ovf(Q);
     int32_t h_fbad = 0;
     BR_CUDA(cudaMemcpyAsync(ovf.data(), b_ovf.p, 4 * Q, cudaMemcpyDeviceToHost, st));
     if (f_bad) BR_CUDA(cudaMemcpyAsync(&h_fbad, f_bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
-    BR_REQUIRE(!h_fbad, BR_ERR_INVALID, "br_cosine_topk: a filter query_row is outside [-1, n_rows)");
+    BR_REQUIRE(!h_fbad, BR_ERR_INVALID, fn + ": a filter query_row is outside [-1, n_rows)");
     // A query with more than COS_CAP candidates at or above its threshold in one launch (masses of duplicate / exactly tied
     // embeddings) cannot be served by the filter: those few queries are answered exactly by scoring every doc row with the
     // gather kernel (same normalisation, ties by doc id) - slow (one pass over the embeddings per query) but exact.
@@ -1018,7 +1314,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         // This also covers a corpus whose row order correlates with the queries (every launch then passes far more
         // than COS_CAP rows above the threshold learnt on the rows before it).
         BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED,
-                   "br_cosine_topk: candidate overflow (more than 1024 rows at or above a query's running threshold in one "
+                   fn + ": candidate overflow (more than 1024 rows at or above a query's running threshold in one "
                    "launch) needs the exact gather pass, which supports d <= 1024");
         const int32_t sub = 64;
         AsyncBuf b_q(st), b_c(st), b_oi(st), b_os(st), b_rows(st);
@@ -1028,6 +1324,21 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         if (!filt) {
             k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr_max, n_docs);
             BR_CUDA(cudaGetLastError());
+        }
+        // grouped: every row's cosine [nr, n_docs], the segmented max over each group's run [nr, n_groups], then the top
+        // k groups by (score desc, group asc); empty groups and groups without an allowed row are empty slots
+        AsyncBuf b_gi(st), b_s(st), b_goff(st), b_gid(st), b_gsc(st), b_qoff(st), b_o64(st);
+        if (grp) {
+            const size_t G = (size_t)grp->n_groups;
+            BR_TRY(b_gi.alloc(4 * (size_t)nr_max)); BR_TRY(b_s.alloc(4 * (size_t)nr_max * (size_t)n_docs));
+            BR_TRY(b_goff.alloc(4 * (G + 1))); BR_TRY(b_gid.alloc(4 * (size_t)nr_max * G)); BR_TRY(b_gsc.alloc(8 * (size_t)nr_max * G));
+            BR_TRY(b_qoff.alloc(8 * ((size_t)nr_max + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nr_max * k));
+            k_group_offsets<<<blocks_for((int64_t)G + 1, 256), 256, 0, st>>>(grp->row_group, n_docs, grp->n_groups, (int32_t*)b_goff.p);
+            BR_CUDA(cudaGetLastError());
+            std::vector<int64_t> qoff((size_t)nr_max + 1);
+            for (int32_t r = 0; r <= nr_max; ++r) qoff[(size_t)r] = (int64_t)r * (int64_t)G;
+            BR_CUDA(cudaMemcpyAsync(b_qoff.p, qoff.data(), 8 * qoff.size(), cudaMemcpyHostToDevice, st));
+            BR_CUDA(cudaStreamSynchronize(st));               // qoff is a local
         }
         for (size_t r0 = 0; r0 < redo.size(); r0 += (size_t)sub) {
             const int32_t nr = (int32_t)std::min<size_t>((size_t)sub, redo.size() - r0);
@@ -1039,8 +1350,22 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
                 k_iota_rows_filtered<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr, n_docs, (const int32_t*)b_rows.p, fv);
                 BR_CUDA(cudaGetLastError());
             }
-            BR_TRY(cosine_rerank(docs, inv_nd, n_docs, d, b_q.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs, k, (int32_t*)b_oi.p,
-                                 (float*)b_os.p, st));             // synchronises: b_rows / b_q may be reused afterwards
+            if (grp) {
+                BR_TRY(row_inv_norms(b_q.p, nr, d, (float*)b_gi.p, st));
+                BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, b_q.p, (const float*)b_gi.p, nr, (const int32_t*)b_c.p,
+                                         (int32_t)n_docs, (float*)b_s.p, st));
+                k_group_max<<<kNumSMs * 8, 256, 0, st>>>((const float*)b_s.p, nr, n_docs, (const int32_t*)b_goff.p, grp->n_groups,
+                                                         (int32_t*)b_gid.p, (double*)b_gsc.p);
+                BR_CUDA(cudaGetLastError());
+                BR_TRY(launch_final_select((const int32_t*)b_gid.p, (const double*)b_gsc.p, (const int64_t*)b_qoff.p, 0, nr, k, 0,
+                                           (int32_t*)b_oi.p, (double*)b_o64.p, nullptr, st));
+                k_rerank_output<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_oi.p, (const double*)b_o64.p,
+                                                                                  (int64_t)nr * k, (float*)b_os.p);
+                BR_CUDA(cudaGetLastError());
+            } else {
+                BR_TRY(cosine_rerank(docs, inv_nd, n_docs, d, b_q.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs, k, (int32_t*)b_oi.p,
+                                     (float*)b_os.p, st));         // synchronises: b_rows / b_q may be reused afterwards
+            }
             k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_rows.p, nr, k, (const int32_t*)b_oi.p,
                                                                           (const float*)b_os.p, doc_base, out_ids, out_sims);
             BR_CUDA(cudaGetLastError());
@@ -1061,17 +1386,7 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
     BR_TRY(b_inq.alloc(4 * (size_t)nq)); BR_TRY(b_s.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
     BR_TRY(b_off.alloc(8 * ((size_t)nq + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
     BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
-    BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim > 1024");
-    const int nv = (d / 8 + 31) / 32;
-    auto launch = [&](auto kern) {
-        kern<<<nq, 256, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, n_docs, d, (const __nv_bfloat16*)queries,
-                                 (const float*)b_inq.p, cand, c, (float*)b_s.p);
-    };
-    if (nv <= 1) launch(k_cosine_rerank<1>);
-    else if (nv == 2) launch(k_cosine_rerank<2>);
-    else if (nv == 3) launch(k_cosine_rerank<3>);
-    else launch(k_cosine_rerank<4>);
-    BR_CUDA(cudaGetLastError());
+    BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, (const float*)b_inq.p, nq, cand, c, (float*)b_s.p, st));
     k_f32_to_f64<<<blocks_for(n_pairs, 256), 256, 0, st>>>((const float*)b_s.p, n_pairs, (double*)b_s64.p);
     BR_CUDA(cudaGetLastError());
     std::vector<int64_t> off((size_t)nq + 1);
@@ -1105,6 +1420,15 @@ int br_cosine_topk_filtered(const void* docs_bf16_dev, const float* doc_inv_norm
                             float* out_sims_dev, const br_doc_filter* filter, void* stream) {
     return br::cosine_topk(docs_bf16_dev, doc_inv_norm_dev, n_docs, d, queries_bf16_dev, nq, k, doc_base, out_ids_dev,
                            out_sims_dev, filter, (cudaStream_t)stream);
+}
+
+int br_cosine_topk_grouped(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_rows, int32_t d,
+                           const int32_t* row_group_dev, int32_t n_groups, const void* queries_bf16_dev, int32_t nq,
+                           int32_t k, int64_t doc_base, int64_t* out_ids_dev, float* out_sims_dev,
+                           const br_doc_filter* filter, void* stream) {
+    const br::CosGroups grp{row_group_dev, n_groups};
+    return br::cosine_topk(docs_bf16_dev, doc_inv_norm_dev, n_rows, d, queries_bf16_dev, nq, k, doc_base, out_ids_dev,
+                           out_sims_dev, filter, (cudaStream_t)stream, &grp);
 }
 
 int br_set_cosine_option(const char* name, int value) { return br::set_cosine_option(name, value); }

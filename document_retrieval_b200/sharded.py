@@ -25,6 +25,18 @@ def shard_bounds(n_docs: int, world: int):
     return [(min(n_docs, r * per), min(n_docs, (r + 1) * per)) for r in range(world)]
 
 
+def group_shard_bounds(row_group, world: int):
+    """Contiguous row ranges that never split a group: the cuts of ``shard_bounds`` moved forward to the next group
+    start.  ``row_group`` is the non-decreasing row -> group map of the whole corpus.  A shard may come out empty when
+    one group spans more than a shard's share of the rows."""
+    rg = np.asarray(torch.as_tensor(row_group).cpu())
+    n = rg.shape[0]
+    starts = np.flatnonzero(np.r_[True, rg[1:] != rg[:-1]]) if n else np.zeros(0, np.int64)
+    starts = np.r_[starts, n]
+    cuts = [0] + [int(starts[np.searchsorted(starts, lo)]) for lo, _ in shard_bounds(n, world)[1:]] + [n]
+    return [(cuts[r], cuts[r + 1]) for r in range(world)]
+
+
 def reduce_stats(local_df: torch.Tensor, n_docs: int, sum_dl: int, group=None):
     """All-reduce (sum) of the df histogram and (N, sum dl) -> (df int64[V] on host, N, sum_dl)."""
     df = local_df.to(torch.int64)
@@ -238,12 +250,24 @@ class ShardedCosineIndex:
     ``[row_base, row_base + n_local)``, queries are replicated (10 k x 768 x 2 B = 15 MB), every rank
     runs the fused GEMM + top-k on its rows and only the [Q, k] (global row, cosine) candidates are
     all-gathered and merged - bit-identical to the single-GPU result because top-k over a row
-    partition is exactly decomposable and ties break on the global row id."""
+    partition is exactly decomposable and ties break on the global row id.
 
-    def __init__(self, local_embeddings, row_base, device=None, group=None, merge=merge_topk_cuda, local=None):
+    ``row_group`` (optional): the GLOBAL group (document) id of each local row, non-decreasing, for ``topk_groups``.
+    Every rank must hold whole groups (split with ``group_shard_bounds``); the local index numbers its groups from the
+    rank's first group, which it adds back to the ids it returns.  ``n_groups``: the global group id bound of this rank
+    (default: its largest group + 1)."""
+
+    def __init__(self, local_embeddings, row_base, device=None, group=None, merge=merge_topk_cuda, local=None,
+                 row_group=None, n_groups=None):
         if local is None:
             from .cosine import CosineIndex
-            local = CosineIndex(local_embeddings, device=device, doc_base=row_base)
+            gkw = {}
+            if row_group is not None:
+                rg = torch.as_tensor(row_group).to(torch.int64)
+                g_lo = int(rg.min()) if rg.numel() else 0
+                hi = int(n_groups) if n_groups is not None else (int(rg.max()) + 1 if rg.numel() else 1)
+                gkw = dict(row_group=rg - g_lo, n_groups=hi - g_lo, group_base=g_lo)
+            local = CosineIndex(local_embeddings, device=device, doc_base=row_base, **gkw)
         self.local, self.group, self.merge = local, group, merge
 
     def topk(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
@@ -254,6 +278,20 @@ class ShardedCosineIndex:
             fkw = dict(doc_filter=local_filter_slice(doc_filter, self.local.doc_base, self.local.n_docs),
                        query_filter=query_filter)
         ids, sims = self.local.topk(query_embeddings, k, **fkw)
+        return self._merge(ids, sims, k)
+
+    def topk_groups(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
+        """Group-level top-k (``CosineIndex.topk_groups``) over all ranks -> (global group ids int64[Q, k], cosine
+        float64[Q, k]) on every rank, identical to one index over all rows.  ``doc_filter``: bool [G] or [F, G] over
+        the GLOBAL group ids (with ``query_filter`` int [Q] for [F, G]); each rank uses its own columns."""
+        fkw = {}
+        if doc_filter is not None or query_filter is not None:
+            fkw = dict(doc_filter=local_filter_slice(doc_filter, self.local.group_base, self.local.n_groups),
+                       query_filter=query_filter)
+        ids, sims = self.local.topk_groups(query_embeddings, k, **fkw)
+        return self._merge(ids, sims, k)
+
+    def _merge(self, ids, sims, k):
         sims = sims.to(torch.float64)
         all_ids, all_sc = gather_candidates(ids, sims, self.group)
         if all_ids.shape[0] == 1:

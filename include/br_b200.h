@@ -254,6 +254,20 @@ int br_cosine_topk(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int
 int br_cosine_topk_filtered(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                             const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base,
                             int64_t* out_ids_dev, float* out_sims_dev, const br_doc_filter* filter, void* stream);
+/* Grouped (document-level) cosine top-k, e.g. documents ranked by the best of their sentence embeddings ("max-sim").
+ * Embedding row r belongs to group row_group_dev[r] (int32[n_rows], device, non-decreasing, values in [0, n_groups): a
+ * group's rows are one contiguous run, e.g. a document's sentences in order).  A group's score is the largest cosine of
+ * its rows, computed exactly as br_cosine_topk computes a row's cosine.  Outputs [nq, k], best first, ordered by
+ * (score desc, group id asc): out_ids_dev int64 = doc_base + group id, -1 pads when fewer than k non-empty groups
+ * (allowed groups, with a filter) exist; out_sims_dev float.  Groups without rows are never returned.  1 <= k <= 256.
+ * filter (may be NULL): a br_doc_filter over GROUP ids (words >= ceil(n_groups / 32)), same rules as
+ * br_cosine_topk_filtered.  A decreasing or out-of-range row_group is BR_ERR_INVALID (checked on the device before any
+ * scoring).  A query whose candidate lists overflow takes the exact gather pass as in br_cosine_topk (d <= 1024).
+ * Synchronises `stream`. */
+int br_cosine_topk_grouped(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_rows, int32_t d,
+                           const int32_t* row_group_dev, int32_t n_groups, const void* queries_bf16_dev, int32_t nq,
+                           int32_t k, int64_t doc_base, int64_t* out_ids_dev, float* out_sims_dev,
+                           const br_doc_filter* filter, void* stream);
 /* Process-wide test switch of br_cosine_topk: name = "kernel" (0 auto: query-stationary CTA pairs for d <= 768, else
  * 2-CTA multicast; 1 always multicast).  Both kernels return bit-identical results.  Any other name: BR_ERR_INVALID. */
 int br_set_cosine_option(const char* name, int value);
