@@ -120,7 +120,8 @@ class CosineIndex:
         return ids, sims
 
     def rerank(self, query_embeddings, candidate_ids, k=10):
-        """Cosine re-rank of per-query candidates [Q, c] (local rows, -1 = empty) -> (ids int32[Q, k], sims)."""
+        """Cosine re-rank of per-query candidates [Q, c] (local rows, -1 = empty) -> (ids int32[Q, k], sims).  Any other
+        id outside [0, n) raises BRError."""
         lib = _lib.load()
         q = _bf16(query_embeddings, self.device)
         cand = torch.as_tensor(candidate_ids).to(device=self.device, dtype=torch.int32).contiguous()

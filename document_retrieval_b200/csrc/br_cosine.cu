@@ -944,13 +944,15 @@ __global__ void k_group_max(const float* __restrict__ sims, int32_t nr, int64_t 
 // candidate re-rank: query q against its own candidate rows
 // ------------------------------------------------------------------------------------------
 // One CTA per query: each warp keeps the query row in registers (d <= 1024: 4 x 16 B per lane) and walks the
-// candidates warp, warp+8, ... four at a time (12-16 independent 128-bit loads in flight per lane).
+// candidates warp, warp+8, ... four at a time (12-16 independent 128-bit loads in flight per lane).  A candidate id
+// outside [-1, n_docs) is never read; it scores -inf and sets *bad (when bad != NULL) in a pass over the list before the
+// gather, which leaves the registers of the gather loop as they are (its occupancy bounds the gather rate).
 template <int NV>   // 16-byte vectors per lane = ceil(d / 256)
 __global__ void __launch_bounds__(256) k_cosine_rerank(const __nv_bfloat16* __restrict__ docs,
                                                        const float* __restrict__ inv_nd, int64_t n_docs, int32_t d,
                                                        const __nv_bfloat16* __restrict__ queries,
                                                        const float* __restrict__ inv_nq, const int32_t* __restrict__ cand,
-                                                       int32_t c, float* __restrict__ out) {
+                                                       int32_t c, float* __restrict__ out, int32_t* __restrict__ bad) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int q = blockIdx.x;
     const int nvec = d / 8;
@@ -960,6 +962,9 @@ __global__ void __launch_bounds__(256) k_cosine_rerank(const __nv_bfloat16* __re
     for (int i = 0; i < NV; ++i) qv[i] = lane + 32 * i < nvec ? __ldg(pq + lane + 32 * i) : make_uint4(0, 0, 0, 0);
     const float iq = inv_nq[q];
     const int32_t* cq = cand + (int64_t)q * c;
+    if (bad)
+        for (int j = threadIdx.x; j < c; j += blockDim.x)
+            if (cq[j] < -1 || cq[j] >= n_docs) *bad = 1;
     for (int j0 = warp * 4; j0 < c; j0 += 32) {
         int32_t doc[4];
         uint4 dv[4][NV];
@@ -1132,13 +1137,16 @@ static int for_each_cos_launch(int n_dt, int warm_tiles, int warm_cap, double gr
     return BR_OK;
 }
 
-// the gather kernel over explicit candidate rows cand[q, 0..c) -> out[q, c] fp32 cosines (-inf for an empty slot)
+// the gather kernel over explicit candidate rows cand[q, 0..c) -> out[q, c] fp32 cosines (-inf for an empty slot);
+// bad (may be NULL) is set when an id is outside [-1, n_docs)
 static int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries,
-                             const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, cudaStream_t st) {
+                             const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, int32_t* bad,
+                             cudaStream_t st) {
     BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim > 1024");
     const int nv = (d / 8 + 31) / 32;
     auto launch = [&](auto kern) {
-        kern<<<nq, 256, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, n_docs, d, (const __nv_bfloat16*)queries, inv_nq, cand, c, out);
+        kern<<<nq, 256, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, n_docs, d, (const __nv_bfloat16*)queries, inv_nq, cand, c, out,
+                                 bad);
     };
     if (nv <= 1) launch(k_cosine_rerank<1>);
     else if (nv == 2) launch(k_cosine_rerank<2>);
@@ -1158,7 +1166,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
                 int32_t k, int64_t doc_base, int64_t* out_ids, float* out_sims, const br_doc_filter* filter, cudaStream_t st,
                 const CosGroups* grp = nullptr) {
     const std::string fn = grp ? "br_cosine_topk_grouped" : "br_cosine_topk";
-    BR_REQUIRE(docs && inv_nd && queries && out_ids && out_sims, BR_ERR_INVALID, fn + ": null pointer");
+    BR_REQUIRE(docs && inv_nd && (nq == 0 || (queries && out_ids && out_sims)), BR_ERR_INVALID, fn + ": null pointer");
     BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31) && nq >= 0, BR_ERR_INVALID, fn + ": bad sizes");
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, fn + ": embedding dim must be a multiple of 8 (16-byte rows for TMA)");
     BR_REQUIRE(k >= 1 && k <= 256, BR_ERR_INVALID, fn + ": k must be in [1, 256]");
@@ -1353,7 +1361,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
             if (grp) {
                 BR_TRY(row_inv_norms(b_q.p, nr, d, (float*)b_gi.p, st));
                 BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, b_q.p, (const float*)b_gi.p, nr, (const int32_t*)b_c.p,
-                                         (int32_t)n_docs, (float*)b_s.p, st));
+                                         (int32_t)n_docs, (float*)b_s.p, nullptr, st));
                 k_group_max<<<kNumSMs * 8, 256, 0, st>>>((const float*)b_s.p, nr, n_docs, (const int32_t*)b_goff.p, grp->n_groups,
                                                          (int32_t*)b_gid.p, (double*)b_gsc.p);
                 BR_CUDA(cudaGetLastError());
@@ -1377,16 +1385,18 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
 
 int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries, int32_t nq,
                   const int32_t* cand, int32_t c, int32_t k, int32_t* out_ids, float* out_sims, cudaStream_t st) {
-    BR_REQUIRE(docs && queries && cand && out_ids && out_sims, BR_ERR_INVALID, "br_cosine_rerank: null pointer");
+    BR_REQUIRE(docs && (nq == 0 || (queries && cand && out_ids && out_sims)), BR_ERR_INVALID, "br_cosine_rerank: null pointer");
     BR_REQUIRE(n_docs > 0 && nq >= 0 && c >= 1 && k >= 1 && k <= BR_MAX_K, BR_ERR_INVALID, "br_cosine_rerank: bad sizes");
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim must be a multiple of 8");
     if (nq == 0) return BR_OK;
     const int64_t n_pairs = (int64_t)nq * c;
     AsyncBuf b_inq(st), b_s(st), b_s64(st), b_off(st), b_o64(st);
-    BR_TRY(b_inq.alloc(4 * (size_t)nq)); BR_TRY(b_s.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
+    BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_s.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
     BR_TRY(b_off.alloc(8 * ((size_t)nq + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
+    int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_docs)
+    BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
     BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
-    BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, (const float*)b_inq.p, nq, cand, c, (float*)b_s.p, st));
+    BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, (const float*)b_inq.p, nq, cand, c, (float*)b_s.p, bad, st));
     k_f32_to_f64<<<blocks_for(n_pairs, 256), 256, 0, st>>>((const float*)b_s.p, n_pairs, (double*)b_s64.p);
     BR_CUDA(cudaGetLastError());
     std::vector<int64_t> off((size_t)nq + 1);
@@ -1396,7 +1406,10 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
                                nullptr, st));
     k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
     BR_CUDA(cudaGetLastError());
+    int32_t h_bad = 0;
+    BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
+    BR_REQUIRE(!h_bad, BR_ERR_INVALID, "br_cosine_rerank: a candidate id is outside [-1, n_docs)");
     return BR_OK;
 }
 

@@ -244,7 +244,7 @@ int br_row_inv_norms(const void* emb_bf16_dev, int64_t n, int32_t d, float* out_
  * out_ids_dev int64 (doc_base + local row, -1 pads), out_sims_dev float.  A query for which one launch finds more
  * than 1024 rows at or above its running threshold (masses of duplicate embeddings, or rows ordered by similarity to
  * the queries) is answered exactly by a full gather pass instead of the filter - any number of such queries, 64 per
- * pass; slower, never wrong.  Synchronises `stream`. */
+ * pass; slower, never wrong.  nq = 0 returns at once (queries and outputs may then be NULL).  Synchronises `stream`. */
 int br_cosine_topk(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                    const void* queries_bf16_dev, int32_t nq, int32_t k, int64_t doc_base,
                    int64_t* out_ids_dev, float* out_sims_dev, void* stream);
@@ -273,8 +273,11 @@ int br_cosine_topk_grouped(const void* docs_bf16_dev, const float* doc_inv_norm_
 int br_set_cosine_option(const char* name, int value);
 /* Re-rank: query q against its own candidates cand_ids_dev[q, 0..c) (local rows, -1 = empty slot),
  * e.g. the BM25 top-1000 (text_preprocessing_and_embedding_setup.py:342).  doc_inv_norm_dev may be
- * NULL (norms are then computed on the fly).  Outputs [nq, k] (k <= BR_MAX_K): out_ids_dev int32,
- * out_sims_dev float, ordered by (cosine desc, doc id asc).  Synchronises `stream`. */
+ * NULL (norms are then computed on the fly, bit-identical to br_row_inv_norms).  Outputs [nq, k] (k <= BR_MAX_K):
+ * out_ids_dev int32, out_sims_dev float, ordered by (cosine desc, doc id asc); a candidate repeated in a row is returned
+ * once; fewer than k distinct candidates pad with -1 / 0.0.  A candidate id outside [-1, n_docs) is BR_ERR_INVALID (its
+ * row is never read).  nq = 0 returns at once (queries, candidates and outputs may then be NULL).  Synchronises
+ * `stream`. */
 int br_cosine_rerank(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                      const void* queries_bf16_dev, int32_t nq, const int32_t* cand_ids_dev, int32_t c,
                      int32_t k, int32_t* out_ids_dev, float* out_sims_dev, void* stream);
