@@ -285,6 +285,7 @@ __device__ __forceinline__ float4 filter4(float4 f, const uint32_t* fr, uint32_t
     return f;
 }
 
+constexpr int SPX = 1;               // postings per lane requested ahead for a sparse slice (2 was measured no faster)
 constexpr int LIST_CAP = 64;         // crossing-list slots per warp and sub-range (overflow -> full scan of the sub-range)
 
 // MaxScore deferral (exact): between launches every query gets a plan (make_plan): the terms with the smallest upper
@@ -320,7 +321,7 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
     int* s_cnt = reinterpret_cast<int*>(s_list_all + TILE_W * LIST_CAP);                 // Ur, Ud, U (streamed), rows, deferred
                                                                                          // terms (padded to x4), sparse terms
     int* s_lcnt_all = s_cnt + 6;                                                         // [W]
-    uint8_t* s_ql = reinterpret_cast<uint8_t*>(s_lcnt_all + TILE_W);                     // [QT] entry indices of the sparse terms
+    uint8_t* s_ql_all = reinterpret_cast<uint8_t*>(s_lcnt_all + TILE_W);                 // [W][umax] non-empty sparse slices
 
     const int g = blockIdx.x;                                           // query position
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -336,7 +337,7 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
         // split the query's entries into streamed and deferred ones (stable: rows, dense postings, sparse)
         const int U0 = a.n_entries[g] & 0x3ff, Ud0 = (a.n_entries[g] >> 10) & 0x3ff, Ur0 = a.n_entries[g] >> 20;
         const uint32_t dm = a.defer_mask[qi];
-        int na = 0, ur = 0, ud = 0, nne = 0, nql = 0;
+        int na = 0, ur = 0, ud = 0, nne = 0;
         bool rows = false;
         for (int base = 0; base < U0; base += 32) {
             const int u = base + lane;
@@ -350,13 +351,6 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
             const bool isa = act != 0.f;
             const unsigned ma = __ballot_sync(0xffffffffu, isa);
             const unsigned lt = (1u << lane) - 1;
-            const bool in = isa && u >= Ud0;                                  // list of streamed sparse terms
-            const unsigned mq = __ballot_sync(0xffffffffu, in);
-            if (in) {
-                const int p = nql + __popc(mq & lt);
-                if (p < QT) s_ql[p] = (uint8_t)(na + __popc(ma & lt));
-            }
-            nql += __popc(mq);
             if (isa) {
                 const int p = na + __popc(ma & lt);
                 ent[p] = e;
@@ -377,13 +371,14 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
         rows = __any_sync(0xffffffffu, rows);
         const int n = min(nne, NE_MAX), n4 = (n + 3) & ~3;
         if (lane >= n && lane < n4) s_ne[lane] = NeEntry{0, 0.f};     // padding: row 0, multiplicity 0
-        if (lane == 0) { s_cnt[0] = ur; s_cnt[1] = ud; s_cnt[2] = na; s_cnt[3] = rows ? 1 : 0; s_cnt[4] = n4; s_cnt[5] = min(nql, QT); }
+        if (lane == 0) { s_cnt[0] = ur; s_cnt[1] = ud; s_cnt[2] = na; s_cnt[3] = rows ? 1 : 0; s_cnt[4] = n4; }
     }
     __syncthreads();                                   // the only block barrier: from here on the warps run independently
     const int Ur = s_cnt[0], Ud = s_cnt[1], U = s_cnt[2];
     const bool rows = s_cnt[3] != 0;
-    const int nne = s_cnt[4], nql = s_cnt[5];
+    const int nne = s_cnt[4];
     uint2* s_bnd = s_bnd_all + w * a.umax;
+    uint8_t* s_ql = s_ql_all + w * a.umax;
     uint16_t* s_list = s_list_all + w * LIST_CAP;
     int* s_lcnt = s_lcnt_all + w;
 
@@ -402,12 +397,20 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
             }
         }
     };
+    // stores the bounds and lists the sparse entries whose slice in this sub-range is not empty (entry order kept);
+    // returns their number
     auto store_bounds = [&]() {
+        int n = 0;
 #pragma unroll
         for (int r = 0; r < NR; ++r) {
             const int u = lane + 32 * r;
             if (u < U) s_bnd[u] = make_uint2(nlo[r], nhi[r]);     // row terms keep empty slices
+            const bool sp = u >= Ud && u < U && nlo[r] < nhi[r];
+            const unsigned m = __ballot_sync(0xffffffffu, sp);
+            if (sp) s_ql[n + __popc(m & ((1u << lane) - 1u))] = (uint8_t)u;
+            n += __popc(m);
         }
+        return n;
     };
     // (large-k path: a launch may start inside its first tile - the warps below sub_begin start one tile later)
     const int tile_begin_w = tile_first + ((tile_first * TILE_W + w < a.sub_begin) ? 1 : 0);
@@ -416,7 +419,7 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
     for (int tile = tile_begin_w; tile < tile_last; ++tile) {
     const int sub = tile * TILE_W + w;
     if (sub >= a.sub_end) break;                                      // warp-uniform; the later tiles are out of range too
-    store_bounds();
+    const int nql = store_bounds();
     if (tile + 1 < tile_last && sub + TILE_W < a.n_sub) load_bounds(sub + TILE_W);     // in flight during this tile
     // threshold of this tile (a stale, lower value is always valid); t1: partial scores below it cannot reach thr.
     // A query that is scanned anyway (streamed rows / no threshold yet) never pushes: its t1 is +inf.
@@ -476,16 +479,16 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
     }
     __syncwarp();
 
-    // Phase A - sparse slices (most (term, sub-range) pairs hold 0-8 postings): the warp walks the query's term list
-    // straight from shared memory - slice bounds, list base and multiplicity of term i are broadcast reads, the posting
-    // of term i+1 is requested before term i is added.  (Pulling the next non-empty slice over by shuffle from the lane
+    // Phase A - sparse slices (most (term, sub-range) pairs hold 0-8 postings): the warp walks the list of the
+    // sub-range's non-empty sparse slices straight from shared memory - slice bounds, list base and multiplicity of slice
+    // i are broadcast reads, the postings of slice i+1 are requested before slice i is added.  (Pulling the next non-empty slice over by shuffle from the lane
     // that fetched its bounds cost three shuffles, a find-first-set and two votes per step and was slower: DESIGN.md 3.2.)
     {
         const uint2* const post2 = reinterpret_cast<const uint2*>(a.post);
         uint32_t c_hi = 0, c_lo = 0, c_pb = 0;
         float c_mu = 1.f;
-        uint2 c_p = make_uint2(0u, 0u);
-        auto fetch = [&](int it, uint32_t& lo, uint32_t& hi, uint32_t& pb, float& mu, uint2& p) {
+        uint2 c_p[SPX];
+        auto fetch = [&](int it, uint32_t& lo, uint32_t& hi, uint32_t& pb, float& mu, uint2* p) {
             lo = hi = 0;
             if (it < nql) {
                 const int u = s_ql[it];
@@ -493,7 +496,9 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
                 lo = bd.x; hi = bd.y;
                 pb = (uint32_t)s_base[u];                           // posting index of the term's list (nnz < 2^32)
                 if (a.has_mult) mu = s_fm[u];
-                if (lo + lane < hi) p = __ldg(post2 + pb + lo + lane);
+#pragma unroll
+                for (int x = 0; x < SPX; ++x)
+                    if (lo + 32 * x + lane < hi) p[x] = __ldg(post2 + pb + lo + 32 * x + lane);
             }
         };
         fetch(0, c_lo, c_hi, c_pb, c_mu, c_p);
@@ -501,16 +506,19 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
         for (int it = 0; it < nql; ++it) {
             uint32_t n_lo, n_hi, n_pb = 0;
             float n_mu = 1.f;
-            uint2 n_p = make_uint2(0u, 0u);
+            uint2 n_p[SPX];
             fetch(it + 1, n_lo, n_hi, n_pb, n_mu, n_p);
-            if (c_lo + lane < c_hi) {
-                const uint32_t idx = c_p.x - doc0;
-                const float val = fmaf(__uint_as_float(c_p.y), c_mu, my[idx]);
-                my[idx] = val;
-                if (val >= t1) push(idx);
+#pragma unroll
+            for (int x = 0; x < SPX; ++x) {
+                if (c_lo + 32 * x + lane < c_hi) {                  // one term: distinct docs
+                    const uint32_t idx = c_p[x].x - doc0;
+                    const float val = fmaf(__uint_as_float(c_p[x].y), c_mu, my[idx]);
+                    my[idx] = val;
+                    if (val >= t1) push(idx);
+                }
             }
-            // a slice longer than the warp (rare for a sparse-class term)
-            for (uint32_t c = c_lo + 32; __any_sync(0xffffffffu, c < c_hi); c += 32) {
+            // a slice longer than the postings fetched ahead
+            for (uint32_t c = c_lo + 32 * SPX; __any_sync(0xffffffffu, c < c_hi); c += 32) {
                 __syncwarp();
                 if (c + lane < c_hi) {
                     const uint2 p = __ldg(post2 + c_pb + c + lane);
@@ -521,7 +529,9 @@ __global__ void __launch_bounds__(TILE_W * 32, 3) k_tile_score(TileArgs a) {
                 }
             }
             __syncwarp();
-            c_lo = n_lo; c_hi = n_hi; c_pb = n_pb; c_mu = n_mu; c_p = n_p;
+            c_lo = n_lo; c_hi = n_hi; c_pb = n_pb; c_mu = n_mu;
+#pragma unroll
+            for (int x = 0; x < SPX; ++x) c_p[x] = n_p[x];
         }
     }
     __syncwarp();
@@ -1238,7 +1248,7 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
     const PlanArgs pa{q_off, pv.u_terms, pv.u_mult, pv.u_cnt, ix->ub, ix->row_slot, n_srows, cos ? 0.f : (float)ix->defer_pm * 1e-3f, defer_mask, ne_ub};
     const size_t smem = sizeof(float) * TILE_W * TILE_S + (size_t)umax * (sizeof(TileEntry) + sizeof(int64_t) + sizeof(float) +
                                                                         sizeof(uint32_t) + sizeof(uint2) * TILE_W) +
-                        sizeof(NeEntry) * NE_MAX + sizeof(uint16_t) * TILE_W * LIST_CAP + 4 * (6 + TILE_W) + umax;
+                        sizeof(NeEntry) * NE_MAX + sizeof(uint16_t) * TILE_W * LIST_CAP + 4 * (6 + TILE_W) + (size_t)TILE_W * umax;
     // threshold exchange with the other shards: only in the regular pass of the first attempt, so that every shard makes
     // exactly 1 + thr_exchange_rounds calls per batch
     const bool exchange = !cos && ix->thr_exchange != nullptr && ix->thr_exchange_rounds >= 0 && !long_pass && attempt == 0 && k <= 32 &&
