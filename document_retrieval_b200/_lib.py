@@ -51,6 +51,8 @@ SIGNATURES = {
                                          _P, _P, _P, _P]),
     "br_set_cosine_option": (C.c_int, [C.c_char_p, C.c_int]),
     "br_cosine_rerank": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
+    "br_cosine_rerank_grouped": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32,
+                                           _P, _P, _P]),
     "br_dedupe_first_docs": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     "br_set_thr_exchange": (C.c_int, [_P, _P, _P, C.c_int, C.c_int]),
     "br_tile_launch_count": (C.c_int, [_P, C.c_int32]),

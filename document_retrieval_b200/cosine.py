@@ -133,6 +133,25 @@ class CosineIndex:
                                        int(k), ptr(ids), ptr(sims), _lib.stream_ptr(self.device)), "br_cosine_rerank")
         return ids, sims
 
+    def rerank_groups(self, query_embeddings, candidate_groups, k=10):
+        """Grouped re-rank of per-query candidate groups [Q, c] (local group ids, -1 = empty) -> (ids int32[Q, k] local
+        group ids, sims float32[Q, k]).  A group scores the best cosine of its rows, each computed as ``rerank`` computes
+        it; order (score desc, group id asc); a repeated group comes back once, groups without rows never, -1 / 0 pad.
+        Any other id outside [0, n_groups) raises BRError."""
+        if self.row_group is None:
+            raise ValueError("rerank_groups needs an index built with row_group")
+        lib = _lib.load()
+        q = _bf16(query_embeddings, self.device)
+        cand = torch.as_tensor(candidate_groups).to(device=self.device, dtype=torch.int32).contiguous()
+        nq, c = cand.shape
+        with torch.cuda.device(self.device):
+            ids = torch.empty((nq, k), dtype=torch.int32, device=self.device)
+            sims = torch.empty((nq, k), dtype=torch.float32, device=self.device)
+            check(lib.br_cosine_rerank_grouped(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(self.row_group),
+                                               self.n_groups, ptr(q), nq, ptr(cand), c, int(k), ptr(ids), ptr(sims),
+                                               _lib.stream_ptr(self.device)), "br_cosine_rerank_grouped")
+        return ids, sims
+
 
 def rerank_bm25_with_cosine(bm25_model, cosine_index, queries, query_embeddings, n_candidates=1000, k=10):
     """BASELINE config 3: BM25 top-``n_candidates`` then cosine re-rank to top-``k`` (the intended
@@ -140,3 +159,14 @@ def rerank_bm25_with_cosine(bm25_model, cosine_index, queries, query_embeddings,
     text_preprocessing_and_embedding_setup.py:342)."""
     cand, _ = bm25_model.retrieve_top_n_batch(queries, min(n_candidates, bm25_model.corpus_size))
     return cosine_index.rerank(query_embeddings, cand, k)
+
+
+def rerank_bm25_with_sentences(bm25_model, cosine_index, queries, query_embeddings, n_candidates=1000, k=10):
+    """Config 3 at sentence granularity: BM25 top-``n_candidates`` documents, then each document scored by the best
+    cosine of its sentence embeddings (``CosineIndex.rerank_groups`` over a sentence-level index whose groups are the
+    BM25 documents) -> (document ids int32[Q, k], sims float32[Q, k])."""
+    if cosine_index.n_groups != bm25_model.corpus_size:
+        raise ValueError(f"the cosine index has {cosine_index.n_groups} groups, the BM25 model {bm25_model.corpus_size} "
+                         "documents: the groups must be the BM25 documents")
+    cand, _ = bm25_model.retrieve_top_n_batch(queries, min(n_candidates, bm25_model.corpus_size))
+    return cosine_index.rerank_groups(query_embeddings, cand, k)

@@ -13,6 +13,8 @@
 //   k_tighten_cos       between doc chunks of doubling size: threshold := k-th best so far, compact list
 //   k_cosine_rerank     per query its own c candidate rows (BM25 top-1000 -> cosine): one warp per
 //                       (query, candidate) dot product with 128-bit loads              (gather / HBM-bound)
+//   k_cosine_rerank_grouped  per query the rows of its c candidate documents, warps split over rows, best row per
+//                       document folded in shared memory                               (gather / HBM-bound)
 // This is the only place tensor cores are used: it is the only dense contraction on the path.
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -943,6 +945,26 @@ __global__ void k_group_max(const float* __restrict__ sims, int32_t nr, int64_t 
 // ------------------------------------------------------------------------------------------
 // candidate re-rank: query q against its own candidate rows
 // ------------------------------------------------------------------------------------------
+// One lane's share of a row's dot product (s) and squared norm (nn): 2 x 4 bf16 pairs per 16-byte vector, in vector
+// order.  Both gather kernels use it, so a row's cosine is the same bits in either.
+template <int NV, class QV>   // QV: the lane's query vectors, qv[i] for i < NV (registers, or shared memory)
+__device__ __forceinline__ void cos_lane_dot(const uint4 (&dv)[NV], const QV& qv, float& s, float& nn) {
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+        const uint32_t wa[4] = {dv[i].x, dv[i].y, dv[i].z, dv[i].w};
+        const uint32_t wb[4] = {qv[i].x, qv[i].y, qv[i].z, qv[i].w};
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const float a0 = __uint_as_float(wa[e] << 16), a1 = __uint_as_float(wa[e] & 0xffff0000u);
+            const float b0 = __uint_as_float(wb[e] << 16), b1 = __uint_as_float(wb[e] & 0xffff0000u);
+            s = fmaf(a0, b0, s);
+            s = fmaf(a1, b1, s);
+            nn = fmaf(a0, a0, nn);
+            nn = fmaf(a1, a1, nn);
+        }
+    }
+}
+
 // One CTA per query: each warp keeps the query row in registers (d <= 1024: 4 x 16 B per lane) and walks the
 // candidates warp, warp+8, ... four at a time (12-16 independent 128-bit loads in flight per lane).  A candidate id
 // outside [-1, n_docs) is never read; it scores -inf and sets *bad (when bad != NULL) in a pass over the list before the
@@ -980,20 +1002,7 @@ __global__ void __launch_bounds__(256) k_cosine_rerank(const __nv_bfloat16* __re
 #pragma unroll
         for (int x = 0; x < 4; ++x) {
             float s = 0.f, nn = 0.f;
-#pragma unroll
-            for (int i = 0; i < NV; ++i) {
-                const uint32_t wa[4] = {dv[x][i].x, dv[x][i].y, dv[x][i].z, dv[x][i].w};
-                const uint32_t wb[4] = {qv[i].x, qv[i].y, qv[i].z, qv[i].w};
-#pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const float a0 = __uint_as_float(wa[e] << 16), a1 = __uint_as_float(wa[e] & 0xffff0000u);
-                    const float b0 = __uint_as_float(wb[e] << 16), b1 = __uint_as_float(wb[e] & 0xffff0000u);
-                    s = fmaf(a0, b0, s);
-                    s = fmaf(a1, b1, s);
-                    nn = fmaf(a0, a0, nn);
-                    nn = fmaf(a1, a1, nn);
-                }
-            }
+            cos_lane_dot<NV>(dv[x], qv, s, nn);
             for (int o = 16; o > 0; o >>= 1) {
                 s += __shfl_xor_sync(0xffffffffu, s, o);
                 nn += __shfl_xor_sync(0xffffffffu, nn, o);
@@ -1015,6 +1024,123 @@ __global__ void k_rerank_output(const int32_t* __restrict__ ids, const double* _
                                 float* __restrict__ out_sims) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out_sims[i] = ids[i] >= 0 ? (float)sc[i] : 0.f;
+}
+
+// Grouped re-rank: query q against the rows of its candidate GROUPS cand[q, 0..c) (local group ids, -1 = empty slot); a
+// group scores the best cosine of its rows.  One CTA per query takes the candidates in chunks of RG_CH: an exclusive
+// prefix of their row counts (int64: a list may repeat a large group) flattens the chunk's rows into one range, which
+// the warps walk 4 rows at a time (warp w: rows 4w.., stride 32), so the work follows rows, not candidates, and one long
+// group keeps every warp busy.  A row finds its candidate by binary search in the prefix; its cosine is computed as
+// k_cosine_rerank computes it and folded into the candidate's slot with an atomicMax on order-preserving bits (max is
+// exact, so the order of the folds does not matter).  Out: per candidate the group id (-1 for an empty slot, an empty
+// group or an id outside [-1, n_groups), which also sets *bad and never addresses off[]) and the best cosine, widened.
+constexpr int RG_T = 256, RG_CH = 1024;
+// Resident CTAs asked of ptxas, per NV: the gather rate follows the loads in flight per SM.  With the query in shared
+// memory this gives 56 / 64 / 80 / 120 registers without spills (4 / 4 / 3 / 2 CTAs, as many as k_cosine_rerank).
+#define RG_MIN_BLOCKS(NV) ((NV) <= 2 ? 4 : (NV) == 3 ? 3 : 2)
+__device__ __forceinline__ uint32_t f32_order(float x) {     // monotone float -> uint32 (for atomicMax)
+    const uint32_t u = __float_as_uint(x);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float f32_unorder(uint32_t e) {
+    return __uint_as_float((e & 0x80000000u) ? (e & 0x7fffffffu) : ~e);
+}
+struct QStrided {                                            // vector i of a lane's query share in shared memory
+    const uint4* p;
+    __device__ __forceinline__ uint4 operator[](int i) const { return p[32 * i]; }
+};
+template <int NV>   // 16-byte vectors per lane = ceil(d / 256)
+__global__ void __launch_bounds__(RG_T, RG_MIN_BLOCKS(NV)) k_cosine_rerank_grouped(const __nv_bfloat16* __restrict__ docs,
+                                                                const float* __restrict__ inv_nd, int32_t d,
+                                                                const int32_t* __restrict__ off, int32_t n_groups,
+                                                                const __nv_bfloat16* __restrict__ queries,
+                                                                const float* __restrict__ inv_nq, const int32_t* __restrict__ cand,
+                                                                int32_t c, int32_t* __restrict__ out_ids,
+                                                                double* __restrict__ out_sc, int32_t* __restrict__ bad) {
+    constexpr int PER = RG_CH / RG_T;                        // candidates per thread in the prefix pass
+    __shared__ int64_t s_pre[RG_CH + 1];                     // exclusive prefix of the row counts; [RG_CH] = chunk total
+    __shared__ int32_t s_row0[RG_CH];                        // first row of each candidate's group
+    __shared__ uint32_t s_best[RG_CH];                       // f32_order(best cosine so far)
+    __shared__ int64_t s_wsum[RG_T / 32];
+    __shared__ uint4 s_q[32 * NV];                           // the query row, zero-padded to 32 x NV vectors
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int q = blockIdx.x;
+    const int nvec = d / 8;
+    const uint4* pq = reinterpret_cast<const uint4*>(queries + (int64_t)q * d);
+    for (int i = threadIdx.x; i < 32 * NV; i += RG_T) s_q[i] = i < nvec ? __ldg(pq + i) : make_uint4(0, 0, 0, 0);
+    const uint4* qv = s_q + lane;                            // qv[32 i]: read at use, so the query holds no registers
+    const float iq = inv_nq[q];
+    const int32_t* cq = cand + (int64_t)q * c;
+    auto group_of = [&](int j) {                             // validated candidate j of the list, -1 = no rows to read
+        const int32_t g = j < c ? cq[j] : -1;
+        if (g < -1 || g >= n_groups) { *bad = 1; return -1; }
+        return g;
+    };
+    for (int j0 = 0; j0 < c; j0 += RG_CH) {
+        // 1. the chunk's row runs and their prefix
+        int64_t cnt[PER], sum = 0;
+#pragma unroll
+        for (int p = 0; p < PER; ++p) {
+            const int jl = threadIdx.x * PER + p;
+            const int32_t g = group_of(j0 + jl);
+            const int32_t r0 = g >= 0 ? off[g] : 0;
+            cnt[p] = g >= 0 ? (int64_t)(off[g + 1] - r0) : 0;
+            sum += cnt[p];
+            s_row0[jl] = r0;
+            s_best[jl] = f32_order(-CUDART_INF_F);
+        }
+        int64_t incl = sum;
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t v = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += v;
+        }
+        if (lane == 31) s_wsum[warp] = incl;
+        __syncthreads();
+        int64_t run = incl - sum;
+        for (int w = 0; w < warp; ++w) run += s_wsum[w];
+#pragma unroll
+        for (int p = 0; p < PER; ++p) {
+            s_pre[threadIdx.x * PER + p] = run;
+            run += cnt[p];
+        }
+        if (threadIdx.x == RG_T - 1) s_pre[RG_CH] = run;
+        __syncthreads();
+        // 2. the rows: 4 in flight per warp, as in k_cosine_rerank
+        const int64_t total = s_pre[RG_CH];
+        for (int64_t f0 = warp * 4; f0 < total; f0 += 32) {
+            // lane x (mod 4) locates row f0 + x: its candidate slot (the last run starting at or before it) and its row
+            const int64_t f = f0 + (lane & 3);
+            int slot = 0;
+#pragma unroll
+            for (int step = RG_CH / 2; step > 0; step >>= 1) slot += s_pre[slot + step] <= f ? step : 0;
+            const int32_t row = f < total ? s_row0[slot] + (int32_t)(f - s_pre[slot]) : -1;
+            uint4 dv[4][NV];
+#pragma unroll
+            for (int x = 0; x < 4; ++x) {
+                const int32_t rx = __shfl_sync(0xffffffffu, row, x);
+                const uint4* pd = reinterpret_cast<const uint4*>(docs + (int64_t)(rx >= 0 ? rx : 0) * d);
+#pragma unroll
+                for (int i = 0; i < NV; ++i)
+                    dv[x][i] = rx >= 0 && lane + 32 * i < nvec ? __ldg(pd + lane + 32 * i) : make_uint4(0, 0, 0, 0);
+            }
+#pragma unroll
+            for (int x = 0; x < 4; ++x) {
+                float s = 0.f, nn = 0.f;
+                cos_lane_dot<NV>(dv[x], QStrided{qv}, s, nn);   // nn is not used: the norms come from inv_nd
+                for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+                if (lane == x && row >= 0) atomicMax(s_best + slot, f32_order(s * inv_nd[row] * iq));
+            }
+        }
+        __syncthreads();
+        // 3. one (group, score) per candidate
+        for (int jl = threadIdx.x; jl < RG_CH && j0 + jl < c; jl += RG_T) {
+            const int64_t i = (int64_t)q * c + j0 + jl;
+            const bool has_rows = s_pre[jl + 1] > s_pre[jl];
+            out_ids[i] = has_rows ? cq[j0 + jl] : -1;
+            out_sc[i] = has_rows ? (double)f32_unorder(s_best[jl]) : 0.0;
+        }
+        __syncthreads();                                     // the next chunk rewrites the shared arrays
+    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1413,6 +1539,65 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
     return BR_OK;
 }
 
+int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows, int32_t d, const int32_t* row_group,
+                          int32_t n_groups, const void* queries, int32_t nq, const int32_t* cand, int32_t c, int32_t k,
+                          int32_t* out_ids, float* out_sims, cudaStream_t st) {
+    const std::string fn = "br_cosine_rerank_grouped";
+    BR_REQUIRE(docs && inv_nd && row_group && (nq == 0 || (queries && cand && out_ids && out_sims)), BR_ERR_INVALID,
+               fn + ": null pointer");
+    BR_REQUIRE(n_rows > 0 && n_rows < (1LL << 31) && n_groups >= 1 && nq >= 0 && c >= 1 && k >= 1 && k <= BR_MAX_K,
+               BR_ERR_INVALID, fn + ": bad sizes");
+    BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, fn + ": embedding dim must be a multiple of 8");
+    BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, fn + ": embedding dim > 1024");
+    if (nq == 0) return BR_OK;
+    // the layout, checked before anything reads a row through it
+    const int32_t n_blk = (int32_t)((n_rows + GC_ROWS - 1) / GC_ROWS);
+    AsyncBuf b_lay(st), b_off(st);
+    BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 16));
+    int32_t* info = (int32_t*)b_lay.p + n_blk;
+    BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
+    k_group_check<<<n_blk, 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_lay.p, info);
+    BR_CUDA(cudaGetLastError());
+    int32_t h_info = 0;
+    BR_CUDA(cudaMemcpyAsync(&h_info, info, 4, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+    BR_REQUIRE(!h_info, BR_ERR_INVALID, fn + ": row_group must be non-decreasing with values in [0, n_groups)");
+    BR_TRY(b_off.alloc(4 * ((size_t)n_groups + 1)));
+    k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_off.p);
+    BR_CUDA(cudaGetLastError());
+    // per candidate (group or -1, best cosine), then the same selection and output as cosine_rerank
+    const int64_t n_pairs = (int64_t)nq * c;
+    AsyncBuf b_inq(st), b_id(st), b_s64(st), b_qoff(st), b_o64(st);
+    BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_id.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
+    BR_TRY(b_qoff.alloc(8 * ((size_t)nq + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
+    int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_groups)
+    BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
+    BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
+    const int nv = (d / 8 + 31) / 32;
+    auto launch = [&](auto kern) {
+        kern<<<nq, RG_T, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, d, (const int32_t*)b_off.p, n_groups,
+                                  (const __nv_bfloat16*)queries, (const float*)b_inq.p, cand, c, (int32_t*)b_id.p,
+                                  (double*)b_s64.p, bad);
+    };
+    if (nv <= 1) launch(k_cosine_rerank_grouped<1>);
+    else if (nv == 2) launch(k_cosine_rerank_grouped<2>);
+    else if (nv == 3) launch(k_cosine_rerank_grouped<3>);
+    else launch(k_cosine_rerank_grouped<4>);
+    BR_CUDA(cudaGetLastError());
+    std::vector<int64_t> qoff((size_t)nq + 1);
+    for (int32_t q = 0; q <= nq; ++q) qoff[(size_t)q] = (int64_t)q * c;
+    BR_CUDA(cudaMemcpyAsync(b_qoff.p, qoff.data(), 8 * ((size_t)nq + 1), cudaMemcpyHostToDevice, st));
+    BR_TRY(launch_final_select((const int32_t*)b_id.p, (const double*)b_s64.p, (const int64_t*)b_qoff.p, 0, nq, k, 0, out_ids,
+                               (double*)b_o64.p, nullptr, st));
+    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
+    BR_CUDA(cudaGetLastError());
+    int32_t h_bad = 0;
+    BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+    BR_REQUIRE(!h_bad, BR_ERR_INVALID, fn + ": a candidate id is outside [-1, n_groups)");
+    return BR_OK;
+}
+
 }  // namespace br
 
 extern "C" {
@@ -1451,6 +1636,14 @@ int br_cosine_rerank(const void* docs_bf16_dev, const float* doc_inv_norm_dev, i
                      int32_t* out_ids_dev, float* out_sims_dev, void* stream) {
     return br::cosine_rerank(docs_bf16_dev, doc_inv_norm_dev, n_docs, d, queries_bf16_dev, nq, cand_ids_dev, c, k, out_ids_dev,
                              out_sims_dev, (cudaStream_t)stream);
+}
+
+int br_cosine_rerank_grouped(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_rows, int32_t d,
+                             const int32_t* row_group_dev, int32_t n_groups, const void* queries_bf16_dev, int32_t nq,
+                             const int32_t* cand_groups_dev, int32_t c, int32_t k, int32_t* out_ids_dev,
+                             float* out_sims_dev, void* stream) {
+    return br::cosine_rerank_grouped(docs_bf16_dev, doc_inv_norm_dev, n_rows, d, row_group_dev, n_groups, queries_bf16_dev, nq,
+                                     cand_groups_dev, c, k, out_ids_dev, out_sims_dev, (cudaStream_t)stream);
 }
 
 }  // extern "C"

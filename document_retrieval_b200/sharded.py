@@ -112,6 +112,14 @@ def local_filter_slice(doc_filter, lo: int, n_local: int):
     return f[..., lo:lo + n_local]
 
 
+def local_group_candidates(candidate_groups, group_base: int, n_groups: int):
+    """GLOBAL candidate group ids [Q, c] (-1 = empty) -> this shard's local ids: ids in [group_base, group_base + n_groups)
+    minus group_base, every other id -1.  -> (local int32 [Q, c], number of ids this shard owns)."""
+    g = torch.as_tensor(candidate_groups).to(torch.int64)
+    own = (g >= group_base) & (g < group_base + n_groups)
+    return torch.where(own, g - group_base, torch.full_like(g, -1)).to(torch.int32), int(own.sum())
+
+
 class ShardedBM25:
     """One rank's view of a doc-sharded index.  ``local`` is this rank's ``BM25`` shard (built with
     ``doc_base`` = first global doc id of the shard and the all-reduced statistics)."""
@@ -289,6 +297,24 @@ class ShardedCosineIndex:
             fkw = dict(doc_filter=local_filter_slice(doc_filter, self.local.group_base, self.local.n_groups),
                        query_filter=query_filter)
         ids, sims = self.local.topk_groups(query_embeddings, k, **fkw)
+        return self._merge(ids, sims, k)
+
+    def rerank_groups(self, query_embeddings, candidate_groups, k=10):
+        """Grouped re-rank (``CosineIndex.rerank_groups``) of candidate groups [Q, c] given as GLOBAL group ids (-1 =
+        empty), the same on every rank -> (global group ids int64[Q, k], cosine float64[Q, k]) on every rank, identical
+        to one index over all rows.  Rank r owns the ids [group_base, group_base + n_groups) of its local index; an id
+        below -1 or owned by no rank raises ValueError on every rank."""
+        cand = torch.as_tensor(candidate_groups).to(device=self.local.device, dtype=torch.int64)
+        if bool((cand < -1).any()):
+            raise ValueError("candidate group ids must be >= -1")
+        local, owned = local_group_candidates(cand, self.local.group_base, self.local.n_groups)
+        t = torch.tensor([owned], dtype=torch.int64, device=cand.device)
+        if dist.is_initialized() and dist.get_world_size(self.group) > 1:
+            dist.all_reduce(t, group=self.group)
+        if int(t) != int((cand >= 0).sum()):
+            raise ValueError("a candidate group id is owned by no rank")
+        ids, sims = self.local.rerank_groups(query_embeddings, local, k)
+        ids = torch.where(ids >= 0, ids.to(torch.int64) + self.local.group_base, torch.full_like(ids, -1, dtype=torch.int64))
         return self._merge(ids, sims, k)
 
     def _merge(self, ids, sims, k):

@@ -281,6 +281,20 @@ int br_set_cosine_option(const char* name, int value);
 int br_cosine_rerank(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_docs, int32_t d,
                      const void* queries_bf16_dev, int32_t nq, const int32_t* cand_ids_dev, int32_t c,
                      int32_t k, int32_t* out_ids_dev, float* out_sims_dev, void* stream);
+/* Grouped re-rank, e.g. BM25's candidate documents re-ranked by the best of their sentence embeddings.  row_group_dev and
+ * n_groups as in br_cosine_topk_grouped (non-decreasing, values in [0, n_groups)); doc_inv_norm_dev (br_row_inv_norms) is
+ * required.  cand_groups_dev int32[nq, c] holds each query's candidate GROUPS (local group ids, -1 = empty slot); c >= 1,
+ * any size.  A group scores the largest cosine of its rows, each computed bit for bit as br_cosine_rerank computes it.
+ * Outputs [nq, k] (1 <= k <= BR_MAX_K): out_ids_dev int32 local group ids, out_sims_dev float, ordered by (score desc,
+ * group id asc); a group repeated in a row is returned once, groups without rows are never returned, and fewer than k
+ * distinct non-empty candidates pad with -1 / 0.0.  A decreasing or out-of-range row_group is BR_ERR_INVALID (checked on
+ * the device before any row is read); so is a candidate id outside [-1, n_groups) (never used to find rows, reported at
+ * the synchronisation).  d not a multiple of 8 or d > 1024: BR_ERR_UNSUPPORTED.  nq = 0 returns at once (queries,
+ * candidates and outputs may then be NULL).  Synchronises `stream`. */
+int br_cosine_rerank_grouped(const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_rows, int32_t d,
+                             const int32_t* row_group_dev, int32_t n_groups, const void* queries_bf16_dev, int32_t nq,
+                             const int32_t* cand_groups_dev, int32_t c, int32_t k, int32_t* out_ids_dev,
+                             float* out_sims_dev, void* stream);
 
 /* Sentence -> document step of the sentence-level retrieval (team_run1.py:286-294): for every query walk its ranked
  * sentences sentence_ids_dev int64[nq, n] (best first, -1 = padding), map each to its parent doc through
