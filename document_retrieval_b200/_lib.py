@@ -92,11 +92,16 @@ def _bit_weights(dev):
     return torch.bitwise_left_shift(torch.ones(32, dtype=torch.int64, device=dev), torch.arange(32, device=dev))
 
 
-def pack_doc_filter(doc_filter, query_filter, nq: int, n_docs: int, device):
+def pack_doc_filter(doc_filter=None, query_filter=None, nq: int = 0, n_docs: int = 0, device=None):
     """``doc_filter`` bool [N] (one allow-list for the whole batch) or [F, N] with ``query_filter`` int [Q] (the row each
-    query uses, -1 = unfiltered) -> (br_doc_filter struct, tensors it points to).  The bits are packed on the device:
-    bit (d & 31) of word (d >> 5) of row f = doc_filter[f, d].  Shape mismatches raise ValueError; a query_filter value
-    outside [-1, F) is left to the library, which rejects it (BRError)."""
+    query uses, -1 = unfiltered) -> (br_doc_filter struct, tensors it points to); (None, None) without a filter, which
+    the library takes as the unfiltered call.  The bits are packed on the device: bit (d & 31) of word (d >> 5) of row
+    f = doc_filter[f, d].  Shape mismatches raise ValueError; a query_filter value outside [-1, F) is left to the
+    library, which rejects it (BRError)."""
+    if doc_filter is None:
+        if query_filter is not None:
+            raise ValueError("query_filter needs a doc_filter")
+        return None, None
     f = torch.as_tensor(doc_filter)
     if f.dtype != torch.bool:
         raise ValueError(f"doc_filter must be a bool array, got {f.dtype}")

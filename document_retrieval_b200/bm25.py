@@ -282,22 +282,14 @@ class BM25:
         nq = q_off.numel() - 1
         dev = self._device
         with torch.cuda.device(dev):
-            filt = None
-            if doc_filter is not None or query_filter is not None:
-                if doc_filter is None:
-                    raise ValueError("query_filter needs a doc_filter")
-                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
+            filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
             ids = torch.empty((nq, n), dtype=torch.int32, device=dev)
             sc = torch.empty((nq, n), dtype=torch.float64, device=dev)
             cnt = torch.empty((nq,), dtype=torch.int32, device=dev)
-            if filt is None:
-                check(lib.br_topk_batch(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                        int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
-                                        _lib.stream_ptr(dev)), "br_topk_batch")
-            else:
-                check(lib.br_topk_batch_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                                 int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
-                                                 C.byref(filt), _lib.stream_ptr(dev)), "br_topk_batch_filtered")
+            check(lib.br_topk_batch_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                             int(self.dedup_query), int(positive_only), ptr(ids), ptr(sc), ptr(cnt),
+                                             None if filt is None else C.byref(filt), _lib.stream_ptr(dev)),
+                  "br_topk_batch_filtered")
         return (ids, sc, cnt) if return_counts else (ids, sc)
 
     def retrieve_records_batch(self, queries, n=10, positive_only=False, doc_filter=None, query_filter=None):
@@ -313,21 +305,12 @@ class BM25:
         nq = q_off.numel() - 1
         dev = self._device
         with torch.cuda.device(dev):
-            filt = None
-            if doc_filter is not None or query_filter is not None:
-                if doc_filter is None:
-                    raise ValueError("query_filter needs a doc_filter")
-                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
+            filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.corpus_size, dev)
             rec = torch.empty((nq, n, 2), dtype=torch.int64, device=dev)
-            if filt is None:
-                check(lib.br_topk_batch_records(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                                int(self.dedup_query), int(positive_only), ptr(rec), None,
-                                                _lib.stream_ptr(dev)), "br_topk_batch_records")
-            else:
-                check(lib.br_topk_batch_records_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
-                                                         int(self.dedup_query), int(positive_only), ptr(rec), None,
-                                                         C.byref(filt), _lib.stream_ptr(dev)),
-                      "br_topk_batch_records_filtered")
+            check(lib.br_topk_batch_records_filtered(self._h, ptr(q_terms), ptr(q_off), nq, int(q_terms.numel()), n,
+                                                     int(self.dedup_query), int(positive_only), ptr(rec), None,
+                                                     None if filt is None else C.byref(filt), _lib.stream_ptr(dev)),
+                  "br_topk_batch_records_filtered")
         return rec
 
     def exact_scores(self, query):

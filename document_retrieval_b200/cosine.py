@@ -79,20 +79,12 @@ class CosineIndex:
         q = _bf16(query_embeddings, self.device)
         nq = q.shape[0]
         with torch.cuda.device(self.device):
-            filt = None
-            if doc_filter is not None or query_filter is not None:
-                if doc_filter is None:
-                    raise ValueError("query_filter needs a doc_filter")
-                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_docs, self.device)
+            filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_docs, self.device)
             ids = torch.empty((nq, k), dtype=torch.int64, device=self.device)
             sims = torch.empty((nq, k), dtype=torch.float32, device=self.device)
-            if filt is None:
-                check(lib.br_cosine_topk(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq, int(k),
-                                         self.doc_base, ptr(ids), ptr(sims), _lib.stream_ptr(self.device)), "br_cosine_topk")
-            else:
-                check(lib.br_cosine_topk_filtered(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq,
-                                                  int(k), self.doc_base, ptr(ids), ptr(sims), C.byref(filt),
-                                                  _lib.stream_ptr(self.device)), "br_cosine_topk_filtered")
+            check(lib.br_cosine_topk_filtered(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(q), nq, int(k),
+                                              self.doc_base, ptr(ids), ptr(sims), None if filt is None else C.byref(filt),
+                                              _lib.stream_ptr(self.device)), "br_cosine_topk_filtered")
         return ids, sims
 
     def topk_groups(self, query_embeddings, k=10, doc_filter=None, query_filter=None):
@@ -106,11 +98,7 @@ class CosineIndex:
         q = _bf16(query_embeddings, self.device)
         nq = q.shape[0]
         with torch.cuda.device(self.device):
-            filt = None
-            if doc_filter is not None or query_filter is not None:
-                if doc_filter is None:
-                    raise ValueError("query_filter needs a doc_filter")
-                filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_groups, self.device)
+            filt, _keep = _lib.pack_doc_filter(doc_filter, query_filter, nq, self.n_groups, self.device)
             ids = torch.empty((nq, k), dtype=torch.int64, device=self.device)
             sims = torch.empty((nq, k), dtype=torch.float32, device=self.device)
             check(lib.br_cosine_topk_grouped(ptr(self.docs), ptr(self.inv_norm), self.n_docs, self.dim, ptr(self.row_group),

@@ -177,16 +177,29 @@ struct CosArgs {
     int32_t d;
     int32_t tile_begin, tile_end;   // doc tiles [tile_begin, tile_end) of CG_BM rows
     int32_t window;                 // query-stationary kernel: doc tiles per L2 window
-    // row filter (the <true> instantiations only; appended so that the fields above keep their offsets)
-    const uint32_t* fbits;          // bitmap rows [n_rows, fwords]
-    int64_t fwords;
-    const int32_t* frow;            // [nq] row of query q, -1 = unfiltered
+    DocFilter f;                    // row filter (the <true> instantiations only; last, so the fields above keep their offsets)
 };
 
 // The filtered kernels keep each query column's filter row in shared memory behind the barriers (beyond the unfiltered
-// layout, so that it stays as it is); a row is tested only where a score has passed the threshold.
+// layout, so that it stays as it is); a row is tested only where a score has passed the threshold.  doc_allowed's test
+// on a row pointer that may be null costs these kernels instructions, so the test stays on frow here.
 __device__ __forceinline__ bool cos_row_allowed(const CosArgs& a, int32_t frow, int64_t doc) {
-    return frow < 0 || ((__ldg(a.fbits + (int64_t)frow * a.fwords + (doc >> 5)) >> (doc & 31)) & 1u) != 0u;
+    return frow < 0 || ((__ldg(a.f.bits + (int64_t)frow * a.f.words + (doc >> 5)) >> (doc & 31)) & 1u) != 0u;
+}
+
+// Epilogue, query column c of the block (query q): the threshold that acc * inv_d is compared against (thr / inv_q,
+// widened so that the rounding of the division keeps a superset), 1 / (||q|| + eps) and, FILT, the column's filter row
+template <bool FILT>
+__device__ __forceinline__ void cos_stage_column(const CosArgs& a, int q, int c, float* s_thr, float* s_inq, int32_t* s_frow) {
+    float th = CUDART_INF_F, iq = 0.f;
+    if (q < a.nq) {
+        iq = a.inv_nq[q];
+        const float raw = __ldcg(a.thr + q) / iq;
+        th = raw - fabsf(raw) * 4e-6f;
+    }
+    s_thr[c] = th;
+    s_inq[c] = iq;
+    if constexpr (FILT) s_frow[c] = q < a.nq ? a.f.row[q] : -1;
 }
 
 // Multicast kernel (d > 768): a CTA computes docs[256-row tile] x queries[256-col tile] with two 128-row UMMAs sharing the
@@ -289,19 +302,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(CG_THREADS, 1) k_cos
         for (int64_t t = t_first; t < n_tiles; t += t_step) {
             const int dt = a.tile_begin + (int)(t / n_qt), qt = 2 * (int)(t % n_qt) + (int)crank;
             asm volatile("bar.sync 1, 256;" ::: "memory");          // previous tile's thresholds no longer in use
-            {
-                const int c = et;
-                const int q = qt * CG_BN + c;
-                float th = CUDART_INF_F, iq = 0.f;
-                if (q < a.nq) {
-                    iq = a.inv_nq[q];
-                    const float raw = __ldcg(a.thr + q) / iq;          // compare acc*inv_d against thr/inv_q
-                    th = raw - fabsf(raw) * 4e-6f;                      // superset: rounding of the division
-                }
-                s_thr[c] = th;
-                s_inq[c] = iq;
-                if constexpr (FILT) s_frow[c] = q < a.nq ? a.frow[q] : -1;
-            }
+            cos_stage_column<FILT>(a, qt * CG_BN + et, et, s_thr, s_inq, s_frow);
             asm volatile("bar.sync 1, 256;" ::: "memory");          // epilogue warps only
             mbar_wait(tfull_bar(half), acc_phase);
             acc_phase ^= 1;
@@ -579,18 +580,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
             if (un.qb != cur_qb) {
                 cur_qb = un.qb;
                 asm volatile("bar.sync 1, 256;" ::: "memory");      // previous block's thresholds no longer in use
-                if (et < QS_BN) {
-                    const int q = un.qb * QS_BN + et;
-                    float th = CUDART_INF_F, iq = 0.f;
-                    if (q < a.nq) {
-                        iq = a.inv_nq[q];
-                        const float raw = __ldcg(a.thr + q) / iq;      // compare acc*inv_d against thr/inv_q
-                        th = raw - fabsf(raw) * 4e-6f;                  // superset: rounding of the division
-                    }
-                    s_thr[et] = th;
-                    s_inq[et] = iq;
-                    if constexpr (FILT) s_frow[et] = q < a.nq ? a.frow[q] : -1;
-                }
+                if (et < QS_BN) cos_stage_column<FILT>(a, un.qb * QS_BN + et, et, s_thr, s_inq, s_frow);
                 asm volatile("bar.sync 1, 256;" ::: "memory");
             }
             const int64_t doc = (int64_t)(a.tile_begin + un.tile) * CG_BM + (int)crank * 128 + quarter * 32 + lane;
@@ -683,14 +673,53 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(QS_THREADS, 1) k_cos
     }
 }
 
-// threshold := k-th best candidate so far; keep the candidates >= threshold, sorted (score desc, id asc)
+// bitonic sort of s_h / s_id [0, n_sort) by (score desc, id asc), or, BY_GROUP, of s_h / s_id / s_g by (group asc,
+// score desc, id asc); n_sort a power of two
 constexpr int TC_T = 256;
+template <bool BY_GROUP>
+__device__ __forceinline__ void cos_sort(float* s_h, int32_t* s_id, int32_t* s_g, int n_sort) {
+    for (int size = 2; size <= n_sort; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            __syncthreads();
+            for (int i = threadIdx.x; i < n_sort / 2; i += blockDim.x) {
+                const int x = 2 * i - (i & (stride - 1)), y = x + stride;
+                const bool up = (x & size) == 0;
+                const float hx = s_h[x], hy = s_h[y];
+                const int32_t ix = s_id[x], iy = s_id[y];
+                bool y_first = hy > hx || (hy == hx && iy < ix);
+                if constexpr (BY_GROUP) y_first = s_g[y] < s_g[x] || (s_g[y] == s_g[x] && y_first);
+                if (y_first == up) {
+                    s_h[x] = hy; s_h[y] = hx; s_id[x] = iy; s_id[y] = ix;
+                    if constexpr (BY_GROUP) { const int32_t g = s_g[x]; s_g[x] = s_g[y]; s_g[y] = g; }
+                }
+            }
+        }
+    }
+    __syncthreads();
+}
+
+// threshold := k-th best candidate so far; keep the candidates >= threshold, sorted (score desc, id asc).
+// GROUPED (row r in group row_group[r]): the list first keeps one entry per group - its best row, the lowest row on ties
+// -, so the threshold is the k-th best DISTINCT-group score so far (only raised) and the kept rows are sorted (score
+// desc, row asc) = (score desc, group asc).  Every threshold is the score of k distinct groups, so it never exceeds the
+// final k-th best group score and no row of a final top-k group is ever filtered out; rows of a group that is already
+// in the list are merged by the next call.
+template <bool GROUPED>
 __global__ void __launch_bounds__(TC_T) k_tighten_cos(float* __restrict__ thr, int32_t* __restrict__ cand_cnt,
                                                       int32_t* __restrict__ prev_cnt, int32_t* __restrict__ cand,
-                                                      float* __restrict__ cand_h, int K, int32_t* __restrict__ overflow) {
+                                                      float* __restrict__ cand_h, const int32_t* __restrict__ row_group,
+                                                      int K, int32_t* __restrict__ overflow) {
     __shared__ float s_h[COS_CAP];
     __shared__ int32_t s_id[COS_CAP];
     __shared__ int s_keep;
+    int32_t* s_g = nullptr;
+    int* s_nd = nullptr;
+    if constexpr (GROUPED) {
+        __shared__ int32_t s_g_[COS_CAP];
+        __shared__ int s_nd_;
+        s_g = s_g_;
+        s_nd = &s_nd_;
+    }
     const int q = blockIdx.x;
     int n = cand_cnt[q];
     if (n == prev_cnt[q]) return;
@@ -703,126 +732,30 @@ __global__ void __launch_bounds__(TC_T) k_tighten_cos(float* __restrict__ thr, i
     int n_sort = 32;                                   // smallest power of two covering the list
     while (n_sort < n) n_sort <<= 1;
     for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
-        s_h[i] = i < n ? hs[i] : -CUDART_INF_F;
-        s_id[i] = i < n ? ids[i] : 0x7fffffff;
-    }
-    if (threadIdx.x == 0) s_keep = 0;
-    for (int size = 2; size <= n_sort; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < n_sort / 2; i += blockDim.x) {
-                const int x = 2 * i - (i & (stride - 1)), y = x + stride;
-                const bool up = (x & size) == 0;
-                const float hx = s_h[x], hy = s_h[y];
-                const int32_t ix = s_id[x], iy = s_id[y];
-                const bool y_first = hy > hx || (hy == hx && iy < ix);
-                if (y_first == up) { s_h[x] = hy; s_h[y] = hx; s_id[x] = iy; s_id[y] = ix; }
-            }
-        }
-    }
-    __syncthreads();
-    float th = thr[q];
-    if (n >= K && s_h[K - 1] > th) th = s_h[K - 1];
-    int keep = 0;
-    for (int i = threadIdx.x; i < n; i += blockDim.x) keep += (s_h[i] >= th) ? 1 : 0;
-    for (int o = 16; o > 0; o >>= 1) keep += __shfl_xor_sync(0xffffffffu, keep, o);
-    if ((threadIdx.x & 31) == 0 && keep) atomicAdd(&s_keep, keep);
-    __syncthreads();
-    keep = s_keep;
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        ids[i] = i < keep ? s_id[i] : -1;
-        hs[i] = i < keep ? s_h[i] : 0.f;
-    }
-    if (threadIdx.x == 0) {
-        thr[q] = th;
-        cand_cnt[q] = keep;
-        prev_cnt[q] = keep;
-    }
-}
-
-__global__ void k_cos_output(const int32_t* __restrict__ cand, const float* __restrict__ cand_h,
-                             const int32_t* __restrict__ cand_cnt, int32_t nq, int32_t k, int64_t doc_base,
-                             int64_t* __restrict__ out_ids, float* __restrict__ out_sims) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (int64_t)nq * k) return;
-    const int q = (int)(i / k), j = (int)(i - (int64_t)q * k);
-    const bool ok = j < cand_cnt[q] && j < COS_CAP;           // lists are sorted by the last k_tighten_cos
-    out_ids[i] = ok ? (int64_t)cand[(int64_t)q * COS_CAP + j] + doc_base : -1;
-    out_sims[i] = ok ? cand_h[(int64_t)q * COS_CAP + j] : 0.f;
-}
-
-// ------------------------------------------------------------------------------------------
-// grouped (document-level) top-k: row r belongs to group row_group[r], a non-decreasing map, so a group's rows are one
-// contiguous run and, between rows of different groups, "row asc" is "group asc".  A group scores the best of its rows.
-// ------------------------------------------------------------------------------------------
-// bitonic sort of s_h / s_id / s_g [0, n_sort) by `before(y, x)` (true: entry y goes first); n_sort a power of two
-template <class Before>
-__device__ __forceinline__ void cos_sort3(float* s_h, int32_t* s_id, int32_t* s_g, int n_sort, Before before) {
-    for (int size = 2; size <= n_sort; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < n_sort / 2; i += blockDim.x) {
-                const int x = 2 * i - (i & (stride - 1)), y = x + stride;
-                const bool up = (x & size) == 0;
-                if (before(y, x) == up) {
-                    const float h = s_h[x]; s_h[x] = s_h[y]; s_h[y] = h;
-                    const int32_t id = s_id[x]; s_id[x] = s_id[y]; s_id[y] = id;
-                    const int32_t g = s_g[x]; s_g[x] = s_g[y]; s_g[y] = g;
-                }
-            }
-        }
-    }
-    __syncthreads();
-}
-
-// k_tighten_cos for a grouped corpus: the list (rows) keeps one entry per group - its best row, the lowest row on ties -,
-// threshold := the k-th best DISTINCT-group score so far (only raised), and the groups at or above it stay, sorted
-// (score desc, row asc) = (score desc, group asc).  Every threshold is the score of k distinct groups, so it never
-// exceeds the final k-th best group score and no row of a final top-k group is ever filtered out; rows of a group that
-// is already in the list are merged by the next call.  Same overflow rule as k_tighten_cos.
-__global__ void __launch_bounds__(TC_T) k_tighten_cos_grouped(float* __restrict__ thr, int32_t* __restrict__ cand_cnt,
-                                                              int32_t* __restrict__ prev_cnt, int32_t* __restrict__ cand,
-                                                              float* __restrict__ cand_h, const int32_t* __restrict__ row_group,
-                                                              int K, int32_t* __restrict__ overflow) {
-    __shared__ float s_h[COS_CAP];
-    __shared__ int32_t s_id[COS_CAP];
-    __shared__ int32_t s_g[COS_CAP];
-    __shared__ int s_keep, s_nd;
-    const int q = blockIdx.x;
-    int n = cand_cnt[q];
-    if (n == prev_cnt[q]) return;
-    if (n > COS_CAP) {
-        if (threadIdx.x == 0) overflow[q] = 1;
-        n = COS_CAP;
-    }
-    int32_t* ids = cand + (int64_t)q * COS_CAP;
-    float* hs = cand_h + (int64_t)q * COS_CAP;
-    int n_sort = 32;
-    while (n_sort < n) n_sort <<= 1;
-    for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
         const int32_t row = i < n ? ids[i] : 0x7fffffff;
         s_h[i] = i < n ? hs[i] : -CUDART_INF_F;
         s_id[i] = row;
-        s_g[i] = i < n ? __ldg(row_group + row) : 0x7fffffff;
+        if constexpr (GROUPED) s_g[i] = i < n ? __ldg(row_group + row) : 0x7fffffff;
     }
-    if (threadIdx.x == 0) { s_keep = 0; s_nd = 0; }
-    // 1. (group asc, score desc, row asc): the first entry of every group run is the group's best row
-    cos_sort3(s_h, s_id, s_g, n_sort, [&](int y, int x) {
-        return s_g[y] < s_g[x] || (s_g[y] == s_g[x] && (s_h[y] > s_h[x] || (s_h[y] == s_h[x] && s_id[y] < s_id[x])));
-    });
-    int nd = 0;                                        // only s_h / s_id change here; s_g is only read
-    for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
-        const bool first = i < n && (i == 0 || s_g[i] != s_g[i - 1]);
-        nd += first ? 1 : 0;
-        if (!first) { s_h[i] = -CUDART_INF_F; s_id[i] = 0x7fffffff; }
+    if (threadIdx.x == 0) {
+        s_keep = 0;
+        if constexpr (GROUPED) *s_nd = 0;
     }
-    for (int o = 16; o > 0; o >>= 1) nd += __shfl_xor_sync(0xffffffffu, nd, o);
-    if ((threadIdx.x & 31) == 0 && nd) atomicAdd(&s_nd, nd);
-    // 2. the distinct groups first, (score desc, row asc); the dropped entries (-inf, INT_MAX) last
-    cos_sort3(s_h, s_id, s_g, n_sort, [&](int y, int x) {
-        return s_h[y] > s_h[x] || (s_h[y] == s_h[x] && s_id[y] < s_id[x]);
-    });
-    nd = s_nd;
+    int nd = n;                                        // distinct entries
+    if constexpr (GROUPED) {
+        // the first entry of every group run is the group's best row; the others become (-inf, INT_MAX) and sort last
+        cos_sort<true>(s_h, s_id, s_g, n_sort);
+        nd = 0;                                        // only s_h / s_id change here; s_g is only read
+        for (int i = threadIdx.x; i < n_sort; i += blockDim.x) {
+            const bool first = i < n && (i == 0 || s_g[i] != s_g[i - 1]);
+            nd += first ? 1 : 0;
+            if (!first) { s_h[i] = -CUDART_INF_F; s_id[i] = 0x7fffffff; }
+        }
+        for (int o = 16; o > 0; o >>= 1) nd += __shfl_xor_sync(0xffffffffu, nd, o);
+        if ((threadIdx.x & 31) == 0 && nd) atomicAdd(s_nd, nd);
+    }
+    cos_sort<false>(s_h, s_id, s_g, n_sort);
+    if constexpr (GROUPED) nd = *s_nd;
     float th = thr[q];
     if (nd >= K && s_h[K - 1] > th) th = s_h[K - 1];
     int keep = 0;
@@ -842,17 +775,23 @@ __global__ void __launch_bounds__(TC_T) k_tighten_cos_grouped(float* __restrict_
     }
 }
 
-__global__ void k_cos_output_grouped(const int32_t* __restrict__ cand, const float* __restrict__ cand_h,
-                                     const int32_t* __restrict__ cand_cnt, const int32_t* __restrict__ row_group, int32_t nq,
-                                     int32_t k, int64_t doc_base, int64_t* __restrict__ out_ids, float* __restrict__ out_sims) {
+// row_group (may be NULL): the lists hold one row per group, returned as its group id
+__global__ void k_cos_output(const int32_t* __restrict__ cand, const float* __restrict__ cand_h,
+                             const int32_t* __restrict__ cand_cnt, const int32_t* __restrict__ row_group, int32_t nq,
+                             int32_t k, int64_t doc_base, int64_t* __restrict__ out_ids, float* __restrict__ out_sims) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int64_t)nq * k) return;
     const int q = (int)(i / k), j = (int)(i - (int64_t)q * k);
-    const bool ok = j < cand_cnt[q] && j < COS_CAP;           // one row per group, sorted by k_tighten_cos_grouped
-    out_ids[i] = ok ? (int64_t)row_group[cand[(int64_t)q * COS_CAP + j]] + doc_base : -1;
+    const bool ok = j < cand_cnt[q] && j < COS_CAP;           // lists are sorted by the last k_tighten_cos
+    const int32_t row = ok ? cand[(int64_t)q * COS_CAP + j] : 0;
+    out_ids[i] = ok ? (int64_t)(row_group ? row_group[row] : row) + doc_base : -1;
     out_sims[i] = ok ? cand_h[(int64_t)q * COS_CAP + j] : 0.f;
 }
 
+// ------------------------------------------------------------------------------------------
+// grouped (document-level) top-k: row r belongs to group row_group[r], a non-decreasing map, so a group's rows are one
+// contiguous run and, between rows of different groups, "row asc" is "group asc".  A group scores the best of its rows.
+// ------------------------------------------------------------------------------------------
 // Layout check, pass 1: block b looks at rows [b * GC_ROWS, (b + 1) * GC_ROWS): a value outside [0, n_groups) or below
 // its predecessor sets info[0]; blk_starts[b] = the rows of the block that start a group run.
 constexpr int GC_ROWS = 1024;
@@ -1189,33 +1128,14 @@ int row_inv_norms(const void* emb, int64_t n, int32_t d, float* out, cudaStream_
     return BR_OK;
 }
 
-int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries, int32_t nq,
-                  const int32_t* cand, int32_t c, int32_t k, int32_t* out_ids, float* out_sims, cudaStream_t st);
-
-__global__ void k_iota_rows(int32_t* __restrict__ out, int32_t rows, int64_t n) {
-    const int64_t total = (int64_t)rows * n;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = (int32_t)(i % n);
-}
-// the same for filtered queries: row r of the list holds the doc rows query qs[r] may return, -1 (an empty slot of the
-// gather pass) for the others
-__global__ void k_iota_rows_filtered(int32_t* __restrict__ out, int32_t rows, int64_t n, const int32_t* __restrict__ qs,
-                                     DocFilter f) {
+// row r of the list: the doc rows [0, n) in order; with a filter (f.row != NULL) -1 (an empty slot of the gather pass)
+// for the rows query qs[r] may not return
+__global__ void k_iota_rows(int32_t* __restrict__ out, int32_t rows, int64_t n, const int32_t* __restrict__ qs, DocFilter f) {
     const int64_t total = (int64_t)rows * n;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = i / n, d = i - r * n;
-        out[i] = doc_allowed(f.row_of(qs[r]), (uint32_t)d) ? (int32_t)d : -1;
+        out[i] = !f.row || doc_allowed(f.row_of(qs[r]), (uint32_t)d) ? (int32_t)d : -1;
     }
-}
-// validated filter rows (the same rule as br_topk_batch_filtered): a value outside [-1, n_rows) sets *bad and becomes -1
-__global__ void k_cos_filter_rows(const int32_t* __restrict__ in, int32_t nq, int32_t n_rows, int32_t* __restrict__ out,
-                                  int32_t* __restrict__ bad) {
-    const int q = blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= nq) return;
-    const int32_t r = in ? in[q] : 0;
-    const bool ok = r >= -1 && r < n_rows;
-    if (!ok) atomicOr(bad, 1);
-    out[q] = ok ? r : -1;
 }
 __global__ void k_cos_patch(const int32_t* __restrict__ rows, int32_t nr, int32_t k, const int32_t* __restrict__ ids,
                             const float* __restrict__ sims, int64_t doc_base, int64_t* __restrict__ out_ids,
@@ -1282,6 +1202,45 @@ static int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_do
     return BR_OK;
 }
 
+// The selection of the re-rank calls: ids / s64 hold nq lists of c (id, float64 score), -1 = an empty slot -> per query
+// the top k ids by (score desc, id asc), a repeated id once, with their scores as fp32; -1 / 0.0 pad the rest.
+static int select_fixed(const int32_t* ids, const double* s64, int32_t nq, int32_t c, int32_t k, int32_t* out_ids,
+                        float* out_sims, cudaStream_t st) {
+    AsyncBuf b_o64(st);
+    BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
+    BR_TRY(launch_final_select(ids, s64, nullptr, 0, nq, k, 0, out_ids, (double*)b_o64.p, nullptr, st, nullptr, c));
+    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
+    BR_CUDA(cudaGetLastError());
+    return BR_OK;
+}
+
+// The layout of a grouped call, checked before anything reads a row through it: a decreasing value or one outside
+// [0, n_groups) fails the call `fn`.  Also returns R_k, the shortest row prefix holding k distinct groups (every row when
+// fewer than k groups are non-empty), and the number of non-empty groups.
+static int check_row_group(const int32_t* row_group, int64_t n_rows, int32_t n_groups, int32_t k, const std::string& fn,
+                           cudaStream_t st, int64_t* r_k, int64_t* n_nonempty) {
+    const int32_t n_blk = (int32_t)((n_rows + GC_ROWS - 1) / GC_ROWS);
+    AsyncBuf b_lay(st);
+    BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 8 * ((size_t)n_blk + 1) + 16));
+    int64_t* excl = (int64_t*)b_lay.p;
+    int32_t* blk = (int32_t*)(excl + n_blk + 1);
+    int32_t* info = blk + n_blk;
+    BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
+    k_group_check<<<n_blk, 256, 0, st>>>(row_group, n_rows, n_groups, blk, info);
+    BR_CUDA(cudaGetLastError());
+    k_exscan<int32_t><<<1, 1024, 0, st>>>(blk, n_blk, excl);
+    BR_CUDA(cudaGetLastError());
+    k_group_prefix<<<n_blk, GC_ROWS, 0, st>>>(row_group, n_rows, excl, n_blk, k, info);
+    BR_CUDA(cudaGetLastError());
+    int32_t h_info[4] = {0, 0, 0, 0};
+    BR_CUDA(cudaMemcpyAsync(h_info, info, 16, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+    BR_REQUIRE(!h_info[0], BR_ERR_INVALID, fn + ": row_group must be non-decreasing with values in [0, n_groups)");
+    *r_k = h_info[1];
+    *n_nonempty = h_info[2];
+    return BR_OK;
+}
+
 // Grouped call: row r belongs to group row_group[r] (device, non-decreasing, in [0, n_groups)).
 struct CosGroups {
     const int32_t* row_group;
@@ -1302,44 +1261,24 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         BR_REQUIRE(grp->n_groups >= 1, BR_ERR_INVALID, fn + ": n_groups must be >= 1");
     }
     // a filter is over the ids the call returns: rows, or groups for a grouped call
-    const int64_t n_ids = grp ? (int64_t)grp->n_groups : n_docs;
-    if (filter) {
-        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, fn + ": filter bitmap is null");
-        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, fn + ": filter n_rows must be >= 1");
-        BR_REQUIRE(filter->words >= (n_ids + 31) / 32, BR_ERR_INVALID,
-                   fn + (grp ? ": filter words < ceil(n_groups / 32)" : ": filter words < ceil(n_docs / 32)"));
-    }
+    BR_TRY(check_doc_filter(filter, grp ? (int64_t)grp->n_groups : n_docs, grp ? "n_groups" : "n_docs", fn));
     if (nq == 0) return BR_OK;
+    const int32_t* row_group = grp ? grp->row_group : nullptr;
     const int n_dt = (int)((n_docs + CG_BM - 1) / CG_BM), n_qt = (nq + CG_BN - 1) / CG_BN;
     // Launch schedule.  Ungrouped, the first launch runs without thresholds: every row is a candidate, and one doc tile
     // (CG_BM rows) fits a query's list of COS_CAP.
     static_assert(CG_BM <= COS_CAP, "the first launch must fit the candidate lists");
     int warm_tiles = 1, warm_cap = 1;
     double grow = 1.0;
-    AsyncBuf b_lay(st);
     if (grp) {
         // One pass over the layout before any GEMM: a decreasing or out-of-range value fails the call, and R_k (the
         // shortest row prefix with k distinct groups) bounds the warm-up.  Until R_k rows are covered a query holds
         // fewer than k groups and no threshold: its list keeps <= k - 1 entries and a launch can emit every row it
         // covers, so warm-up launches cover at most (COS_CAP - (k - 1)) / CG_BM tiles (>= 3).  With singleton groups
         // R_k = k <= CG_BM: one tile, then the ungrouped doubling - the same launches as br_cosine_topk.
-        const int32_t n_blk = (int32_t)((n_docs + GC_ROWS - 1) / GC_ROWS);
-        BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 8 * ((size_t)n_blk + 1) + 16));
-        int64_t* excl = (int64_t*)b_lay.p;
-        int32_t* blk = (int32_t*)(excl + n_blk + 1);
-        int32_t* info = blk + n_blk;
-        BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
-        k_group_check<<<n_blk, 256, 0, st>>>(grp->row_group, n_docs, grp->n_groups, blk, info);
-        BR_CUDA(cudaGetLastError());
-        k_exscan<int32_t><<<1, 1024, 0, st>>>(blk, n_blk, excl);
-        BR_CUDA(cudaGetLastError());
-        k_group_prefix<<<n_blk, GC_ROWS, 0, st>>>(grp->row_group, n_docs, excl, n_blk, k, info);
-        BR_CUDA(cudaGetLastError());
-        int32_t h_info[4] = {0, 0, 0, 0};
-        BR_CUDA(cudaMemcpyAsync(h_info, info, 16, cudaMemcpyDeviceToHost, st));
-        BR_CUDA(cudaStreamSynchronize(st));
-        BR_REQUIRE(!h_info[0], BR_ERR_INVALID, fn + ": row_group must be non-decreasing with values in [0, n_groups)");
-        const int64_t r_k = h_info[1], n_nonempty = std::max<int64_t>(h_info[2], 1);
+        int64_t r_k, n_nonempty;
+        BR_TRY(check_row_group(row_group, n_docs, grp->n_groups, k, fn, st, &r_k, &n_nonempty));
+        n_nonempty = std::max<int64_t>(n_nonempty, 1);
         warm_tiles = (int)((r_k + CG_BM - 1) / CG_BM);
         warm_cap = (COS_CAP - (k - 1)) / CG_BM;
         // After the warm-up a launch over R new rows passes about k R / S of the groups seen in S rows, and the rows of
@@ -1375,7 +1314,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         BR_TRY(b_frow.alloc(4 * Q + 16));
         f_bad = (int32_t*)b_frow.p + Q;
         BR_CUDA(cudaMemsetAsync(f_bad, 0, 4, st));
-        k_cos_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, (int32_t*)b_frow.p, f_bad);
+        k_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, (int32_t*)b_frow.p, f_bad);
         BR_CUDA(cudaGetLastError());
         fv = DocFilter{filter->bits_dev, filter->words, (const int32_t*)b_frow.p};
     }
@@ -1384,7 +1323,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         const int64_t rwords = (n_docs + 31) / 32, n_words = (int64_t)filter->n_rows * rwords;
         BR_TRY(b_rbits.alloc(4 * (size_t)n_words));
         k_group_filter_rows<<<(unsigned)std::min<int64_t>((n_words + 7) / 8, kNumSMs * 64), 256, 0, st>>>(
-            filter->bits_dev, filter->words, filter->n_rows, grp->row_group, n_docs, rwords, (uint32_t*)b_rbits.p);
+            filter->bits_dev, filter->words, filter->n_rows, row_group, n_docs, rwords, (uint32_t*)b_rbits.p);
         BR_CUDA(cudaGetLastError());
         fv.bits = (const uint32_t*)b_rbits.p;
         fv.words = rwords;
@@ -1402,9 +1341,10 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     // wall time, which makes doubling (13 launches, ~120 emissions per query) faster than 3x / 4x / 8x growth
     // candidate lists are ~2k long after the first rounds: small CTAs (more of them resident, cheaper barriers)
     constexpr int tighten_t = 64;
+    const auto tighten = grp ? k_tighten_cos<true> : k_tighten_cos<false>;
     BR_TRY(for_each_cos_launch(n_dt, warm_tiles, warm_cap, grow, [&](int t0, int nt) {
         CosArgs a{inv_nd, inv_nq, thr, (int32_t*)b_cnt.p, (int32_t*)b_cand.p, (float*)b_h.p, n_docs, nq, d, t0, t0 + nt,
-                  QS_WINDOW, fv.bits, fv.words, fv.row};
+                  QS_WINDOW, fv};
         if (use_qs) {
             const int64_t units = (int64_t)nt * ((nq + QS_BN - 1) / QS_BN);
             const int grid = 2 * (int)std::min<int64_t>(units, kNumSMs / 2);
@@ -1416,21 +1356,13 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
             else k_cosine_gemm_mc<false><<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
         }
         BR_CUDA(cudaGetLastError());
-        if (grp)
-            k_tighten_cos_grouped<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p,
-                                                            (float*)b_h.p, grp->row_group, k, (int32_t*)b_ovf.p);
-        else
-            k_tighten_cos<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, k,
-                                               (int32_t*)b_ovf.p);
+        tighten<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, row_group, k,
+                                          (int32_t*)b_ovf.p);
         BR_CUDA(cudaGetLastError());
         return BR_OK;
     }));
-    if (grp)
-        k_cos_output_grouped<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p,
-                                                                                grp->row_group, nq, k, doc_base, out_ids, out_sims);
-    else
-        k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, nq, k,
-                                                                        doc_base, out_ids, out_sims);
+    k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, row_group,
+                                                                    nq, k, doc_base, out_ids, out_sims);
     BR_CUDA(cudaGetLastError());
     std::vector<int32_t> ovf(Q);
     int32_t h_fbad = 0;
@@ -1443,68 +1375,54 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     // gather kernel (same normalisation, ties by doc id) - slow (one pass over the embeddings per query) but exact.
     std::vector<int32_t> redo;
     for (int32_t q = 0; q < nq; ++q) if (ovf[(size_t)q]) redo.push_back(q);
-    if (!redo.empty()) {
-        // Any number of such queries: sub-batches of at most 64 bound the scratch (4 B x 64 x n_docs candidate ids).
-        // This also covers a corpus whose row order correlates with the queries (every launch then passes far more
-        // than COS_CAP rows above the threshold learnt on the rows before it).
-        BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED,
-                   fn + ": candidate overflow (more than 1024 rows at or above a query's running threshold in one "
-                   "launch) needs the exact gather pass, which supports d <= 1024");
-        const int32_t sub = 64;
-        AsyncBuf b_q(st), b_c(st), b_oi(st), b_os(st), b_rows(st);
-        const int32_t nr_max = (int32_t)std::min<size_t>(redo.size(), (size_t)sub);
-        BR_TRY(b_q.alloc((size_t)nr_max * d * 2)); BR_TRY(b_c.alloc(4 * (size_t)nr_max * (size_t)n_docs));
-        BR_TRY(b_oi.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_os.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_rows.alloc(4 * (size_t)nr_max));
-        if (!filt) {
-            k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr_max, n_docs);
-            BR_CUDA(cudaGetLastError());
-        }
-        // grouped: every row's cosine [nr, n_docs], the segmented max over each group's run [nr, n_groups], then the top
-        // k groups by (score desc, group asc); empty groups and groups without an allowed row are empty slots
-        AsyncBuf b_gi(st), b_s(st), b_goff(st), b_gid(st), b_gsc(st), b_qoff(st), b_o64(st);
-        if (grp) {
-            const size_t G = (size_t)grp->n_groups;
-            BR_TRY(b_gi.alloc(4 * (size_t)nr_max)); BR_TRY(b_s.alloc(4 * (size_t)nr_max * (size_t)n_docs));
-            BR_TRY(b_goff.alloc(4 * (G + 1))); BR_TRY(b_gid.alloc(4 * (size_t)nr_max * G)); BR_TRY(b_gsc.alloc(8 * (size_t)nr_max * G));
-            BR_TRY(b_qoff.alloc(8 * ((size_t)nr_max + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nr_max * k));
-            k_group_offsets<<<blocks_for((int64_t)G + 1, 256), 256, 0, st>>>(grp->row_group, n_docs, grp->n_groups, (int32_t*)b_goff.p);
-            BR_CUDA(cudaGetLastError());
-            std::vector<int64_t> qoff((size_t)nr_max + 1);
-            for (int32_t r = 0; r <= nr_max; ++r) qoff[(size_t)r] = (int64_t)r * (int64_t)G;
-            BR_CUDA(cudaMemcpyAsync(b_qoff.p, qoff.data(), 8 * qoff.size(), cudaMemcpyHostToDevice, st));
-            BR_CUDA(cudaStreamSynchronize(st));               // qoff is a local
-        }
-        for (size_t r0 = 0; r0 < redo.size(); r0 += (size_t)sub) {
-            const int32_t nr = (int32_t)std::min<size_t>((size_t)sub, redo.size() - r0);
-            for (int32_t i = 0; i < nr; ++i)
-                BR_CUDA(cudaMemcpyAsync((char*)b_q.p + (size_t)i * d * 2, (const char*)queries + (size_t)redo[r0 + (size_t)i] * d * 2,
-                                        (size_t)d * 2, cudaMemcpyDeviceToDevice, st));
-            BR_CUDA(cudaMemcpyAsync(b_rows.p, redo.data() + r0, 4 * (size_t)nr, cudaMemcpyHostToDevice, st));
-            if (filt) {                                   // each redone query gathers only the rows it may return
-                k_iota_rows_filtered<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr, n_docs, (const int32_t*)b_rows.p, fv);
-                BR_CUDA(cudaGetLastError());
-            }
-            if (grp) {
-                BR_TRY(row_inv_norms(b_q.p, nr, d, (float*)b_gi.p, st));
-                BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, b_q.p, (const float*)b_gi.p, nr, (const int32_t*)b_c.p,
-                                         (int32_t)n_docs, (float*)b_s.p, nullptr, st));
-                k_group_max<<<kNumSMs * 8, 256, 0, st>>>((const float*)b_s.p, nr, n_docs, (const int32_t*)b_goff.p, grp->n_groups,
-                                                         (int32_t*)b_gid.p, (double*)b_gsc.p);
-                BR_CUDA(cudaGetLastError());
-                BR_TRY(launch_final_select((const int32_t*)b_gid.p, (const double*)b_gsc.p, (const int64_t*)b_qoff.p, 0, nr, k, 0,
-                                           (int32_t*)b_oi.p, (double*)b_o64.p, nullptr, st));
-                k_rerank_output<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_oi.p, (const double*)b_o64.p,
-                                                                                  (int64_t)nr * k, (float*)b_os.p);
-                BR_CUDA(cudaGetLastError());
-            } else {
-                BR_TRY(cosine_rerank(docs, inv_nd, n_docs, d, b_q.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs, k, (int32_t*)b_oi.p,
-                                     (float*)b_os.p, st));         // synchronises: b_rows / b_q may be reused afterwards
-            }
-            k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_rows.p, nr, k, (const int32_t*)b_oi.p,
-                                                                          (const float*)b_os.p, doc_base, out_ids, out_sims);
-            BR_CUDA(cudaGetLastError());
-            BR_CUDA(cudaStreamSynchronize(st));
-        }
+    if (redo.empty()) return BR_OK;
+    // Any number of such queries: sub-batches of at most 64 bound the scratch (4 B x 64 x n_docs candidate ids).
+    // This also covers a corpus whose row order correlates with the queries (every launch then passes far more
+    // than COS_CAP rows above the threshold learnt on the rows before it).
+    BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED,
+               fn + ": candidate overflow (more than 1024 rows at or above a query's running threshold in one "
+               "launch) needs the exact gather pass, which supports d <= 1024");
+    // Per sub-batch: every row's cosine [nr, n_docs] over the list of all rows (of the allowed rows, filtered), then per
+    // (query, id) a float64 score and the re-rank's selection.  The ids are the rows, or for a grouped call the groups
+    // [nr, n_groups] with the best of their rows' cosines (a group without rows, or without an allowed row, is an empty
+    // slot).
+    const int32_t sub = 64;
+    const int32_t nr_max = (int32_t)std::min<size_t>(redo.size(), (size_t)sub);
+    const int32_t c = grp ? grp->n_groups : (int32_t)n_docs;   // ids per redone query
+    AsyncBuf b_q(st), b_inr(st), b_rows(st), b_c(st), b_s(st), b_id(st), b_s64(st), b_goff(st), b_oi(st), b_os(st);
+    BR_TRY(b_q.alloc((size_t)nr_max * d * 2)); BR_TRY(b_inr.alloc(4 * (size_t)nr_max)); BR_TRY(b_rows.alloc(4 * (size_t)nr_max));
+    BR_TRY(b_c.alloc(4 * (size_t)nr_max * (size_t)n_docs)); BR_TRY(b_s.alloc(4 * (size_t)nr_max * (size_t)n_docs));
+    BR_TRY(b_s64.alloc(8 * (size_t)nr_max * (size_t)c));
+    BR_TRY(b_oi.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_os.alloc(4 * (size_t)nr_max * k));
+    if (grp) {
+        BR_TRY(b_id.alloc(4 * (size_t)nr_max * (size_t)c)); BR_TRY(b_goff.alloc(4 * ((size_t)c + 1)));
+        k_group_offsets<<<blocks_for((int64_t)c + 1, 256), 256, 0, st>>>(row_group, n_docs, c, (int32_t*)b_goff.p);
+        BR_CUDA(cudaGetLastError());
+    }
+    const int32_t* ids = grp ? (const int32_t*)b_id.p : (const int32_t*)b_c.p;
+    for (size_t r0 = 0; r0 < redo.size(); r0 += (size_t)sub) {
+        const int32_t nr = (int32_t)std::min<size_t>((size_t)sub, redo.size() - r0);
+        for (int32_t i = 0; i < nr; ++i)
+            BR_CUDA(cudaMemcpyAsync((char*)b_q.p + (size_t)i * d * 2, (const char*)queries + (size_t)redo[r0 + (size_t)i] * d * 2,
+                                    (size_t)d * 2, cudaMemcpyDeviceToDevice, st));
+        BR_CUDA(cudaMemcpyAsync(b_rows.p, redo.data() + r0, 4 * (size_t)nr, cudaMemcpyHostToDevice, st));
+        BR_TRY(row_inv_norms(b_q.p, nr, d, (float*)b_inr.p, st));
+        k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr, n_docs, (const int32_t*)b_rows.p, fv);
+        BR_CUDA(cudaGetLastError());
+        BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, b_q.p, (const float*)b_inr.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs,
+                                 (float*)b_s.p, nullptr, st));
+        if (grp)
+            k_group_max<<<kNumSMs * 8, 256, 0, st>>>((const float*)b_s.p, nr, n_docs, (const int32_t*)b_goff.p, c, (int32_t*)b_id.p,
+                                                     (double*)b_s64.p);
+        else
+            k_f32_to_f64<<<blocks_for((int64_t)nr * n_docs, 256), 256, 0, st>>>((const float*)b_s.p, (int64_t)nr * n_docs,
+                                                                               (double*)b_s64.p);
+        BR_CUDA(cudaGetLastError());
+        BR_TRY(select_fixed(ids, (const double*)b_s64.p, nr, c, k, (int32_t*)b_oi.p, (float*)b_os.p, st));
+        k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_rows.p, nr, k, (const int32_t*)b_oi.p,
+                                                                      (const float*)b_os.p, doc_base, out_ids, out_sims);
+        BR_CUDA(cudaGetLastError());
+        BR_CUDA(cudaStreamSynchronize(st));               // the next sub-batch rewrites b_q and b_rows
     }
     return BR_OK;
 }
@@ -1516,22 +1434,15 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim must be a multiple of 8");
     if (nq == 0) return BR_OK;
     const int64_t n_pairs = (int64_t)nq * c;
-    AsyncBuf b_inq(st), b_s(st), b_s64(st), b_off(st), b_o64(st);
+    AsyncBuf b_inq(st), b_s(st), b_s64(st);
     BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_s.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
-    BR_TRY(b_off.alloc(8 * ((size_t)nq + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
     int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_docs)
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
     BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
     BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, (const float*)b_inq.p, nq, cand, c, (float*)b_s.p, bad, st));
     k_f32_to_f64<<<blocks_for(n_pairs, 256), 256, 0, st>>>((const float*)b_s.p, n_pairs, (double*)b_s64.p);
     BR_CUDA(cudaGetLastError());
-    std::vector<int64_t> off((size_t)nq + 1);
-    for (int32_t q = 0; q <= nq; ++q) off[(size_t)q] = (int64_t)q * c;
-    BR_CUDA(cudaMemcpyAsync(b_off.p, off.data(), 8 * ((size_t)nq + 1), cudaMemcpyHostToDevice, st));
-    BR_TRY(launch_final_select(cand, (const double*)b_s64.p, (const int64_t*)b_off.p, 0, nq, k, 0, out_ids, (double*)b_o64.p,
-                               nullptr, st));
-    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
-    BR_CUDA(cudaGetLastError());
+    BR_TRY(select_fixed(cand, (const double*)b_s64.p, nq, c, k, out_ids, out_sims, st));
     int32_t h_bad = 0;
     BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
@@ -1550,26 +1461,16 @@ int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows,
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, fn + ": embedding dim must be a multiple of 8");
     BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, fn + ": embedding dim > 1024");
     if (nq == 0) return BR_OK;
-    // the layout, checked before anything reads a row through it
-    const int32_t n_blk = (int32_t)((n_rows + GC_ROWS - 1) / GC_ROWS);
-    AsyncBuf b_lay(st), b_off(st);
-    BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 16));
-    int32_t* info = (int32_t*)b_lay.p + n_blk;
-    BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
-    k_group_check<<<n_blk, 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_lay.p, info);
-    BR_CUDA(cudaGetLastError());
-    int32_t h_info = 0;
-    BR_CUDA(cudaMemcpyAsync(&h_info, info, 4, cudaMemcpyDeviceToHost, st));
-    BR_CUDA(cudaStreamSynchronize(st));
-    BR_REQUIRE(!h_info, BR_ERR_INVALID, fn + ": row_group must be non-decreasing with values in [0, n_groups)");
+    int64_t r_k, n_nonempty;                               // not used here
+    BR_TRY(check_row_group(row_group, n_rows, n_groups, k, fn, st, &r_k, &n_nonempty));
+    AsyncBuf b_off(st);
     BR_TRY(b_off.alloc(4 * ((size_t)n_groups + 1)));
     k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_off.p);
     BR_CUDA(cudaGetLastError());
-    // per candidate (group or -1, best cosine), then the same selection and output as cosine_rerank
+    // per candidate (group or -1, best cosine), then the same selection as cosine_rerank
     const int64_t n_pairs = (int64_t)nq * c;
-    AsyncBuf b_inq(st), b_id(st), b_s64(st), b_qoff(st), b_o64(st);
+    AsyncBuf b_inq(st), b_id(st), b_s64(st);
     BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_id.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
-    BR_TRY(b_qoff.alloc(8 * ((size_t)nq + 1))); BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
     int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_groups)
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
     BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
@@ -1584,13 +1485,7 @@ int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows,
     else if (nv == 3) launch(k_cosine_rerank_grouped<3>);
     else launch(k_cosine_rerank_grouped<4>);
     BR_CUDA(cudaGetLastError());
-    std::vector<int64_t> qoff((size_t)nq + 1);
-    for (int32_t q = 0; q <= nq; ++q) qoff[(size_t)q] = (int64_t)q * c;
-    BR_CUDA(cudaMemcpyAsync(b_qoff.p, qoff.data(), 8 * ((size_t)nq + 1), cudaMemcpyHostToDevice, st));
-    BR_TRY(launch_final_select((const int32_t*)b_id.p, (const double*)b_s64.p, (const int64_t*)b_qoff.p, 0, nq, k, 0, out_ids,
-                               (double*)b_o64.p, nullptr, st));
-    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
-    BR_CUDA(cudaGetLastError());
+    BR_TRY(select_fixed((const int32_t*)b_id.p, (const double*)b_s64.p, nq, c, k, out_ids, out_sims, st));
     int32_t h_bad = 0;
     BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));

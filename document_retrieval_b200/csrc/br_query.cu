@@ -660,9 +660,9 @@ int launch_rescore_heads(br_index* ix, const int32_t* q_off, const PrepView& pv,
 
 int launch_final_select(const int32_t* cand, const double* cand_score, const int64_t* cand_off, int32_t q_begin,
                         int32_t nq, int32_t k, int positive_only, int32_t* out_ids, double* out_scores,
-                        int32_t* out_counts, cudaStream_t st, const int32_t* cnt_hint) {
-    k_final_select<int32_t><<<nq, FS_T, 0, st>>>(cand, cand_score, cand_off, q_begin, 1, 0, 0, k, 0, positive_only, out_ids,
-                                                 out_scores, out_counts, cnt_hint);
+                        int32_t* out_counts, cudaStream_t st, const int32_t* cnt_hint, int32_t fixed_cnt) {
+    k_final_select<int32_t><<<nq, FS_T, 0, st>>>(cand, cand_score, cand_off, q_begin, 1, 0, fixed_cnt, k, 0, positive_only,
+                                                 out_ids, out_scores, out_counts, cnt_hint);
     BR_CUDA(cudaGetLastError());
     return BR_OK;
 }
@@ -794,9 +794,15 @@ __global__ void k_pack_records(const int32_t* __restrict__ ids, const double* __
     out[i] = br_record{d >= 0 ? (int64_t)d + doc_base : (int64_t)-1, sc[i]};
 }
 
-// Filter rows of a batch (br_doc_filter::query_row_dev, NULL = row 0 for every query), validated on the device: a value
-// outside [-1, n_rows) sets *bad (reported when the call returns) and becomes -1, so no kernel ever addresses a row that
-// does not exist.
+int check_doc_filter(const br_doc_filter* filter, int64_t n_ids, const char* ids, const std::string& fn) {
+    if (!filter) return BR_OK;
+    BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, fn + ": filter bitmap is null");
+    BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, fn + ": filter n_rows must be >= 1");
+    BR_REQUIRE(filter->words >= (n_ids + 31) / 32, BR_ERR_INVALID, fn + ": filter words < ceil(" + ids + " / 32)");
+    return BR_OK;
+}
+
+// *bad is reported when the call returns; the -1 for a bad value means no kernel ever addresses a row that does not exist.
 __global__ void k_filter_rows(const int32_t* __restrict__ in, int32_t nq, int32_t n_rows, int32_t* __restrict__ out,
                               int32_t* __restrict__ bad) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -908,11 +914,7 @@ int topk_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32
     BR_REQUIRE(ix->finalized, BR_ERR_STATE, "br_topk_batch: call br_index_finalize first");
     BR_REQUIRE(k >= 1 && k <= BR_MAX_K, BR_ERR_INVALID, "br_topk_batch: k must be in [1, BR_MAX_K]");
     BR_REQUIRE(nq >= 0, BR_ERR_INVALID, "br_topk_batch: nq < 0");
-    if (filter) {
-        BR_REQUIRE(filter->bits_dev, BR_ERR_INVALID, "br_topk_batch: filter bitmap is null");
-        BR_REQUIRE(filter->n_rows >= 1, BR_ERR_INVALID, "br_topk_batch: filter n_rows must be >= 1");
-        BR_REQUIRE(filter->words >= (ix->n_docs + 31) / 32, BR_ERR_INVALID, "br_topk_batch: filter words < ceil(n_docs / 32)");
-    }
+    BR_TRY(check_doc_filter(filter, ix->n_docs, "n_docs", "br_topk_batch"));
     if (nq == 0) return BR_OK;
     BR_CUDA(cudaSetDevice(ix->device));
     ix->stats = br_query_stats{};
