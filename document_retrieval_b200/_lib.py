@@ -53,6 +53,10 @@ SIGNATURES = {
     "br_cosine_rerank": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "br_cosine_rerank_grouped": (C.c_int, [_P, _P, C.c_int64, C.c_int32, _P, C.c_int32, _P, C.c_int32, _P, C.c_int32, C.c_int32,
                                            _P, _P, _P]),
+    "br_fuse_rrf": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int64, C.c_int32, C.c_double, C.c_double, C.c_double,
+                              C.c_int32, _P, _P, _P, _P]),
+    "br_fuse_linear": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int, _P, _P, C.c_int64, C.c_int32, _P, _P, _P,
+                                 C.c_int32, _P, C.c_int32, C.c_double, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "br_dedupe_first_docs": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
     "br_set_thr_exchange": (C.c_int, [_P, _P, _P, C.c_int, C.c_int]),
     "br_tile_launch_count": (C.c_int, [_P, C.c_int32]),

@@ -95,6 +95,16 @@ inline int scratch_alloc(void** p, size_t bytes, cudaStream_t st) {
     BR_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 1, pool, st));
     return BR_OK;
 }
+struct AsyncBuf {   // stream-ordered scratch
+    void* p = nullptr;
+    cudaStream_t st;
+    explicit AsyncBuf(cudaStream_t s) : st(s) {}
+    int alloc(size_t bytes) {
+        BR_TRY(scratch_alloc(&p, bytes, st));
+        return BR_OK;
+    }
+    ~AsyncBuf() { if (p) cudaFreeAsync(p, st); }
+};
 
 constexpr int kNumSMs = 148;          // B200
 constexpr float kBandRel = 1e-5f;     // fp32 candidate band kept below the k-th fp32 score (see DESIGN.md)

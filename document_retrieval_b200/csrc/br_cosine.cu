@@ -1109,17 +1109,6 @@ static int make_map(CUtensorMap* m, const void* ptr, int64_t rows, int32_t d, in
     return BR_OK;
 }
 
-struct AsyncBuf {   // stream-ordered scratch
-    void* p = nullptr;
-    cudaStream_t st;
-    explicit AsyncBuf(cudaStream_t s) : st(s) {}
-    int alloc(size_t bytes) {
-        BR_TRY(scratch_alloc(&p, bytes, st));
-        return BR_OK;
-    }
-    ~AsyncBuf() { if (p) cudaFreeAsync(p, st); }
-};
-
 int row_inv_norms(const void* emb, int64_t n, int32_t d, float* out, cudaStream_t st) {
     BR_REQUIRE(emb && out && n >= 0 && d > 0, BR_ERR_INVALID, "br_row_inv_norms: bad arguments");
     if (n == 0) return BR_OK;
@@ -1185,9 +1174,9 @@ static int for_each_cos_launch(int n_dt, int warm_tiles, int warm_cap, double gr
 
 // the gather kernel over explicit candidate rows cand[q, 0..c) -> out[q, c] fp32 cosines (-inf for an empty slot);
 // bad (may be NULL) is set when an id is outside [-1, n_docs)
-static int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries,
-                             const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, int32_t* bad,
-                             cudaStream_t st) {
+int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries,
+                      const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, int32_t* bad,
+                      cudaStream_t st) {
     BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim > 1024");
     const int nv = (d / 8 + 31) / 32;
     auto launch = [&](auto kern) {
@@ -1450,6 +1439,29 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
     return BR_OK;
 }
 
+int launch_cos_gather_grouped(const void* docs, const float* inv_nd, int64_t n_rows, int32_t d, const int32_t* row_group,
+                              int32_t n_groups, const void* queries, const float* inv_nq, int32_t nq, const int32_t* cand,
+                              int32_t c, int32_t* out_ids, double* out_s64, int32_t* bad, const std::string& fn,
+                              cudaStream_t st) {
+    int64_t r_k, n_nonempty;                               // not used here
+    BR_TRY(check_row_group(row_group, n_rows, n_groups, 1, fn, st, &r_k, &n_nonempty));
+    AsyncBuf b_off(st);
+    BR_TRY(b_off.alloc(4 * ((size_t)n_groups + 1)));
+    k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_off.p);
+    BR_CUDA(cudaGetLastError());
+    const int nv = (d / 8 + 31) / 32;
+    auto launch = [&](auto kern) {
+        kern<<<nq, RG_T, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, d, (const int32_t*)b_off.p, n_groups,
+                                  (const __nv_bfloat16*)queries, inv_nq, cand, c, out_ids, out_s64, bad);
+    };
+    if (nv <= 1) launch(k_cosine_rerank_grouped<1>);
+    else if (nv == 2) launch(k_cosine_rerank_grouped<2>);
+    else if (nv == 3) launch(k_cosine_rerank_grouped<3>);
+    else launch(k_cosine_rerank_grouped<4>);
+    BR_CUDA(cudaGetLastError());
+    return BR_OK;
+}
+
 int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows, int32_t d, const int32_t* row_group,
                           int32_t n_groups, const void* queries, int32_t nq, const int32_t* cand, int32_t c, int32_t k,
                           int32_t* out_ids, float* out_sims, cudaStream_t st) {
@@ -1461,12 +1473,6 @@ int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows,
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, fn + ": embedding dim must be a multiple of 8");
     BR_REQUIRE(d <= 1024, BR_ERR_UNSUPPORTED, fn + ": embedding dim > 1024");
     if (nq == 0) return BR_OK;
-    int64_t r_k, n_nonempty;                               // not used here
-    BR_TRY(check_row_group(row_group, n_rows, n_groups, k, fn, st, &r_k, &n_nonempty));
-    AsyncBuf b_off(st);
-    BR_TRY(b_off.alloc(4 * ((size_t)n_groups + 1)));
-    k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_off.p);
-    BR_CUDA(cudaGetLastError());
     // per candidate (group or -1, best cosine), then the same selection as cosine_rerank
     const int64_t n_pairs = (int64_t)nq * c;
     AsyncBuf b_inq(st), b_id(st), b_s64(st);
@@ -1474,17 +1480,8 @@ int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows,
     int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_groups)
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
     BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
-    const int nv = (d / 8 + 31) / 32;
-    auto launch = [&](auto kern) {
-        kern<<<nq, RG_T, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, d, (const int32_t*)b_off.p, n_groups,
-                                  (const __nv_bfloat16*)queries, (const float*)b_inq.p, cand, c, (int32_t*)b_id.p,
-                                  (double*)b_s64.p, bad);
-    };
-    if (nv <= 1) launch(k_cosine_rerank_grouped<1>);
-    else if (nv == 2) launch(k_cosine_rerank_grouped<2>);
-    else if (nv == 3) launch(k_cosine_rerank_grouped<3>);
-    else launch(k_cosine_rerank_grouped<4>);
-    BR_CUDA(cudaGetLastError());
+    BR_TRY(launch_cos_gather_grouped(docs, inv_nd, n_rows, d, row_group, n_groups, queries, (const float*)b_inq.p, nq, cand, c,
+                                     (int32_t*)b_id.p, (double*)b_s64.p, bad, fn, st));
     BR_TRY(select_fixed((const int32_t*)b_id.p, (const double*)b_s64.p, nq, c, k, out_ids, out_sims, st));
     int32_t h_bad = 0;
     BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));

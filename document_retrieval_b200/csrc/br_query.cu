@@ -667,8 +667,8 @@ int launch_final_select(const int32_t* cand, const double* cand_score, const int
     return BR_OK;
 }
 // n_terms >= 0: the caller knows q_offsets[nq] (or an upper bound) - no device read, no stream synchronisation.
-static int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int dedup,
-                        cudaStream_t st, PrepView* pv, int64_t** chunk_start, int32_t* total_terms, int32_t n_terms = -1) {
+int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int dedup, cudaStream_t st,
+                 PrepView* pv, int64_t** chunk_start, int32_t* total_terms, int32_t n_terms) {
     int32_t T = n_terms;
     if (T < 0) {
         BR_CUDA(cudaMemcpyAsync(&T, q_off + nq, sizeof(int32_t), cudaMemcpyDeviceToHost, st));

@@ -1,5 +1,5 @@
 // br_query.cuh - declarations shared by br_query.cu (dense path, re-score, final select, doc filters) with
-// br_tile.cu (fused tiled path) and br_cosine.cu (dense cosine).
+// br_tile.cu (fused tiled path), br_cosine.cu (dense cosine) and br_hybrid.cu (BM25 + dense fusion).
 #pragma once
 #include "br_common.cuh"
 
@@ -21,6 +21,9 @@ struct PrepView {
 };
 
 
+// The query preparation of br_topk_batch (k_prep_queries into ix->ws_prep); n_terms < 0: read q_offsets[nq] back.
+int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int dedup, cudaStream_t st,
+                 PrepView* pv, int64_t** chunk_start, int32_t* total_terms, int32_t n_terms = -1);
 int launch_rescore(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, const int64_t* cand_off,
                    int32_t q_begin, int32_t nq, const int32_t* cand, double* cand_score, int64_t total, cudaStream_t st);
 int launch_rescore_heads(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, int32_t nq, int32_t stride,
@@ -42,5 +45,20 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
                int positive_only, int32_t* out_ids, double* out_scores, int32_t* out_counts, cudaStream_t st,
                std::vector<int32_t>* h_flags, bool long_pass = false, const br_posting* post_table = nullptr,
                const DocFilter* filt = nullptr);
+
+// br_cosine.cu: the gather kernels of br_cosine_rerank / br_cosine_rerank_grouped over fixed-stride candidate lists
+// cand[q, 0..c) (-1 = empty slot), for callers that need the per-candidate cosines rather than a selection.
+int row_inv_norms(const void* emb, int64_t n, int32_t d, float* out, cudaStream_t st);
+// out[q, c] fp32 cosines (-inf for an empty slot); bad (may be NULL) is set when an id is outside [-1, n_docs).  d <= 1024.
+int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d, const void* queries,
+                      const float* inv_nq, int32_t nq, const int32_t* cand, int32_t c, float* out, int32_t* bad,
+                      cudaStream_t st);
+// Checks the row_group layout (failing the call `fn`), then per candidate: out_ids = its group, -1 for an empty slot, a
+// group without rows or an id outside [-1, n_groups) (which sets *bad); out_s64 = the group's best cosine, widened
+// (0.0 without rows).  d <= 1024.
+int launch_cos_gather_grouped(const void* docs, const float* inv_nd, int64_t n_rows, int32_t d, const int32_t* row_group,
+                              int32_t n_groups, const void* queries, const float* inv_nq, int32_t nq, const int32_t* cand,
+                              int32_t c, int32_t* out_ids, double* out_s64, int32_t* bad, const std::string& fn,
+                              cudaStream_t st);
 
 }  // namespace br

@@ -296,6 +296,41 @@ int br_cosine_rerank_grouped(const void* docs_bf16_dev, const float* doc_inv_nor
                              const int32_t* cand_groups_dev, int32_t c, int32_t k, int32_t* out_ids_dev,
                              float* out_sims_dev, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Hybrid retrieval: one ranking from a BM25 candidate list and a dense cosine candidate list per query.
+ * bm25_ids_dev int32[nq, nb] and dense_ids_dev int32[nq, nd] hold LOCAL doc ids of the BM25 index, -1 = an empty slot
+ * (anywhere in a list).  A doc's rank in a list is 1 + the slot of its first occurrence; later repeats are ignored and
+ * empty slots do not renumber the slots after them.  The union is the set of distinct valid ids of both lists.
+ * 0 <= nb, nd <= BR_MAX_K, nb + nd >= 1, 1 <= k <= BR_MAX_K.  Outputs [nq, k]: the top k union members by (fused score
+ * desc, doc id asc), out_ids_dev int32 (-1 pads when the union has fewer than k members), out_scores_dev double (0.0
+ * pads), out_counts_dev int32[nq] = valid entries (may be NULL).  An id outside [-1, n_docs) is BR_ERR_INVALID: it is
+ * detected on the device and never used to address anything.  nq = 0 returns at once (lists and outputs may then be
+ * NULL).  Both calls synchronise `stream`.
+ * ------------------------------------------------------------------------------------------- */
+/* Reciprocal rank fusion: f(d) = w_bm25 / (rrf_c + r_b(d)) + w_dense / (rrf_c + r_d(d)), a term omitted when d is not in
+ * that list; float64, one correctly rounded division per term and one addition (a numpy restatement gives the same
+ * bits).  rrf_c >= 0 (60 is usual), w_bm25, w_dense >= 0 and not both 0, all finite; BR_ERR_INVALID otherwise. */
+int br_fuse_rrf(const int32_t* bm25_ids_dev, int32_t nb, const int32_t* dense_ids_dev, int32_t nd, int64_t n_docs,
+                int32_t nq, double rrf_c, double w_bm25, double w_dense, int32_t k, int32_t* out_ids_dev,
+                double* out_scores_dev, int32_t* out_counts_dev, void* stream);
+/* Linear fusion of min-max-normalised exact scores: f = alpha * n_b + (1 - alpha) * n_c, alpha in [0, 1].
+ *   s_b(d): float64 BM25 of d for the query (q_terms_dev / q_offsets_dev / n_terms / dedup as in br_topk_batch),
+ *           bit-identical to br_rescore_docs and to the scores br_topk_batch returns; 0.0 when no query term matches.
+ *   s_c(d): fp32 cosine, bit-identical to br_cosine_rerank for row d (row_group_dev == NULL: row = doc, and n_rows must
+ *           equal the index's n_docs), or to br_cosine_rerank_grouped for group d (row_group_dev as there, with the
+ *           index's docs as the groups: n_groups = n_docs); a doc without rows has no cosine.  doc_inv_norm_dev from
+ *           br_row_inv_norms; d a multiple of 8 and <= 1024, BR_ERR_UNSUPPORTED otherwise.
+ *   Per query over the union: n_b = (s_b - min_b) / (max_b - min_b); n_c = ((double)s_c - min_c) / (max_c - min_c) over
+ *   the members with a cosine, 0.0 for a doc without rows; a normalised value is 0.0 when max == min.  (1 - alpha) is
+ *   formed once; every operation is one float64 rounding, no contraction.
+ * out_bm25_dev double[nq, k] = s_b and out_cos_dev float[nq, k] = s_c of each returned doc (NaN: no rows; 0 pads); both
+ * may be NULL.  The row_group layout is checked as in the grouped calls. */
+int br_fuse_linear(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev, int32_t nq, int32_t n_terms,
+                   int dedup, const void* docs_bf16_dev, const float* doc_inv_norm_dev, int64_t n_rows, int32_t d,
+                   const int32_t* row_group_dev, const void* queries_bf16_dev, const int32_t* bm25_ids_dev, int32_t nb,
+                   const int32_t* dense_ids_dev, int32_t nd, double alpha, int32_t k, int32_t* out_ids_dev,
+                   double* out_scores_dev, double* out_bm25_dev, float* out_cos_dev, int32_t* out_counts_dev, void* stream);
+
 /* Sentence -> document step of the sentence-level retrieval (team_run1.py:286-294): for every query walk its ranked
  * sentences sentence_ids_dev int64[nq, n] (best first, -1 = padding), map each to its parent doc through
  * sentence_to_doc_dev int32[n_sentences], keep the first occurrence of every doc and stop at k docs (k <= 32; the
