@@ -268,9 +268,8 @@ int fuse_linear(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
     // BM25: br_topk_batch's query preparation and float64 re-score over the union
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
-    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, &T, n_terms));
-    BR_TRY(launch_rescore_heads(ix, q_off, pv, dedup, nq, W, u_cnt, u_ids, s_b, st));
+    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, n_terms));
+    BR_TRY(launch_rescore_heads(ix, Formula::BM25, q_off, pv, dedup, nq, W, u_cnt, u_ids, s_b, st));
     // cosine: the re-rank gather over the union
     BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
     const int32_t* g_ids = nullptr;

@@ -7,8 +7,12 @@
 //   k_select_radix   per query row: exact k-th largest fp32 score by 3-pass radix select, then the
 //                    candidate band  s >= kth - 1e-5*|kth|   (retrieve_top_n, :206-213)
 //   k_emit_cands     band members -> candidate list (doc-id order; zero-score tail in doc-id order)
-//   k_rescore        exact float64 re-evaluation of the reference formula for every candidate
+//   k_rescore<F>     exact float64 re-evaluation of formula F (BM25, TF-IDF cosine, V3 re-rank) for every candidate,
+//                    candidates in per-query ranges cand_off (dense path, br_rescore_docs, br_rerank_v3_scores)
+//   k_rescore_heads<F>  the same over fixed-stride per-query regions with a live count, one CTA per query (tiled
+//                    path, br_fuse_linear)
 //   k_final_select   (score64 desc, doc id asc) order, top-k, duplicate ids removed
+// k_select_radix, k_emit_cands and the tiled path's k_seed_thr take a doc filter; a null row table means unfiltered.
 //
 // Why a band + float64 re-score: the reference ranks float64 scores; fp32 accumulation can swap
 // near-ties.  Every doc outside the band has fp32 score < kth32*(1-1e-5), hence (fp32 error of a
@@ -157,11 +161,13 @@ struct SelView {
 
 constexpr int SEL_T = 1024;
 
-// FILT: a doc the query's filter row excludes gets key 0, below every allowed doc, so kth_key == 0 means "fewer than k
+// A doc the query's filter row excludes gets key 0, below every allowed doc, so kth_key == 0 means "fewer than k
 // allowed docs (with a hit, for positive_only)": mode 2 then takes every allowed doc (with a hit).  Disallowed docs are
-// neither counted nor emitted, so the zero-score tail of mode 1 is made of allowed docs in doc-id order.
-template <bool FILT>
-__global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict__ scores, int64_t n_docs, int32_t k,
+// neither counted nor emitted, so the zero-score tail of mode 1 is made of allowed docs in doc-id order.  Unfiltered,
+// kth_key == 0 needs positive_only: without it no non-NaN score has key 0, and k_rem <= n_docs makes the k-th key a
+// doc's own key.  Two CTAs per SM (at most 32 registers): the filter test must not halve the occupancy of the unfiltered
+// select.
+__global__ void __launch_bounds__(SEL_T, 2) k_select_radix(const float* __restrict__ scores, int64_t n_docs, int32_t k,
                                                         int positive_only, SelView sv, int32_t q_begin,
                                                         const int32_t* __restrict__ n_terms, DocFilter f) {
     __shared__ uint32_t hist[2048];
@@ -169,20 +175,16 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     __shared__ unsigned long long s_cnt[2];
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
-    const uint32_t* fr = nullptr;
-    if constexpr (FILT) fr = f.row_of(q);
+    const uint32_t* fr = f.row ? f.row_of(q) : nullptr;
     uint32_t prefix = 0, mask = 0;
     uint32_t k_rem = (uint32_t)min((int64_t)k, n_docs);
-    const int shifts[3] = {21, 10, 0};
-    const int widths[3] = {11, 11, 10};
 #pragma unroll 1
     for (int pass = 0; pass < 3; ++pass) {
-        const int shift = shifts[pass], nb = 1 << widths[pass];
+        const int shift = pass == 0 ? 21 : pass == 1 ? 10 : 0, nb = pass == 2 ? 1024 : 2048;
         for (int i = threadIdx.x; i < 2048; i += SEL_T) hist[i] = 0;
         __syncthreads();
         for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
-            uint32_t u = score_key(row[i], positive_only);
-            if constexpr (FILT) u = doc_allowed(fr, (uint32_t)i) ? u : 0u;
+            const uint32_t u = doc_allowed(fr, (uint32_t)i) ? score_key(row[i], positive_only) : 0u;
             if ((u & mask) == prefix) atomicAdd(&hist[(u >> shift) & (nb - 1)], 1u);
         }
         __syncthreads();
@@ -203,10 +205,8 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     const uint32_t kth_key = prefix;
     int mode = 0;
     float lo = 0.f;
-    bool take_all = positive_only && kth_key == 0u;
-    if constexpr (FILT) take_all = kth_key == 0u;  // fewer than k allowed docs (with a hit): take them all
-    if (take_all) {
-        mode = 2;                                   // fewer than k docs with a hit: take them all
+    if (kth_key == 0u) {
+        mode = 2;                                   // fewer than k allowed docs with a hit: take them all
     } else {
         const float kth = key_score(kth_key);
         if (!positive_only && kth == 0.0f) mode = 1; // fewer than k positive docs: zero tail in doc order
@@ -219,16 +219,10 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     unsigned long long c_band = 0, c_pos = 0;
     for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
         const float s = row[i];
-        if constexpr (FILT) {
-            const bool ok = doc_allowed(fr, (uint32_t)i);
-            if (mode == 2) c_band += (ok && (!positive_only || s != 0.0f));
-            else if (mode == 1) c_pos += (ok && s > 0.0f);
-            else c_band += (ok && s >= lo && !(positive_only && s == 0.0f));
-        } else {
-            if (mode == 2) c_band += (s != 0.0f);
-            else if (mode == 1) c_pos += (s > 0.0f);
-            else c_band += (s >= lo && !(positive_only && s == 0.0f));
-        }
+        const bool ok = doc_allowed(fr, (uint32_t)i);
+        if (mode == 2) c_band += (ok && (!positive_only || s != 0.0f));
+        else if (mode == 1) c_pos += (ok && s > 0.0f);
+        else c_band += (ok && s >= lo && !(positive_only && s == 0.0f));
     }
     for (int o = 16; o > 0; o >>= 1) {
         c_band += __shfl_xor_sync(0xffffffffu, c_band, o);
@@ -250,15 +244,13 @@ __global__ void __launch_bounds__(SEL_T) k_select_radix(const float* __restrict_
     }
 }
 
-template <bool FILT>
 __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ scores, int64_t n_docs,
                                                       int positive_only, SelView sv, int32_t q_begin,
                                                       const int64_t* __restrict__ cand_off, int32_t* __restrict__ cand,
                                                       DocFilter f) {
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
-    const uint32_t* fr = nullptr;
-    if constexpr (FILT) fr = f.row_of(q);
+    const uint32_t* fr = f.row ? f.row_of(q) : nullptr;
     const int mode = sv.mode[q];
     const float lo = sv.lo[q];
     const uint32_t zfill = (uint32_t)sv.zfill[q];
@@ -268,16 +260,10 @@ __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ 
         const int64_t i = base + threadIdx.x;
         const float s = i < n_docs ? row[i] : -CUDART_INF_F;
         bool take, zero = false;
-        if constexpr (FILT) {
-            const bool ok = i < n_docs && doc_allowed(fr, (uint32_t)i);
-            if (mode == 2) take = ok && (!positive_only || s != 0.0f);
-            else if (mode == 1) { take = ok && s > 0.0f; zero = ok && s == 0.0f; }
-            else take = ok && s >= lo && !(positive_only && s == 0.0f);
-        } else {
-            if (mode == 2) take = i < n_docs && s != 0.0f;
-            else if (mode == 1) { take = s > 0.0f; zero = i < n_docs && s == 0.0f; }
-            else take = i < n_docs && s >= lo && !(positive_only && s == 0.0f);
-        }
+        const bool ok = i < n_docs && doc_allowed(fr, (uint32_t)i);
+        if (mode == 2) take = ok && (!positive_only || s != 0.0f);
+        else if (mode == 1) { take = ok && s > 0.0f; zero = ok && s == 0.0f; }
+        else take = ok && s >= lo && !(positive_only && s == 0.0f);
         uint32_t total, ztotal = 0, zex = 0;
         if (mode == 1) {
             zex = block_excl_scan(zero ? 1u : 0u, &ztotal);
@@ -299,6 +285,7 @@ struct RescoreIndex {
     const int64_t* row_ptr;
     const uint32_t* dl;
     const double* idf;
+    const double* inv_norm;   // 1/||d|| of the TF-IDF doc vectors (Formula::COS only)
     const int32_t* hot_slot;
     const uint32_t* skip;
     int32_t n_sub;
@@ -307,50 +294,137 @@ struct RescoreIndex {
     int variant;
 };
 
-// float64 score of one doc for one query: the reference loop body (bm25_ranking.ipynb:199-203)
-// doc-at-a-time; terms are visited in the given order (ascending id / query order) so the sum is
-// reproducible.  Hot terms use the skip table to narrow the search to one sub-range.
-__device__ __forceinline__ double rescore_one(const RescoreIndex& r, const int32_t* __restrict__ terms, int32_t nt,
-                                              uint32_t doc) {
+// Index of posting (t, doc) in the packed lists, -1 when doc does not contain t.  Hot terms use the skip table to narrow
+// the search to one sub-range.
+__device__ __forceinline__ int64_t find_posting(const RescoreIndex& r, int32_t t, uint32_t doc) {
+    const int64_t base = r.row_ptr[t];
+    int64_t lo = base, hi = r.row_ptr[t + 1];
+    const int32_t slot = r.skip ? r.hot_slot[t] : -1;
+    if (slot >= 0) {
+        const uint32_t* sk = r.skip + (int64_t)slot * (r.n_sub + 1) + (doc >> r.sub_shift);
+        lo = base + sk[0];
+        hi = base + sk[1];
+    }
+    const int64_t stop = hi;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (r.post[mid].doc < doc) lo = mid + 1; else hi = mid;
+    }
+    return lo < stop && r.post[lo].doc == doc ? lo : -1;
+}
+
+// BM25: the reference loop body (bm25_ranking.ipynb:199-203) doc-at-a-time; terms are visited in the given order
+// (ascending id / query order) so the sum is reproducible.
+__device__ __forceinline__ double score_bm25(const RescoreIndex& r, const int32_t* __restrict__ terms, int32_t nt,
+                                             uint32_t doc) {
     double s = 0.0;
     const double dld = (double)r.dl[doc];
     for (int32_t i = 0; i < nt; ++i) {
         const int32_t t = terms[i];
-        const int64_t base = r.row_ptr[t], end = r.row_ptr[t + 1];
-        int64_t lo = base, hi = end;
-        const int32_t slot = r.skip ? r.hot_slot[t] : -1;
-        if (slot >= 0) {
-            const uint32_t* sk = r.skip + (int64_t)slot * (r.n_sub + 1) + (doc >> r.sub_shift);
-            lo = base + sk[0];
-            hi = base + sk[1];
-        }
-        const int64_t stop = hi;
-        while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (r.post[mid].doc < doc) lo = mid + 1; else hi = mid;
-        }
-        if (lo < stop && r.post[lo].doc == doc)
-            s = __dadd_rn(s, bm25_contrib(r.idf[t], (double)r.tf[lo], dld, r.avgdl, r.k1, r.b, r.variant));
+        const int64_t p = find_posting(r, t, doc);
+        if (p >= 0) s = __dadd_rn(s, bm25_contrib(r.idf[t], (double)r.tf[p], dld, r.avgdl, r.k1, r.b, r.variant));
     }
     return s;
 }
 
+// TF-IDF cosine with the reference's mixed precision (cosine_similarity_bm25_reranking.py:88,121-126,210-226): doc
+// entries float32(tf*idf) scaled by the float64 1/doc_norm, query entries float32(float32(idf) * float32(1/||q||)),
+// products and sum in float64, terms in ascending id.  ||q|| is a float32 BLAS dot in the reference (platform-dependent
+// last bit); here float32(sqrt(float64 sum)).
+__device__ __forceinline__ double score_cos(const RescoreIndex& r, const int32_t* __restrict__ terms, int32_t nt,
+                                            uint32_t doc) {
+    double n2 = 0.0;
+    for (int32_t i = 0; i < nt; ++i) { const double x = (double)(float)r.idf[terms[i]]; n2 += x * x; }
+    const float inv_q = 1.0f / (float)sqrt(n2);
+    const double inv_d = r.inv_norm[doc];
+    double s = 0.0;
+    for (int32_t i = 0; i < nt; ++i) {
+        const int32_t t = terms[i];
+        const int64_t p = find_posting(r, t, doc);
+        if (p < 0 || r.tf[p] == 0) continue;
+        const double e = (double)(float)((double)r.tf[p] * r.idf[t]);
+        const double qn = (double)((float)r.idf[t] * inv_q);
+        s = __dadd_rn(s, __dmul_rn(__dmul_rn(e, inv_d), qn));
+    }
+    return s;
+}
+
+// "V3" re-rank: bm25_score, cosine_similarity_bm25_reranking.py:185-195
+//   doc_length = sum of the tf of the query's term occurrences in this doc (:187)
+//   score += idf * ((tf*(k1+1)) / (tf + k1*(1 - b + b*(doc_length/avgdl))))   for every occurrence whose
+//   term is in the corpus (duplicates counted, idf without +1)
+__device__ __forceinline__ double score_v3(const RescoreIndex& r, const int32_t* __restrict__ terms, int32_t nt,
+                                           uint32_t doc) {
+    int64_t doc_length = 0;
+    for (int32_t i = 0; i < nt; ++i) {
+        const int64_t p = find_posting(r, terms[i], doc);
+        doc_length += p >= 0 ? r.tf[p] : 0;
+    }
+    const double norm = __dadd_rn(__dsub_rn(1.0, r.b), __dmul_rn(r.b, __ddiv_rn((double)doc_length, r.avgdl)));
+    const double kn = __dmul_rn(r.k1, norm);
+    double s = 0.0;
+    for (int32_t i = 0; i < nt; ++i) {
+        const int32_t t = terms[i];
+        const int64_t p = find_posting(r, t, doc);
+        const double tf = p >= 0 ? (double)r.tf[p] : 0.0;
+        const double num = __dmul_rn(tf, __dadd_rn(r.k1, 1.0));
+        const double den = __dadd_rn(tf, kn);
+        s = __dadd_rn(s, __dmul_rn(r.idf[t], __ddiv_rn(num, den)));
+    }
+    return s;
+}
+
+// The terms formula F sums over for query q: BM25 the distinct terms ascending (dedup) or the occurrences in query
+// order; COS the distinct terms; V3 the occurrences.
+template <Formula F>
+__device__ __forceinline__ const int32_t* formula_terms(const PrepView& v, int32_t off, int32_t q, int dedup, int32_t* nt) {
+    const bool uniq = F == Formula::COS || (F == Formula::BM25 && dedup);
+    *nt = uniq ? v.u_cnt[q] : v.o_cnt[q];
+    return (uniq ? v.u_terms : v.o_terms) + off;
+}
+
+template <Formula F>
+__device__ __forceinline__ double formula_score(const RescoreIndex& r, const int32_t* terms, int32_t nt, uint32_t doc) {
+    if constexpr (F == Formula::BM25) return score_bm25(r, terms, nt, doc);
+    else if constexpr (F == Formula::COS) return score_cos(r, terms, nt, doc);
+    else return score_v3(r, terms, nt, doc);
+}
+
+// Ranges layout, grid-stride over every candidate: query q owns [cand_off[q], cand_off[q+1]) (dense path, explicit
+// candidate lists of br_rescore_docs / br_rerank_v3_scores).
+template <Formula F>
 __global__ void k_rescore(RescoreIndex r, const int32_t* __restrict__ q_off, PrepView v, int dedup,
                           const int64_t* __restrict__ cand_off, int32_t q_begin, int32_t nq,
                           const int32_t* __restrict__ cand, double* __restrict__ cand_score) {
     const int64_t c0 = cand_off[q_begin], c1 = cand_off[q_begin + nq];
     for (int64_t c = c0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < c1; c += (int64_t)gridDim.x * blockDim.x) {
         const int32_t doc = cand[c];
-        if (doc < 0) continue;                       // unused candidate slot
+        if (doc < 0) { cand_score[c] = 0.0; continue; }          // empty candidate slot
         int32_t lo = q_begin, hi = q_begin + nq;
         while (hi - lo > 1) {
             const int32_t mid = (lo + hi) >> 1;
             if (cand_off[mid] <= c) lo = mid; else hi = mid;
         }
-        const int32_t q = lo, off = q_off[q];
-        const int32_t* terms = dedup ? v.u_terms + off : v.o_terms + off;
-        const int32_t nt = dedup ? v.u_cnt[q] : v.o_cnt[q];
-        cand_score[c] = rescore_one(r, terms, nt, (uint32_t)doc);
+        int32_t nt;
+        const int32_t* terms = formula_terms<F>(v, q_off[lo], lo, dedup, &nt);
+        cand_score[c] = formula_score<F>(r, terms, nt, (uint32_t)doc);
+    }
+}
+
+// Stride layout, one CTA per query: query q owns [q*stride, (q+1)*stride), only its first cnt[q] slots are live (tiled
+// path, br_fuse_linear's candidate union).
+template <Formula F>
+__global__ void __launch_bounds__(64) k_rescore_heads(RescoreIndex r, const int32_t* __restrict__ q_off, PrepView v, int dedup,
+                                                      int32_t stride, const int32_t* __restrict__ cnt,
+                                                      const int32_t* __restrict__ cand, double* __restrict__ cand_score) {
+    const int q = blockIdx.x;
+    const int n = min(cnt[q], stride);
+    int32_t nt;
+    const int32_t* terms = formula_terms<F>(v, q_off[q], q, dedup, &nt);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const int64_t c = (int64_t)q * stride + i;
+        const int32_t doc = cand[c];
+        cand_score[c] = doc < 0 ? 0.0 : formula_score<F>(r, terms, nt, (uint32_t)doc);   // 0.0: empty candidate slot
     }
 }
 
@@ -463,59 +537,6 @@ __global__ void __launch_bounds__(FS_T) k_final_select(const IdT* __restrict__ i
 }
 
 
-// ------------------------------------------------------------------------------------------
-// "V3" re-rank formula: bm25_score, cosine_similarity_bm25_reranking.py:185-195
-//   doc_length = sum of the tf of the query's term occurrences in this doc (:187)
-//   score += idf * ((tf*(k1+1)) / (tf + k1*(1 - b + b*(doc_length/avgdl))))   for every occurrence whose
-//   term is in the corpus (duplicates counted, idf without +1)
-// ------------------------------------------------------------------------------------------
-__device__ __forceinline__ int32_t lookup_tf(const RescoreIndex& r, int32_t t, uint32_t doc) {
-    const int64_t base = r.row_ptr[t], end = r.row_ptr[t + 1];
-    int64_t lo = base, hi = end;
-    const int32_t slot = r.skip ? r.hot_slot[t] : -1;
-    if (slot >= 0) {
-        const uint32_t* sk = r.skip + (int64_t)slot * (r.n_sub + 1) + (doc >> r.sub_shift);
-        lo = base + sk[0];
-        hi = base + sk[1];
-    }
-    const int64_t stop = hi;
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (r.post[mid].doc < doc) lo = mid + 1; else hi = mid;
-    }
-    return (lo < stop && r.post[lo].doc == doc) ? (int32_t)r.tf[lo] : 0;
-}
-
-__global__ void k_rescore_v3(RescoreIndex r, const int32_t* __restrict__ q_off, PrepView v,
-                             const int64_t* __restrict__ cand_off, int32_t nq, const int32_t* __restrict__ cand,
-                             double* __restrict__ out) {
-    const int64_t c1 = cand_off[nq];
-    for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < c1; c += (int64_t)gridDim.x * blockDim.x) {
-        const int32_t doc = cand[c];
-        if (doc < 0) { out[c] = 0.0; continue; }
-        int32_t lo = 0, hi = nq;
-        while (hi - lo > 1) {
-            const int32_t mid = (lo + hi) >> 1;
-            if (cand_off[mid] <= c) lo = mid; else hi = mid;
-        }
-        const int32_t q = lo, off = q_off[q], nt = v.o_cnt[q];
-        const int32_t* terms = v.o_terms + off;              // in-corpus terms, query order, duplicates kept
-        int64_t doc_length = 0;
-        for (int32_t i = 0; i < nt; ++i) doc_length += lookup_tf(r, terms[i], (uint32_t)doc);
-        const double norm = __dadd_rn(__dsub_rn(1.0, r.b), __dmul_rn(r.b, __ddiv_rn((double)doc_length, r.avgdl)));
-        const double kn = __dmul_rn(r.k1, norm);
-        double s = 0.0;
-        for (int32_t i = 0; i < nt; ++i) {
-            const int32_t t = terms[i];
-            const double tf = (double)lookup_tf(r, t, (uint32_t)doc);
-            const double num = __dmul_rn(tf, __dadd_rn(r.k1, 1.0));
-            const double den = __dadd_rn(tf, kn);
-            s = __dadd_rn(s, __dmul_rn(r.idf[t], __ddiv_rn(num, den)));
-        }
-        out[c] = s;
-    }
-}
-
 // TF-IDF cosine first stage (cosine_similarity_bm25_reranking.py:72-110,121-126,210-226): doc vector tf*idf,
 // query vector idf per distinct in-corpus term, both L2-normalised.  cos(d,q) = sum_t (tf*idf_t)*idf_t /
 // (||d|| ||q||); ||q|| is constant per query, so ranking needs only w'[d,t] = tf*idf_t^2/||d|| per posting -
@@ -555,72 +576,6 @@ __global__ void k_tfidf_weights(const int64_t* __restrict__ row_ptr, int32_t voc
     out[j].w = (float)((double)e * (double)(float)idf[lo] * inv_norm[d]);
 }
 
-// Exact (float64) cosine of explicit (query, doc) candidates with the reference's mixed precision
-// (cosine_similarity_bm25_reranking.py:88,121-126,210-226): doc entries float32(tf*idf) scaled by the float64
-// 1/doc_norm, query entries float32(float32(idf) * float32(1/||q||)), products and sum in float64, terms in ascending
-// id.  ||q|| is a float32 BLAS dot in the reference (platform-dependent last bit); here float32(sqrt(float64 sum)).
-__device__ __forceinline__ double rescore_cos_one(const RescoreIndex& r, const double* __restrict__ inv_norm, const int32_t* terms,
-                                                  int32_t nt, int32_t doc) {
-    double n2 = 0.0;
-    for (int32_t i = 0; i < nt; ++i) { const double x = (double)(float)r.idf[terms[i]]; n2 += x * x; }
-    const float inv_q = 1.0f / (float)sqrt(n2);
-    const double inv_d = inv_norm[doc];
-    double s = 0.0;
-    for (int32_t i = 0; i < nt; ++i) {
-        const int32_t t = terms[i];
-        const int32_t tf = lookup_tf(r, t, (uint32_t)doc);
-        if (tf == 0) continue;
-        const double e = (double)(float)((double)tf * r.idf[t]);
-        const double qn = (double)((float)r.idf[t] * inv_q);
-        s = __dadd_rn(s, __dmul_rn(__dmul_rn(e, inv_d), qn));
-    }
-    return s;
-}
-__global__ void k_rescore_cos(RescoreIndex r, const double* __restrict__ inv_norm, const int32_t* __restrict__ q_off, PrepView v,
-                              const int64_t* __restrict__ cand_off, int32_t q_begin, int32_t nq,
-                              const int32_t* __restrict__ cand, double* __restrict__ out) {
-    const int64_t c0 = cand_off[q_begin], c1 = cand_off[q_begin + nq];
-    for (int64_t c = c0 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < c1; c += (int64_t)gridDim.x * blockDim.x) {
-        const int32_t doc = cand[c];
-        if (doc < 0) continue;
-        int32_t lo = q_begin, hi = q_begin + nq;
-        while (hi - lo > 1) {
-            const int32_t mid = (lo + hi) >> 1;
-            if (cand_off[mid] <= c) lo = mid; else hi = mid;
-        }
-        const int32_t q = lo;
-        out[c] = rescore_cos_one(r, inv_norm, v.u_terms + q_off[q], v.u_cnt[q], doc);   // distinct in-corpus terms, ascending
-    }
-}
-// the same over the fixed-stride candidate regions of the fused path
-__global__ void __launch_bounds__(64) k_rescore_cos_heads(RescoreIndex r, const double* __restrict__ inv_norm,
-                                                          const int32_t* __restrict__ q_off, PrepView v, int32_t stride,
-                                                          const int32_t* __restrict__ cnt, const int32_t* __restrict__ cand,
-                                                          double* __restrict__ cand_score) {
-    const int q = blockIdx.x;
-    const int n = min(cnt[q], stride);
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        const int64_t c = (int64_t)q * stride + i;
-        const int32_t doc = cand[c];
-        if (doc >= 0) cand_score[c] = rescore_cos_one(r, inv_norm, v.u_terms + q_off[q], v.u_cnt[q], doc);
-    }
-}
-// fused path: query q owns the fixed-stride region [q*stride, (q+1)*stride), only its first cnt[q] slots are live
-__global__ void __launch_bounds__(64) k_rescore_heads(RescoreIndex r, const int32_t* __restrict__ q_off, PrepView v, int dedup,
-                                                      int32_t stride, const int32_t* __restrict__ cnt,
-                                                      const int32_t* __restrict__ cand, double* __restrict__ cand_score) {
-    const int q = blockIdx.x;
-    const int n = min(cnt[q], stride);
-    const int32_t off = q_off[q];
-    const int32_t* terms = dedup ? v.u_terms + off : v.o_terms + off;
-    const int32_t nt = dedup ? v.u_cnt[q] : v.o_cnt[q];
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        const int64_t c = (int64_t)q * stride + i;
-        const int32_t doc = cand[c];
-        if (doc >= 0) cand_score[c] = rescore_one(r, terms, nt, (uint32_t)doc);
-    }
-}
-
 __global__ void k_scatter_rows(const int32_t* __restrict__ rows, int32_t ns, int32_t k, const int32_t* __restrict__ ids,
                                const double* __restrict__ sc, const int32_t* __restrict__ cnt, int32_t* __restrict__ out_ids,
                                double* __restrict__ out_sc, int32_t* __restrict__ out_cnt) {
@@ -638,22 +593,24 @@ __global__ void k_scatter_rows(const int32_t* __restrict__ rows, int32_t ns, int
 // ------------------------------------------------------------------------------------------
 
 static RescoreIndex rescore_view(const br_index* ix) {
-    return RescoreIndex{ix->post, ix->tf, ix->row_ptr, ix->dl, ix->idf, ix->hot_slot, ix->skip, ix->n_sub,
+    return RescoreIndex{ix->post, ix->tf, ix->row_ptr, ix->dl, ix->idf, ix->cos_inv_norm, ix->hot_slot, ix->skip, ix->n_sub,
                         ix->sub_shift, ix->avgdl, ix->k1, ix->b, ix->variant};
 }
 
-int launch_rescore(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, const int64_t* cand_off,
+int launch_rescore(br_index* ix, Formula f, const int32_t* q_off, const PrepView& pv, int dedup, const int64_t* cand_off,
                    int32_t q_begin, int32_t nq, const int32_t* cand, double* cand_score, int64_t total, cudaStream_t st) {
-    const unsigned rb = (unsigned)std::max<int64_t>(1, std::min<int64_t>((total + 127) / 128, kNumSMs * 16));
-    k_rescore<<<rb, 128, 0, st>>>(rescore_view(ix), q_off, pv, dedup, cand_off, q_begin, nq, cand, cand_score);
+    const int64_t blocks = total < 0 ? kNumSMs * 16 : std::max<int64_t>(1, std::min<int64_t>((total + 127) / 128, kNumSMs * 16));
+    auto* kern = f == Formula::BM25 ? &k_rescore<Formula::BM25> : f == Formula::COS ? &k_rescore<Formula::COS> : &k_rescore<Formula::V3>;
+    kern<<<(unsigned)blocks, 128, 0, st>>>(rescore_view(ix), q_off, pv, dedup, cand_off, q_begin, nq, cand, cand_score);
     BR_CUDA(cudaGetLastError());
     return BR_OK;
 }
 
-int launch_rescore_heads(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, int32_t nq, int32_t stride,
-                         const int32_t* cnt, const int32_t* cand, double* cand_score, cudaStream_t st, bool cos) {
-    if (cos) k_rescore_cos_heads<<<nq, 64, 0, st>>>(rescore_view(ix), ix->cos_inv_norm, q_off, pv, stride, cnt, cand, cand_score);
-    else k_rescore_heads<<<nq, 64, 0, st>>>(rescore_view(ix), q_off, pv, dedup, stride, cnt, cand, cand_score);
+int launch_rescore_heads(br_index* ix, Formula f, const int32_t* q_off, const PrepView& pv, int dedup, int32_t nq,
+                         int32_t stride, const int32_t* cnt, const int32_t* cand, double* cand_score, cudaStream_t st) {
+    auto* kern = f == Formula::BM25 ? &k_rescore_heads<Formula::BM25>
+               : f == Formula::COS  ? &k_rescore_heads<Formula::COS> : &k_rescore_heads<Formula::V3>;
+    kern<<<nq, 64, 0, st>>>(rescore_view(ix), q_off, pv, dedup, stride, cnt, cand, cand_score);
     BR_CUDA(cudaGetLastError());
     return BR_OK;
 }
@@ -668,14 +625,13 @@ int launch_final_select(const int32_t* cand, const double* cand_score, const int
 }
 // n_terms >= 0: the caller knows q_offsets[nq] (or an upper bound) - no device read, no stream synchronisation.
 int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int dedup, cudaStream_t st,
-                 PrepView* pv, int64_t** chunk_start, int32_t* total_terms, int32_t n_terms) {
+                 PrepView* pv, int64_t** chunk_start, int32_t n_terms) {
     int32_t T = n_terms;
     if (T < 0) {
         BR_CUDA(cudaMemcpyAsync(&T, q_off + nq, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         BR_CUDA(cudaStreamSynchronize(st));
     }
     BR_REQUIRE(T >= 0, BR_ERR_INVALID, "query offsets: negative total");
-    *total_terms = T;
     const size_t Tn = (size_t)T + 1, Q = (size_t)nq + 2;
     // carve ws_prep
     size_t bytes = 0;
@@ -710,8 +666,7 @@ int score_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
     ix->stats = br_query_stats{};
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
-    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, &T));
+    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start));
     BR_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)nq * (size_t)ix->n_docs, st));
     k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(ix->post, ix->row_ptr, q_off, pv, chunk_start, 0, nq, out, ix->n_docs);
     BR_CUDA(cudaGetLastError());
@@ -725,10 +680,11 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
                       int32_t q_begin, int32_t nq, int32_t k, int dedup, int positive_only, int32_t* out_ids,
                       double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table = nullptr,
                       const DocFilter* filt = nullptr) {
-    // post_table != nullptr: score with that weight table and rank by the fp32 dense scores themselves
-    // (TF-IDF cosine stage); otherwise BM25 weights + exact float64 re-score of the candidate band.
-    const bool fp32_rank = post_table != nullptr;
-    const br_posting* post = fp32_rank ? post_table : ix->post;
+    // post_table != nullptr: score with that weight table (TF-IDF cosine stage) and re-score the candidate band with the
+    // float64 cosine; otherwise BM25 weights + exact float64 BM25 re-score of the band.
+    const Formula formula = post_table ? Formula::COS : Formula::BM25;
+    const br_posting* post = post_table ? post_table : ix->post;
+    const DocFilter f = filt ? *filt : DocFilter{};
     const int64_t N = ix->n_docs;
     // queries per pass: dense fp32 rows within ~1 GiB
     int32_t qb = (int32_t)std::max<int64_t>(1, std::min<int64_t>(nq, (1LL << 30) / (4 * N)));
@@ -752,8 +708,7 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
         BR_CUDA(cudaGetLastError());
         ix->prof_end(st);
         // (query chunks keep batch-wide query indices b0 + i, so the filter rows need no remapping here)
-        if (filt) k_select_radix<true><<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, *filt);
-        else k_select_radix<false><<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, DocFilter{});
+        k_select_radix<<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, f);
         BR_CUDA(cudaGetLastError());
         BR_CUDA(cudaMemcpyAsync(h_cnt.data(), sv.cnt + b0, sizeof(int64_t) * (size_t)bn, cudaMemcpyDeviceToHost, st));
         BR_CUDA(cudaStreamSynchronize(st));
@@ -764,17 +719,9 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
         BR_TRY(ix->ws_cand.reserve((size_t)(total + 1) * (sizeof(int32_t) + sizeof(double)) + 256));
         int32_t* cand = ix->ws_cand.as<int32_t>();
         double* cand_sc = (double*)(ix->ws_cand.as<char>() + (((size_t)(total + 1) * sizeof(int32_t) + 255) & ~(size_t)255));
-        if (filt) k_emit_cands<true><<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, *filt);
-        else k_emit_cands<false><<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, DocFilter{});
+        k_emit_cands<<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, f);
         BR_CUDA(cudaGetLastError());
-        if (total > 0 && fp32_rank) {
-            // TF-IDF stage: the fp32 row only selects the band; the candidates are re-scored in float64
-            k_rescore_cos<<<(unsigned)std::min<int64_t>((total + 127) / 128, kNumSMs * 16), 128, 0, st>>>(
-                rescore_view(ix), ix->cos_inv_norm, q_off, pv, cand_off, b0, bn, cand, cand_sc);
-            BR_CUDA(cudaGetLastError());
-        } else if (total > 0) {
-            BR_TRY(launch_rescore(ix, q_off, pv, dedup, cand_off, b0, bn, cand, cand_sc, total, st));
-        }
+        if (total > 0) BR_TRY(launch_rescore(ix, formula, q_off, pv, dedup, cand_off, b0, bn, cand, cand_sc, total, st));
         BR_TRY(launch_final_select(cand, cand_sc, cand_off, b0, bn, k, positive_only, out_ids, out_scores, out_counts, st));
         // cand_off/h_off are reused by the next pass
         BR_CUDA(cudaStreamSynchronize(st));
@@ -821,7 +768,7 @@ __global__ void k_gather_rows(const int32_t* __restrict__ idx, int32_t n, const 
 // A prepared batch through the tiled path, then - for the queries it cannot serve exactly - the long-query pass and the
 // dense path.  post_table: weight table of the TF-IDF cosine stage (nullptr: BM25).  filt: the batch's doc filter
 // (nullptr: none); sub_rows: int32[nq] scratch for the filter rows of the compacted sub-batches.
-static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int32_t T, int32_t k, int dedup,
+static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int32_t k, int dedup,
                           int positive_only, const PrepView& pv, const int64_t* chunk_start, int32_t* out_ids,
                           double* out_scores, int32_t* out_counts, cudaStream_t st, const br_posting* post_table,
                           const DocFilter* filt = nullptr, int32_t* sub_rows = nullptr) {
@@ -845,9 +792,13 @@ static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q
             // The queries the regular pass cannot serve exactly (more than 32 terms / 20 hot terms, candidate overflow,
             // fewer than k docs with a hit) are compacted into a sub-batch: first the long-query pass of the tiled
             // scorer (up to 64 terms / 40 hot terms: bigram-expanded queries), then, for what is still left, the dense path.
-            std::vector<int32_t> h_off((size_t)nq + 1), h_terms((size_t)std::max(T, 1));
+            // n_terms may be an upper bound of q_offsets[nq]: copy the batch's own terms only (q_offsets[nq] <= n_terms
+            // was checked above)
+            std::vector<int32_t> h_off((size_t)nq + 1);
             BR_CUDA(cudaMemcpyAsync(h_off.data(), q_off, 4 * ((size_t)nq + 1), cudaMemcpyDeviceToHost, st));
-            BR_CUDA(cudaMemcpyAsync(h_terms.data(), q_terms, 4 * (size_t)T, cudaMemcpyDeviceToHost, st));
+            BR_CUDA(cudaStreamSynchronize(st));
+            std::vector<int32_t> h_terms((size_t)h_off[(size_t)nq]);
+            BR_CUDA(cudaMemcpyAsync(h_terms.data(), q_terms, 4 * h_terms.size(), cudaMemcpyDeviceToHost, st));
             BR_CUDA(cudaStreamSynchronize(st));
             for (int pass = 0; pass < 2 && !redo.empty(); ++pass) {
                 const bool long_pass = pass == 0;
@@ -883,8 +834,7 @@ static int serve_prepared(br_index* ix, const int32_t* q_terms, const int32_t* q
                 const DocFilter* sf = filt ? &sfilt : nullptr;
                 PrepView spv;
                 int64_t* s_chunk;
-                int32_t sT;
-                BR_TRY(prep_queries(ix, d_t, d_o, ns, dedup, st, &spv, &s_chunk, &sT, (int32_t)s_terms.size()));
+                BR_TRY(prep_queries(ix, d_t, d_o, ns, dedup, st, &spv, &s_chunk, (int32_t)s_terms.size()));
                 std::vector<int32_t> next;
                 if (long_pass) {
                     std::vector<int32_t> f2;
@@ -944,12 +894,11 @@ int topk_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32
     }
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
-    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, &T, n_terms));
+    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, n_terms));
     // algorithmic bytes of this batch: 8 B per posting of every distinct in-vocab query term
     std::vector<int64_t> hP((size_t)nq);
     BR_CUDA(cudaMemcpyAsync(hP.data(), pv.P, sizeof(int64_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
-    BR_TRY(serve_prepared(ix, q_terms, q_off, nq, T, k, dedup, positive_only, pv, chunk_start, out_ids, out_scores, out_counts, st,
+    BR_TRY(serve_prepared(ix, q_terms, q_off, nq, k, dedup, positive_only, pv, chunk_start, out_ids, out_scores, out_counts, st,
                           nullptr, filt, f_sub));
     if (out_recs) {
         k_pack_records<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, out_scores, (int64_t)nq * k, ix->doc_base, out_recs);
@@ -975,11 +924,8 @@ int rescore_docs(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int
     BR_CUDA(cudaSetDevice(ix->device));
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
-    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start, &T));
-    k_rescore<<<kNumSMs * 16, 128, 0, st>>>(rescore_view(ix), q_off, pv, dedup, cand_off, 0, nq, cand_ids, out_scores);
-    BR_CUDA(cudaGetLastError());
-    return BR_OK;
+    BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start));
+    return launch_rescore(ix, Formula::BM25, q_off, pv, dedup, cand_off, 0, nq, cand_ids, out_scores, -1, st);
 }
 
 int enable_tfidf(br_index* ix, cudaStream_t st) {
@@ -1018,11 +964,10 @@ int tfidf_topk(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32
     ix->stats = br_query_stats{};
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
     BR_TRY(prep_queries(ix, q_terms, q_off, nq, 1 /* binary query tf: generate_query_embedding sets, not adds */, st, &pv,
-                        &chunk_start, &T));
+                        &chunk_start));
     // same tiled scorer as BM25 over the tf*idf^2/||d|| table (round 2 ran this stage on the dense scatter-add path)
-    BR_TRY(serve_prepared(ix, q_terms, q_off, nq, T, k, 1, 0, pv, chunk_start, out_ids, out_scores, out_counts, st, ix->post_cos));
+    BR_TRY(serve_prepared(ix, q_terms, q_off, nq, k, 1, 0, pv, chunk_start, out_ids, out_scores, out_counts, st, ix->post_cos));
     BR_CUDA(cudaStreamSynchronize(st));
     ix->prof_collect();
     return BR_OK;
@@ -1036,11 +981,8 @@ int rerank_v3(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_
     BR_CUDA(cudaSetDevice(ix->device));
     PrepView pv;
     int64_t* chunk_start;
-    int32_t T;
-    BR_TRY(prep_queries(ix, q_terms, q_off, nq, 0, st, &pv, &chunk_start, &T));
-    k_rescore_v3<<<kNumSMs * 16, 128, 0, st>>>(rescore_view(ix), q_off, pv, cand_off, nq, cand_ids, out_scores);
-    BR_CUDA(cudaGetLastError());
-    return BR_OK;
+    BR_TRY(prep_queries(ix, q_terms, q_off, nq, 0, st, &pv, &chunk_start));
+    return launch_rescore(ix, Formula::V3, q_off, pv, 0, cand_off, 0, nq, cand_ids, out_scores, -1, st);
 }
 
 int topk_merge(const int64_t* ids, const double* scores, int32_t n_parts, int32_t nq, int32_t k, int64_t* out_ids,

@@ -23,11 +23,17 @@ struct PrepView {
 
 // The query preparation of br_topk_batch (k_prep_queries into ix->ws_prep); n_terms < 0: read q_offsets[nq] back.
 int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int32_t nq, int dedup, cudaStream_t st,
-                 PrepView* pv, int64_t** chunk_start, int32_t* total_terms, int32_t n_terms = -1);
-int launch_rescore(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, const int64_t* cand_off,
+                 PrepView* pv, int64_t** chunk_start, int32_t n_terms = -1);
+// The float64 formula of an exact re-score: BM25 (br_topk_batch, br_rescore_docs), TF-IDF cosine (br_tfidf_cosine_topk),
+// V3 re-rank (br_rerank_v3_scores).  An empty candidate slot (id -1) gets 0.0.
+enum class Formula { BM25, COS, V3 };
+// Candidates of query q in [cand_off[q], cand_off[q+1]), q in [q_begin, q_begin + nq); total: their number, -1 when
+// only the device knows it.
+int launch_rescore(br_index* ix, Formula f, const int32_t* q_off, const PrepView& pv, int dedup, const int64_t* cand_off,
                    int32_t q_begin, int32_t nq, const int32_t* cand, double* cand_score, int64_t total, cudaStream_t st);
-int launch_rescore_heads(br_index* ix, const int32_t* q_off, const PrepView& pv, int dedup, int32_t nq, int32_t stride,
-                         const int32_t* cnt, const int32_t* cand, double* cand_score, cudaStream_t st, bool cos = false);
+// Candidates of query q in the fixed-stride region [q * stride, (q+1) * stride), of which the first cnt[q] are live.
+int launch_rescore_heads(br_index* ix, Formula f, const int32_t* q_off, const PrepView& pv, int dedup, int32_t nq,
+                         int32_t stride, const int32_t* cnt, const int32_t* cand, double* cand_score, cudaStream_t st);
 // cand_off == NULL: query q's candidates are [q * fixed_cnt, (q + 1) * fixed_cnt)
 int launch_final_select(const int32_t* cand, const double* cand_score, const int64_t* cand_off, int32_t q_begin,
                         int32_t nq, int32_t k, int positive_only, int32_t* out_ids, double* out_scores,

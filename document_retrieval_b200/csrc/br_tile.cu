@@ -775,17 +775,15 @@ __device__ __forceinline__ void make_plan(const PlanArgs& pa, int q, float thr, 
 // is a valid lower bound of the K-th best score, and the first launches already run with a deferral plan instead of
 // streaming every term against a zero threshold.  One warp per query; a running top-32 is kept sorted across the lanes
 // (each batch of 32 weights is sorted, reversed and merged bitonically).
-// FILT: only the postings of docs the query's filter row allows count (K distinct ALLOWED docs score at least the seed).
+// Only the postings of docs the query's filter row allows count (K distinct ALLOWED docs score at least the seed).
 constexpr int SEED_MAX = 256;
-template <bool FILT>
 __global__ void __launch_bounds__(128) k_seed_thr(const br_posting* __restrict__ post, const int64_t* __restrict__ row_ptr,
                                                   int32_t nq, int K, const int32_t* __restrict__ elig, float* __restrict__ thr,
                                                   PlanArgs pa, DocFilter f) {
     const int lane = threadIdx.x & 31;
     const int q = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (q >= nq || !elig[q]) return;
-    const uint32_t* fr = nullptr;
-    if constexpr (FILT) fr = f.row_of(q);
+    const uint32_t* fr = f.row ? f.row_of(q) : nullptr;
     const int32_t off = pa.q_off[q], nu = pa.u_cnt[q];
     float best = 0.f;
     for (int j = nu - 1; j >= 0; --j) {         // descending term id: in a frequency-ranked vocabulary the rare (high-bound)
@@ -796,8 +794,7 @@ __global__ void __launch_bounds__(128) k_seed_thr(const br_posting* __restrict__
         const int n = (int)min(df, (int64_t)SEED_MAX);
         float run = 0.f;                                            // lane i: i-th largest weight so far
         for (int base = 0; base < n; base += 32) {
-            float wv = base + lane < n ? post[lo + base + lane].w * m : 0.f;
-            if constexpr (FILT) wv = base + lane < n && doc_allowed(fr, post[lo + base + lane].doc) ? wv : 0.f;
+            const float wv = base + lane < n && doc_allowed(fr, post[lo + base + lane].doc) ? post[lo + base + lane].w * m : 0.f;
             const float srt = warp_sort_desc(fmaxf(wv, 0.f), lane);
             float x = fmaxf(run, __shfl_sync(0xffffffffu, srt, 31 - lane));     // bitonic: top 32 of the union
 #pragma unroll
@@ -1138,7 +1135,7 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
                std::vector<int32_t>* h_flags, bool long_pass, const br_posting* post_table, const DocFilter* filt) {
     // post_table != nullptr: the TF-IDF cosine stage (br_tfidf_cosine_topk) - same kernels over the weight table
     // tf*idf^2/||d|| (all weights >= 0 whatever the idf variant), no deferral (the look-up rows and upper bounds hold
-    // BM25 weights), candidates re-scored by k_rescore_cos
+    // BM25 weights), candidates re-scored with Formula::COS
     const bool cos = post_table != nullptr;
     const br_posting* const post = cos ? post_table : ix->post;
     const int n_srows = cos ? 0 : ix->n_srows;
@@ -1255,8 +1252,8 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
                           ix->thr_exchange_world * (int)k <= 32 * XCHG_PER;
     const int xr = exchange ? ix->thr_exchange_rounds : 0;
     if (k <= 32) {
-        if (filt) k_seed_thr<true><<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa, *filt);
-        else k_seed_thr<false><<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa, DocFilter{});
+        k_seed_thr<<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(post, ix->row_ptr, nq, (int)k, elig, thr, pa,
+                                                                      filt ? *filt : DocFilter{});
         BR_CUDA(cudaGetLastError());
         ix->stats.kernel_launches += 1;
     }
@@ -1267,7 +1264,7 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
     else if (long_pass) BR_TRY((launch_tiles<TILE_QT_LONG, false>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
     else if (filt) BR_TRY((launch_tiles<TILE_QT, true>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
     else BR_TRY((launch_tiles<TILE_QT, false>(a, smem, st, ix, prev_cnt, overflow, pa, xr, x_local, x_gathered)));
-    BR_TRY(launch_rescore_heads(ix, q_off, pv, dedup, nq, cap, cand_cnt, cand, cand_sc, st, cos));
+    BR_TRY(launch_rescore_heads(ix, cos ? Formula::COS : Formula::BM25, q_off, pv, dedup, nq, cap, cand_cnt, cand, cand_sc, st));
     BR_TRY(launch_final_select(cand, cand_sc, cand_off, 0, nq, k, positive_only, out_ids, out_scores, cnt_tmp, st, cand_cnt));
     // with shared thresholds a shard legitimately returns fewer than k docs (the rest of the corpus holds better ones)
     const int32_t need = exchange ? 0 : (int32_t)std::min<int64_t>(k, ix->n_docs);

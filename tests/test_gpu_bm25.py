@@ -333,6 +333,19 @@ def test_long_and_duplicate_heavy_queries():
         ids, sc = m.retrieve_top_n_batch((q_terms, q_off), 10)
         assert np.array_equal(ids.cpu().numpy(), oi) and np.array_equal(sc.cpu().numpy(), os_)
         assert m.query_stats()["queries_dense"] == len(qs)
+        # the same batch through the C entry point with n_terms an upper bound of q_offsets[nq]: the redo pass reads
+        # back only the batch's own terms (q_terms is the head of a larger buffer)
+        from document_retrieval_b200 import _lib
+        from document_retrieval_b200._lib import ptr
+        buf = torch.full((q_terms.size + 4096,), 7, dtype=torch.int32, device="cuda")
+        buf[:q_terms.size] = torch.from_numpy(q_terms).cuda()
+        d_off = torch.from_numpy(q_off).cuda()
+        ids_c = torch.empty_like(ids)
+        sc_c = torch.empty_like(sc)
+        _lib.check(_lib.load().br_topk_batch(m._h, ptr(buf), ptr(d_off), len(qs), buf.numel(), 10, int(dedup), 0, ptr(ids_c),
+                                             ptr(sc_c), None, _lib.stream_ptr(ids.device)), "br_topk_batch")
+        torch.cuda.synchronize()
+        assert torch.equal(ids_c, ids) and torch.equal(sc_c, sc) and m.query_stats()["queries_dense"] == len(qs)
         # 33..64 term occurrences (a 17-token query with its bigrams is 33 terms, bm25_ranking.ipynb:105-107): the
         # long-query pass of the tiled scorer, nothing left for the dense path
         mid = [np.concatenate([q[:36], q[:4]]) for q in qs] + [q[:33] for q in qs]
