@@ -17,6 +17,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <memory>
 #include <thread>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -271,24 +272,21 @@ __global__ void k_export(const br_posting* __restrict__ post, const uint16_t* __
 
 void index_free(br_index* ix) {
     if (!ix) return;
-    cudaSetDevice(ix->device);
-    cudaFree(ix->row_ptr); cudaFree(ix->post); cudaFree(ix->post_cos); cudaFree(ix->cos_inv_norm); cudaFree(ix->tf); cudaFree(ix->dl); cudaFree(ix->df);
-    cudaFree(ix->idf); cudaFree(ix->ub); cudaFree(ix->hot_slot); cudaFree(ix->skip); cudaFree(ix->sig_bit); cudaFree(ix->dense_rows); cudaFree(ix->row_slot);
-    ix->ws_prep.release(); ix->ws_dense.release(); ix->ws_sel.release(); ix->ws_cand.release();
-    ix->ws_misc.release(); ix->ws_tile.release(); ix->ws_sort.release(); ix->ws_cold.release(); ix->ws_rec.release();
-    for (cudaEvent_t e : ix->ev_pool) cudaEventDestroy(e);
+    cudaSetDevice(ix->device);   // the members free their memory on the handle's device
     delete ix;
 }
 
 static int alloc_common(br_index* ix) {
-    BR_CUDA(cudaMalloc(&ix->row_ptr, sizeof(int64_t) * ((size_t)ix->vocab + 1)));
-    BR_CUDA(cudaMalloc(&ix->dl, sizeof(uint32_t) * (size_t)ix->n_docs));
-    BR_CUDA(cudaMalloc(&ix->df, sizeof(uint32_t) * (size_t)ix->vocab));
-    BR_CUDA(cudaMalloc(&ix->idf, sizeof(double) * (size_t)ix->vocab));
-    BR_CUDA(cudaMalloc(&ix->hot_slot, sizeof(int32_t) * (size_t)ix->vocab));
-    BR_CUDA(cudaMalloc(&ix->ub, sizeof(float) * (size_t)ix->vocab));
+    BR_TRY(ix->row_ptr.alloc((size_t)ix->vocab + 1));
+    BR_TRY(ix->dl.alloc((size_t)ix->n_docs));
+    BR_TRY(ix->df.alloc((size_t)ix->vocab));
+    BR_TRY(ix->idf.alloc((size_t)ix->vocab));
+    BR_TRY(ix->hot_slot.alloc((size_t)ix->vocab));
+    BR_TRY(ix->ub.alloc((size_t)ix->vocab));
     return BR_OK;
 }
+
+using IndexOwner = std::unique_ptr<br_index, decltype(&index_free)>;   // a half-built handle: freed unless released
 
 int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int32_t vocab, int64_t doc_base,
                 cudaStream_t st, br_index** out) {
@@ -298,10 +296,9 @@ int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int3
                "bm25_ranking.ipynb:171)");
     BR_REQUIRE(vocab > 0, BR_ERR_INVALID, "br_index_build: vocab must be positive");
     *out = nullptr;
-    br_index* ix = new br_index();
+    IndexOwner ix(new br_index(), index_free);
     BR_CUDA(cudaGetDevice(&ix->device));
     ix->n_docs = n_docs; ix->vocab = vocab; ix->doc_base = doc_base;
-    struct Guard { br_index* p; ~Guard() { if (p) index_free(p); } } guard{ix};
 
     int64_t n_tok = 0;
     BR_CUDA(cudaMemcpyAsync(&n_tok, doc_off + n_docs, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
@@ -309,25 +306,18 @@ int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int3
     BR_REQUIRE(n_tok >= 0 && n_tok < (1LL << 32), BR_ERR_UNSUPPORTED,
                "br_index_build: more than 2^32 tokens in one shard");
     ix->sum_dl = n_tok;
-    BR_TRY(alloc_common(ix));
+    BR_TRY(alloc_common(ix.get()));
 
-    int* d_bad = nullptr;
-    uint32_t *keys_a = nullptr, *keys_b = nullptr, *vals_a = nullptr, *vals_b = nullptr;
-    uint32_t *block_counts = nullptr, *post_term = nullptr, *head_pos = nullptr, *tstart = nullptr, *tend = nullptr;
-    int64_t* block_off = nullptr;
-    void* sort_tmp = nullptr;
-    struct Tmp { void** p; ~Tmp() { if (*p) cudaFree(*p); } };
-    Tmp t0{(void**)&d_bad}, t1{(void**)&keys_a}, t2{(void**)&keys_b}, t3{(void**)&block_counts},
-        t4{(void**)&post_term}, t5{(void**)&head_pos}, t6{(void**)&tstart}, t7{(void**)&tend},
-        t8{(void**)&block_off}, t9{&sort_tmp}, t10{(void**)&vals_a}, t11{(void**)&vals_b};
-
-    BR_CUDA(cudaMalloc(&d_bad, sizeof(int)));
+    DevArray<int> d_bad;
+    DevArray<uint32_t> keys_a, keys_b, vals_a, vals_b, block_counts, post_term, head_pos, tstart, tend;
+    DevArray<int64_t> block_off;
+    DevArray<unsigned char> sort_tmp;
+    BR_TRY(d_bad.alloc(1));
     BR_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
-    const size_t nk = (size_t)(n_tok > 0 ? n_tok : 1);
-    BR_CUDA(cudaMalloc(&keys_a, sizeof(uint32_t) * nk));
-    BR_CUDA(cudaMalloc(&keys_b, sizeof(uint32_t) * nk));
-    BR_CUDA(cudaMalloc(&vals_a, sizeof(uint32_t) * nk));
-    BR_CUDA(cudaMalloc(&vals_b, sizeof(uint32_t) * nk));
+    BR_TRY(keys_a.alloc((size_t)n_tok));
+    BR_TRY(keys_b.alloc((size_t)n_tok));
+    BR_TRY(vals_a.alloc((size_t)n_tok));
+    BR_TRY(vals_b.alloc((size_t)n_tok));
     k_make_keys<<<kNumSMs * 8, 256, 0, st>>>(tok, doc_off, n_docs, vocab, keys_a, vals_a, ix->dl, d_bad);
     BR_CUDA(cudaGetLastError());
 
@@ -339,15 +329,15 @@ int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int3
     cub::DoubleBuffer<uint32_t> dkeys(keys_a, keys_b), dvals(vals_a, vals_b);
     size_t tmp_bytes = 0;
     BR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, dkeys, dvals, (int64_t)n_tok, 0, term_bits, st));
-    BR_CUDA(cudaMalloc(&sort_tmp, tmp_bytes + 16));
+    BR_TRY(sort_tmp.alloc(tmp_bytes + 16));
     BR_CUDA(cub::DeviceRadixSort::SortPairs(sort_tmp, tmp_bytes, dkeys, dvals, (int64_t)n_tok, 0, term_bits, st));
     const uint32_t* keys = dkeys.Current();
     const uint32_t* vals = dvals.Current();
 
     // run-length encode
     const int64_t n_blocks = (n_tok + RLE_TILE - 1) / RLE_TILE;
-    BR_CUDA(cudaMalloc(&block_counts, sizeof(uint32_t) * (size_t)(n_blocks + 1)));
-    BR_CUDA(cudaMalloc(&block_off, sizeof(int64_t) * (size_t)(n_blocks + 2)));
+    BR_TRY(block_counts.alloc((size_t)n_blocks + 1));
+    BR_TRY(block_off.alloc((size_t)n_blocks + 2));
     if (n_blocks > 0) {
         k_rle_count<<<(unsigned)n_blocks, RLE_T, 0, st>>>(keys, vals, n_tok, block_counts);
         BR_CUDA(cudaGetLastError());
@@ -362,13 +352,12 @@ int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int3
     BR_REQUIRE(!(bad & 1), BR_ERR_INVALID, "br_index_build: token id outside [0, vocab)");
     BR_REQUIRE(!(bad & 2), BR_ERR_INVALID, "br_index_build: doc_offsets not non-decreasing");
     ix->nnz = nnz;
-    const size_t np = (size_t)(nnz > 0 ? nnz : 1);
-    BR_CUDA(cudaMalloc(&ix->post, sizeof(br_posting) * np));
-    BR_CUDA(cudaMalloc(&ix->tf, sizeof(uint16_t) * np));
-    BR_CUDA(cudaMalloc(&post_term, sizeof(uint32_t) * np));
-    BR_CUDA(cudaMalloc(&head_pos, sizeof(uint32_t) * np));
-    BR_CUDA(cudaMalloc(&tstart, sizeof(uint32_t) * (size_t)vocab));
-    BR_CUDA(cudaMalloc(&tend, sizeof(uint32_t) * (size_t)vocab));
+    BR_TRY(ix->post.alloc((size_t)nnz));
+    BR_TRY(ix->tf.alloc((size_t)nnz));
+    BR_TRY(post_term.alloc((size_t)nnz));
+    BR_TRY(head_pos.alloc((size_t)nnz));
+    BR_TRY(tstart.alloc((size_t)vocab));
+    BR_TRY(tend.alloc((size_t)vocab));
     BR_CUDA(cudaMemsetAsync(tstart, 0, sizeof(uint32_t) * (size_t)vocab, st));
     BR_CUDA(cudaMemsetAsync(tend, 0, sizeof(uint32_t) * (size_t)vocab, st));
     if (n_blocks > 0) {
@@ -389,8 +378,7 @@ int index_build(const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int3
     BR_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
     BR_REQUIRE(!(bad & 4), BR_ERR_UNSUPPORTED, "br_index_build: a term occurs more than 65535 times in one doc");
-    guard.p = nullptr;
-    *out = ix;
+    *out = ix.release();
     return BR_OK;
 }
 
@@ -402,20 +390,16 @@ int index_import_dev(const int64_t* row_ptr, const int32_t* doc, const uint16_t*
     BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31) && vocab > 0 && nnz >= 0 && nnz < (1LL << 32), BR_ERR_INVALID,
                "br_index_import_csr_dev: bad sizes");
     *out = nullptr;
-    br_index* ix = new br_index();
+    IndexOwner ix(new br_index(), index_free);
     BR_CUDA(cudaGetDevice(&ix->device));
     ix->n_docs = n_docs; ix->vocab = vocab; ix->doc_base = doc_base; ix->nnz = nnz;
-    struct Guard { br_index* p; ~Guard() { if (p) index_free(p); } } guard{ix};
-    BR_TRY(alloc_common(ix));
-    const size_t np = (size_t)(nnz > 0 ? nnz : 1);
-    BR_CUDA(cudaMalloc(&ix->post, sizeof(br_posting) * np));
-    BR_CUDA(cudaMalloc(&ix->tf, sizeof(uint16_t) * np));
-    int* d_bad = nullptr;
-    unsigned long long* d_sum = nullptr;
-    struct Tmp { void** p; ~Tmp() { if (*p) cudaFree(*p); } };
-    Tmp t0{(void**)&d_bad}, t1{(void**)&d_sum};
-    BR_CUDA(cudaMalloc(&d_bad, sizeof(int)));
-    BR_CUDA(cudaMalloc(&d_sum, sizeof(unsigned long long)));
+    BR_TRY(alloc_common(ix.get()));
+    BR_TRY(ix->post.alloc((size_t)nnz));
+    BR_TRY(ix->tf.alloc((size_t)nnz));
+    DevArray<int> d_bad;
+    DevArray<unsigned long long> d_sum;
+    BR_TRY(d_bad.alloc(1));
+    BR_TRY(d_sum.alloc(1));
     BR_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
     BR_CUDA(cudaMemsetAsync(d_sum, 0, sizeof(unsigned long long), st));
     BR_CUDA(cudaMemcpyAsync(ix->row_ptr, row_ptr, sizeof(int64_t) * ((size_t)vocab + 1), cudaMemcpyDeviceToDevice, st));
@@ -442,8 +426,7 @@ int index_import_dev(const int64_t* row_ptr, const int32_t* doc, const uint16_t*
     BR_REQUIRE(!(bad & 4), BR_ERR_INVALID, "br_index_import_csr: tf outside [1, 65535]");
     BR_REQUIRE(!(bad & 16), BR_ERR_INVALID, "br_index_import_csr: negative doc length");
     ix->sum_dl = (int64_t)sum;
-    guard.p = nullptr;
-    *out = ix;
+    *out = ix.release();
     return BR_OK;
 }
 
@@ -455,19 +438,16 @@ int index_import(const int64_t* row_ptr, const int32_t* doc, const int32_t* tf, 
     *out = nullptr;
     const int64_t nnz = row_ptr[vocab];
     BR_REQUIRE(nnz >= 0 && nnz < (1LL << 32) && row_ptr[0] == 0, BR_ERR_INVALID, "br_index_import_csr: bad row_ptr");
-    int64_t* d_rp = nullptr;
-    int32_t *d_doc = nullptr, *d_tf = nullptr, *d_dl = nullptr;
-    uint16_t* d_tf16 = nullptr;
-    int* d_bad = nullptr;
-    struct Tmp { void** p; ~Tmp() { if (*p) cudaFree(*p); } };
-    Tmp t0{(void**)&d_rp}, t1{(void**)&d_doc}, t2{(void**)&d_tf}, t3{(void**)&d_dl}, t4{(void**)&d_tf16}, t5{(void**)&d_bad};
-    const size_t np = (size_t)(nnz > 0 ? nnz : 1);
-    BR_CUDA(cudaMalloc(&d_rp, sizeof(int64_t) * ((size_t)vocab + 1)));
-    BR_CUDA(cudaMalloc(&d_doc, sizeof(int32_t) * np));
-    BR_CUDA(cudaMalloc(&d_tf, sizeof(int32_t) * np));
-    BR_CUDA(cudaMalloc(&d_tf16, sizeof(uint16_t) * np));
-    BR_CUDA(cudaMalloc(&d_dl, sizeof(int32_t) * (size_t)n_docs));
-    BR_CUDA(cudaMalloc(&d_bad, sizeof(int)));
+    DevArray<int64_t> d_rp;
+    DevArray<int32_t> d_doc, d_tf, d_dl;
+    DevArray<uint16_t> d_tf16;
+    DevArray<int> d_bad;
+    BR_TRY(d_rp.alloc((size_t)vocab + 1));
+    BR_TRY(d_doc.alloc((size_t)nnz));
+    BR_TRY(d_tf.alloc((size_t)nnz));
+    BR_TRY(d_tf16.alloc((size_t)nnz));
+    BR_TRY(d_dl.alloc((size_t)n_docs));
+    BR_TRY(d_bad.alloc(1));
     BR_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
     BR_CUDA(cudaMemcpyAsync(d_rp, row_ptr, sizeof(int64_t) * ((size_t)vocab + 1), cudaMemcpyHostToDevice, st));
     BR_CUDA(cudaMemcpyAsync(d_doc, doc, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
@@ -489,10 +469,8 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
     BR_REQUIRE(ix, BR_ERR_INVALID, "br_index_finalize: null handle");
     BR_REQUIRE(variant >= 0 && variant <= 2, BR_ERR_INVALID, "br_index_finalize: unknown variant");
     BR_CUDA(cudaSetDevice(ix->device));
-    if (ix->post_cos) {                      // the TF-IDF tables depend on idf: rebuilt on demand after a re-finalise
-        cudaFree(ix->post_cos); cudaFree(ix->cos_inv_norm);
-        ix->post_cos = nullptr; ix->cos_inv_norm = nullptr;
-    }
+    ix->post_cos.reset();                    // the TF-IDF tables depend on idf: rebuilt on demand after a re-finalise
+    ix->cos_inv_norm.reset();
     ix->k1 = k1; ix->b = b; ix->variant = variant;
     ix->n_stat = n_stat > 0 ? n_stat : (double)ix->n_docs;
     const double sum_dl = sum_dl_stat > 0 ? sum_dl_stat : (double)ix->sum_dl;
@@ -542,16 +520,15 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
         BR_CUDA(cudaMemcpyAsync(ix->hot_slot, slot.data(), sizeof(int32_t) * V, cudaMemcpyHostToDevice, st));
         if (ix->n_hot > 0) {
             const int64_t n_entries = (int64_t)ix->n_hot * ((int64_t)ix->n_sub + 1);
-            int32_t* d_hot = nullptr;
-            BR_CUDA(cudaMalloc(&ix->skip, sizeof(uint32_t) * (size_t)n_entries));
-            BR_CUDA(cudaMalloc(&d_hot, sizeof(int32_t) * (size_t)ix->n_hot));
+            DevArray<int32_t> d_hot;
+            BR_TRY(ix->skip.alloc((size_t)n_entries));
+            BR_TRY(d_hot.alloc((size_t)ix->n_hot));
             BR_CUDA(cudaMemcpyAsync(d_hot, hot_terms.data(), sizeof(int32_t) * (size_t)ix->n_hot,
                                     cudaMemcpyHostToDevice, st));
             k_skip<<<blocks_for(n_entries, 256), 256, 0, st>>>(ix->row_ptr, ix->post, d_hot, ix->n_hot, ix->n_sub,
                                                                ix->sub_shift, ix->skip);
             BR_CUDA(cudaGetLastError());
             BR_CUDA(cudaStreamSynchronize(st));
-            cudaFree(d_hot);
         }
     }
     {   // dense rows (rebuilt at every finalize: they hold the weights)
@@ -571,24 +548,23 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
         int32_t n_s = 0;
         for (int32_t t : cand_terms)
             if ((double)ix->h_df[(size_t)t] >= frac * (double)ix->n_docs && n_s < 32) ++n_s;
-        cudaFree(ix->dense_rows); ix->dense_rows = nullptr;
+        ix->dense_rows.reset();
         ix->n_rows = (int32_t)cand_terms.size();
         ix->n_srows = n_s;
         std::vector<int16_t> slot(V, (int16_t)-1);
         for (size_t r = 0; r < cand_terms.size(); ++r) slot[(size_t)cand_terms[r]] = (int16_t)r;
-        if (!ix->row_slot) BR_CUDA(cudaMalloc(&ix->row_slot, sizeof(int16_t) * V));
+        if (!ix->row_slot) BR_TRY(ix->row_slot.alloc(V));
         BR_CUDA(cudaMemcpyAsync(ix->row_slot, slot.data(), sizeof(int16_t) * V, cudaMemcpyHostToDevice, st));
         if (ix->n_rows > 0) {
-            int32_t* d_terms = nullptr;
-            BR_CUDA(cudaMalloc(&ix->dense_rows, sizeof(float) * (size_t)ix->n_rows * (size_t)ix->n_pad));
-            BR_CUDA(cudaMalloc(&d_terms, sizeof(int32_t) * (size_t)ix->n_rows));
+            DevArray<int32_t> d_terms;
+            BR_TRY(ix->dense_rows.alloc((size_t)ix->n_rows * (size_t)ix->n_pad));
+            BR_TRY(d_terms.alloc((size_t)ix->n_rows));
             BR_CUDA(cudaMemsetAsync(ix->dense_rows, 0, sizeof(float) * (size_t)ix->n_rows * (size_t)ix->n_pad, st));
             BR_CUDA(cudaMemcpyAsync(d_terms, cand_terms.data(), sizeof(int32_t) * (size_t)ix->n_rows, cudaMemcpyHostToDevice, st));
             k_rows_fill<<<dim3(kNumSMs * 4, (unsigned)ix->n_rows), 256, 0, st>>>(ix->row_ptr, ix->post, d_terms, ix->n_rows, ix->n_pad,
                                                                               ix->dense_rows);
             BR_CUDA(cudaGetLastError());
             BR_CUDA(cudaStreamSynchronize(st));
-            cudaFree(d_terms);
         }
         BR_CUDA(cudaStreamSynchronize(st));
     }
@@ -603,7 +579,7 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
         std::vector<int8_t> bit(V, (int8_t)-1);
         for (size_t r = 0; r < top; ++r)
             if (ix->h_df[(size_t)order[r]] > 0) bit[(size_t)order[r]] = (int8_t)r;
-        BR_CUDA(cudaMalloc(&ix->sig_bit, V));
+        BR_TRY(ix->sig_bit.alloc(V));
         BR_CUDA(cudaMemcpyAsync(ix->sig_bit, bit.data(), V, cudaMemcpyHostToDevice, st));
         BR_CUDA(cudaStreamSynchronize(st));
     }
@@ -671,7 +647,7 @@ int br_index_stats(const br_index* ix, int64_t* n_docs, int32_t* vocab, int64_t*
     return BR_OK;
 }
 
-const uint32_t* br_index_df_dev(const br_index* ix) { return ix ? ix->df : nullptr; }
+const uint32_t* br_index_df_dev(const br_index* ix) { return ix ? ix->df.get() : nullptr; }
 
 int br_index_stats_in_force(const br_index* ix, double* n_stat, double* sum_dl_stat) {
     BR_REQUIRE(ix && ix->finalized, BR_ERR_STATE, "br_index_stats_in_force: call br_index_finalize first");
@@ -703,19 +679,12 @@ int br_index_export_csr(const br_index* ix, int64_t* row_ptr_host, int32_t* doc_
     if (dl_host) BR_CUDA(cudaMemcpy(dl_host, ix->dl, sizeof(uint32_t) * (size_t)ix->n_docs, cudaMemcpyDeviceToHost));
     if ((doc_host || tf_host) && ix->nnz > 0) {
         BR_REQUIRE(doc_host && tf_host, BR_ERR_INVALID, "br_index_export_csr: doc_host and tf_host go together");
-        int32_t *d_doc = nullptr, *d_tf = nullptr;
-        BR_CUDA(cudaMalloc(&d_doc, sizeof(int32_t) * (size_t)ix->nnz));
-        if (cudaMalloc(&d_tf, sizeof(int32_t) * (size_t)ix->nnz) != cudaSuccess) {
-            cudaFree(d_doc);
-            br::set_error("br_index_export_csr: out of device memory");
-            return BR_ERR_CUDA;
-        }
+        br::DevArray<int32_t> d_doc, d_tf;
+        BR_TRY(d_doc.alloc((size_t)ix->nnz));
+        BR_TRY(d_tf.alloc((size_t)ix->nnz));
         br::k_export<<<br::blocks_for(ix->nnz, 256), 256>>>(ix->post, ix->tf, ix->nnz, d_doc, d_tf);
-        cudaError_t e1 = cudaMemcpy(doc_host, d_doc, sizeof(int32_t) * (size_t)ix->nnz, cudaMemcpyDeviceToHost);
-        cudaError_t e2 = cudaMemcpy(tf_host, d_tf, sizeof(int32_t) * (size_t)ix->nnz, cudaMemcpyDeviceToHost);
-        cudaFree(d_doc); cudaFree(d_tf);
-        BR_CUDA(e1);
-        BR_CUDA(e2);
+        BR_CUDA(cudaMemcpy(doc_host, d_doc, sizeof(int32_t) * (size_t)ix->nnz, cudaMemcpyDeviceToHost));
+        BR_CUDA(cudaMemcpy(tf_host, d_tf, sizeof(int32_t) * (size_t)ix->nnz, cudaMemcpyDeviceToHost));
     }
     return BR_OK;
 }

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -39,27 +40,58 @@ void set_error(const std::string& msg);
         }                             \
     } while (0)
 
-// Grow-only device scratch buffer (never shrinks; freed with the handle).
+// One cudaMalloc allocation of T, freed with cudaFree by its owner: at the next alloc, at reset() or when it goes away.
+// Converts to T* so that it reads like the raw device pointer it owns.
+template <class T>
+class DevArray {
+  public:
+    DevArray() = default;
+    DevArray(DevArray&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+    DevArray& operator=(DevArray&& o) noexcept {
+        if (this != &o) {
+            reset();
+            p_ = o.p_;
+            o.p_ = nullptr;
+        }
+        return *this;
+    }
+    ~DevArray() { reset(); }
+    // max(n, 1) elements; a failure names the caller's file and line
+    int alloc(size_t n, const char* file = __builtin_FILE(), int line = __builtin_LINE()) {
+        reset();
+        const size_t bytes = sizeof(T) * std::max<size_t>(n, 1);
+        const cudaError_t e = cudaMalloc(&p_, bytes);
+        if (e == cudaSuccess) return BR_OK;
+        p_ = nullptr;
+        set_error("cudaMalloc(" + std::to_string(bytes) + " bytes): " + cudaGetErrorString(e) + " (" + file + ":" +
+                  std::to_string(line) + ")");
+        return BR_ERR_CUDA;
+    }
+    void reset() {
+        if (p_) cudaFree(p_);
+        p_ = nullptr;
+    }
+    T* get() const { return p_; }
+    operator T*() const { return p_; }
+
+  private:
+    T* p_ = nullptr;
+};
+
+// Grow-only device workspace (never shrinks; freed with its owner).
 struct DevBuf {
-    void* p = nullptr;
+    DevArray<unsigned char> mem;
     size_t cap = 0;
     int reserve(size_t bytes) {
         if (bytes <= cap) return BR_OK;
-        if (p) BR_CUDA(cudaFree(p));
-        p = nullptr;
         cap = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        BR_CUDA(cudaMalloc(&p, want));
+        const size_t want = bytes + bytes / 4 + 256;
+        BR_TRY(mem.alloc(want));
         cap = want;
         return BR_OK;
     }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
     template <class T>
-    T* as() const { return reinterpret_cast<T*>(p); }
+    T* as() const { return reinterpret_cast<T*>(mem.get()); }
 };
 
 // Stream-ordered scratch comes from a PRIVATE memory pool of the library, one per device: with a release threshold of 0
@@ -95,15 +127,28 @@ inline int scratch_alloc(void** p, size_t bytes, cudaStream_t st) {
     BR_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 1, pool, st));
     return BR_OK;
 }
-struct AsyncBuf {   // stream-ordered scratch
-    void* p = nullptr;
-    cudaStream_t st;
-    explicit AsyncBuf(cudaStream_t s) : st(s) {}
-    int alloc(size_t bytes) {
-        BR_TRY(scratch_alloc(&p, bytes, st));
+// The stream-ordered temporaries of one call: every alloc comes from the scratch pool and is freed on the same stream
+// (cudaFreeAsync) when the scope ends, whichever way the call returns.
+class StreamScratch {
+  public:
+    explicit StreamScratch(cudaStream_t st) : st_(st) {}
+    StreamScratch(const StreamScratch&) = delete;
+    StreamScratch& operator=(const StreamScratch&) = delete;
+    ~StreamScratch() {
+        for (void* p : ptrs_) cudaFreeAsync(p, st_);
+    }
+    template <class T>
+    int alloc(T** out, size_t n) {   // max(n, 1) elements
+        void* p = nullptr;
+        BR_TRY(scratch_alloc(&p, sizeof(T) * std::max<size_t>(n, 1), st_));
+        ptrs_.push_back(p);
+        *out = static_cast<T*>(p);
         return BR_OK;
     }
-    ~AsyncBuf() { if (p) cudaFreeAsync(p, st); }
+
+  private:
+    cudaStream_t st_;
+    std::vector<void*> ptrs_;
 };
 
 constexpr int kNumSMs = 148;          // B200
@@ -148,16 +193,16 @@ struct br_index {
     double k1 = 1.5, b = 0.75, n_stat = 0, sum_dl_stat = 0, avgdl = 0;
 
     // CSR by term (device)
-    int64_t* row_ptr = nullptr;     // [V+1]
-    br_posting* post = nullptr;     // [nnz]   doc ids ascending inside a term
-    br_posting* post_cos = nullptr; // [nnz]   optional TF-IDF cosine weights tf*idf^2/||d|| (br_index_enable_tfidf)
-    double* cos_inv_norm = nullptr; // [N]     1/||d|| of the doc's float32 tf*idf vector, float64 (with post_cos)
-    uint16_t* tf = nullptr;         // [nnz]   raw term frequency (for the float64 re-score)
-    uint32_t* dl = nullptr;         // [N]
-    uint32_t* df = nullptr;         // [V]     shard-local document frequency
-    double* idf = nullptr;          // [V]     statistics in force (NaN where df_stat == 0)
-    float* ub = nullptr;            // [V]     largest posting weight of the term on this shard (0 when none / negative):
-                                    //         the per-term score upper bound of the tiled scorer's MaxScore deferral
+    br::DevArray<int64_t> row_ptr;     // [V+1]
+    br::DevArray<br_posting> post;     // [nnz]   doc ids ascending inside a term
+    br::DevArray<br_posting> post_cos; // [nnz]   optional TF-IDF cosine weights tf*idf^2/||d|| (br_index_enable_tfidf)
+    br::DevArray<double> cos_inv_norm; // [N]     1/||d|| of the doc's float32 tf*idf vector, float64 (with post_cos)
+    br::DevArray<uint16_t> tf;         // [nnz]   raw term frequency (for the float64 re-score)
+    br::DevArray<uint32_t> dl;         // [N]
+    br::DevArray<uint32_t> df;         // [V]     shard-local document frequency
+    br::DevArray<double> idf;          // [V]     statistics in force (NaN where df_stat == 0)
+    br::DevArray<float> ub;            // [V]     largest posting weight of the term on this shard (0 when none / negative):
+                                       //         the per-term score upper bound of the tiled scorer's MaxScore deferral
 
     // hot-term skip tables for the tiled scorer: term t is "hot" when hot_slot[t] >= 0; then
     // skip[hot_slot[t] * (n_sub+1) + j] = offset (relative to row_ptr[t]) of the first posting
@@ -165,17 +210,17 @@ struct br_index {
     int sub_shift = 0;
     int32_t n_sub = 0, n_hot = 0;
     uint32_t hot_min = 0;           // smallest df with a skip table
-    int32_t* hot_slot = nullptr;    // [V]
-    uint32_t* skip = nullptr;       // [n_hot, n_sub+1]
+    br::DevArray<int32_t> hot_slot;    // [V]
+    br::DevArray<uint32_t> skip;       // [n_hot, n_sub+1]
     // dense rows: w[row][doc] as plain fp32 rows (0 where the doc lacks the term), most frequent term first.
     // Rows [0, n_srows) - terms present in >= ~20% of the docs - are STREAMED by the tiled scorer (accumulators are
     // initialised from them instead of walking their postings); all n_rows rows (terms with df >= N/64) serve as
     // LOOK-UP tables: a term the scorer has deferred (MaxScore) is added to a candidate doc with one 4-byte load.
-    float* dense_rows = nullptr;    // [n_rows, n_pad]
-    int16_t* row_slot = nullptr;    // [V] row index or -1
+    br::DevArray<float> dense_rows;    // [n_rows, n_pad]
+    br::DevArray<int16_t> row_slot;    // [V] row index or -1
     int32_t n_rows = 0, n_srows = 0;
     int64_t n_pad = 0;
-    int8_t* sig_bit = nullptr;      // [V] rank (0 = largest df) among the 32 most frequent terms, -1 otherwise
+    br::DevArray<int8_t> sig_bit;      // [V] rank (0 = largest df) among the 32 most frequent terms, -1 otherwise
 
     // host mirrors
     std::vector<uint32_t> h_df;     // shard-local
@@ -200,6 +245,9 @@ struct br_index {
     bool profiling = false;
     std::vector<cudaEvent_t> ev_pool;   // pairs (start, stop)
     size_t ev_used = 0;
+    ~br_index() {
+        for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
+    }
     void prof_begin(cudaStream_t st) {
         if (!profiling) return;
         if (ev_used + 2 > ev_pool.size()) {

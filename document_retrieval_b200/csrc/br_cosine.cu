@@ -1195,10 +1195,11 @@ int launch_cos_gather(const void* docs, const float* inv_nd, int64_t n_docs, int
 // the top k ids by (score desc, id asc), a repeated id once, with their scores as fp32; -1 / 0.0 pad the rest.
 static int select_fixed(const int32_t* ids, const double* s64, int32_t nq, int32_t c, int32_t k, int32_t* out_ids,
                         float* out_sims, cudaStream_t st) {
-    AsyncBuf b_o64(st);
-    BR_TRY(b_o64.alloc(8 * (size_t)nq * k));
-    BR_TRY(launch_final_select(ids, s64, nullptr, 0, nq, k, 0, out_ids, (double*)b_o64.p, nullptr, st, nullptr, c));
-    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, (const double*)b_o64.p, (int64_t)nq * k, out_sims);
+    StreamScratch tmp(st);
+    double* o64;
+    BR_TRY(tmp.alloc(&o64, (size_t)nq * k));
+    BR_TRY(launch_final_select(ids, s64, nullptr, 0, nq, k, 0, out_ids, o64, nullptr, st, nullptr, c));
+    k_rerank_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, o64, (int64_t)nq * k, out_sims);
     BR_CUDA(cudaGetLastError());
     return BR_OK;
 }
@@ -1209,9 +1210,10 @@ static int select_fixed(const int32_t* ids, const double* s64, int32_t nq, int32
 static int check_row_group(const int32_t* row_group, int64_t n_rows, int32_t n_groups, int32_t k, const std::string& fn,
                            cudaStream_t st, int64_t* r_k, int64_t* n_nonempty) {
     const int32_t n_blk = (int32_t)((n_rows + GC_ROWS - 1) / GC_ROWS);
-    AsyncBuf b_lay(st);
-    BR_TRY(b_lay.alloc(4 * (size_t)n_blk + 8 * ((size_t)n_blk + 1) + 16));
-    int64_t* excl = (int64_t*)b_lay.p;
+    StreamScratch tmp(st);
+    unsigned char* lay;
+    BR_TRY(tmp.alloc(&lay, 4 * (size_t)n_blk + 8 * ((size_t)n_blk + 1) + 16));
+    int64_t* excl = (int64_t*)lay;
     int32_t* blk = (int32_t*)(excl + n_blk + 1);
     int32_t* info = blk + n_blk;
     BR_CUDA(cudaMemsetAsync(info, 0, 16, st));
@@ -1294,37 +1296,38 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
         BR_CUDA(cudaFuncSetAttribute(k_cosine_gemm_mc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CG_SMEM));
     }
     const size_t Q = (size_t)nq;
-    AsyncBuf b_inq(st), b_thr(st), b_cnt(st), b_prev(st), b_ovf(st), b_cand(st), b_h(st), b_frow(st);
-    BR_TRY(b_inq.alloc(4 * Q)); BR_TRY(b_thr.alloc(4 * Q)); BR_TRY(b_cnt.alloc(4 * Q)); BR_TRY(b_prev.alloc(4 * Q));
-    BR_TRY(b_ovf.alloc(4 * Q)); BR_TRY(b_cand.alloc(4 * Q * COS_CAP)); BR_TRY(b_h.alloc(4 * Q * COS_CAP));
+    StreamScratch tmp(st);
+    float *inv_nq, *thr, *h;
+    int32_t *cnt, *prev, *ovf_d, *cand;
+    BR_TRY(tmp.alloc(&inv_nq, Q)); BR_TRY(tmp.alloc(&thr, Q)); BR_TRY(tmp.alloc(&cnt, Q)); BR_TRY(tmp.alloc(&prev, Q));
+    BR_TRY(tmp.alloc(&ovf_d, Q)); BR_TRY(tmp.alloc(&cand, Q * COS_CAP)); BR_TRY(tmp.alloc(&h, Q * COS_CAP));
     DocFilter fv{};
     int32_t* f_bad = nullptr;
     if (filt) {                                           // [nq] validated rows + the "bad row" flag
-        BR_TRY(b_frow.alloc(4 * Q + 16));
-        f_bad = (int32_t*)b_frow.p + Q;
+        int32_t* frow;
+        BR_TRY(tmp.alloc(&frow, Q + 4));
+        f_bad = frow + Q;
         BR_CUDA(cudaMemsetAsync(f_bad, 0, 4, st));
-        k_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, (int32_t*)b_frow.p, f_bad);
+        k_filter_rows<<<blocks_for(nq, 256), 256, 0, st>>>(filter->query_row_dev, nq, filter->n_rows, frow, f_bad);
         BR_CUDA(cudaGetLastError());
-        fv = DocFilter{filter->bits_dev, filter->words, (const int32_t*)b_frow.p};
+        fv = DocFilter{filter->bits_dev, filter->words, frow};
     }
-    AsyncBuf b_rbits(st);
     if (filt && grp) {                                    // the group filter as a row filter: the GEMMs test rows
         const int64_t rwords = (n_docs + 31) / 32, n_words = (int64_t)filter->n_rows * rwords;
-        BR_TRY(b_rbits.alloc(4 * (size_t)n_words));
+        uint32_t* rbits;
+        BR_TRY(tmp.alloc(&rbits, (size_t)n_words));
         k_group_filter_rows<<<(unsigned)std::min<int64_t>((n_words + 7) / 8, kNumSMs * 64), 256, 0, st>>>(
-            filter->bits_dev, filter->words, filter->n_rows, row_group, n_docs, rwords, (uint32_t*)b_rbits.p);
+            filter->bits_dev, filter->words, filter->n_rows, row_group, n_docs, rwords, rbits);
         BR_CUDA(cudaGetLastError());
-        fv.bits = (const uint32_t*)b_rbits.p;
+        fv.bits = rbits;
         fv.words = rwords;
     }
-    float* inv_nq = (float*)b_inq.p;
-    float* thr = (float*)b_thr.p;
     BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
     std::vector<float> ninf(Q, -INFINITY);
     BR_CUDA(cudaMemcpyAsync(thr, ninf.data(), 4 * Q, cudaMemcpyHostToDevice, st));
-    BR_CUDA(cudaMemsetAsync(b_cnt.p, 0, 4 * Q, st));
-    BR_CUDA(cudaMemsetAsync(b_prev.p, 0, 4 * Q, st));
-    BR_CUDA(cudaMemsetAsync(b_ovf.p, 0, 4 * Q, st));
+    BR_CUDA(cudaMemsetAsync(cnt, 0, 4 * Q, st));
+    BR_CUDA(cudaMemsetAsync(prev, 0, 4 * Q, st));
+    BR_CUDA(cudaMemsetAsync(ovf_d, 0, 4 * Q, st));
     // doc chunks of growing size: thresholds learnt on the docs so far filter the next chunk.  A launch emits about
     // k (growth - 1) candidates per query whatever its size; measured on the config-5 shard an emission costs ~1.7 ns of
     // wall time, which makes doubling (13 launches, ~120 emissions per query) faster than 3x / 4x / 8x growth
@@ -1332,8 +1335,7 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     constexpr int tighten_t = 64;
     const auto tighten = grp ? k_tighten_cos<true> : k_tighten_cos<false>;
     BR_TRY(for_each_cos_launch(n_dt, warm_tiles, warm_cap, grow, [&](int t0, int nt) {
-        CosArgs a{inv_nd, inv_nq, thr, (int32_t*)b_cnt.p, (int32_t*)b_cand.p, (float*)b_h.p, n_docs, nq, d, t0, t0 + nt,
-                  QS_WINDOW, fv};
+        CosArgs a{inv_nd, inv_nq, thr, cnt, cand, h, n_docs, nq, d, t0, t0 + nt, QS_WINDOW, fv};
         if (use_qs) {
             const int64_t units = (int64_t)nt * ((nq + QS_BN - 1) / QS_BN);
             const int grid = 2 * (int)std::min<int64_t>(units, kNumSMs / 2);
@@ -1345,17 +1347,15 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
             else k_cosine_gemm_mc<false><<<grid, CG_THREADS, CG_SMEM, st>>>(map_d, map_q, a);
         }
         BR_CUDA(cudaGetLastError());
-        tighten<<<nq, tighten_t, 0, st>>>(thr, (int32_t*)b_cnt.p, (int32_t*)b_prev.p, (int32_t*)b_cand.p, (float*)b_h.p, row_group, k,
-                                          (int32_t*)b_ovf.p);
+        tighten<<<nq, tighten_t, 0, st>>>(thr, cnt, prev, cand, h, row_group, k, ovf_d);
         BR_CUDA(cudaGetLastError());
         return BR_OK;
     }));
-    k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>((int32_t*)b_cand.p, (float*)b_h.p, (int32_t*)b_cnt.p, row_group,
-                                                                    nq, k, doc_base, out_ids, out_sims);
+    k_cos_output<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(cand, h, cnt, row_group, nq, k, doc_base, out_ids, out_sims);
     BR_CUDA(cudaGetLastError());
     std::vector<int32_t> ovf(Q);
     int32_t h_fbad = 0;
-    BR_CUDA(cudaMemcpyAsync(ovf.data(), b_ovf.p, 4 * Q, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaMemcpyAsync(ovf.data(), ovf_d, 4 * Q, cudaMemcpyDeviceToHost, st));
     if (f_bad) BR_CUDA(cudaMemcpyAsync(&h_fbad, f_bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
     BR_REQUIRE(!h_fbad, BR_ERR_INVALID, fn + ": a filter query_row is outside [-1, n_rows)");
@@ -1378,40 +1378,39 @@ int cosine_topk(const void* docs, const float* inv_nd, int64_t n_docs, int32_t d
     const int32_t sub = 64;
     const int32_t nr_max = (int32_t)std::min<size_t>(redo.size(), (size_t)sub);
     const int32_t c = grp ? grp->n_groups : (int32_t)n_docs;   // ids per redone query
-    AsyncBuf b_q(st), b_inr(st), b_rows(st), b_c(st), b_s(st), b_id(st), b_s64(st), b_goff(st), b_oi(st), b_os(st);
-    BR_TRY(b_q.alloc((size_t)nr_max * d * 2)); BR_TRY(b_inr.alloc(4 * (size_t)nr_max)); BR_TRY(b_rows.alloc(4 * (size_t)nr_max));
-    BR_TRY(b_c.alloc(4 * (size_t)nr_max * (size_t)n_docs)); BR_TRY(b_s.alloc(4 * (size_t)nr_max * (size_t)n_docs));
-    BR_TRY(b_s64.alloc(8 * (size_t)nr_max * (size_t)c));
-    BR_TRY(b_oi.alloc(4 * (size_t)nr_max * k)); BR_TRY(b_os.alloc(4 * (size_t)nr_max * k));
+    char* r_q;
+    float *r_inr, *r_s, *r_os;
+    int32_t *r_rows, *r_c, *r_id = nullptr, *r_goff, *r_oi;
+    double* r_s64;
+    BR_TRY(tmp.alloc(&r_q, (size_t)nr_max * d * 2)); BR_TRY(tmp.alloc(&r_inr, (size_t)nr_max)); BR_TRY(tmp.alloc(&r_rows, (size_t)nr_max));
+    BR_TRY(tmp.alloc(&r_c, (size_t)nr_max * (size_t)n_docs)); BR_TRY(tmp.alloc(&r_s, (size_t)nr_max * (size_t)n_docs));
+    BR_TRY(tmp.alloc(&r_s64, (size_t)nr_max * (size_t)c));
+    BR_TRY(tmp.alloc(&r_oi, (size_t)nr_max * k)); BR_TRY(tmp.alloc(&r_os, (size_t)nr_max * k));
     if (grp) {
-        BR_TRY(b_id.alloc(4 * (size_t)nr_max * (size_t)c)); BR_TRY(b_goff.alloc(4 * ((size_t)c + 1)));
-        k_group_offsets<<<blocks_for((int64_t)c + 1, 256), 256, 0, st>>>(row_group, n_docs, c, (int32_t*)b_goff.p);
+        BR_TRY(tmp.alloc(&r_id, (size_t)nr_max * (size_t)c)); BR_TRY(tmp.alloc(&r_goff, (size_t)c + 1));
+        k_group_offsets<<<blocks_for((int64_t)c + 1, 256), 256, 0, st>>>(row_group, n_docs, c, r_goff);
         BR_CUDA(cudaGetLastError());
     }
-    const int32_t* ids = grp ? (const int32_t*)b_id.p : (const int32_t*)b_c.p;
+    const int32_t* ids = grp ? r_id : r_c;
     for (size_t r0 = 0; r0 < redo.size(); r0 += (size_t)sub) {
         const int32_t nr = (int32_t)std::min<size_t>((size_t)sub, redo.size() - r0);
         for (int32_t i = 0; i < nr; ++i)
-            BR_CUDA(cudaMemcpyAsync((char*)b_q.p + (size_t)i * d * 2, (const char*)queries + (size_t)redo[r0 + (size_t)i] * d * 2,
+            BR_CUDA(cudaMemcpyAsync(r_q + (size_t)i * d * 2, (const char*)queries + (size_t)redo[r0 + (size_t)i] * d * 2,
                                     (size_t)d * 2, cudaMemcpyDeviceToDevice, st));
-        BR_CUDA(cudaMemcpyAsync(b_rows.p, redo.data() + r0, 4 * (size_t)nr, cudaMemcpyHostToDevice, st));
-        BR_TRY(row_inv_norms(b_q.p, nr, d, (float*)b_inr.p, st));
-        k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>((int32_t*)b_c.p, nr, n_docs, (const int32_t*)b_rows.p, fv);
+        BR_CUDA(cudaMemcpyAsync(r_rows, redo.data() + r0, 4 * (size_t)nr, cudaMemcpyHostToDevice, st));
+        BR_TRY(row_inv_norms(r_q, nr, d, r_inr, st));
+        k_iota_rows<<<kNumSMs * 8, 256, 0, st>>>(r_c, nr, n_docs, r_rows, fv);
         BR_CUDA(cudaGetLastError());
-        BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, b_q.p, (const float*)b_inr.p, nr, (const int32_t*)b_c.p, (int32_t)n_docs,
-                                 (float*)b_s.p, nullptr, st));
+        BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, r_q, r_inr, nr, r_c, (int32_t)n_docs, r_s, nullptr, st));
         if (grp)
-            k_group_max<<<kNumSMs * 8, 256, 0, st>>>((const float*)b_s.p, nr, n_docs, (const int32_t*)b_goff.p, c, (int32_t*)b_id.p,
-                                                     (double*)b_s64.p);
+            k_group_max<<<kNumSMs * 8, 256, 0, st>>>(r_s, nr, n_docs, r_goff, c, r_id, r_s64);
         else
-            k_f32_to_f64<<<blocks_for((int64_t)nr * n_docs, 256), 256, 0, st>>>((const float*)b_s.p, (int64_t)nr * n_docs,
-                                                                               (double*)b_s64.p);
+            k_f32_to_f64<<<blocks_for((int64_t)nr * n_docs, 256), 256, 0, st>>>(r_s, (int64_t)nr * n_docs, r_s64);
         BR_CUDA(cudaGetLastError());
-        BR_TRY(select_fixed(ids, (const double*)b_s64.p, nr, c, k, (int32_t*)b_oi.p, (float*)b_os.p, st));
-        k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>((const int32_t*)b_rows.p, nr, k, (const int32_t*)b_oi.p,
-                                                                      (const float*)b_os.p, doc_base, out_ids, out_sims);
+        BR_TRY(select_fixed(ids, r_s64, nr, c, k, r_oi, r_os, st));
+        k_cos_patch<<<blocks_for((int64_t)nr * k, 256), 256, 0, st>>>(r_rows, nr, k, r_oi, r_os, doc_base, out_ids, out_sims);
         BR_CUDA(cudaGetLastError());
-        BR_CUDA(cudaStreamSynchronize(st));               // the next sub-batch rewrites b_q and b_rows
+        BR_CUDA(cudaStreamSynchronize(st));               // the next sub-batch rewrites r_q and r_rows
     }
     return BR_OK;
 }
@@ -1423,15 +1422,17 @@ int cosine_rerank(const void* docs, const float* inv_nd, int64_t n_docs, int32_t
     BR_REQUIRE(d > 0 && d % 8 == 0, BR_ERR_UNSUPPORTED, "br_cosine_rerank: embedding dim must be a multiple of 8");
     if (nq == 0) return BR_OK;
     const int64_t n_pairs = (int64_t)nq * c;
-    AsyncBuf b_inq(st), b_s(st), b_s64(st);
-    BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_s.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
-    int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_docs)
+    StreamScratch tmp(st);
+    float *inv_nq, *s;
+    double* s64;
+    BR_TRY(tmp.alloc(&inv_nq, (size_t)nq + 4)); BR_TRY(tmp.alloc(&s, (size_t)n_pairs)); BR_TRY(tmp.alloc(&s64, (size_t)n_pairs));
+    int32_t* bad = (int32_t*)(inv_nq + nq);                // a candidate id outside [-1, n_docs)
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
-    BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
-    BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, (const float*)b_inq.p, nq, cand, c, (float*)b_s.p, bad, st));
-    k_f32_to_f64<<<blocks_for(n_pairs, 256), 256, 0, st>>>((const float*)b_s.p, n_pairs, (double*)b_s64.p);
+    BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
+    BR_TRY(launch_cos_gather(docs, inv_nd, n_docs, d, queries, inv_nq, nq, cand, c, s, bad, st));
+    k_f32_to_f64<<<blocks_for(n_pairs, 256), 256, 0, st>>>(s, n_pairs, s64);
     BR_CUDA(cudaGetLastError());
-    BR_TRY(select_fixed(cand, (const double*)b_s64.p, nq, c, k, out_ids, out_sims, st));
+    BR_TRY(select_fixed(cand, s64, nq, c, k, out_ids, out_sims, st));
     int32_t h_bad = 0;
     BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));
@@ -1445,13 +1446,14 @@ int launch_cos_gather_grouped(const void* docs, const float* inv_nd, int64_t n_r
                               cudaStream_t st) {
     int64_t r_k, n_nonempty;                               // not used here
     BR_TRY(check_row_group(row_group, n_rows, n_groups, 1, fn, st, &r_k, &n_nonempty));
-    AsyncBuf b_off(st);
-    BR_TRY(b_off.alloc(4 * ((size_t)n_groups + 1)));
-    k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, (int32_t*)b_off.p);
+    StreamScratch tmp(st);
+    int32_t* goff;
+    BR_TRY(tmp.alloc(&goff, (size_t)n_groups + 1));
+    k_group_offsets<<<blocks_for((int64_t)n_groups + 1, 256), 256, 0, st>>>(row_group, n_rows, n_groups, goff);
     BR_CUDA(cudaGetLastError());
     const int nv = (d / 8 + 31) / 32;
     auto launch = [&](auto kern) {
-        kern<<<nq, RG_T, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, d, (const int32_t*)b_off.p, n_groups,
+        kern<<<nq, RG_T, 0, st>>>((const __nv_bfloat16*)docs, inv_nd, d, goff, n_groups,
                                   (const __nv_bfloat16*)queries, inv_nq, cand, c, out_ids, out_s64, bad);
     };
     if (nv <= 1) launch(k_cosine_rerank_grouped<1>);
@@ -1475,14 +1477,17 @@ int cosine_rerank_grouped(const void* docs, const float* inv_nd, int64_t n_rows,
     if (nq == 0) return BR_OK;
     // per candidate (group or -1, best cosine), then the same selection as cosine_rerank
     const int64_t n_pairs = (int64_t)nq * c;
-    AsyncBuf b_inq(st), b_id(st), b_s64(st);
-    BR_TRY(b_inq.alloc(4 * (size_t)nq + 16)); BR_TRY(b_id.alloc(4 * (size_t)n_pairs)); BR_TRY(b_s64.alloc(8 * (size_t)n_pairs));
-    int32_t* bad = (int32_t*)b_inq.p + nq;                 // a candidate id outside [-1, n_groups)
+    StreamScratch tmp(st);
+    float* inv_nq;
+    int32_t* ids;
+    double* s64;
+    BR_TRY(tmp.alloc(&inv_nq, (size_t)nq + 4)); BR_TRY(tmp.alloc(&ids, (size_t)n_pairs)); BR_TRY(tmp.alloc(&s64, (size_t)n_pairs));
+    int32_t* bad = (int32_t*)(inv_nq + nq);                // a candidate id outside [-1, n_groups)
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
-    BR_TRY(row_inv_norms(queries, nq, d, (float*)b_inq.p, st));
-    BR_TRY(launch_cos_gather_grouped(docs, inv_nd, n_rows, d, row_group, n_groups, queries, (const float*)b_inq.p, nq, cand, c,
-                                     (int32_t*)b_id.p, (double*)b_s64.p, bad, fn, st));
-    BR_TRY(select_fixed((const int32_t*)b_id.p, (const double*)b_s64.p, nq, c, k, out_ids, out_sims, st));
+    BR_TRY(row_inv_norms(queries, nq, d, inv_nq, st));
+    BR_TRY(launch_cos_gather_grouped(docs, inv_nd, n_rows, d, row_group, n_groups, queries, inv_nq, nq, cand, c, ids, s64, bad,
+                                     fn, st));
+    BR_TRY(select_fixed(ids, s64, nq, c, k, out_ids, out_sims, st));
     int32_t h_bad = 0;
     BR_CUDA(cudaMemcpyAsync(&h_bad, bad, 4, cudaMemcpyDeviceToHost, st));
     BR_CUDA(cudaStreamSynchronize(st));

@@ -224,15 +224,15 @@ int fuse_rrf(const int32_t* B, int32_t nb, const int32_t* D, int32_t nd, int64_t
     if (nq == 0) return BR_OK;
     const int32_t W = nb + nd;
     const size_t n = (size_t)nq * W;
-    AsyncBuf b_ids(st), b_f(st), b_cnt(st);
-    BR_TRY(b_ids.alloc(4 * n)); BR_TRY(b_f.alloc(8 * n)); BR_TRY(b_cnt.alloc(4 * (size_t)nq + 16));
-    int32_t* u_cnt = (int32_t*)b_cnt.p;
+    StreamScratch tmp(st);
+    int32_t *u_ids, *u_cnt;
+    double* f;
+    BR_TRY(tmp.alloc(&u_ids, n)); BR_TRY(tmp.alloc(&f, n)); BR_TRY(tmp.alloc(&u_cnt, (size_t)nq + 4));
     int32_t* bad = u_cnt + nq;
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
-    k_fuse_union<<<nq, FU_T, 0, st>>>(B, nb, D, nd, n_docs, 1, rrf_c, w_b, w_d, (int32_t*)b_ids.p, u_cnt, (double*)b_f.p, bad);
+    k_fuse_union<<<nq, FU_T, 0, st>>>(B, nb, D, nd, n_docs, 1, rrf_c, w_b, w_d, u_ids, u_cnt, f, bad);
     BR_CUDA(cudaGetLastError());
-    BR_TRY(launch_final_select((const int32_t*)b_ids.p, (const double*)b_f.p, nullptr, 0, nq, k, 0, out_ids, out_scores,
-                               out_counts, st, u_cnt, W));
+    BR_TRY(launch_final_select(u_ids, f, nullptr, 0, nq, k, 0, out_ids, out_scores, out_counts, st, u_cnt, W));
     return report_bad(bad, nullptr, fn, "n_docs", st);
 }
 
@@ -253,15 +253,14 @@ int fuse_linear(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
     BR_CUDA(cudaSetDevice(ix->device));
     const int32_t W = nb + nd;
     const size_t n = (size_t)nq * W;
-    AsyncBuf b_ids(st), b_f(st), b_sb(st), b_sc(st), b_cnt(st), b_gid(st), b_g64(st);
-    BR_TRY(b_ids.alloc(4 * n)); BR_TRY(b_f.alloc(8 * n)); BR_TRY(b_sb.alloc(8 * n)); BR_TRY(b_sc.alloc(4 * n));
-    BR_TRY(b_cnt.alloc(8 * (size_t)nq + 16));
-    int32_t* u_ids = (int32_t*)b_ids.p;
-    int32_t* u_cnt = (int32_t*)b_cnt.p;
+    StreamScratch tmp(st);
+    int32_t *u_ids, *u_cnt;
+    double *f, *s_b;
+    float* s_c;
+    BR_TRY(tmp.alloc(&u_ids, n)); BR_TRY(tmp.alloc(&f, n)); BR_TRY(tmp.alloc(&s_b, n)); BR_TRY(tmp.alloc(&s_c, n));
+    BR_TRY(tmp.alloc(&u_cnt, 2 * (size_t)nq + 4));
     float* inv_nq = (float*)(u_cnt + nq);
     int32_t* bad = u_cnt + 2 * nq;
-    double* s_b = (double*)b_sb.p;
-    float* s_c = (float*)b_sc.p;
     BR_CUDA(cudaMemsetAsync(bad, 0, 4, st));
     k_fuse_union<<<nq, FU_T, 0, st>>>(B, nb, D, nd, ix->n_docs, 0, 0.0, 0.0, 0.0, u_ids, u_cnt, nullptr, bad);
     BR_CUDA(cudaGetLastError());
@@ -275,17 +274,19 @@ int fuse_linear(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
     const int32_t* g_ids = nullptr;
     const double* g_s64 = nullptr;
     if (row_group) {
-        BR_TRY(b_gid.alloc(4 * n)); BR_TRY(b_g64.alloc(8 * n));
+        int32_t* gid;
+        double* g64;
+        BR_TRY(tmp.alloc(&gid, n)); BR_TRY(tmp.alloc(&g64, n));
         BR_TRY(launch_cos_gather_grouped(docs, inv_nd, n_rows, d, row_group, (int32_t)ix->n_docs, queries, inv_nq, nq, u_ids, W,
-                                         (int32_t*)b_gid.p, (double*)b_g64.p, bad, fn, st));
-        g_ids = (const int32_t*)b_gid.p;
-        g_s64 = (const double*)b_g64.p;
+                                         gid, g64, bad, fn, st));
+        g_ids = gid;
+        g_s64 = g64;
     } else {
         BR_TRY(launch_cos_gather(docs, inv_nd, n_rows, d, queries, inv_nq, nq, u_ids, W, s_c, nullptr, st));
     }
-    k_fuse_linear<<<nq, FL_T, 0, st>>>(u_cnt, W, s_b, s_c, g_ids, g_s64, alpha, (double*)b_f.p, s_c);
+    k_fuse_linear<<<nq, FL_T, 0, st>>>(u_cnt, W, s_b, s_c, g_ids, g_s64, alpha, f, s_c);
     BR_CUDA(cudaGetLastError());
-    BR_TRY(launch_final_select(u_ids, (const double*)b_f.p, nullptr, 0, nq, k, 0, out_ids, out_scores, out_counts, st, u_cnt, W));
+    BR_TRY(launch_final_select(u_ids, f, nullptr, 0, nq, k, 0, out_ids, out_scores, out_counts, st, u_cnt, W));
     if (out_bm25 || out_cos) {
         k_fuse_components<<<blocks_for((int64_t)nq * k, 256), 256, 0, st>>>(out_ids, nq, k, u_ids, u_cnt, W, s_b, s_c, out_bm25,
                                                                             out_cos);

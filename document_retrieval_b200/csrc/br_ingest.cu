@@ -17,6 +17,8 @@
 //                 collision is reported as an error instead of silently merging two terms
 //   k_pool_len / k_pool_fill     vocabulary strings into one byte pool (-> Python `terms`, query-time verification)
 //   k_lookup      query tokens: binary search in the sorted hash table + byte compare -> term id or -1 (OOV)
+#include <memory>
+
 #include <cub/cub.cuh>
 
 #include "br_kernels.cuh"
@@ -24,10 +26,10 @@
 struct br_vocab {
     int device = 0;
     int64_t n_terms = 0, pool_bytes = 0;
-    uint64_t* hash_sorted = nullptr;   // [V] ascending
-    int32_t* term_sorted = nullptr;    // [V] term id of hash_sorted[i]
-    int64_t* pool_off = nullptr;       // [V+1]
-    uint8_t* pool = nullptr;           // [pool_bytes]
+    br::DevArray<uint64_t> hash_sorted;   // [V] ascending
+    br::DevArray<int32_t> term_sorted;    // [V] term id of hash_sorted[i]
+    br::DevArray<int64_t> pool_off;       // [V+1]
+    br::DevArray<uint8_t> pool;           // [pool_bytes]
 };
 
 namespace br {
@@ -320,21 +322,6 @@ __global__ void __launch_bounds__(256) k_lookup(const uint8_t* __restrict__ text
     token_ids[i] = term;
 }
 
-struct Tmp {   // stream-ordered temporaries, released when the call returns
-    cudaStream_t st;
-    std::vector<void*> ptrs;
-    explicit Tmp(cudaStream_t s) : st(s) {}
-    ~Tmp() { for (void* p : ptrs) if (p) cudaFreeAsync(p, st); }
-    template <class T>
-    int alloc(T** out, size_t n) {
-        void* p = nullptr;
-        BR_TRY(scratch_alloc(&p, sizeof(T) * (n > 0 ? n : 1), st));
-        ptrs.push_back(p);
-        *out = reinterpret_cast<T*>(p);
-        return BR_OK;
-    }
-};
-
 int report_bad(int bad, const char* who) {
     if (bad & 2) { set_error(std::string(who) + ": byte offsets not non-decreasing"); return BR_ERR_INVALID; }
     if (bad & 4) { set_error(std::string(who) + ": a document of 2 GiB or more"); return BR_ERR_UNSUPPORTED; }
@@ -343,7 +330,7 @@ int report_bad(int bad, const char* who) {
 }
 
 // (start, len) of every token, given the per-document token offsets of tokenize_count
-int emit_tokens(Tmp& tmp, const uint8_t* text, const int64_t* doc_off, int64_t n_docs, int bigrams,
+int emit_tokens(StreamScratch& tmp, const uint8_t* text, const int64_t* doc_off, int64_t n_docs, int bigrams,
                 const int64_t* doc_tok_off, int64_t n_tok, cudaStream_t st, int64_t** tok_start, uint32_t** tok_len) {
     BR_TRY(tmp.alloc(tok_start, (size_t)n_tok));
     BR_TRY(tmp.alloc(tok_len, (size_t)n_tok));
@@ -355,7 +342,7 @@ int emit_tokens(Tmp& tmp, const uint8_t* text, const int64_t* doc_off, int64_t n
 }
 
 template <class K, class V>
-int sort_pairs(Tmp& tmp, K** keys, V** vals, int64_t n, int end_bit, cudaStream_t st) {
+int sort_pairs(StreamScratch& tmp, K** keys, V** vals, int64_t n, int end_bit, cudaStream_t st) {
     if (n <= 1) return BR_OK;
     K* k2 = nullptr;
     V* v2 = nullptr;
@@ -373,12 +360,6 @@ int sort_pairs(Tmp& tmp, K** keys, V** vals, int64_t n, int end_bit, cudaStream_
     return BR_OK;
 }
 
-void vocab_free(br_vocab* v) {
-    if (!v) return;
-    cudaFree(v->hash_sorted); cudaFree(v->term_sorted); cudaFree(v->pool_off); cudaFree(v->pool);
-    delete v;
-}
-
 }  // namespace
 }  // namespace br
 
@@ -391,7 +372,7 @@ int br_tokenize_count(const uint8_t* text_dev, const int64_t* doc_byte_off_dev, 
     cudaStream_t st = (cudaStream_t)stream;
     BR_REQUIRE(doc_byte_off_dev && doc_tok_off_dev && n_tokens_host && n_docs >= 0, BR_ERR_INVALID,
                "br_tokenize_count: null pointer / negative n_docs");
-    Tmp tmp(st);
+    StreamScratch tmp(st);
     uint32_t* counts = nullptr;
     int* d_bad = nullptr;
     BR_TRY(tmp.alloc(&counts, (size_t)n_docs));
@@ -420,10 +401,9 @@ int br_vocab_build(const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int
     BR_REQUIRE(n_tokens >= 0 && n_tokens < (1LL << 31), BR_ERR_UNSUPPORTED, "br_vocab_build: 2^31 or more tokens");
     BR_REQUIRE(n_tokens == 0 || token_ids_dev, BR_ERR_INVALID, "br_vocab_build: null token_ids");
     *out = nullptr;
-    br_vocab* v = new br_vocab();
-    struct Guard { br_vocab* p; ~Guard() { if (p) vocab_free(p); } } guard{v};
+    std::unique_ptr<br_vocab> v(new br_vocab());   // a half-built handle: freed unless released
     BR_CUDA(cudaGetDevice(&v->device));
-    Tmp tmp(st);
+    StreamScratch tmp(st);
     const int64_t T = n_tokens;
 
     int64_t* tok_start = nullptr;
@@ -454,9 +434,9 @@ int br_vocab_build(const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int
         BR_CUDA(cudaStreamSynchronize(st));
     }
     v->n_terms = V;
-    BR_CUDA(cudaMalloc(&v->hash_sorted, sizeof(uint64_t) * (size_t)(V > 0 ? V : 1)));
-    BR_CUDA(cudaMalloc(&v->term_sorted, sizeof(int32_t) * (size_t)(V > 0 ? V : 1)));
-    BR_CUDA(cudaMalloc(&v->pool_off, sizeof(int64_t) * (size_t)(V + 1)));
+    BR_TRY(v->hash_sorted.alloc((size_t)V));
+    BR_TRY(v->term_sorted.alloc((size_t)V));
+    BR_TRY(v->pool_off.alloc((size_t)V + 1));
     if (V > 0) {
         BR_TRY(tmp.alloc(&first_tok, (size_t)V));
         BR_TRY(tmp.alloc(&run_id, (size_t)V));
@@ -488,16 +468,15 @@ int br_vocab_build(const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int
         BR_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
         BR_CUDA(cudaStreamSynchronize(st));
         BR_TRY(report_bad(bad, "br_vocab_build"));
-        BR_CUDA(cudaMalloc(&v->pool, (size_t)(v->pool_bytes > 0 ? v->pool_bytes : 1)));
+        BR_TRY(v->pool.alloc((size_t)v->pool_bytes));
         k_pool_fill<<<blocks_for(V, 256), 256, 0, st>>>(text_dev, tok_start, tok_len, first_by_rank, V, v->pool_off, v->pool);
         BR_CUDA(cudaGetLastError());
     } else {
         BR_CUDA(cudaMemsetAsync(v->pool_off, 0, sizeof(int64_t), st));
-        BR_CUDA(cudaMalloc(&v->pool, 1));
+        BR_TRY(v->pool.alloc(0));
     }
     BR_CUDA(cudaStreamSynchronize(st));   // temporaries are freed when tmp goes out of scope
-    guard.p = nullptr;
-    *out = v;
+    *out = v.release();
     return BR_OK;
 }
 
@@ -508,7 +487,7 @@ int br_vocab_lookup(const br_vocab* v, const uint8_t* text_dev, const int64_t* d
     BR_REQUIRE(n_tokens >= 0 && n_tokens < (1LL << 31), BR_ERR_UNSUPPORTED, "br_vocab_lookup: 2^31 or more tokens");
     if (n_tokens == 0) return BR_OK;
     BR_REQUIRE(token_ids_dev, BR_ERR_INVALID, "br_vocab_lookup: null token_ids");
-    Tmp tmp(st);
+    StreamScratch tmp(st);
     int64_t* tok_start = nullptr;
     uint32_t* tok_len = nullptr;
     BR_TRY(emit_tokens(tmp, text_dev, doc_byte_off_dev, n_docs, bigrams, doc_tok_off_dev, n_tokens, st, &tok_start, &tok_len));
@@ -540,21 +519,20 @@ int br_vocab_import(const int64_t* pool_off_host, const uint8_t* pool_host, int6
     cudaStream_t st = (cudaStream_t)stream;
     BR_REQUIRE(out && pool_off_host && n_terms >= 0 && n_terms < (1LL << 31), BR_ERR_INVALID, "br_vocab_import: bad arguments");
     *out = nullptr;
-    br_vocab* v = new br_vocab();
-    struct Guard { br_vocab* p; ~Guard() { if (p) vocab_free(p); } } guard{v};
+    std::unique_ptr<br_vocab> v(new br_vocab());   // a half-built handle: freed unless released
     BR_CUDA(cudaGetDevice(&v->device));
     const int64_t V = n_terms;
     v->n_terms = V;
     v->pool_bytes = pool_off_host[V];
     BR_REQUIRE(pool_off_host[0] == 0 && v->pool_bytes >= 0, BR_ERR_INVALID, "br_vocab_import: bad pool offsets");
-    BR_CUDA(cudaMalloc(&v->hash_sorted, sizeof(uint64_t) * (size_t)(V > 0 ? V : 1)));
-    BR_CUDA(cudaMalloc(&v->term_sorted, sizeof(int32_t) * (size_t)(V > 0 ? V : 1)));
-    BR_CUDA(cudaMalloc(&v->pool_off, sizeof(int64_t) * (size_t)(V + 1)));
-    BR_CUDA(cudaMalloc(&v->pool, (size_t)(v->pool_bytes > 0 ? v->pool_bytes : 1)));
+    BR_TRY(v->hash_sorted.alloc((size_t)V));
+    BR_TRY(v->term_sorted.alloc((size_t)V));
+    BR_TRY(v->pool_off.alloc((size_t)V + 1));
+    BR_TRY(v->pool.alloc((size_t)v->pool_bytes));
     BR_CUDA(cudaMemcpyAsync(v->pool_off, pool_off_host, sizeof(int64_t) * (size_t)(V + 1), cudaMemcpyHostToDevice, st));
     if (v->pool_bytes > 0)
         BR_CUDA(cudaMemcpyAsync(v->pool, pool_host, (size_t)v->pool_bytes, cudaMemcpyHostToDevice, st));
-    Tmp tmp(st);
+    StreamScratch tmp(st);
     if (V > 0) {
         uint64_t* hash = nullptr;
         uint32_t* term = nullptr;
@@ -577,11 +555,10 @@ int br_vocab_import(const int64_t* pool_off_host, const uint8_t* pool_host, int6
         BR_REQUIRE(!(bad & 8), BR_ERR_INVALID, "br_vocab_import: duplicate term (or 64-bit hash collision) in the vocabulary");
     }
     BR_CUDA(cudaStreamSynchronize(st));
-    guard.p = nullptr;
-    *out = v;
+    *out = v.release();
     return BR_OK;
 }
 
-void br_vocab_destroy(br_vocab* v) { vocab_free(v); }
+void br_vocab_destroy(br_vocab* v) { delete v; }
 
 }  // extern "C"

@@ -21,6 +21,8 @@
 // reference's ranking exactly (DESIGN.md, "exactness").
 #include <math_constants.h>
 
+#include <utility>
+
 #include "br_common.cuh"
 #include "br_kernels.cuh"
 #include "br_query.cuh"
@@ -932,14 +934,12 @@ int enable_tfidf(br_index* ix, cudaStream_t st) {
     BR_REQUIRE(ix && ix->finalized, BR_ERR_STATE, "br_index_enable_tfidf: call br_index_finalize first");
     if (ix->post_cos) return BR_OK;
     BR_CUDA(cudaSetDevice(ix->device));
-    BR_CUDA(cudaMalloc(&ix->cos_inv_norm, sizeof(double) * (size_t)ix->n_docs));
-    if (cudaMalloc(&ix->post_cos, sizeof(br_posting) * (size_t)std::max<int64_t>(ix->nnz, 1)) != cudaSuccess) {
-        cudaFree(ix->cos_inv_norm);
-        ix->cos_inv_norm = nullptr;
-        ix->post_cos = nullptr;
-        set_error("br_index_enable_tfidf: out of device memory");
-        return BR_ERR_CUDA;
-    }
+    DevArray<double> inv_norm;               // owned by the index only once both allocations succeed
+    DevArray<br_posting> post_cos;
+    BR_TRY(inv_norm.alloc((size_t)ix->n_docs));
+    BR_TRY(post_cos.alloc((size_t)ix->nnz));
+    ix->cos_inv_norm = std::move(inv_norm);
+    ix->post_cos = std::move(post_cos);
     BR_CUDA(cudaMemsetAsync(ix->cos_inv_norm, 0, sizeof(double) * (size_t)ix->n_docs, st));
     if (ix->nnz > 0) {
         k_tfidf_norm2<<<blocks_for(ix->nnz, 256), 256, 0, st>>>(ix->row_ptr, ix->vocab, ix->nnz, ix->post, ix->tf, ix->idf,

@@ -54,17 +54,16 @@ extern "C" int br_dedupe_first_docs(const int64_t* sentence_ids_dev, const int32
     BR_REQUIRE(nq >= 0 && n >= 0 && k >= 1 && k <= 32, BR_ERR_INVALID, "br_dedupe_first_docs: need nq, n >= 0 and 1 <= k <= 32");
     if (nq == 0) return BR_OK;
     cudaStream_t st = (cudaStream_t)stream;
+    br::StreamScratch tmp(st);
     int* d_bad = nullptr;
-    BR_TRY(br::scratch_alloc((void**)&d_bad, sizeof(int), st));
+    BR_TRY(tmp.alloc(&d_bad, 1));
     BR_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
     br::k_dedupe_first_docs<<<br::blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(sentence_ids_dev, sentence_to_doc_dev, n_sentences,
                                                                                   nq, n, k, out_docs_dev, d_bad);
+    BR_CUDA(cudaGetLastError());
     int bad = 0;
-    cudaError_t e1 = cudaGetLastError();
-    cudaError_t e2 = cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st);
-    cudaError_t e3 = cudaStreamSynchronize(st);
-    cudaFreeAsync(d_bad, st);
-    BR_CUDA(e1); BR_CUDA(e2); BR_CUDA(e3);
+    BR_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
     BR_REQUIRE(!bad, BR_ERR_INVALID, "br_dedupe_first_docs: sentence id outside [0, n_sentences)");
     return BR_OK;
 }

@@ -1197,7 +1197,7 @@ int topk_fused(br_index* ix, const int32_t* q_off, const PrepView& pv, int32_t n
         size_t tmp_bytes = 0;
         BR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, key_in, key_out, val_in, perm, nq, 0, 32, st));
         BR_TRY(ix->ws_sort.reserve(tmp_bytes + 16));
-        BR_CUDA(cub::DeviceRadixSort::SortPairs(ix->ws_sort.p, tmp_bytes, key_in, key_out, val_in, perm, nq, 0, 32, st));
+        BR_CUDA(cub::DeviceRadixSort::SortPairs(ix->ws_sort.as<void>(), tmp_bytes, key_in, key_out, val_in, perm, nq, 0, 32, st));
         k_invert_perm<<<blocks_for(nq, 256), 256, 0, st>>>(perm, nq, inv_perm);
         BR_CUDA(cudaGetLastError());
         ix->stats.kernel_launches += 2;
