@@ -258,8 +258,8 @@ class BM25:
         return out
 
     def get_scores(self, query):
-        """bm25_ranking.ipynb:191-204 -> np.ndarray[float64, (N,)] (fp32 accumulation widened;
-        within 1e-5 relative of the reference)."""
+        """bm25_ranking.ipynb:191-204 -> np.ndarray[float64, (N,)] (fp32 accumulation widened; the
+        error bound of br_score_batch in include/br_b200.h)."""
         return self.get_scores_batch([query])[0].double().cpu().numpy()
 
     calculate_scores = get_scores          # final_implementation.py:127

@@ -123,7 +123,7 @@ __global__ void k_df(const uint32_t* __restrict__ tstart, const uint32_t* __rest
 __global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, int64_t nnz,
                           br_posting* __restrict__ post, const uint16_t* __restrict__ tf,
                           const uint32_t* __restrict__ dl, const double* __restrict__ idf, double avgdl,
-                          double k1, double b, int variant, float* __restrict__ ub) {
+                          double k1, double b, int variant, float* __restrict__ ub, float* __restrict__ amax) {
     const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
     int32_t lo = -1;
@@ -158,7 +158,7 @@ __global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, in
     }
     // ub[t] = max posting weight of term t (the score upper bound of the tiled scorer's deferral): one atomic per
     // (warp, term) - the lanes of a warp hold consecutive postings, i.e. mostly one term.  Weights < 0 (idf without
-    // +1) count as 0; non-negative floats order like their bit patterns.
+    // +1) count as 0; non-negative floats order like their bit patterns.  amax (when not null) gets max |w| the same way.
     unsigned todo = __ballot_sync(0xffffffffu, lo >= 0);
     while (todo) {
         const int leader = __ffs(todo) - 1;
@@ -166,6 +166,10 @@ __global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, in
         const bool mine = lo == t;
         const unsigned mx = __reduce_max_sync(0xffffffffu, mine ? __float_as_uint(fmaxf(wv, 0.f)) : 0u);
         if (lane == leader) atomicMax(reinterpret_cast<unsigned*>(ub) + t, mx);
+        if (amax) {
+            const unsigned ma = __reduce_max_sync(0xffffffffu, mine ? __float_as_uint(fabsf(wv)) : 0u);
+            if (lane == leader) atomicMax(reinterpret_cast<unsigned*>(amax) + t, ma);
+        }
         todo &= ~__ballot_sync(0xffffffffu, mine);
     }
 }
@@ -502,9 +506,16 @@ int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat
     }
     BR_CUDA(cudaMemcpyAsync(ix->idf, ix->h_idf.data(), sizeof(double) * V, cudaMemcpyHostToDevice, st));
     BR_CUDA(cudaMemsetAsync(ix->ub, 0, sizeof(float) * V, st));
+    // only okapi_no_plus1 has negative idf, i.e. queries whose weights can have mixed signs (br_query.cu)
+    if (variant == BR_OKAPI_NO_PLUS1) {
+        if (!ix->amax) BR_TRY(ix->amax.alloc(V));
+        BR_CUDA(cudaMemsetAsync(ix->amax, 0, sizeof(float) * V, st));
+    } else {
+        ix->amax.reset();
+    }
     if (ix->nnz > 0) {
         k_weights<<<blocks_for(ix->nnz, 256), 256, 0, st>>>(ix->row_ptr, ix->vocab, ix->nnz, ix->post, ix->tf,
-                                                            ix->dl, ix->idf, ix->avgdl, k1, b, variant, ix->ub);
+                                                            ix->dl, ix->idf, ix->avgdl, k1, b, variant, ix->ub, ix->amax);
         BR_CUDA(cudaGetLastError());
     }
     // hot-term skip tables (shard-local structure: decided from the local df)

@@ -203,6 +203,8 @@ struct br_index {
     br::DevArray<double> idf;          // [V]     statistics in force (NaN where df_stat == 0)
     br::DevArray<float> ub;            // [V]     largest posting weight of the term on this shard (0 when none / negative):
                                        //         the per-term score upper bound of the tiled scorer's MaxScore deferral
+    br::DevArray<float> amax;          // [V]     largest |posting weight| of the term on this shard; okapi_no_plus1 only
+                                       //         (null otherwise): the fp32 error bound of a query with mixed signs
 
     // hot-term skip tables for the tiled scorer: term t is "hot" when hot_slot[t] >= 0; then
     // skip[hot_slot[t] * (n_sub+1) + j] = offset (relative to row_ptr[t]) of the first posting

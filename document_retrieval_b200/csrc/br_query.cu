@@ -18,7 +18,9 @@
 // near-ties.  Every doc outside the band has fp32 score < kth32*(1-1e-5), hence (fp32 error of a
 // <=64-term positive sum is < 4e-6 relative) a float64 score below that of the k band members that
 // define kth32 - so the true top-k is inside the band, and re-scoring the band in float64 gives the
-// reference's ranking exactly (DESIGN.md, "exactness").
+// reference's ranking exactly (DESIGN.md, "exactness").  A query with a term of negative idf (okapi_no_plus1) sums
+// weights of both signs: its band also reaches kth32 - slack, an absolute bound of the fp32 error, and a hit row tells
+// its docs with a hit from those without (k_select_radix).
 #include <math_constants.h>
 
 #include <utility>
@@ -36,7 +38,7 @@ constexpr int SCORE_CHUNK = 8192;
 
 __global__ void k_prep_queries(const int32_t* __restrict__ q_terms, const int32_t* __restrict__ q_off, int32_t nq,
                                int32_t vocab, const int64_t* __restrict__ row_ptr, const int8_t* __restrict__ sig_bit, int dedup,
-                               PrepView v) {
+                               const double* __restrict__ idf, const float* __restrict__ amax, PrepView v) {
     const int lane = threadIdx.x & 31;
     const int q = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (q >= nq) return;
@@ -96,16 +98,40 @@ __global__ void k_prep_queries(const int32_t* __restrict__ q_terms, const int32_
     if (lane == 0) {
         v.sig[q] = sig;
         int64_t cum = 0;
+        float wsum = 0.f;
+        bool neg = false;
         for (int32_t i = 0; i < n_uniq; ++i) {
             const int32_t t = v.u_terms[off + i];
             v.u_cum[off + i] = cum;
             cum += row_ptr[t + 1] - row_ptr[t];
+            if (amax) {
+                neg |= idf[t] < 0.0;
+                wsum += (float)v.u_mult[off + i] * amax[t];
+            }
         }
+        v.slack[q] = neg ? ldexpf((float)(2 * n_uniq + 6), -24) * wsum : 0.f;
         v.u_cnt[q] = n_uniq;
         v.o_cnt[q] = n_valid;
         v.P[q] = cum;
         v.n_chunks[q] = (uint32_t)((cum + SCORE_CHUNK - 1) / SCORE_CHUNK);
     }
+}
+
+// Hit rows of the dense path's queries with a term of negative idf (PrepView::slack[q] > 0): bit (d & 31) of word
+// (d >> 5) of the query's row is set when doc d holds at least one of its terms.  With mixed signs a doc's fp32 sum can
+// be exactly 0 while its float64 score is not, so "fp32 score 0" no longer means "no hit" for such a query.  slack ==
+// nullptr (other variants, the TF-IDF weight table): no query has a row.  Rows follow the pass's query order.
+struct HitRows {
+    const float* slack;
+    uint32_t* bits;
+    int64_t words;
+    __device__ __forceinline__ uint32_t* row_of(int q, int row) const {
+        return slack && slack[q] > 0.f ? bits + (int64_t)row * words : nullptr;
+    }
+};
+// hr: the query's hit row (nullptr: a query whose weights are all >= 0, where fp32 score 0 means no hit)
+__device__ __forceinline__ bool no_hit(const uint32_t* hr, float s, uint32_t doc) {
+    return hr ? ((hr[doc >> 5] >> (doc & 31)) & 1u) == 0u : s == 0.0f;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -115,7 +141,7 @@ __global__ void __launch_bounds__(256) k_score_dense(const br_posting* __restric
                                                      const int64_t* __restrict__ row_ptr,
                                                      const int32_t* __restrict__ q_off, PrepView v,
                                                      const int64_t* __restrict__ chunk_start, int32_t q_begin,
-                                                     int32_t nq, float* __restrict__ out, int64_t n_docs) {
+                                                     int32_t nq, float* __restrict__ out, int64_t n_docs, HitRows h) {
     const int64_t w_begin = chunk_start[q_begin], w_end = chunk_start[q_begin + nq];
     for (int64_t w = w_begin + blockIdx.x; w < w_end; w += gridDim.x) {
         // query of this work item: last q with chunk_start[q] <= w
@@ -129,6 +155,7 @@ __global__ void __launch_bounds__(256) k_score_dense(const br_posting* __restric
         const int64_t e0 = (w - chunk_start[q]) * SCORE_CHUNK;
         const int64_t e1 = min(e0 + (int64_t)SCORE_CHUNK, v.P[q]);
         float* row = out + (int64_t)(q - q_begin) * n_docs;
+        uint32_t* hr = h.row_of(q, q - q_begin);
         for (int64_t e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
             int32_t a = 0, b = nt;  // last term index with u_cum <= e
             while (b - a > 1) {
@@ -138,6 +165,7 @@ __global__ void __launch_bounds__(256) k_score_dense(const br_posting* __restric
             const int32_t t = v.u_terms[off + a];
             const br_posting p = post[row_ptr[t] + (e - v.u_cum[off + a])];
             atomicAdd(row + p.doc, p.w * (float)v.u_mult[off + a]);
+            if (hr) atomicOr(hr + (p.doc >> 5), 1u << (p.doc & 31));
         }
     }
 }
@@ -145,8 +173,9 @@ __global__ void __launch_bounds__(256) k_score_dense(const br_posting* __restric
 // ------------------------------------------------------------------------------------------
 // radix select
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t score_key(float s, int positive_only) {
-    if (positive_only && s == 0.0f) return 0u;
+// nh: the doc has no hit (no_hit); under positive_only such a doc gets key 0, below every doc with a hit
+__device__ __forceinline__ uint32_t score_key(float s, bool nh, int positive_only) {
+    if (positive_only && nh) return 0u;
     const uint32_t u = __float_as_uint(s);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
@@ -156,8 +185,8 @@ __device__ __forceinline__ float key_score(uint32_t k) {
 
 struct SelView {
     float* lo;         // [nq] band lower bound
-    int32_t* mode;     // [nq] 0 band, 1 band over positives + zero fill, 2 all non-zero
-    int32_t* zfill;    // [nq] number of zero-score docs to take in doc-id order (mode 1)
+    int32_t* mode;     // [nq] 0 band, 1 band over docs with a hit + zero fill, 2 all (with a hit, positive_only)
+    int32_t* zfill;    // [nq] number of docs without a hit to take in doc-id order (mode 1)
     int64_t* cnt;      // [nq] number of candidates the emit kernel writes
 };
 
@@ -169,24 +198,46 @@ constexpr int SEL_T = 1024;
 // kth_key == 0 needs positive_only: without it no non-NaN score has key 0, and k_rem <= n_docs makes the k-th key a
 // doc's own key.  Two CTAs per SM (at most 32 registers): the filter test must not halve the occupancy of the unfiltered
 // select.
+// A query with a term of negative idf (slack sl > 0, hit row hr) widens the band to kth - sl, which bounds the fp32
+// error of a mixed-sign sum where the relative band does not.  Once the band reaches 0 (mode 1) it takes every doc WITH
+// a hit whose fp32 score is >= lo, fp32 zeros included, and fills with docs WITHOUT a hit in doc-id order: all of them
+// score exactly 0, and at most k minus the docs with fp32 score > sl (surely > 0 in float64) belong to the top k.  Under
+// positive_only a doc with a hit can score exactly 0 in float64 (dropped later, by k_final_select); only docs with
+// |fp32| <= sl can, so the select looks for the (k + their number)-th key instead of the k-th.  For every other query
+// (sl == 0, fp32 zero == no hit) each rule reduces to the positive-weight one.
 __global__ void __launch_bounds__(SEL_T, 2) k_select_radix(const float* __restrict__ scores, int64_t n_docs, int32_t k,
                                                         int positive_only, SelView sv, int32_t q_begin,
-                                                        const int32_t* __restrict__ n_terms, DocFilter f) {
+                                                        const int32_t* __restrict__ n_terms, DocFilter f, HitRows h) {
     __shared__ uint32_t hist[2048];
     __shared__ uint32_t s_bin, s_above;
-    __shared__ unsigned long long s_cnt[2];
+    __shared__ unsigned long long s_cnt[3];
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
     const uint32_t* fr = f.row ? f.row_of(q) : nullptr;
+    const uint32_t* hr = h.row_of(q, blockIdx.x);
+    const float sl = hr ? h.slack[q] : 0.f;
     uint32_t prefix = 0, mask = 0;
-    uint32_t k_rem = (uint32_t)min((int64_t)k, n_docs);
+    int64_t k_sel = k;
+    if (threadIdx.x < 3) s_cnt[threadIdx.x] = 0;
+    __syncthreads();
+    if (hr && positive_only) {
+        uint32_t n_amb = 0;
+        for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T)
+            n_amb += doc_allowed(fr, (uint32_t)i) && !no_hit(hr, row[i], (uint32_t)i) && fabsf(row[i]) <= sl;
+        n_amb = __reduce_add_sync(0xffffffffu, n_amb);
+        if ((threadIdx.x & 31) == 0) atomicAdd(&s_cnt[2], (unsigned long long)n_amb);
+        __syncthreads();
+        k_sel += (int64_t)s_cnt[2];
+    }
+    uint32_t k_rem = (uint32_t)min(k_sel, n_docs);
 #pragma unroll 1
     for (int pass = 0; pass < 3; ++pass) {
         const int shift = pass == 0 ? 21 : pass == 1 ? 10 : 0, nb = pass == 2 ? 1024 : 2048;
         for (int i = threadIdx.x; i < 2048; i += SEL_T) hist[i] = 0;
         __syncthreads();
         for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
-            const uint32_t u = doc_allowed(fr, (uint32_t)i) ? score_key(row[i], positive_only) : 0u;
+            const float s = row[i];
+            const uint32_t u = doc_allowed(fr, (uint32_t)i) ? score_key(s, no_hit(hr, s, (uint32_t)i), positive_only) : 0u;
             if ((u & mask) == prefix) atomicAdd(&hist[(u >> shift) & (nb - 1)], 1u);
         }
         __syncthreads();
@@ -211,48 +262,47 @@ __global__ void __launch_bounds__(SEL_T, 2) k_select_radix(const float* __restri
         mode = 2;                                   // fewer than k allowed docs with a hit: take them all
     } else {
         const float kth = key_score(kth_key);
-        if (!positive_only && kth == 0.0f) mode = 1; // fewer than k positive docs: zero tail in doc order
         // fp32 error of an n-term sum grows with n: widen the band for unusually long queries
         const float band = kBandRel * (float)max(1, (n_terms[q] + 31) / 32);
-        lo = kth - band * fabsf(kth);
+        lo = fminf(kth - band * fabsf(kth), kth - sl);
+        if (!positive_only && lo <= 0.0f) mode = 1; // the band reaches the zero-score docs: zero tail in doc order
     }
-    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    if (threadIdx.x < 3) s_cnt[threadIdx.x] = 0;
     __syncthreads();
-    unsigned long long c_band = 0, c_pos = 0;
+    unsigned long long c_band = 0, c_sure = 0, c_zero = 0;
     for (int64_t i = threadIdx.x; i < n_docs; i += SEL_T) {
         const float s = row[i];
         const bool ok = doc_allowed(fr, (uint32_t)i);
-        if (mode == 2) c_band += (ok && (!positive_only || s != 0.0f));
-        else if (mode == 1) c_pos += (ok && s > 0.0f);
-        else c_band += (ok && s >= lo && !(positive_only && s == 0.0f));
+        const bool nh = no_hit(hr, s, (uint32_t)i);
+        if (mode == 2) c_band += (ok && (!positive_only || !nh));
+        else if (mode == 1) { c_band += (ok && s >= lo && !nh); c_sure += (ok && s > sl); c_zero += (ok && nh); }
+        else c_band += (ok && s >= lo && !(positive_only && nh));
     }
     for (int o = 16; o > 0; o >>= 1) {
         c_band += __shfl_xor_sync(0xffffffffu, c_band, o);
-        c_pos += __shfl_xor_sync(0xffffffffu, c_pos, o);
+        c_sure += __shfl_xor_sync(0xffffffffu, c_sure, o);
+        c_zero += __shfl_xor_sync(0xffffffffu, c_zero, o);
     }
-    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_cnt[0], c_band); atomicAdd(&s_cnt[1], c_pos); }
+    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_cnt[0], c_band); atomicAdd(&s_cnt[1], c_sure); atomicAdd(&s_cnt[2], c_zero); }
     __syncthreads();
     if (threadIdx.x == 0) {
         const int64_t kk = min((int64_t)k, n_docs);
         sv.lo[q] = lo;
         sv.mode[q] = mode;
-        if (mode == 1) {
-            sv.zfill[q] = (int32_t)(kk - (int64_t)s_cnt[1]);
-            sv.cnt[q] = kk;
-        } else {
-            sv.zfill[q] = 0;
-            sv.cnt[q] = (int64_t)s_cnt[0];
-        }
+        const int64_t zfill = mode == 1 ? min(kk - (int64_t)s_cnt[1], (int64_t)s_cnt[2]) : 0;
+        sv.zfill[q] = (int32_t)zfill;
+        sv.cnt[q] = (int64_t)s_cnt[0] + zfill;
     }
 }
 
 __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ scores, int64_t n_docs,
                                                       int positive_only, SelView sv, int32_t q_begin,
                                                       const int64_t* __restrict__ cand_off, int32_t* __restrict__ cand,
-                                                      DocFilter f) {
+                                                      DocFilter f, HitRows h) {
     const float* row = scores + (int64_t)blockIdx.x * n_docs;
     const int q = q_begin + blockIdx.x;
     const uint32_t* fr = f.row ? f.row_of(q) : nullptr;
+    const uint32_t* hr = h.row_of(q, blockIdx.x);
     const int mode = sv.mode[q];
     const float lo = sv.lo[q];
     const uint32_t zfill = (uint32_t)sv.zfill[q];
@@ -263,9 +313,10 @@ __global__ void __launch_bounds__(SEL_T) k_emit_cands(const float* __restrict__ 
         const float s = i < n_docs ? row[i] : -CUDART_INF_F;
         bool take, zero = false;
         const bool ok = i < n_docs && doc_allowed(fr, (uint32_t)i);
-        if (mode == 2) take = ok && (!positive_only || s != 0.0f);
-        else if (mode == 1) { take = ok && s > 0.0f; zero = ok && s == 0.0f; }
-        else take = ok && s >= lo && !(positive_only && s == 0.0f);
+        const bool nh = ok && no_hit(hr, s, (uint32_t)i);
+        if (mode == 2) take = ok && (!positive_only || !nh);
+        else if (mode == 1) { take = ok && s >= lo && !nh; zero = nh; }
+        else take = ok && s >= lo && !(positive_only && nh);
         uint32_t total, ztotal = 0, zex = 0;
         if (mode == 1) {
             zex = block_excl_scan(zero ? 1u : 0u, &ztotal);
@@ -491,7 +542,7 @@ __global__ void __launch_bounds__(FS_T) k_final_select(const IdT* __restrict__ i
                 if (recs) { const br_record r = recs[base + pos + i]; id = (IdT)r.id; scv = r.score; }   // packed {id, score}
                 else { id = ids[base + pos + i]; scv = sc[base + pos + i]; }
                 FsKey kk = {scv, (int64_t)id};
-                if (id < 0) kk = pad;
+                if (id < 0 || (positive_only && scv == 0.0)) kk = pad;      // positive_only: float64 score != 0 only
                 keys[filled + i] = kk;
             }
             filled += (int)take;
@@ -527,15 +578,11 @@ __global__ void __launch_bounds__(FS_T) k_final_select(const IdT* __restrict__ i
         n_best = (int)min(total, (uint32_t)k);
     }
     for (int i = threadIdx.x; i < k; i += FS_T) {
-        const bool valid = i < n_best && !(positive_only && keys[i].s == 0.0);
+        const bool valid = i < n_best;
         out_ids[(int64_t)q * k + i] = valid ? (IdT)(keys[i].id + id_base) : (IdT)-1;
         out_sc[(int64_t)q * k + i] = valid ? keys[i].s : 0.0;
     }
-    if (out_cnt && threadIdx.x == 0) {
-        int c = n_best;
-        if (positive_only) { c = 0; while (c < n_best && keys[c].s != 0.0) ++c; }
-        out_cnt[q] = c;
-    }
+    if (out_cnt && threadIdx.x == 0) out_cnt[q] = n_best;
 }
 
 
@@ -640,17 +687,19 @@ int prep_queries(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int
     auto carve = [&](size_t n) { size_t o = bytes; bytes += (n + 255) & ~(size_t)255; return o; };
     const size_t o_ut = carve(Tn * 4), o_um = carve(Tn * 4), o_uc = carve(Tn * 8), o_un = carve(Q * 4),
                  o_ot = carve(Tn * 4), o_on = carve(Q * 4), o_P = carve(Q * 8), o_nc = carve(Q * 4),
-                 o_tmp = carve(Tn * 4), o_cs = carve(Q * 8), o_sig = carve(Q * 4), o_bad = carve(16);
+                 o_tmp = carve(Tn * 4), o_cs = carve(Q * 8), o_sig = carve(Q * 4), o_sl = carve(Q * 4), o_bad = carve(16);
     BR_TRY(ix->ws_prep.reserve(bytes));
     char* p = ix->ws_prep.as<char>();
     pv->u_terms = (int32_t*)(p + o_ut); pv->u_mult = (int32_t*)(p + o_um); pv->u_cum = (int64_t*)(p + o_uc);
     pv->u_cnt = (int32_t*)(p + o_un); pv->o_terms = (int32_t*)(p + o_ot); pv->o_cnt = (int32_t*)(p + o_on);
     pv->P = (int64_t*)(p + o_P); pv->n_chunks = (uint32_t*)(p + o_nc); pv->tmp = (int32_t*)(p + o_tmp); pv->sig = (uint32_t*)(p + o_sig);
+    pv->slack = (float*)(p + o_sl);
     *chunk_start = (int64_t*)(p + o_cs);
     pv->t_cap = T;
     pv->bad = (int32_t*)(p + o_bad);
     BR_CUDA(cudaMemsetAsync(pv->bad, 0, 4, st));
-    k_prep_queries<<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(q_terms, q_off, nq, ix->vocab, ix->row_ptr, ix->sig_bit, dedup, *pv);
+    k_prep_queries<<<blocks_for((int64_t)nq * 32, 128), 128, 0, st>>>(q_terms, q_off, nq, ix->vocab, ix->row_ptr, ix->sig_bit, dedup,
+                                                                    ix->idf, ix->amax, *pv);
     BR_CUDA(cudaGetLastError());
     k_exscan<uint32_t><<<1, 1024, 0, st>>>(pv->n_chunks, nq, *chunk_start);
     BR_CUDA(cudaGetLastError());
@@ -670,7 +719,8 @@ int score_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_off, int3
     int64_t* chunk_start;
     BR_TRY(prep_queries(ix, q_terms, q_off, nq, dedup, st, &pv, &chunk_start));
     BR_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)nq * (size_t)ix->n_docs, st));
-    k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(ix->post, ix->row_ptr, q_off, pv, chunk_start, 0, nq, out, ix->n_docs);
+    k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(ix->post, ix->row_ptr, q_off, pv, chunk_start, 0, nq, out, ix->n_docs,
+                                               HitRows{});
     BR_CUDA(cudaGetLastError());
     ix->stats.kernel_launches += 1;
     ix->stats.queries_dense += nq;
@@ -690,8 +740,18 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
     const int64_t N = ix->n_docs;
     // queries per pass: dense fp32 rows within ~1 GiB
     int32_t qb = (int32_t)std::max<int64_t>(1, std::min<int64_t>(nq, (1LL << 30) / (4 * N)));
-    BR_TRY(ix->ws_dense.reserve(sizeof(float) * (size_t)qb * (size_t)N));
+    // BM25 under okapi_no_plus1: a hit row per query (used only by the queries with a term of negative idf) after the
+    // fp32 rows, 1/32 of their size
+    const bool mixed = !post_table && ix->amax;
+    const size_t dense_bytes = (sizeof(float) * (size_t)qb * (size_t)N + 255) & ~(size_t)255;
+    HitRows hits{};
+    hits.words = (N + 31) / 32;
+    BR_TRY(ix->ws_dense.reserve(dense_bytes + (mixed ? sizeof(uint32_t) * (size_t)qb * (size_t)hits.words : 0)));
     float* dense = ix->ws_dense.as<float>();
+    if (mixed) {
+        hits.slack = pv.slack;
+        hits.bits = (uint32_t*)(ix->ws_dense.as<char>() + dense_bytes);
+    }
     // selection scratch for the whole batch slice
     size_t bytes = 0;
     auto carve = [&](size_t n) { size_t o = bytes; bytes += (n + 255) & ~(size_t)255; return o; };
@@ -705,12 +765,13 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
     for (int32_t s = 0; s < nq; s += qb) {
         const int32_t b0 = q_begin + s, bn = std::min(qb, nq - s);
         BR_CUDA(cudaMemsetAsync(dense, 0, sizeof(float) * (size_t)bn * (size_t)N, st));
+        if (mixed) BR_CUDA(cudaMemsetAsync(hits.bits, 0, sizeof(uint32_t) * (size_t)bn * (size_t)hits.words, st));
         ix->prof_begin(st);
-        k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(post, ix->row_ptr, q_off, pv, chunk_start, b0, bn, dense, N);
+        k_score_dense<<<kNumSMs * 8, 256, 0, st>>>(post, ix->row_ptr, q_off, pv, chunk_start, b0, bn, dense, N, hits);
         BR_CUDA(cudaGetLastError());
         ix->prof_end(st);
         // (query chunks keep batch-wide query indices b0 + i, so the filter rows need no remapping here)
-        k_select_radix<<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, f);
+        k_select_radix<<<bn, SEL_T, 0, st>>>(dense, N, k, positive_only, sv, b0, dedup ? pv.u_cnt : pv.o_cnt, f, hits);
         BR_CUDA(cudaGetLastError());
         BR_CUDA(cudaMemcpyAsync(h_cnt.data(), sv.cnt + b0, sizeof(int64_t) * (size_t)bn, cudaMemcpyDeviceToHost, st));
         BR_CUDA(cudaStreamSynchronize(st));
@@ -721,7 +782,7 @@ static int topk_dense(br_index* ix, const int32_t* q_off, const PrepView& pv, co
         BR_TRY(ix->ws_cand.reserve((size_t)(total + 1) * (sizeof(int32_t) + sizeof(double)) + 256));
         int32_t* cand = ix->ws_cand.as<int32_t>();
         double* cand_sc = (double*)(ix->ws_cand.as<char>() + (((size_t)(total + 1) * sizeof(int32_t) + 255) & ~(size_t)255));
-        k_emit_cands<<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, f);
+        k_emit_cands<<<bn, SEL_T, 0, st>>>(dense, N, positive_only, sv, b0, cand_off, cand, f, hits);
         BR_CUDA(cudaGetLastError());
         if (total > 0) BR_TRY(launch_rescore(ix, formula, q_off, pv, dedup, cand_off, b0, bn, cand, cand_sc, total, st));
         BR_TRY(launch_final_select(cand, cand_sc, cand_off, b0, bn, k, positive_only, out_ids, out_scores, out_counts, st));

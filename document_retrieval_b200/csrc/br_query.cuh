@@ -16,6 +16,8 @@ struct PrepView {
     uint32_t* n_chunks; // [nq]
     int32_t* tmp;       // [T]
     uint32_t* sig;      // [nq] bit (31 - r) set when the query contains the r-th most frequent term
+    float* slack;       // [nq] > 0 for a query with a term of negative idf: twice the bound on |fp32 sum - float64
+                        //      score| of any doc, (2n + 6) 2^-24 sum_t mult_t amax_t over its n distinct terms; else 0
     int32_t t_cap;      // term slots the scratch arrays hold (caller's n_terms)
     int32_t* bad;       // [1] set when q_offsets runs past t_cap
 };

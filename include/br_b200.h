@@ -112,8 +112,10 @@ int br_index_import_csr_dev(const int64_t* row_ptr_dev, const int32_t* doc_dev, 
 
 /* Replaces BM25.get_scores (bm25_ranking.ipynb:191-204) / calculate_scores
  * (final_implementation.py:127-145) for a batch: out_scores_dev float32[nq, n_docs] (fp32
- * accumulation of the precomputed posting weights; within 1e-5 relative of the float64
- * reference). */
+ * accumulation of the precomputed posting weights: per doc, |fp32 - float64 reference| <=
+ * (n + 2) * 2^-24 * sum_t mult_t * |w_t,d| over the query's n distinct terms with multiplicity mult_t
+ * and float64 weights w_t,d; for weights of one sign that is within 1e-5 relative, while under
+ * okapi_no_plus1 a query with a term of negative idf can cancel to an fp32 0 of a non-zero score). */
 int br_score_batch(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_offsets_dev,
                    int32_t nq, int dedup, float* out_scores_dev, void* stream);
 
@@ -123,9 +125,11 @@ int br_score_batch(br_index* ix, const int32_t* q_terms_dev, const int32_t* q_of
  * descending, doc id ascending): out_ids_dev int32 (local ids; -1 pads a short result),
  * out_scores_dev double (exact float64 re-evaluation of the reference formula, terms summed in
  * ascending term id for dedup != 0 and in query order otherwise), out_counts_dev int32[nq]
- * (number of valid entries; may be NULL).  positive_only != 0 keeps only docs with at least one
- * matching posting (team_run1.py:196); otherwise zero-score docs fill the tail in doc-id order
- * like the dense argpartition (bm25_ranking.ipynb:211).  1 <= k <= BR_MAX_K.
+ * (number of valid entries; may be NULL).  positive_only != 0 keeps only docs whose float64 score
+ * is not 0 (team_run1.py:196 ranks the docs with a hit; a doc whose only hits are terms of idf 0 -
+ * df = N/2 under okapi_no_plus1 - scores exactly 0 and is dropped too); otherwise zero-score docs
+ * fill the tail in doc-id order like the dense argpartition (bm25_ranking.ipynb:211).
+ * 1 <= k <= BR_MAX_K.
  * The call synchronises `stream` before returning. */
 /* n_terms = q_offsets[nq], the number of term slots of the batch, which the caller knows from packing it (an upper
  * bound works too); pass -1 when it is unknown - the library then reads it back from the device, which costs a
