@@ -22,6 +22,7 @@ SIGNATURES = {
     "br_index_build": (C.c_int, [_P, _P, C.c_int64, C.c_int32, C.c_int64, _P, C.POINTER(_P)]),
     "br_index_finalize": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_double, C.c_double, _P, _P]),
     "br_index_destroy": (None, [_P]),
+    "br_index_append": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, _P]),
     "br_index_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int64),
                                  C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "br_index_stats_in_force": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
@@ -67,6 +68,7 @@ SIGNATURES = {
     "br_tokenize_count": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, C.POINTER(C.c_int64), _P]),
     "br_vocab_build": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, C.POINTER(_P)]),
     "br_vocab_lookup": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, _P, C.c_int64, _P, _P]),
+    "br_vocab_extend": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, _P, C.c_int64, _P, _P]),
     "br_vocab_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "br_vocab_export": (C.c_int, [_P, _P, _P]),
     "br_vocab_import": (C.c_int, [_P, _P, C.c_int64, _P, C.POINTER(_P)]),

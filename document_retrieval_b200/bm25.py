@@ -8,8 +8,9 @@ this file only converts between the reference's Python types and device buffers.
 
 Added on top of the reference surface (SURVEY 8b): ``from_token_ids`` (int32 term ids instead of
 strings), ``retrieve_top_n_batch`` / ``get_scores_batch`` (whole batches, torch CUDA tensors),
-``variant`` / ``dedup_query`` (the three BM25 formulas in the reference, SURVEY appendix A) and
-``get_top_n`` as an alias of ``retrieve_top_n``.
+``variant`` / ``dedup_query`` (the three BM25 formulas in the reference, SURVEY appendix A),
+``get_top_n`` as an alias of ``retrieve_top_n``, and ``add_documents`` / ``add_texts`` / ``add_token_ids`` (grow a
+built or loaded index, bit-identical to rebuilding the whole corpus).
 """
 from __future__ import annotations
 
@@ -168,6 +169,113 @@ class BM25:
         self.avgdl = st["avgdl"]
         self._df_idf = None
         return self
+
+    # ------------------------------------------------------------------ append
+    # Each add_* is the append counterpart of one constructor: the new docs get ids corpus_size .., and the index is
+    # re-finalised with this model's k1 / b / variant, bit-identical to building the concatenated corpus from scratch.
+    def add_documents(self, tokenized_corpus):
+        """Append token lists (``list[list[str]]``, as for ``BM25(...)`` / ``build``).  New term strings are appended to
+        ``terms`` in first-seen order.  Returns ``self``."""
+        if self.bigrams:
+            raise ValueError("add_documents: this model expands its texts with bigrams, which token lists would skip; "
+                             "use add_texts")
+        if len(tokenized_corpus) == 0:
+            return self
+        self._check_appendable()
+        terms = self.terms
+        if terms is None:
+            raise ValueError("add_documents needs a model with a string vocabulary (use add_token_ids)")
+        import pandas as pd
+        n_docs = len(tokenized_corpus)
+        lens = np.fromiter((len(d) for d in tokenized_corpus), dtype=np.int64, count=n_docs)
+        doc_offsets = np.zeros(n_docs + 1, dtype=np.int64)
+        np.cumsum(lens, out=doc_offsets[1:])
+        flat = [w for d in tokenized_corpus for w in d]
+        codes, uniques = pd.factorize(np.asarray(flat, dtype=object)) if flat else (np.zeros(0, np.int64), [])
+        vocab, new_terms = self.vocab, []
+        ids_of_unique = np.empty(len(uniques), dtype=np.int32)
+        for i, u in enumerate(uniques):
+            t = vocab.get(str(u))
+            if t is None:
+                t = len(terms) + len(new_terms)
+                new_terms.append(str(u))
+            ids_of_unique[i] = t
+        grown = terms + new_terms
+        self._append_ids(doc_offsets, ids_of_unique[codes], max(len(grown), self.vocab_size))
+        if new_terms:
+            self.vocabulary = None     # a GPU vocabulary lacks the new terms: retrieve_top_n_texts rebuilds it from terms
+            self.terms = grown
+        return self
+
+    def add_texts(self, texts):
+        """Append preprocessed texts (as for ``from_texts``), tokenised on the GPU; new terms are added to the GPU
+        vocabulary (br_vocab_extend), with the model's 2-gram expansion when it has one.  A model with string terms but
+        no GPU vocabulary (built by ``build``, loaded from a file, unpickled) first gets one from its terms.  Returns
+        ``self``."""
+        from .ingest import Vocabulary
+        if not isinstance(texts, tuple) and len(texts) == 0:
+            return self
+        self._check_appendable()
+        if self.vocabulary is None:
+            if self.terms is None:
+                raise BRError("add_texts needs a model with a string vocabulary")
+            self.vocabulary = Vocabulary.from_terms(self.terms, bigrams=self.bigrams, device=self._device)
+        voc = self.vocabulary
+        n_terms = len(voc)
+        doc_off, ids = voc.extend_texts(texts)
+        try:
+            self._append_ids(doc_off, ids, max(len(voc), self.vocab_size))
+        except Exception:
+            voc._truncate(n_terms)     # the index refused the documents: their new terms leave the vocabulary too
+            raise
+        self.terms = None              # decoded again from the grown vocabulary
+        return self
+
+    def add_token_ids(self, doc_offsets, token_ids, vocab_size=None):
+        """Append int32 term ids (as for ``from_token_ids``): ``doc_offsets`` int64[n+1], ``token_ids`` int32[T], numpy or
+        torch, host or device.  ``vocab_size`` (default: the current one) may grow the vocabulary of a model without
+        term strings only.  Returns ``self``."""
+        vocab_size = self.vocab_size if vocab_size is None else int(vocab_size)
+        if vocab_size > self.vocab_size and self.terms is not None:
+            raise ValueError("add_token_ids cannot add terms without strings to a model with a string vocabulary "
+                             "(use add_documents or add_texts)")
+        if len(doc_offsets) <= 1:
+            return self
+        self._check_appendable()
+        self._append_ids(doc_offsets, token_ids, vocab_size)
+        return self
+
+    def _check_appendable(self):
+        """A doc shard is finalised with global statistics; re-finalising it with its local ones would silently break
+        it, so it only grows through a sharded wrapper."""
+        self._require()
+        lib = _lib.load()
+        n_stat, sum_dl_stat = C.c_double(), C.c_double()
+        check(lib.br_index_stats_in_force(self._h, C.byref(n_stat), C.byref(sum_dl_stat)), "br_index_stats_in_force")
+        st = self.stats()
+        df, _ = self._export_df_idf()
+        if (n_stat.value != st["n_docs"] or sum_dl_stat.value != st["sum_dl"]
+                or not np.array_equal(df, self.local_df_tensor().cpu().numpy())):
+            raise BRError("this index is a doc shard finalised with global statistics: documents cannot be added to it "
+                          "alone")
+
+    def _append_ids(self, doc_offsets, token_ids, vocab_size):
+        lib = _lib.load()
+        dev = self._device
+        with torch.cuda.device(dev):
+            d_off = torch.as_tensor(doc_offsets).to(device=dev, dtype=torch.int64).contiguous()
+            d_tok = torch.as_tensor(token_ids).to(device=dev, dtype=torch.int32).contiguous()
+            n_docs = d_off.numel() - 1
+            if n_docs <= 0:
+                return
+            if d_tok.numel() == 0:
+                d_tok = torch.zeros(1, dtype=torch.int32, device=dev)      # only empty docs: nothing is read
+            check(lib.br_index_append(self._h, ptr(d_tok), ptr(d_off), n_docs, int(vocab_size), _lib.stream_ptr(dev)),
+                  "br_index_append")
+        self.vocab_size = int(vocab_size)
+        self.corpus_size += n_docs
+        self._csr = None
+        self.finalize()
 
     def stats(self):
         lib = _lib.load()

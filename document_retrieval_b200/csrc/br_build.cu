@@ -14,6 +14,10 @@
 //   [host]           idf[t] = log(..) in float64 with libm (bit-identical to math.log)
 //   k_weights        w = fp32(idf * ((tf*(k1+1)) / (tf + k1*norm(dl))))  evaluated in float64, no FMA
 //   k_skip           per hot term: offset of the first posting of every 2^sub_shift-doc sub-range
+//
+// Append (br_index_append): the new docs go through the same pipeline as a build of their own, then
+//   k_append_rows    row_ptr / df of the grown index (old + new part, per term)
+//   k_append_merge   thread per output posting: a term's old postings, then its new ones with doc + N_old  (10 B in, 10 B out)
 #include <math.h>
 
 #include <algorithm>
@@ -120,17 +124,12 @@ __global__ void k_df(const uint32_t* __restrict__ tstart, const uint32_t* __rest
     if (t < vocab) df[t] = tend[t] - tstart[t];
 }
 
-__global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, int64_t nnz,
-                          br_posting* __restrict__ post, const uint16_t* __restrict__ tf,
-                          const uint32_t* __restrict__ dl, const double* __restrict__ idf, double avgdl,
-                          double k1, double b, int variant, float* __restrict__ ub, float* __restrict__ amax) {
-    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int lane = threadIdx.x & 31;
-    int32_t lo = -1;
-    float wv = 0.f;
-    // term of posting j: last t with row_ptr[t] <= j.  The 32 postings of a warp are consecutive, so their terms lie
-    // between the term of the warp's first and last posting: two full binary searches per warp, the other lanes search
-    // only that (mostly one-term) range.
+// Term of posting j = blockIdx.x * blockDim.x + threadIdx.x: the last t with row_ptr[t] <= j, -1 for j >= nnz.  Every
+// lane of the warp must call.  The 32 postings of a warp are consecutive, so their terms lie between the term of the
+// warp's first and last posting: two full binary searches per warp, the other lanes search only that (mostly one-term)
+// range.
+__device__ __forceinline__ int32_t warp_term_of(const int64_t* __restrict__ row_ptr, int32_t vocab, int64_t nnz,
+                                                int64_t j, int lane) {
     const int64_t j_first = min(j - lane, nnz - 1), j_last = min(j - lane + 31, nnz - 1);
     int32_t t_first = 0, t_last = 0;
     if (j_first >= 0 && (lane == 0 || lane == 31)) {
@@ -144,13 +143,24 @@ __global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, in
     }
     t_first = __shfl_sync(0xffffffffu, t_first, 0);
     t_last = __shfl_sync(0xffffffffu, t_last, 31);
-    if (j < nnz) {
-        lo = t_first;
-        int32_t hi = t_last + 1;  // invariant: row_ptr[lo] <= j < row_ptr[hi]
-        while (hi - lo > 1) {
-            const int32_t mid = (lo + hi) >> 1;
-            if (row_ptr[mid] <= j) lo = mid; else hi = mid;
-        }
+    if (j >= nnz) return -1;
+    int32_t lo = t_first, hi = t_last + 1;  // invariant: row_ptr[lo] <= j < row_ptr[hi]
+    while (hi - lo > 1) {
+        const int32_t mid = (lo + hi) >> 1;
+        if (row_ptr[mid] <= j) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, int64_t nnz,
+                          br_posting* __restrict__ post, const uint16_t* __restrict__ tf,
+                          const uint32_t* __restrict__ dl, const double* __restrict__ idf, double avgdl,
+                          double k1, double b, int variant, float* __restrict__ ub, float* __restrict__ amax) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    float wv = 0.f;
+    const int32_t lo = warp_term_of(row_ptr, vocab, nnz, j, lane);
+    if (lo >= 0) {
         const uint32_t d = post[j].doc;
         const double c = bm25_contrib(idf[lo], (double)tf[j], (double)dl[d], avgdl, k1, b, variant);
         wv = isnan(c) ? 0.f : (float)c;
@@ -172,6 +182,45 @@ __global__ void k_weights(const int64_t* __restrict__ row_ptr, int32_t vocab, in
         }
         todo &= ~__ballot_sync(0xffffffffu, mine);
     }
+}
+
+// Append: row_ptr and df of the grown index over the grown vocabulary.  Terms t >= the old vocabulary have no old
+// postings; rp_old[v_old] = the old nnz.
+__global__ void k_append_rows(const int64_t* __restrict__ rp_old, const uint32_t* __restrict__ df_old, int32_t v_old,
+                              const int64_t* __restrict__ rp_new_part, const uint32_t* __restrict__ df_new_part,
+                              int32_t vocab, int64_t* __restrict__ row_ptr, uint32_t* __restrict__ df) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t > vocab) return;
+    row_ptr[t] = rp_old[min(t, v_old)] + rp_new_part[t];
+    if (t < vocab) df[t] = (t < v_old ? df_old[t] : 0u) + df_new_part[t];
+}
+
+// Append: posting j of the grown index.  Its term's row is the term's old postings followed by the new documents'
+// postings (doc ids shifted by the old N), so every output posting has exactly one source posting: one 10-byte read and
+// one 10-byte write per posting.  Weights are left 0 for br_index_finalize.
+__global__ void k_append_merge(const int64_t* __restrict__ row_ptr, int32_t vocab, int64_t nnz,
+                               const int64_t* __restrict__ rp_old, int32_t v_old, const br_posting* __restrict__ post_old,
+                               const uint16_t* __restrict__ tf_old, const int64_t* __restrict__ rp_new_part,
+                               const br_posting* __restrict__ post_new_part, const uint16_t* __restrict__ tf_new_part,
+                               uint32_t n_docs_old, br_posting* __restrict__ post, uint16_t* __restrict__ tf) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int32_t t = warp_term_of(row_ptr, vocab, nnz, j, threadIdx.x & 31);
+    if (t < 0) return;
+    const int64_t off = j - row_ptr[t];
+    const int64_t old_lo = rp_old[min(t, v_old)], old_len = t < v_old ? rp_old[t + 1] - old_lo : 0;
+    br_posting p;
+    uint16_t f;
+    if (off < old_len) {
+        p.doc = post_old[old_lo + off].doc;
+        f = tf_old[old_lo + off];
+    } else {
+        const int64_t s = rp_new_part[t] + (off - old_len);
+        p.doc = post_new_part[s].doc + n_docs_old;
+        f = tf_new_part[s];
+    }
+    p.w = 0.f;
+    post[j] = p;
+    tf[j] = f;
 }
 
 __global__ void k_skip(const int64_t* __restrict__ row_ptr, const br_posting* __restrict__ post,
@@ -468,6 +517,86 @@ int index_import(const int64_t* row_ptr, const int32_t* doc, const int32_t* tf, 
     return index_import_dev(d_rp, d_doc, d_tf16, d_dl, n_docs, vocab, nnz, doc_base, st, out);
 }
 
+// Append documents: the new documents' postings come from index_build (the same sort and run-length encoding, over the
+// grown vocabulary), then one streaming pass merges them behind each term's old postings.  Every grown array is
+// allocated and filled before any of them replaces the handle's, so that an error leaves the handle as it was.
+int index_append(br_index* ix, const int32_t* tok, const int64_t* doc_off, int64_t n_docs, int32_t vocab,
+                 cudaStream_t st) {
+    BR_REQUIRE(ix && tok && doc_off, BR_ERR_INVALID, "br_index_append: null pointer");
+    BR_REQUIRE(n_docs > 0 && n_docs < (1LL << 31), BR_ERR_INVALID, "br_index_append: n_docs must be in [1, 2^31)");
+    BR_REQUIRE(vocab >= ix->vocab, BR_ERR_INVALID, "br_index_append: vocab must be at least the index's vocab");
+    BR_CUDA(cudaSetDevice(ix->device));
+    br_index* part_raw = nullptr;
+    BR_TRY(index_build(tok, doc_off, n_docs, vocab, 0, st, &part_raw));
+    IndexOwner part(part_raw, index_free);
+    const int64_t n_docs_new = ix->n_docs + n_docs, sum_dl = ix->sum_dl + part->sum_dl, nnz = ix->nnz + part->nnz;
+    BR_REQUIRE(n_docs_new < (1LL << 31), BR_ERR_UNSUPPORTED, "br_index_append: 2^31 or more docs in one shard");
+    BR_REQUIRE(sum_dl < (1LL << 32), BR_ERR_UNSUPPORTED, "br_index_append: 2^32 or more tokens in one shard");
+    BR_REQUIRE(nnz < (1LL << 32), BR_ERR_UNSUPPORTED, "br_index_append: 2^32 or more postings in one shard");
+
+    const size_t V = (size_t)vocab;
+    const bool grow_v = vocab > ix->vocab;
+    DevArray<int64_t> row_ptr;
+    DevArray<br_posting> post;
+    DevArray<uint16_t> tf;
+    DevArray<uint32_t> dl, df;
+    DevArray<double> idf;
+    DevArray<int32_t> hot_slot;
+    DevArray<float> ub;
+    BR_TRY(row_ptr.alloc(V + 1));
+    BR_TRY(df.alloc(V));
+    BR_TRY(dl.alloc((size_t)n_docs_new));
+    BR_TRY(post.alloc((size_t)nnz));
+    BR_TRY(tf.alloc((size_t)nnz));
+    if (grow_v) {
+        BR_TRY(idf.alloc(V));
+        BR_TRY(hot_slot.alloc(V));
+        BR_TRY(ub.alloc(V));
+    }
+    k_append_rows<<<blocks_for((int64_t)V + 1, 256), 256, 0, st>>>(ix->row_ptr, ix->df, ix->vocab, part->row_ptr, part->df,
+                                                                   vocab, row_ptr, df);
+    BR_CUDA(cudaGetLastError());
+    if (nnz > 0) {
+        k_append_merge<<<blocks_for(nnz, 256), 256, 0, st>>>(row_ptr, vocab, nnz, ix->row_ptr, ix->vocab, ix->post, ix->tf,
+                                                             part->row_ptr, part->post, part->tf, (uint32_t)ix->n_docs,
+                                                             post, tf);
+        BR_CUDA(cudaGetLastError());
+    }
+    BR_CUDA(cudaMemcpyAsync(dl, ix->dl, sizeof(uint32_t) * (size_t)ix->n_docs, cudaMemcpyDeviceToDevice, st));
+    BR_CUDA(cudaMemcpyAsync(dl + ix->n_docs, part->dl, sizeof(uint32_t) * (size_t)n_docs, cudaMemcpyDeviceToDevice, st));
+    std::vector<uint32_t> h_df(V);
+    BR_CUDA(cudaMemcpyAsync(h_df.data(), df, sizeof(uint32_t) * V, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+
+    // nothing below can fail: the handle takes the grown arrays and frees the old ones
+    ix->row_ptr = std::move(row_ptr);
+    ix->post = std::move(post);
+    ix->tf = std::move(tf);
+    ix->dl = std::move(dl);
+    ix->df = std::move(df);
+    ix->h_df.swap(h_df);
+    if (grow_v) {
+        ix->idf = std::move(idf);
+        ix->hot_slot = std::move(hot_slot);
+        ix->ub = std::move(ub);
+        ix->amax.reset();       // [V] arrays that index_finalize allocates when they are missing
+        ix->row_slot.reset();
+    }
+    // structures index_finalize builds only when they are missing: they depend on the local df and N
+    ix->skip.reset();
+    ix->sig_bit.reset();
+    ix->dense_rows.reset();
+    ix->n_rows = ix->n_srows = 0;
+    ix->post_cos.reset();
+    ix->cos_inv_norm.reset();
+    ix->n_docs = n_docs_new;
+    ix->vocab = vocab;
+    ix->sum_dl = sum_dl;
+    ix->nnz = nnz;
+    ix->finalized = false;
+    return BR_OK;
+}
+
 int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat, double sum_dl_stat,
                    const int64_t* df_stat_host, cudaStream_t st) {
     BR_REQUIRE(ix, BR_ERR_INVALID, "br_index_finalize: null handle");
@@ -609,6 +738,11 @@ extern "C" {
 int br_index_build(const int32_t* token_ids_dev, const int64_t* doc_offsets_dev, int64_t n_docs, int32_t vocab,
                    int64_t doc_base, void* stream, br_index** out) {
     return br::index_build(token_ids_dev, doc_offsets_dev, n_docs, vocab, doc_base, (cudaStream_t)stream, out);
+}
+
+int br_index_append(br_index* ix, const int32_t* token_ids_dev, const int64_t* doc_offsets_dev, int64_t n_docs,
+                    int32_t vocab, void* stream) {
+    return br::index_append(ix, token_ids_dev, doc_offsets_dev, n_docs, vocab, (cudaStream_t)stream);
 }
 
 int br_index_finalize(br_index* ix, double k1, double b, int variant, double n_stat, double sum_dl_stat,

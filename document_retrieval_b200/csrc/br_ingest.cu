@@ -17,6 +17,10 @@
 //                 collision is reported as an error instead of silently merging two terms
 //   k_pool_len / k_pool_fill     vocabulary strings into one byte pool (-> Python `terms`, query-time verification)
 //   k_lookup      query tokens: binary search in the sorted hash table + byte compare -> term id or -1 (OOV)
+// Extension (br_vocab_extend): the new text's own vocabulary (the pipeline above), then
+//   k_extend_find its terms looked up in the existing table (hash + byte compare), k_exscan numbers the new ones
+//   k_extend_map  local id -> global id; k_remap the new tokens; k_extend_pool appends the new strings; the new
+//                 (hash, id) pairs are sorted into the table together with the old ones
 #include <memory>
 
 #include <cub/cub.cuh>
@@ -322,6 +326,74 @@ __global__ void __launch_bounds__(256) k_lookup(const uint8_t* __restrict__ text
     token_ids[i] = term;
 }
 
+// Vocabulary extension, thread per entry i of the new text's own (local) hash table: is its term in v?  A hash hit is
+// byte-compared like k_lookup; a hit with other bytes is a collision.  By local id r: known[r] = the term id in v or -1,
+// is_new[r] = known[r] < 0, hash_of[r] = the term's hash.
+__global__ void k_extend_find(const uint64_t* __restrict__ loc_hash, const int32_t* __restrict__ loc_term, int64_t n_loc,
+                              const int64_t* __restrict__ loc_pool_off, const uint8_t* __restrict__ loc_pool,
+                              const uint64_t* __restrict__ hash_sorted, const int32_t* __restrict__ term_sorted,
+                              int64_t n_terms, const int64_t* __restrict__ pool_off, const uint8_t* __restrict__ pool,
+                              int32_t* __restrict__ known, uint32_t* __restrict__ is_new, uint64_t* __restrict__ hash_of,
+                              int* __restrict__ bad) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_loc) return;
+    const uint64_t h = loc_hash[i];
+    const int32_t r = loc_term[i];
+    int64_t lo = 0, hi = n_terms;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (hash_sorted[mid] < h) lo = mid + 1; else hi = mid;
+    }
+    int32_t term = -1;
+    if (lo < n_terms && hash_sorted[lo] == h) {
+        const int32_t t = term_sorted[lo];
+        const int64_t s = pool_off[t], ls = loc_pool_off[r];
+        if (canon_equal(Canon(loc_pool, ls, (uint32_t)(loc_pool_off[r + 1] - ls)), Canon(pool, s, (uint32_t)(pool_off[t + 1] - s))))
+            term = t;
+        else
+            atomicOr(bad, 8);
+    }
+    known[r] = term;
+    is_new[r] = term < 0 ? 1u : 0u;
+    hash_of[r] = h;
+}
+
+// By local id r: map[r] = the global term id (a new term's is n_terms + its rank among the new terms in local, i.e.
+// first-occurrence, order); a new term also gets its slot in the appended hash entries and its string length.
+__global__ void k_extend_map(const int32_t* __restrict__ known, const int64_t* __restrict__ rank, const uint64_t* __restrict__ hash_of,
+                             const int64_t* __restrict__ loc_pool_off, int64_t n_loc, int64_t n_terms,
+                             int32_t* __restrict__ map, uint64_t* __restrict__ new_hash, uint32_t* __restrict__ new_term,
+                             uint32_t* __restrict__ new_src, uint32_t* __restrict__ new_len) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= n_loc) return;
+    if (known[r] >= 0) { map[r] = known[r]; return; }
+    const int64_t s = rank[r];
+    map[r] = (int32_t)(n_terms + s);
+    new_hash[s] = hash_of[r];
+    new_term[s] = (uint32_t)(n_terms + s);
+    new_src[s] = (uint32_t)r;
+    new_len[s] = (uint32_t)(loc_pool_off[r + 1] - loc_pool_off[r]);
+}
+
+__global__ void k_remap(int32_t* __restrict__ ids, int64_t n, const int32_t* __restrict__ map) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) ids[i] = map[ids[i]];
+}
+
+// New term s: its string goes to the end of the pool, pool_off[n_terms + s + 1] = end of it (off: exclusive scan of
+// the new strings' lengths).
+__global__ void k_extend_pool(const uint32_t* __restrict__ new_src, const int64_t* __restrict__ off, int64_t n_new,
+                              const int64_t* __restrict__ loc_pool_off, const uint8_t* __restrict__ loc_pool,
+                              int64_t n_terms, int64_t pool_bytes, int64_t* __restrict__ pool_off, uint8_t* __restrict__ pool) {
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n_new) return;
+    const uint32_t r = new_src[s];
+    const int64_t a = loc_pool_off[r], n = loc_pool_off[r + 1] - a;
+    uint8_t* o = pool + pool_bytes + off[s];
+    for (int64_t b = 0; b < n; ++b) o[b] = loc_pool[a + b];
+    pool_off[n_terms + s + 1] = pool_bytes + off[s + 1];
+}
+
 int report_bad(int bad, const char* who) {
     if (bad & 2) { set_error(std::string(who) + ": byte offsets not non-decreasing"); return BR_ERR_INVALID; }
     if (bad & 4) { set_error(std::string(who) + ": a document of 2 GiB or more"); return BR_ERR_UNSUPPORTED; }
@@ -495,6 +567,108 @@ int br_vocab_lookup(const br_vocab* v, const uint8_t* text_dev, const int64_t* d
                                                         v->term_sorted, v->n_terms, v->pool_off, v->pool, token_ids_dev);
     BR_CUDA(cudaGetLastError());
     BR_CUDA(cudaStreamSynchronize(st));
+    return BR_OK;
+}
+
+// The new text gets a vocabulary of its own (br_vocab_build: its terms in first-occurrence order, its tokens' local ids);
+// its terms are looked up in v, the ones not found are numbered after v's terms in local order, the tokens are
+// remapped, the new strings appended to the pool and the new (hash, id) pairs sorted into the hash table.  The grown
+// tables are complete before they replace v's.
+int br_vocab_extend(br_vocab* v, const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int64_t n_docs, int bigrams,
+                    const int64_t* doc_tok_off_dev, int64_t n_tokens, int32_t* token_ids_dev, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    BR_REQUIRE(v && doc_byte_off_dev && doc_tok_off_dev && n_docs >= 0, BR_ERR_INVALID, "br_vocab_extend: null pointer");
+    BR_REQUIRE(n_tokens >= 0 && n_tokens < (1LL << 31), BR_ERR_UNSUPPORTED, "br_vocab_extend: 2^31 or more tokens");
+    BR_REQUIRE(n_tokens == 0 || token_ids_dev, BR_ERR_INVALID, "br_vocab_extend: null token_ids");
+    if (n_tokens == 0) return BR_OK;
+    BR_CUDA(cudaSetDevice(v->device));
+    br_vocab* loc_raw = nullptr;
+    BR_TRY(br_vocab_build(text_dev, doc_byte_off_dev, n_docs, bigrams, doc_tok_off_dev, n_tokens, token_ids_dev, stream,
+                          &loc_raw));
+    std::unique_ptr<br_vocab> loc(loc_raw);
+    const int64_t L = loc->n_terms, V = v->n_terms;
+    StreamScratch tmp(st);
+    int32_t *known = nullptr, *map = nullptr;
+    uint32_t* is_new = nullptr;
+    uint64_t* hash_of = nullptr;
+    int64_t* rank = nullptr;
+    int* d_bad = nullptr;
+    BR_TRY(tmp.alloc(&known, (size_t)L));
+    BR_TRY(tmp.alloc(&map, (size_t)L));
+    BR_TRY(tmp.alloc(&is_new, (size_t)L));
+    BR_TRY(tmp.alloc(&hash_of, (size_t)L));
+    BR_TRY(tmp.alloc(&rank, (size_t)L + 1));
+    BR_TRY(tmp.alloc(&d_bad, 1));
+    BR_CUDA(cudaMemsetAsync(d_bad, 0, sizeof(int), st));
+    k_extend_find<<<blocks_for(L, 256), 256, 0, st>>>(loc->hash_sorted, loc->term_sorted, L, loc->pool_off, loc->pool,
+                                                      v->hash_sorted, v->term_sorted, V, v->pool_off, v->pool, known,
+                                                      is_new, hash_of, d_bad);
+    BR_CUDA(cudaGetLastError());
+    k_exscan<uint32_t><<<1, 1024, 0, st>>>(is_new, L, rank);
+    BR_CUDA(cudaGetLastError());
+    int64_t n_new = 0;
+    int bad = 0;
+    BR_CUDA(cudaMemcpyAsync(&n_new, rank + L, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+    BR_TRY(report_bad(bad, "br_vocab_extend"));
+    BR_REQUIRE(V + n_new < (1LL << 31), BR_ERR_UNSUPPORTED, "br_vocab_extend: 2^31 or more terms");
+
+    const int64_t W = V + n_new;
+    uint64_t* cat_hash = nullptr;
+    uint32_t *cat_term = nullptr, *new_src = nullptr, *new_len = nullptr;
+    int64_t* new_off = nullptr;
+    BR_TRY(tmp.alloc(&cat_hash, (size_t)W));
+    BR_TRY(tmp.alloc(&cat_term, (size_t)W));
+    BR_TRY(tmp.alloc(&new_src, (size_t)n_new));
+    BR_TRY(tmp.alloc(&new_len, (size_t)n_new));
+    BR_TRY(tmp.alloc(&new_off, (size_t)n_new + 1));
+    if (V > 0) {
+        BR_CUDA(cudaMemcpyAsync(cat_hash, v->hash_sorted, sizeof(uint64_t) * (size_t)V, cudaMemcpyDeviceToDevice, st));
+        BR_CUDA(cudaMemcpyAsync(cat_term, v->term_sorted, sizeof(int32_t) * (size_t)V, cudaMemcpyDeviceToDevice, st));
+    }
+    k_extend_map<<<blocks_for(L, 256), 256, 0, st>>>(known, rank, hash_of, loc->pool_off, L, V, map, cat_hash + V,
+                                                     cat_term + V, new_src, new_len);
+    BR_CUDA(cudaGetLastError());
+    k_remap<<<blocks_for(n_tokens, 256), 256, 0, st>>>(token_ids_dev, n_tokens, map);
+    BR_CUDA(cudaGetLastError());
+    k_exscan<uint32_t><<<1, 1024, 0, st>>>(new_len, n_new, new_off);
+    BR_CUDA(cudaGetLastError());
+    int64_t new_bytes = 0;
+    BR_CUDA(cudaMemcpyAsync(&new_bytes, new_off + n_new, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    // the hash tables' entries are distinct (a new term's hash is not in v), so sorting the concatenation by hash gives
+    // exactly the table br_vocab_build makes over old text + new text
+    BR_TRY(sort_pairs(tmp, &cat_hash, &cat_term, W, 64, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+
+    DevArray<uint64_t> hash_sorted;
+    DevArray<int32_t> term_sorted;
+    DevArray<int64_t> pool_off;
+    DevArray<uint8_t> pool;
+    BR_TRY(hash_sorted.alloc((size_t)W));
+    BR_TRY(term_sorted.alloc((size_t)W));
+    BR_TRY(pool_off.alloc((size_t)W + 1));
+    BR_TRY(pool.alloc((size_t)(v->pool_bytes + new_bytes)));
+    BR_CUDA(cudaMemcpyAsync(hash_sorted, cat_hash, sizeof(uint64_t) * (size_t)W, cudaMemcpyDeviceToDevice, st));
+    k_u32_to_i32<<<blocks_for(W, 256), 256, 0, st>>>(cat_term, W, term_sorted);
+    BR_CUDA(cudaGetLastError());
+    BR_CUDA(cudaMemcpyAsync(pool_off, v->pool_off, sizeof(int64_t) * (size_t)(V + 1), cudaMemcpyDeviceToDevice, st));
+    if (v->pool_bytes > 0)
+        BR_CUDA(cudaMemcpyAsync(pool, v->pool, (size_t)v->pool_bytes, cudaMemcpyDeviceToDevice, st));
+    if (n_new > 0) {
+        k_extend_pool<<<blocks_for(n_new, 256), 256, 0, st>>>(new_src, new_off, n_new, loc->pool_off, loc->pool, V,
+                                                              v->pool_bytes, pool_off, pool);
+        BR_CUDA(cudaGetLastError());
+    }
+    BR_CUDA(cudaStreamSynchronize(st));
+
+    // nothing below can fail
+    v->hash_sorted = std::move(hash_sorted);
+    v->term_sorted = std::move(term_sorted);
+    v->pool_off = std::move(pool_off);
+    v->pool = std::move(pool);
+    v->n_terms = W;
+    v->pool_bytes += new_bytes;
     return BR_OK;
 }
 

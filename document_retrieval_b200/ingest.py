@@ -80,6 +80,27 @@ class Vocabulary:
                                      _lib.stream_ptr(dev), C.byref(h)), "br_vocab_build")
         return cls(h, dev, bigrams), tok_off, ids
 
+    def extend_texts(self, texts):
+        """Grow the vocabulary with the terms of new documents -> (doc_offsets int64[N+1], token_ids int32[T]) on the
+        device, like ``from_texts``.  Known terms keep their ids; new terms are numbered after the existing ones in order
+        of first occurrence, so ``from_texts(A)`` extended with B equals ``from_texts(A + B)``."""
+        lib = _lib.load()
+        dev = self.device
+        with torch.cuda.device(dev):
+            d_text, d_off, n_docs, tok_off, n_tok = self._tokenize_count(lib, dev, texts, self.bigrams)
+            ids = torch.empty(max(n_tok, 1), dtype=torch.int32, device=dev)[:n_tok]
+            check(lib.br_vocab_extend(self._h, ptr(d_text), ptr(d_off), n_docs, int(self.bigrams), ptr(tok_off), n_tok,
+                                      ptr(ids), _lib.stream_ptr(dev)), "br_vocab_extend")
+        self._terms = None
+        return tok_off, ids
+
+    def _truncate(self, n_terms):
+        """Keep the first ``n_terms`` terms (takes back an ``extend_texts`` whose documents an index refused)."""
+        off, pool = self._export()
+        old = self._h
+        self.__setstate__(dict(pool_off=off[:n_terms + 1], pool=pool[:off[n_terms]], bigrams=self.bigrams))
+        _lib.load().br_vocab_destroy(old)
+
     def encode_texts(self, texts):
         """Query texts -> (q_terms int32[T], q_offsets int64[Q+1]) on the device; -1 = out of vocabulary."""
         lib = _lib.load()

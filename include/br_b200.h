@@ -68,6 +68,21 @@ int br_index_finalize(br_index* ix, double k1, double b, int variant, double n_s
                       double sum_dl_stat, const int64_t* df_stat_host, void* stream);
 void br_index_destroy(br_index* ix);
 
+/* Append n_docs documents to a built index.  token_ids_dev / doc_offsets_dev: the same layout as br_index_build.
+ * vocab is the new vocabulary size, >= the handle's; token ids must be in [0, vocab).  The appended docs get local ids
+ * n_docs_old .. n_docs_old + n_docs - 1.  On success the handle is NOT finalised: every query entry point returns
+ * BR_ERR_STATE until br_index_finalize is called again (N, avgdl and df changed, so every weight changes).
+ * On any error the handle is left exactly as it was, including its finalised state, and still answers queries with the
+ * same results.
+ * Appending B to the index of A and finalising gives the same bits as building A followed by B from scratch and
+ * finalising: the same CSR, df, idf, weights, skip tables and dense rows, hence the same results from every query.
+ * Works on any handle (built, imported, loaded from an index file); doc_base is kept.  n_docs < 1, vocab below the
+ * handle's, a token id outside [0, vocab) or decreasing offsets: BR_ERR_INVALID.  A term occurring more than 65535
+ * times in one doc, or a grown index of 2^31 docs, 2^32 tokens or 2^32 postings or more: BR_ERR_UNSUPPORTED.  A
+ * doc-sharded caller re-finalises every shard with the all-reduced statistics afterwards. */
+int br_index_append(br_index* ix, const int32_t* token_ids_dev, const int64_t* doc_offsets_dev, int64_t n_docs,
+                    int32_t vocab, void* stream);
+
 /* corpus_size / nnz / avgdl / sum(dl) attributes (bm25_ranking.ipynb:170-171). Any out may be NULL. */
 int br_index_stats(const br_index* ix, int64_t* n_docs, int32_t* vocab, int64_t* nnz,
                    double* avgdl, int64_t* sum_dl, int64_t* doc_base);
@@ -401,6 +416,13 @@ int br_vocab_build(const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int
 int br_vocab_lookup(const br_vocab* v, const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int64_t n_docs,
                     int bigrams, const int64_t* doc_tok_off_dev, int64_t n_tokens, int32_t* token_ids_dev,
                     void* stream);
+/* Grow a vocabulary with the tokens of new documents (call order as for br_vocab_build: br_tokenize_count first).
+ * Writes the term id of every token to token_ids_dev.  A term already in v keeps its id.  New terms get ids
+ * n_terms_old .. in order of first occurrence in the new text, which is the id br_vocab_build would give them over
+ * old text + new text.  A 64-bit hash collision with an existing or another new term is BR_ERR_UNSUPPORTED.
+ * On any error v is unchanged.  Synchronises `stream`. */
+int br_vocab_extend(br_vocab* v, const uint8_t* text_dev, const int64_t* doc_byte_off_dev, int64_t n_docs, int bigrams,
+                    const int64_t* doc_tok_off_dev, int64_t n_tokens, int32_t* token_ids_dev, void* stream);
 int br_vocab_stats(const br_vocab* v, int64_t* n_terms, int64_t* pool_bytes);
 /* Vocabulary strings: term t = pool[pool_off[t] .. pool_off[t+1]) (UTF-8).  Export for the Python
  * dict attributes (df / idf / inverted_index keys) and for pickling; import rebuilds the hash table. */
