@@ -23,6 +23,7 @@ SIGNATURES = {
     "br_index_finalize": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_double, C.c_double, _P, _P]),
     "br_index_destroy": (None, [_P]),
     "br_index_append": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, _P]),
+    "br_index_remove": (C.c_int, [_P, _P, _P]),
     "br_index_stats": (C.c_int, [_P, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int64),
                                  C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "br_index_stats_in_force": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_double)]),

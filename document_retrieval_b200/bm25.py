@@ -9,8 +9,9 @@ this file only converts between the reference's Python types and device buffers.
 Added on top of the reference surface (SURVEY 8b): ``from_token_ids`` (int32 term ids instead of
 strings), ``retrieve_top_n_batch`` / ``get_scores_batch`` (whole batches, torch CUDA tensors),
 ``variant`` / ``dedup_query`` (the three BM25 formulas in the reference, SURVEY appendix A),
-``get_top_n`` as an alias of ``retrieve_top_n``, and ``add_documents`` / ``add_texts`` / ``add_token_ids`` (grow a
-built or loaded index, bit-identical to rebuilding the whole corpus).
+``get_top_n`` as an alias of ``retrieve_top_n``, ``add_documents`` / ``add_texts`` / ``add_token_ids`` (grow a
+built or loaded index, bit-identical to rebuilding the whole corpus) and ``remove_documents`` (shrink it, bit-identical
+to rebuilding the kept documents).
 """
 from __future__ import annotations
 
@@ -181,7 +182,7 @@ class BM25:
                              "use add_texts")
         if len(tokenized_corpus) == 0:
             return self
-        self._check_appendable()
+        self._check_mutable()
         terms = self.terms
         if terms is None:
             raise ValueError("add_documents needs a model with a string vocabulary (use add_token_ids)")
@@ -215,7 +216,7 @@ class BM25:
         from .ingest import Vocabulary
         if not isinstance(texts, tuple) and len(texts) == 0:
             return self
-        self._check_appendable()
+        self._check_mutable()
         if self.vocabulary is None:
             if self.terms is None:
                 raise BRError("add_texts needs a model with a string vocabulary")
@@ -241,13 +242,13 @@ class BM25:
                              "(use add_documents or add_texts)")
         if len(doc_offsets) <= 1:
             return self
-        self._check_appendable()
+        self._check_mutable()
         self._append_ids(doc_offsets, token_ids, vocab_size)
         return self
 
-    def _check_appendable(self):
+    def _check_mutable(self):
         """A doc shard is finalised with global statistics; re-finalising it with its local ones would silently break
-        it, so it only grows through a sharded wrapper."""
+        it, so documents are only added to or removed from it through a sharded wrapper."""
         self._require()
         lib = _lib.load()
         n_stat, sum_dl_stat = C.c_double(), C.c_double()
@@ -256,8 +257,8 @@ class BM25:
         df, _ = self._export_df_idf()
         if (n_stat.value != st["n_docs"] or sum_dl_stat.value != st["sum_dl"]
                 or not np.array_equal(df, self.local_df_tensor().cpu().numpy())):
-            raise BRError("this index is a doc shard finalised with global statistics: documents cannot be added to it "
-                          "alone")
+            raise BRError("this index is a doc shard finalised with global statistics: documents cannot be added to or "
+                          "removed from it alone")
 
     def _append_ids(self, doc_offsets, token_ids, vocab_size):
         lib = _lib.load()
@@ -274,6 +275,64 @@ class BM25:
                   "br_index_append")
         self.vocab_size = int(vocab_size)
         self.corpus_size += n_docs
+        self._csr = None
+        self.finalize()
+
+    # ------------------------------------------------------------------ remove
+    def remove_documents(self, docs):
+        """Remove documents: ``docs`` is a bool mask [N] (True = remove) or integer local doc ids (duplicates count
+        once), numpy or torch, host or device.  Returns ``self``.
+
+        The kept docs keep their order and are renumbered by rank: with ``kept = np.flatnonzero(~mask)``, new id ``i`` is
+        old id ``kept[i]`` (update a ``doc_id_maps`` list with ``[old_map[d] for d in kept]``).  ``doc_base``, the term
+        ids, ``vocab_size``, ``terms`` and the GPU vocabulary do not change; a term left in no doc keeps its id with
+        df 0 and drops out of the ``df`` / ``idf`` / ``inverted_index`` dicts.  The index is re-finalised with this
+        model's k1 / b / variant and equals, bit for bit, the index built from scratch from the kept docs over the same
+        vocabulary.  Removing nothing is a no-op; removing every doc is refused (ValueError).
+
+        A ``CosineIndex`` holding the same docs is not changed: rebuild it from the kept rows (``emb[kept]``; for a
+        grouped index the kept rows with ``row_group`` remapped by the same rank), which is exact because a row's norm
+        depends on that row only."""
+        self._require()
+        N = self.corpus_size
+        if isinstance(docs, (list, tuple)):
+            if len(docs) == 0:
+                return self
+            docs = np.asarray(docs)
+        t = torch.as_tensor(docs)
+        if t.dtype == torch.bool:
+            if tuple(t.shape) != (N,):
+                raise ValueError(f"remove_documents: a mask must have shape [{N}], got {list(t.shape)}")
+        elif t.is_floating_point() or t.is_complex():
+            raise ValueError(f"remove_documents: docs must be a bool mask or integer doc ids, got {t.dtype}")
+        else:
+            t = t.reshape(-1)
+            if t.numel() == 0:
+                return self
+            lo, hi = int(t.min()), int(t.max())
+            if lo < 0 or hi >= N:
+                raise ValueError(f"remove_documents: doc ids must be in [0, {N}), got [{lo}, {hi}]")
+        dev = self._device
+        with torch.cuda.device(dev):
+            if t.dtype == torch.bool:
+                mask = t.to(device=dev, dtype=torch.uint8).contiguous()
+            else:
+                mask = torch.zeros(N, dtype=torch.uint8, device=dev)
+                mask[t.to(device=dev, dtype=torch.int64)] = 1
+            n_removed = int(mask.sum())
+        if n_removed == 0:
+            return self
+        if n_removed == N:
+            raise ValueError("remove_documents: every document would be removed; an index holds at least one")
+        self._check_mutable()
+        self._remove_mask(mask, n_removed)
+        return self
+
+    def _remove_mask(self, mask, n_removed):
+        dev = self._device
+        with torch.cuda.device(dev):
+            check(_lib.load().br_index_remove(self._h, ptr(mask), _lib.stream_ptr(dev)), "br_index_remove")
+        self.corpus_size -= n_removed
         self._csr = None
         self.finalize()
 

@@ -18,6 +18,17 @@
 // Append (br_index_append): the new docs go through the same pipeline as a build of their own, then
 //   k_append_rows    row_ptr / df of the grown index (old + new part, per term)
 //   k_append_merge   thread per output posting: a term's old postings, then its new ones with doc + N_old  (10 B in, 10 B out)
+//
+// Remove (br_index_remove): one order-preserving stream compaction of the docs, then of the postings (no term search:
+// the CSR is term-major with docs ascending inside a term, and dropping postings keeps that order)
+//   k_docmap_count   kept docs per 2048-doc tile, sum(dl) of the kept docs (integer atomics: exact)
+//   k_exscan         -> first new id of every tile
+//   k_docmap_emit    new_id[doc] = rank among the kept docs (~0u = removed), compacted dl
+//   k_remove_count   surviving postings per 2048-posting tile                                  (8 B in + new_id gather)
+//   k_exscan         -> first output posting of every tile
+//   k_remove_emit    survivors as {new_id[doc], 0.f} + tf; row_ptr of the terms whose rows start in the tile, from the
+//                    tile's own ballots                                           (10 B in, 10 B out per kept posting)
+//   k_remove_df      df = diff(row_ptr)
 #include <math.h>
 
 #include <algorithm>
@@ -221,6 +232,155 @@ __global__ void k_append_merge(const int64_t* __restrict__ row_ptr, int32_t voca
     p.w = 0.f;
     post[j] = p;
     tf[j] = f;
+}
+
+// Remove.  Both compactions use tiles of RLE_TILE items (RLE_T threads x RLE_I); new_id[doc] == kRemovedDoc marks a removed
+// doc.
+constexpr uint32_t kRemovedDoc = 0xffffffffu;
+
+__global__ void __launch_bounds__(RLE_T) k_docmap_count(const uint8_t* __restrict__ remove, const uint32_t* __restrict__ dl,
+                                                        int64_t n, uint32_t* __restrict__ block_counts,
+                                                        unsigned long long* __restrict__ sum_dl) {
+    const int64_t base = (int64_t)blockIdx.x * RLE_TILE;
+    uint32_t c = 0;
+    unsigned long long s = 0;
+#pragma unroll
+    for (int j = 0; j < RLE_I; ++j) {
+        const int64_t i = base + j * RLE_T + threadIdx.x;   // striped: coalesced, order irrelevant
+        if (i < n && !remove[i]) {
+            ++c;
+            s += dl[i];
+        }
+    }
+    uint32_t total;
+    block_excl_scan(c, &total);
+    if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if ((threadIdx.x & 31) == 0 && s) atomicAdd(sum_dl, s);
+}
+
+__global__ void __launch_bounds__(RLE_T) k_docmap_emit(const uint8_t* __restrict__ remove, const uint32_t* __restrict__ dl,
+                                                       int64_t n, const int64_t* __restrict__ block_off,
+                                                       uint32_t* __restrict__ new_id, uint32_t* __restrict__ dl_new) {
+    const int64_t base = (int64_t)blockIdx.x * RLE_TILE + (int64_t)threadIdx.x * RLE_I;  // blocked: ordered
+    bool keep[RLE_I];
+    uint32_t c = 0;
+#pragma unroll
+    for (int j = 0; j < RLE_I; ++j) {
+        keep[j] = base + j < n && !remove[base + j];
+        c += keep[j] ? 1u : 0u;
+    }
+    uint32_t total;
+    uint32_t o = (uint32_t)block_off[blockIdx.x] + block_excl_scan(c, &total);   // new ids are < 2^31
+#pragma unroll
+    for (int j = 0; j < RLE_I; ++j) {
+        if (base + j >= n) break;
+        if (keep[j]) {
+            new_id[base + j] = o;
+            dl_new[o] = dl[base + j];
+            ++o;
+        } else {
+            new_id[base + j] = kRemovedDoc;
+        }
+    }
+}
+
+// Posting tile layout: warp w reads postings [32 * RLE_I * w, 32 * RLE_I * (w + 1)) of the tile in RLE_I coalesced rounds of
+// 32; round r of warp w is chunk w * RLE_I + r of the tile.
+__global__ void __launch_bounds__(RLE_T) k_remove_count(const br_posting* __restrict__ post, int64_t nnz,
+                                                        const uint32_t* __restrict__ new_id,
+                                                        uint32_t* __restrict__ block_counts) {
+    const int64_t base = (int64_t)blockIdx.x * RLE_TILE + (threadIdx.x >> 5) * (32 * RLE_I) + (threadIdx.x & 31);
+    uint32_t c = 0;
+#pragma unroll
+    for (int r = 0; r < RLE_I; ++r) {
+        const int64_t i = base + r * 32;
+        if (i < nnz && new_id[post[i].doc] != kRemovedDoc) ++c;
+    }
+    uint32_t total;
+    block_excl_scan(c, &total);
+    if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
+}
+
+// Writes the tile's surviving postings from block_off[tile] on, in order, with their new doc ids and weight 0 (for
+// br_index_finalize), and row_ptr_new[t] = the number of survivors before row_ptr[t] for every term whose row starts in
+// the tile; the last tile also takes the terms whose rows start at nnz (trailing empty rows and t = vocab).  The count
+// before a position p of the tile is the prefix of its chunk plus a popcount of the chunk's keep ballot below p.
+__global__ void __launch_bounds__(RLE_T) k_remove_emit(const int64_t* __restrict__ row_ptr, int32_t vocab,
+                                                       const br_posting* __restrict__ post, const uint16_t* __restrict__ tf,
+                                                       int64_t nnz, const uint32_t* __restrict__ new_id,
+                                                       const int64_t* __restrict__ block_off,
+                                                       br_posting* __restrict__ post_new, uint16_t* __restrict__ tf_new,
+                                                       int64_t* __restrict__ row_ptr_new) {
+    constexpr int NC = RLE_TILE / 32;                      // chunks of 32 postings per tile
+    __shared__ uint32_t s_ballot[NC + 1], s_pre[NC + 1];   // [NC]: position RLE_TILE (the end of a full last tile)
+    __shared__ int32_t s_terms[2];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t tile_lo = (int64_t)blockIdx.x * RLE_TILE;
+    if (w == (RLE_T >> 5) - 1 && lane < 2) {
+        // the terms whose rows start in the tile: [first t with row_ptr[t] >= tile_lo, first t with row_ptr[t] >= key)
+        const int64_t key = lane == 0 ? tile_lo : (tile_lo + RLE_TILE >= nnz ? nnz + 1 : tile_lo + RLE_TILE);
+        int32_t a = 0, b = vocab + 1;
+        while (a < b) {
+            const int32_t mid = (a + b) >> 1;
+            if (row_ptr[mid] < key) a = mid + 1; else b = mid;
+        }
+        s_terms[lane] = a;
+    }
+    const int64_t base = tile_lo + w * (32 * RLE_I) + lane;
+    uint32_t nid[RLE_I], bal[RLE_I];
+    uint16_t f[RLE_I];
+#pragma unroll
+    for (int r = 0; r < RLE_I; ++r) {
+        const int64_t i = base + r * 32;
+        nid[r] = kRemovedDoc;
+        f[r] = 0;
+        if (i < nnz) {
+            nid[r] = new_id[post[i].doc];
+            f[r] = tf[i];
+        }
+        bal[r] = __ballot_sync(0xffffffffu, nid[r] != kRemovedDoc);
+    }
+    if (lane < RLE_I) {
+        uint32_t mine = bal[0];
+#pragma unroll
+        for (int r = 1; r < RLE_I; ++r) if (lane == r) mine = bal[r];
+        s_ballot[w * RLE_I + lane] = mine;
+    }
+    if (threadIdx.x == 0) s_ballot[NC] = 0;
+    __syncthreads();
+    if (w == 0) {                                          // exclusive prefix over the NC chunks, two per lane
+        static_assert(NC == 64, "two chunks per lane of one warp");
+        const uint32_t v0 = __popc(s_ballot[2 * lane]), v1 = __popc(s_ballot[2 * lane + 1]);
+        const uint32_t incl = warp_incl_scan(v0 + v1, lane);
+        s_pre[2 * lane] = incl - v0 - v1;
+        s_pre[2 * lane + 1] = incl - v1;
+        if (lane == 31) s_pre[NC] = incl;
+    }
+    __syncthreads();
+    const int64_t out0 = block_off[blockIdx.x];
+    const uint32_t below = (1u << lane) - 1u;
+#pragma unroll
+    for (int r = 0; r < RLE_I; ++r) {
+        if (nid[r] != kRemovedDoc) {
+            const int64_t o = out0 + s_pre[w * RLE_I + r] + __popc(bal[r] & below);
+            br_posting p;
+            p.doc = nid[r];
+            p.w = 0.f;
+            post_new[o] = p;
+            tf_new[o] = f[r];
+        }
+    }
+    for (int32_t t = s_terms[0] + threadIdx.x; t < s_terms[1]; t += RLE_T) {
+        const uint32_t pos = (uint32_t)(row_ptr[t] - tile_lo);   // in [0, RLE_TILE]
+        const uint32_t c = pos >> 5;
+        row_ptr_new[t] = out0 + s_pre[c] + __popc(s_ballot[c] & ((1u << (pos & 31)) - 1u));
+    }
+}
+
+__global__ void k_remove_df(const int64_t* __restrict__ row_ptr, int32_t vocab, uint32_t* __restrict__ df) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < vocab) df[t] = (uint32_t)(row_ptr[t + 1] - row_ptr[t]);
 }
 
 __global__ void k_skip(const int64_t* __restrict__ row_ptr, const br_posting* __restrict__ post,
@@ -597,6 +757,94 @@ int index_append(br_index* ix, const int32_t* tok, const int64_t* doc_off, int64
     return BR_OK;
 }
 
+// Remove documents: compact the docs (new id = rank among the kept docs), then the postings, which keeps every row's docs
+// ascending.  Terms keep their ids; a term that loses all its postings keeps an empty row.  As in index_append, every
+// new array is allocated and filled before any of them replaces the handle's, so that an error leaves the handle as it
+// was.
+int index_remove(br_index* ix, const uint8_t* remove, cudaStream_t st) {
+    BR_REQUIRE(ix && remove, BR_ERR_INVALID, "br_index_remove: null pointer");
+    BR_CUDA(cudaSetDevice(ix->device));
+    const int64_t N = ix->n_docs, nnz = ix->nnz;
+    const size_t V = (size_t)ix->vocab;
+
+    // doc map
+    const int64_t nb_docs = (N + RLE_TILE - 1) / RLE_TILE;
+    DevArray<uint32_t> new_id, doc_counts, post_counts, dl, df;
+    DevArray<int64_t> doc_off, post_off, row_ptr;
+    DevArray<unsigned long long> d_sum;
+    BR_TRY(new_id.alloc((size_t)N));
+    BR_TRY(doc_counts.alloc((size_t)nb_docs));
+    BR_TRY(doc_off.alloc((size_t)nb_docs + 1));
+    BR_TRY(d_sum.alloc(1));
+    BR_CUDA(cudaMemsetAsync(d_sum, 0, sizeof(unsigned long long), st));
+    k_docmap_count<<<(unsigned)nb_docs, RLE_T, 0, st>>>(remove, ix->dl, N, doc_counts, d_sum);
+    BR_CUDA(cudaGetLastError());
+    k_exscan<uint32_t><<<1, 1024, 0, st>>>(doc_counts, nb_docs, doc_off);
+    BR_CUDA(cudaGetLastError());
+    int64_t n_kept = 0;
+    unsigned long long sum_dl = 0;
+    BR_CUDA(cudaMemcpyAsync(&n_kept, doc_off + nb_docs, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaMemcpyAsync(&sum_dl, d_sum, sizeof(sum_dl), cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+    if (n_kept == N) return BR_OK;                         // nothing to remove: the handle stays as it is, finalised
+    BR_REQUIRE(n_kept > 0, BR_ERR_INVALID, "br_index_remove: every document would be removed (an index holds at least one)");
+    BR_TRY(dl.alloc((size_t)n_kept));
+    k_docmap_emit<<<(unsigned)nb_docs, RLE_T, 0, st>>>(remove, ix->dl, N, doc_off, new_id, dl);
+    BR_CUDA(cudaGetLastError());
+
+    // postings
+    const int64_t nb_post = (nnz + RLE_TILE - 1) / RLE_TILE;
+    int64_t nnz_new = 0;
+    BR_TRY(row_ptr.alloc(V + 1));
+    BR_TRY(df.alloc(V));
+    BR_TRY(post_counts.alloc((size_t)nb_post));
+    BR_TRY(post_off.alloc((size_t)nb_post + 1));
+    if (nnz > 0) {
+        k_remove_count<<<(unsigned)nb_post, RLE_T, 0, st>>>(ix->post, nnz, new_id, post_counts);
+        BR_CUDA(cudaGetLastError());
+        k_exscan<uint32_t><<<1, 1024, 0, st>>>(post_counts, nb_post, post_off);
+        BR_CUDA(cudaGetLastError());
+        BR_CUDA(cudaMemcpyAsync(&nnz_new, post_off + nb_post, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        BR_CUDA(cudaStreamSynchronize(st));
+    }
+    DevArray<br_posting> post;
+    DevArray<uint16_t> tf;
+    BR_TRY(post.alloc((size_t)nnz_new));
+    BR_TRY(tf.alloc((size_t)nnz_new));
+    if (nnz > 0) {
+        k_remove_emit<<<(unsigned)nb_post, RLE_T, 0, st>>>(ix->row_ptr, ix->vocab, ix->post, ix->tf, nnz, new_id, post_off,
+                                                            post, tf, row_ptr);
+        BR_CUDA(cudaGetLastError());
+    } else {
+        BR_CUDA(cudaMemsetAsync(row_ptr, 0, sizeof(int64_t) * (V + 1), st));
+    }
+    k_remove_df<<<blocks_for((int64_t)V, 256), 256, 0, st>>>(row_ptr, ix->vocab, df);
+    BR_CUDA(cudaGetLastError());
+    std::vector<uint32_t> h_df(V);
+    BR_CUDA(cudaMemcpyAsync(h_df.data(), df, sizeof(uint32_t) * V, cudaMemcpyDeviceToHost, st));
+    BR_CUDA(cudaStreamSynchronize(st));
+
+    // nothing below can fail: the handle takes the compacted arrays and frees the old ones
+    ix->row_ptr = std::move(row_ptr);
+    ix->post = std::move(post);
+    ix->tf = std::move(tf);
+    ix->dl = std::move(dl);
+    ix->df = std::move(df);
+    ix->h_df.swap(h_df);
+    // structures index_finalize builds only when they are missing: they depend on the local df and N
+    ix->skip.reset();
+    ix->sig_bit.reset();
+    ix->dense_rows.reset();
+    ix->n_rows = ix->n_srows = 0;
+    ix->post_cos.reset();
+    ix->cos_inv_norm.reset();
+    ix->n_docs = n_kept;
+    ix->sum_dl = (int64_t)sum_dl;
+    ix->nnz = nnz_new;
+    ix->finalized = false;
+    return BR_OK;
+}
+
 int index_finalize(br_index* ix, double k1, double b, int variant, double n_stat, double sum_dl_stat,
                    const int64_t* df_stat_host, cudaStream_t st) {
     BR_REQUIRE(ix, BR_ERR_INVALID, "br_index_finalize: null handle");
@@ -743,6 +991,10 @@ int br_index_build(const int32_t* token_ids_dev, const int64_t* doc_offsets_dev,
 int br_index_append(br_index* ix, const int32_t* token_ids_dev, const int64_t* doc_offsets_dev, int64_t n_docs,
                     int32_t vocab, void* stream) {
     return br::index_append(ix, token_ids_dev, doc_offsets_dev, n_docs, vocab, (cudaStream_t)stream);
+}
+
+int br_index_remove(br_index* ix, const uint8_t* remove_dev, void* stream) {
+    return br::index_remove(ix, remove_dev, (cudaStream_t)stream);
 }
 
 int br_index_finalize(br_index* ix, double k1, double b, int variant, double n_stat, double sum_dl_stat,

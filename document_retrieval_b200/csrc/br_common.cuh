@@ -286,6 +286,7 @@ int index_import_dev(const int64_t* row_ptr, const int32_t* doc, const uint16_t*
                      int32_t vocab, int64_t nnz, int64_t doc_base, cudaStream_t st, br_index** out);
 int index_append(br_index* ix, const int32_t* token_ids, const int64_t* doc_offsets, int64_t n_docs, int32_t vocab,
                  cudaStream_t st);
+int index_remove(br_index* ix, const uint8_t* remove, cudaStream_t st);
 void index_free(br_index* ix);
 // br_query.cu
 int score_batch(br_index* ix, const int32_t* q_terms, const int32_t* q_offsets, int32_t nq, int dedup,

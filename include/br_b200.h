@@ -83,6 +83,20 @@ void br_index_destroy(br_index* ix);
 int br_index_append(br_index* ix, const int32_t* token_ids_dev, const int64_t* doc_offsets_dev, int64_t n_docs,
                     int32_t vocab, void* stream);
 
+/* Remove documents from a built index.  remove_dev is uint8[n_docs] on the device; a nonzero byte removes that local doc.
+ * The kept docs keep their order: a kept doc's new local id is its rank among the kept docs (old id kept[i] becomes i,
+ * kept = the ids with a zero byte, ascending).  doc_base, term ids and vocab do not change; a term that loses every
+ * posting keeps its id with df 0, like an id no doc uses in br_index_build.  On success the handle is NOT finalised:
+ * every query entry point returns BR_ERR_STATE until br_index_finalize is called again (N, avgdl and df changed).
+ * Removing R from the index of C and finalising gives the same bits as building the docs of C not in R, in order, over
+ * the same vocab and finalising: the same CSR, df, idf, weights, skip tables and dense rows, hence the same results from
+ * every query.
+ * No nonzero byte: BR_OK, and the handle is left as it was, still finalised.  Null pointers or a mask that removes every
+ * doc: BR_ERR_INVALID.  On any error the handle is left exactly as it was, including its finalised state, and still
+ * answers queries with the same results.  Works on any handle (built, imported, appended to).  A doc-sharded caller
+ * re-finalises every shard with the all-reduced statistics afterwards. */
+int br_index_remove(br_index* ix, const uint8_t* remove_dev, void* stream);
+
 /* corpus_size / nnz / avgdl / sum(dl) attributes (bm25_ranking.ipynb:170-171). Any out may be NULL. */
 int br_index_stats(const br_index* ix, int64_t* n_docs, int32_t* vocab, int64_t* nnz,
                    double* avgdl, int64_t* sum_dl, int64_t* doc_base);
